@@ -2,6 +2,7 @@
 """bench.py -- Schnorr verifications per second on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload single|double|vargen] [--log2n 20]
+                    [--dump-outputs DIR]
 
 A step is one pass of the verify path over one synthetic batch (default: BASELINE.json configs[1], 2^20 single
 signatures with 10 % invalid items per GPU; weak scaling, every rank owns its own batch).
@@ -20,6 +21,8 @@ signatures with 10 % invalid items per GPU; weak scaling, every rank owns its ow
             algorithm on all host threads
 --impl reference times that CPU port on a bounded sample of the GPU arm's workload (same invalid mix; the reference is
 Rust and cannot be built here; see DESIGN.md).
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs), so that two builds run with the same
+arguments, and therefore the same seeded inputs, can be compared output for output.
 """
 from __future__ import annotations
 
@@ -285,6 +288,26 @@ class Part:
         return s
 
 
+DUMP_ITEMS = 1 << 19    # items dumped over the whole job, 68 bytes each: at most 34 MiB
+
+
+def dump_outputs(out_dir, shards, rank, n_shards_total):
+    """Writes, for every part of every shard of this process, what the device path returned in the last timed step:
+    shard<g>_<kind>_status.npy (float32 status codes) and shard<g>_<kind>_challenge.npy (float64 [items, 8], the challenge
+    scalar as eight little-endian 32-bit words, exact in float64).  A part larger than its share of DUMP_ITEMS is represented
+    by a fixed sample of its items (sorted indices drawn with the part's size as the seed), the same in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    per_part = DUMP_ITEMS // (n_shards_total * len(shards[0]))
+    for k, parts in enumerate(shards):
+        g = rank * len(shards) + k
+        for p in parts:
+            idx = np.arange(p.n) if p.n <= per_part else np.sort(np.random.default_rng(p.n).choice(p.n, size=per_part, replace=False))
+            status = p.d_status.cpu().numpy()[idx]
+            c = p.d_c.cpu().numpy()[idx]
+            np.save(os.path.join(out_dir, f"shard{g}_{p.kind}_status.npy"), status.astype(np.float32))
+            np.save(os.path.join(out_dir, f"shard{g}_{p.kind}_challenge.npy"), np.ascontiguousarray(c).view("<u4").astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -297,7 +320,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the 2^24 strong-scaling sub-record")
     ap.add_argument("--strong-log2n", type=int, default=24)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if not args.log2n:
         args.log2n = 24 if args.workload == "mixed5" else 20
     rank = int(os.environ.get("RANK", "0"))
@@ -389,6 +417,8 @@ def main():
     ms_dev = max_over_ranks(max(e0.elapsed_time(e1) for e0, e1 in events))
     launches = bv.launch_count - launches0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, shards, rank, n_gpus_total)
     # Stage breakdown from a second, untimed pass of the same K steps: with the per-stage timers on, the library keeps
     # every launch on one stream (the timed pass above overlaps neighbouring sub-chunks on two streams, which per-stage
     # CUDA events cannot attribute), so the stage times add up to slightly more than ms_per_step.
@@ -547,7 +577,7 @@ def strong_scaling_record(args, torch, wl, BatchVerifier, n_devices):
     enqueued through the device entry points, CUDA events per device, max over devices."""
     log2n = args.strong_log2n
     half = 1 << (log2n - 1)
-    steps, warm = max(1, min(args.steps, 4)), 1
+    steps, warm = args.steps, 1
     with BatchVerifier(list(range(n_devices))) as sv:
         batches = [(wl.SINGLE,) + tuple(wl.make_batch(sv, wl.SINGLE, half, 0.10, seed=0x24A)[:4]), (wl.DOUBLE,) + tuple(wl.make_batch(sv, wl.DOUBLE, half, 0.10, seed=0x24B)[:4])]
         n = 2 * half

@@ -303,7 +303,7 @@ def test_typed_inputs_match_oracle(bv, vi, kind):
     assert set(st_b.tolist()) == {0, 1, 2, 3}
 
 
-def test_multisig_combine_matches_oracle(bv, tmp_path):
+def test_multisig_combine_matches_oracle(bv):
     """jjs_multisig_combine (SURVEY 8(f) row 2): the pinned KAT, then 6000 generated sessions with tampered shares,
     swapped commitments, undecodable fields and empty sessions, item by item against the oracle; every combined
     signature is then verified under its aggregate key by the GPU verify path."""
@@ -354,11 +354,8 @@ def test_multisig_combine_matches_oracle(bv, tmp_path):
     assert (st_b == 0).all() and (ok_b == 1).all()
     st_s, _, sig_s, _ = co.multisig_combine(pks[:3 * 256], Rs[:3 * 256], Ss[:3 * 256], zs[:3 * 256], off[:257], msg[:256])
     assert np.array_equal(st_s, st_b[:256]) and np.array_equal(sig_s, sig_b[:256])
-    out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out")
-    os.makedirs(out, exist_ok=True)
-    with open(os.path.join(out, "multisig_combine.json"), "w") as f:
-        _json.dump({"path": "jjs_multisig_combine (host buffers, 3 participants per session)", "sessions": nb, "participants": int(off[-1]),
-                    "seconds": dt, "sessions_per_s": nb / dt, "shares_per_s": int(off[-1]) / dt}, f)
+    print(_json.dumps({"path": "jjs_multisig_combine (host buffers, 3 participants per session)", "sessions": nb, "participants": int(off[-1]),
+                       "seconds": dt, "sessions_per_s": nb / dt, "shares_per_s": int(off[-1]) / dt}))
 
 
 def test_fp64_pipe_multiplier_equals_integer_multiplier_on_device():
