@@ -155,6 +155,37 @@ int jjs_verify_aggregate_device(jjs_ctx* ctx, int device_index, const uint8_t* d
                                 const uint32_t* h_offsets, const uint8_t* d_sig64, const uint8_t* d_msg32, size_t n,
                                 uint8_t* d_status, uint8_t* d_c32_or_null, uint8_t* d_aggpk32_or_null, void* cuda_stream);
 
+/* ---- registered key sets: many signatures under a small, stable set of keys (validators, frequent senders, a
+ *      service's registered devices).  A key set is decoded and validated once, and every key point gets a table of
+ *      32 windows x 128 points j 2^(8 w) PK in affine Niels form, 96 B each: 393 216 B per single key, 786 432 B per
+ *      double key (pk with G, pk' with G'), on every device of the context.  Verification against it then evaluates
+ *      u G + c PK == R from precomputed tables only, and returns exactly what jjs_verify_single (single key sets) or
+ *      jjs_verify_double (double key sets) returns for the same items with the keys written out.  A key set is named by
+ *      an int handle owned by the context; jjs_destroy frees the key sets still registered. --- */
+
+/* Register n_keys >= 1 keys of kind JJS_KIND_SINGLE (pk: n_keys x 32 B, PublicKey) or JJS_KIND_DOUBLE (pk: n_keys x 64 B,
+ * PublicKeyDouble) on every device of the context.  Keys that do not decode or fail is_valid() are registered too, so that
+ * indices stay dense: items under them get the status verify() gives for those key bytes.  key_status_or_null receives per
+ * key 0 (valid), 2 (InvalidPoint) or 3 (BytesError).  Returns JJS_ERR_ARGUMENT for another kind or n_keys == 0 and
+ * JJS_ERR_NOMEM, with nothing left allocated, when the tables do not fit.  Synchronous. */
+int jjs_keyset_create(jjs_ctx* ctx, int kind, const uint8_t* pk, size_t n_keys, uint8_t* key_status_or_null, int* keyset_out);
+/* Free a key set (waits for the devices first).  An unknown or already destroyed handle returns JJS_ERR_ARGUMENT. */
+int jjs_keyset_destroy(jjs_ctx* ctx, int keyset);
+/* Item i is verified under key key_index[i] of the set, with signature sig (64 B single, 96 B double) and message msg32.
+ * An index >= n_keys is reported as a key that does not decode: status JJS_BYTES_ERROR, zero challenge.  Host buffers,
+ * sharded over the context's devices like the other host-buffer entry points; status_or_null and accept_bitmap_or_null
+ * (layout of jjs_verify_batch) are not both NULL. */
+int jjs_verify_keyed(jjs_ctx* ctx, int keyset, const uint32_t* key_index, const uint8_t* sig, const uint8_t* msg32, size_t n,
+                     uint8_t* status_or_null, uint8_t* c32_or_null, uint32_t* accept_bitmap_or_null);
+/* The same on device buffers of device `device_index`, enqueue-only on cuda_stream like the other device-buffer entry points. */
+int jjs_verify_keyed_device(jjs_ctx* ctx, int device_index, int keyset, const uint32_t* d_key_index, const uint8_t* d_sig,
+                            const uint8_t* d_msg32, size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream);
+/* Key-set table self-check (a cross-check hook for the tests, like jjs_fb_table_check): recompute the n entries named by
+ * `entries` from their definition j 2^(8 w) PK by plain double-and-add on device 0 and count those that differ.  Flat index
+ * (key * points_per_key + point) * 4096 + w * 128 + j - 1, reduced modulo the table size; points_per_key is 1 (single) or
+ * 2 (double: pk, then pk').  The table of a key that failed is_valid() is that of the identity.  Host buffers. */
+int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* entries, size_t n, uint32_t* mismatches);
+
 /* Typed inputs (what a Rust caller holds before any to_bytes()): every point is given by its JubJubExtended
  * coordinates (u, v, z, t1, t2), each the in-memory BlsScalar of the reference (4 x u64 little-endian Montgomery limbs,
  * R = 2^256): 160 bytes per point.  points_ext160 is item-major, the points of one item in the order

@@ -18,6 +18,7 @@ EXPORTS = [
     "jjs_challenge_only", "jjs_sign_batch", "jjs_profile_enable", "jjs_profile_collect", "jjs_subgroup_check", "jjs_fb_table_check", "jjs_verify_aggregate_device", "jjs_sign_aggregate_batch", "jjs_verify_ext", "jjs_points_to_ext", "jjs_multisig_combine",
     "jjs_verify_batch", "jjs_status_bitmap_device", "jjs_verify_batch_double", "jjs_verify_batch_vargen", "jjs_verify_batch_aggregate",
     "jjs_verify_mixed",
+    "jjs_keyset_create", "jjs_keyset_destroy", "jjs_verify_keyed", "jjs_verify_keyed_device", "jjs_keyset_table_check",
 ]
 
 
@@ -98,5 +99,15 @@ def lib():
     L.jjs_points_to_ext.restype = C.c_int
     L.jjs_multisig_combine.argtypes = [vp, vp, vp, vp, vp, vp, vp, sz, vp, vp, vp, vp]
     L.jjs_multisig_combine.restype = C.c_int
+    L.jjs_keyset_create.argtypes = [vp, C.c_int, vp, sz, vp, C.POINTER(C.c_int)]
+    L.jjs_keyset_create.restype = C.c_int
+    L.jjs_keyset_destroy.argtypes = [vp, C.c_int]
+    L.jjs_keyset_destroy.restype = C.c_int
+    L.jjs_verify_keyed.argtypes = [vp, C.c_int, vp, vp, vp, sz, vp, vp, vp]
+    L.jjs_verify_keyed.restype = C.c_int
+    L.jjs_verify_keyed_device.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, sz, vp, vp, vp]
+    L.jjs_verify_keyed_device.restype = C.c_int
+    L.jjs_keyset_table_check.argtypes = [vp, C.c_int, vp, sz, vp]
+    L.jjs_keyset_table_check.restype = C.c_int
     _lib = L
     return L

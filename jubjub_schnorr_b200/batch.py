@@ -17,6 +17,14 @@ class JjsError(RuntimeError):
     pass
 
 
+class KeySet:
+    """A key set registered with BatchVerifier.keyset_create: its handle in the context, kind (SINGLE or DOUBLE), number of keys
+    and per-key status (0 valid, 2 InvalidPoint, 3 BytesError)."""
+
+    def __init__(self, handle, kind, n_keys, key_status):
+        self.handle, self.kind, self.n_keys, self.key_status = handle, kind, n_keys, key_status
+
+
 def _u8(a, width, name):
     a = np.ascontiguousarray(a, dtype=np.uint8)
     if a.size % width:
@@ -290,6 +298,49 @@ class BatchVerifier:
         h_offsets = np.ascontiguousarray(h_offsets, dtype=np.uint32)
         self._check(self._lib.jjs_verify_aggregate_device(self._ctx, device_index, d_pks, d_offsets, h_offsets.ctypes.data, d_sig, d_msg, n,
                                                           d_status, d_c, d_agg, stream), "jjs_verify_aggregate_device")
+
+    # ---- registered key sets ---------------------------------------------------------------------
+    def keyset_create(self, kind, pks):
+        """Register keys of kind SINGLE (pks: n x 32 bytes) or DOUBLE (n x 64) on every device (jjs_keyset_create)."""
+        if kind not in (SINGLE, DOUBLE):
+            raise ValueError("key sets hold SINGLE or DOUBLE keys")
+        pk = _u8(pks, PK_SIZE[kind], "pks")
+        status = np.empty(pk.shape[0], dtype=np.uint8)
+        handle = C.c_int(-1)
+        self._check(self._lib.jjs_keyset_create(self._ctx, kind, pk.ctypes.data, pk.shape[0], status.ctypes.data, C.byref(handle)), "jjs_keyset_create")
+        return KeySet(handle.value, kind, pk.shape[0], status)
+
+    def keyset_destroy(self, ks):
+        self._check(self._lib.jjs_keyset_destroy(self._ctx, ks.handle), "jjs_keyset_destroy")
+
+    def verify_keyed(self, ks, key_index, sig, msg32, want_challenge=False, want_bitmap=False):
+        """Item i under key key_index[i] of the key set (jjs_verify_keyed).  Returns status, plus c and / or the accept bitmap
+        when asked for (in that order)."""
+        idx = np.ascontiguousarray(key_index, dtype=np.uint32).reshape(-1)
+        sig, msg = _u8(sig, SIG_SIZE[ks.kind], "sig"), _u8(msg32, 32, "msg")
+        n = msg.shape[0]
+        if idx.shape[0] != n or sig.shape[0] != n:
+            raise ValueError("key_index, sig and msg must describe the same number of items")
+        status = np.empty(n, dtype=np.uint8)
+        c = np.empty((n, 32), dtype=np.uint8) if want_challenge else None
+        words = np.zeros((n + 31) // 32, dtype=np.uint32) if want_bitmap else None
+        self._check(self._lib.jjs_verify_keyed(self._ctx, ks.handle, idx.ctypes.data, sig.ctypes.data, msg.ctypes.data, n, status.ctypes.data,
+                                               c.ctypes.data if want_challenge else None, words.ctypes.data if want_bitmap else None),
+                    "jjs_verify_keyed")
+        out = [status] + ([c] if want_challenge else []) + ([words] if want_bitmap else [])
+        return out[0] if len(out) == 1 else tuple(out)
+
+    def verify_keyed_device(self, ks, d_key_index, d_sig, d_msg, n, d_status, d_c=None, stream=None, device_index=0):
+        """jjs_verify_keyed_device on raw device pointers (uint32 key indices), enqueued on `stream`."""
+        self._check(self._lib.jjs_verify_keyed_device(self._ctx, device_index, ks.handle, d_key_index, d_sig, d_msg, n, d_status, d_c, stream),
+                    "jjs_verify_keyed_device")
+
+    def keyset_table_check(self, ks, entries):
+        """Number of the given key-table entries (flat indices, see jjs_keyset_table_check) that differ from their definition."""
+        idx = np.ascontiguousarray(entries, dtype=np.uint32)
+        bad = np.zeros(1, dtype=np.uint32)
+        self._check(self._lib.jjs_keyset_table_check(self._ctx, ks.handle, idx.ctypes.data, idx.shape[0], bad.ctypes.data), "jjs_keyset_table_check")
+        return int(bad[0])
 
     # ---- raw host / device pointers (pinned torch tensors, device tensors: pass .data_ptr()) ----------
     def verify_host_ptr(self, variant, pk_ptr, sig_ptr, msg_ptr, n, status_ptr, c_ptr=None):

@@ -15,6 +15,7 @@
 #include <vector>
 
 #include "../../include/jjschnorr_b200.h"
+#include "keyset.cuh"
 #include "multisig_core.cuh"
 #include "sign_core.cuh"
 #include "verify_core.cuh"
@@ -409,6 +410,81 @@ __global__ void __launch_bounds__(BLOCK) k_fb_check(const niels* table, int whic
     if (!(fq_eq(e.ypx, g.ypx) && fq_eq(e.ymx, g.ymx) && fq_eq(e.t2d, g.t2d))) atomicAdd(mismatches, 1u);
 }
 
+// ---- registered key sets (keyset.cuh) --------------------------------------------------------------------------------
+// Key points are numbered key-major (point p = key * nk + s, the order of the tables); the decoded points are slot-major
+// (s * n_keys + key, as k_decode writes them).
+// Table pass 1: thread p computes the window bases of key point p, bases[w * npts + p].
+__global__ void __launch_bounds__(BLOCK) k_keyset_bases(int variant, const fq* keys_u, const fq* keys_v, const uint8_t* kflags, size_t n_keys,
+                                                        ext* bases) {
+    const int nk = keyed_points(variant);
+    const size_t npts = (size_t)nk * n_keys, p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npts) return;
+    const size_t k = (size_t)(p % nk) * n_keys + p / nk;
+    fq u, v;
+    keyed_table_base(u, v, keys_u[k], keys_v[k], kflags[k]);
+    keyed_window_bases(bases + p, npts, u, v);
+}
+// Table pass 2: one thread per batch of KEYED_BATCH entries of one window of one key point.
+constexpr int KEYED_GROUPS = KEYED_ENTRIES / KEYED_BATCH;
+__global__ void __launch_bounds__(BLOCK) k_keyset_combine(const ext* bases, size_t npts, niels* table) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= npts * KEYED_WINDOWS * KEYED_GROUPS) return;
+    const size_t p = t / (KEYED_WINDOWS * KEYED_GROUPS);
+    const int r = (int)(t % (KEYED_WINDOWS * KEYED_GROUPS)), w = r / KEYED_GROUPS, g = r % KEYED_GROUPS;
+    keyed_combine_entries(table + p * KEYED_POINT_ENTRIES + (size_t)w * KEYED_ENTRIES + (size_t)g * KEYED_BATCH, bases[(size_t)w * npts + p],
+                          g * KEYED_BATCH + 1);
+}
+// the definition, entry by entry (jjs_keyset_table_check): flat index p * KEYED_POINT_ENTRIES + w * KEYED_ENTRIES + j - 1
+__global__ void __launch_bounds__(BLOCK) k_keyset_check(int variant, const fq* keys_u, const fq* keys_v, const uint8_t* kflags, size_t n_keys,
+                                                        const niels* table, const uint32_t* entries, size_t n, uint32_t* mismatches) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const int nk = keyed_points(variant);
+    const size_t idx = (size_t)entries[t] % ((size_t)nk * n_keys * KEYED_POINT_ENTRIES), p = idx / KEYED_POINT_ENTRIES;
+    const int e = (int)(idx % KEYED_POINT_ENTRIES);
+    const size_t k = (size_t)(p % nk) * n_keys + p / nk;
+    fq u, v;
+    keyed_table_base(u, v, keys_u[k], keys_v[k], kflags[k]);
+    niels ref;
+    keyed_table_entry(ref, u, v, e / KEYED_ENTRIES, e % KEYED_ENTRIES + 1);
+    const niels& g = table[idx];
+    if (!(fq_eq(ref.ypx, g.ypx) && fq_eq(ref.ymx, g.ymx) && fq_eq(ref.t2d, g.t2d))) atomicAdd(mismatches, 1u);
+}
+// key slots of the chunk's items from the key set, by index
+__global__ void __launch_bounds__(BLOCK) k_keyed_gather(int variant, const fq* keys_u, const fq* keys_v, const uint8_t* kflags, size_t n_keys,
+                                                        const uint32_t* key_index, size_t n, fq* pts_u, fq* pts_v, uint8_t* pflags) {
+    const size_t item = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (item >= n) return;
+    stage_keyed_gather(variant, keys_u, keys_v, kflags, n_keys, key_index[item], pts_u, pts_v, pflags, n, item);
+}
+// thread t < neq * *count: equation t % neq of item list[t / neq] under its registered key (stage_equation_keyed).  No per-thread
+// table scratch: both products read precomputed tables.
+#ifndef JJS_EQK_MINBLOCKS
+#define JJS_EQK_MINBLOCKS 4
+#endif
+__global__ void __launch_bounds__(BLOCK, JJS_EQK_MINBLOCKS) k_equation_keyed(int variant, const fq* pts_u, const fq* pts_v, uint8_t* pflags, size_t n,
+                                                                             const uint32_t* list, const uint32_t* lcount, WireField usc,
+                                                                             const uint32_t* cwords, uint8_t* eqflags, const niels* ktab,
+                                                                             const uint32_t* key_index, size_t n_keys, Tables T, uint32_t* rlist,
+                                                                             uint32_t* rcount) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int neq = keyed_points(variant);
+    if (t >= (size_t)neq * *lcount) return;
+    const int eq = (int)(t % neq);
+    const size_t item = list[t / neq];
+    const uint32_t key = key_index[item];   // in range: items under an unknown index never reach the work list
+    bool need_r_test = false;
+    const bool ok = key < n_keys &&
+                    stage_equation_keyed(variant, eq, pts_u, pts_v, pflags, n, item, eq == 1 ? T.fb_gn : T.fb_g,
+                                         ktab + ((size_t)key * neq + eq) * KEYED_POINT_ENTRIES, usc, cwords, &need_r_test);
+    if (need_r_test) {
+        int pk_slot, r_slot, base_slot;
+        equation_slots(variant, eq, pk_slot, r_slot, base_slot);
+        rlist[atomicAdd(rcount, 1u)] = (uint32_t)((size_t)r_slot * n + item);
+    }
+    eqflags[(size_t)eq * n + item] = ok ? 1 : 0;
+}
+
 // one thread signs one item; inputs are 32-byte little-endian scalars, outputs the reference's wire bytes.
 // The variant is a template parameter so that every array index below is static.
 template <int VARIANT>
@@ -596,6 +672,20 @@ constexpr size_t SUB_CHUNK = size_t(1) << JJS_SUB_CHUNK_LOG2;      // items per 
 inline Region region_whole(const DeviceState& d) { return region_of(d, 0, CHUNK_ITEMS, 0); }
 inline Region region_half(const DeviceState& d, size_t j) { return region_of(d, (j & 1) * SUB_ITEMS, SUB_ITEMS, (int)(j & 1)); }
 
+// A registered key set (jjs_keyset_create), copied to every device of the context: the decoded key points slot-major as k_decode
+// writes them (point s of key k at s * n_keys + k), their flags, and the window tables key-major (keyset.cuh; the table of point
+// s of key k starts at entry (k * nk + s) * KEYED_POINT_ENTRIES).
+struct KeySetDev {
+    fq *u = nullptr, *v = nullptr;
+    uint8_t* flags = nullptr;
+    niels* table = nullptr;
+};
+struct KeySet {
+    int variant = VAR_SINGLE;
+    size_t n_keys = 0;
+    std::vector<KeySetDev> dev;
+};
+
 }  // namespace
 
 struct StageRecord {
@@ -613,6 +703,7 @@ struct jjs_ctx {
     bool profile = false;
     std::vector<StageRecord> records;
     std::vector<fq> tags;            // host copy of the SAFE tag table
+    std::vector<KeySet*> keysets;    // registered key sets by handle (nullptr once destroyed; handles are not reused)
 };
 
 namespace {
@@ -927,6 +1018,41 @@ int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uin
     return JJS_SUCCESS;
 }
 
+// The pipeline for one chunk of m <= R.cap items under a registered key set (device pointers, key_index: the chunk's first
+// index).  The key slots are gathered from the key set instead of decoded; only the signature points go through k_decode,
+// with their subgroup test deferred.  Hash, deferred tests and status are the kernels of run_chunk.
+int run_chunk_keyed(jjs_ctx* ctx, DeviceState& d, const Region& R, const KeySet& ks, const KeySetDev& kd, const uint32_t* key_index, const uint8_t* sig,
+                    const uint8_t* msg, size_t m, uint8_t* status, uint8_t* c_out, cudaStream_t stream) {
+    const int variant = ks.variant, nk = keyed_points(variant);
+    const uint32_t sgs = (uint32_t)sig_size(variant);
+    Tables T = d.tables();
+    Fields fr;
+    fr.f[0] = WireField{sig + 32, sgs};
+    fr.f[1] = variant == VAR_DOUBLE ? WireField{sig + 64, sgs} : WireField{nullptr, 0};
+    fr.f[2] = fr.f[3] = WireField{nullptr, 0};
+    WireField fmsg{msg, 32}, fu{sig, sgs};
+    StageTimer t0(ctx, d.device, 0, stream);
+    k_keyed_gather<<<blocks_for(m), BLOCK, 0, stream>>>(variant, kd.u, kd.v, kd.flags, ks.n_keys, key_index, m, R.pts_u, R.pts_v, R.pflags);
+    k_decode<<<blocks_for(nk * m), BLOCK, 0, stream>>>(fr, nk, nk, m, R.pts_u, R.pts_v, R.pflags, T, 0u);
+    t0.stop(stream);
+    ctx->launches += 2;
+    int rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
+    if (rc) return rc;
+    StageTimer t3(ctx, d.device, 3, stream);
+    JJS_CUDA(ctx, cudaMemsetAsync(R.rcount, 0, sizeof(uint32_t), stream));
+    k_equation_keyed<<<blocks_for(nk * m), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, R.eqlist, R.rcount + 2, fu, R.cwords, R.eqflags,
+                                                              kd.table, key_index, ks.n_keys, T, R.rlist, R.rcount);
+    t3.stop(stream);
+    StageTimer t5(ctx, d.device, 5, stream);
+    k_rtest<<<blocks_for(nk * m), BLOCK, 0, stream>>>(R.pts_u, R.pts_v, R.pflags, R.rlist, R.rcount);
+    t5.stop(stream);
+    StageTimer t4(ctx, d.device, 4, stream);
+    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.eqflags, R.cwords, m, status, c_out);
+    t4.stop(stream);
+    ctx->launches += 3;
+    return JJS_SUCCESS;
+}
+
 // Sub-chunks of an overlapped batch alternate between the two internal streams and scratch halves: kernels of neighbouring
 // sub-chunks overlap, which hides the partially filled last wave of every launch (per-thread work is uniform, so a launch
 // ends with SMs idling for up to one block duration).  With per-stage profiling on, everything stays on `stream` so that
@@ -972,6 +1098,28 @@ int run_device(jjs_ctx* ctx, DeviceState& d, int variant, const uint8_t* pk, con
         size_t m = n - off < step ? n - off : step;
         rc = run_chunk(ctx, d, ov.next_region(), variant, pk + off * pk_size(variant), sig + off * sig_size(variant), msg + off * 32, m,
                        status ? status + off : nullptr, c_out ? c_out + off * 32 : nullptr, ov.next_stream(), challenge_only);
+        if (rc) return rc;
+    }
+    rc = ov.end();
+    if (rc) return rc;
+    JJS_CUDA(ctx, cudaGetLastError());
+    return JJS_SUCCESS;
+}
+
+// run_device for items under a registered key set
+int run_keyed_device(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, const KeySetDev& kd, const uint32_t* key_index, const uint8_t* sig,
+                     const uint8_t* msg, size_t n, uint8_t* status, uint8_t* c_out, cudaStream_t stream) {
+    int rc = ensure_scratch(ctx, d);
+    if (rc) return rc;
+    JJS_CUDA(ctx, cudaSetDevice(d.device));
+    Overlap ov(ctx, d, stream, n > SUB_CHUNK);
+    rc = ov.begin();
+    if (rc) return rc;
+    const size_t step = ov.on ? SUB_CHUNK : CHUNK_ITEMS;
+    for (size_t off = 0; off < n; off += step, ov.advance()) {
+        size_t m = n - off < step ? n - off : step;
+        rc = run_chunk_keyed(ctx, d, ov.next_region(), ks, kd, key_index + off, sig + off * sig_size(ks.variant), msg + off * 32, m, status + off,
+                             c_out ? c_out + off * 32 : nullptr, ov.next_stream());
         if (rc) return rc;
     }
     rc = ov.end();
@@ -1035,15 +1183,16 @@ int run_aggregate_device(jjs_ctx* ctx, DeviceState& d, const uint8_t* d_pks, con
 // loaded device), and every device is driven by its own host thread: copies in on the copy stream, pipeline slices alternating
 // between the two compute streams, results copied out at the end, one synchronisation.  A single host thread would serialise
 // the devices whenever the caller's memory is pageable (cudaMemcpyAsync from pageable memory returns only after staging).
-enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2 };
+enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2, PART_KEYED = 3 };
 struct HostPart {
     int mode, variant;
-    const uint8_t *pk, *sig, *msg;    // typed: pk = points_ext160, sig = u32
+    const uint8_t *pk, *sig, *msg;    // typed: pk = points_ext160, sig = u32;  keyed: pk = the uint32 key indices
     const uint32_t* offsets;          // aggregate only
     size_t n;
     uint8_t *status, *c_out, *agg_out;
     uint32_t* bitmap;
     bool challenge_only;
+    const KeySet* keys = nullptr;     // keyed only
 };
 struct Shard {
     size_t lo, hi;
@@ -1098,6 +1247,9 @@ inline size_t part_in_bytes(const HostPart& p, size_t lo, size_t hi, size_t* pk_
     } else if (p.mode == PART_TYPED) {
         *pk_bytes = 160 * (size_t)variant_slots(p.variant) * m;
         *sig_bytes = 32 * m;
+    } else if (p.mode == PART_KEYED) {
+        *pk_bytes = sizeof(uint32_t) * m;
+        *sig_bytes = sig_size(p.variant) * m;
     } else {
         *pk_bytes = pk_size(p.variant) * m;
         *sig_bytes = sig_size(p.variant) * m;
@@ -1162,7 +1314,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
             JJS_CUDA(ctx, cudaMemcpyAsync(S.offsets, P.offsets + lo, 4 * (m + 1), cudaMemcpyHostToDevice, d.copy_stream));
         }
         const bool want_c = P.c_out != nullptr || P.challenge_only;
-        const size_t pks = P.mode == PART_TYPED ? 160 * (size_t)variant_slots(P.variant) : pk_size(P.variant);
+        const size_t pks = P.mode == PART_TYPED ? 160 * (size_t)variant_slots(P.variant) : (P.mode == PART_KEYED ? sizeof(uint32_t) : pk_size(P.variant));
         const size_t sgs = P.mode == PART_TYPED ? 32 : (P.mode == PART_AGGREGATE ? 64 : sig_size(P.variant));
         // Pipeline slices: slice j + 1 is copied in on the copy stream while slice j is being verified (the kernels of one
         // slice run far longer than its copy); the first slice of a device is short so that compute starts early.
@@ -1193,6 +1345,9 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
                 if (P.mode == PART_TYPED)
                     rc = run_chunk_ext(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * 32, S.msg + off * 32, cnt, S.status + off,
                                        want_c ? S.c + off * 32 : nullptr, cs);
+                else if (P.mode == PART_KEYED)
+                    rc = run_chunk_keyed(ctx, d, R, *P.keys, P.keys->dev[k], reinterpret_cast<const uint32_t*>(S.pk + off * pks), S.sig + off * sgs,
+                                         S.msg + off * 32, cnt, S.status + off, want_c ? S.c + off * 32 : nullptr, cs);
                 else
                     rc = run_chunk(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * sgs, S.msg + off * 32, cnt, S.status + off,
                                    want_c ? S.c + off * 32 : nullptr, cs, P.challenge_only);
@@ -1237,7 +1392,7 @@ int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& part
 }
 
 int validate_part(jjs_ctx* ctx, const HostPart& P) {
-    if (P.mode == PART_WIRE || P.mode == PART_TYPED) {
+    if (P.mode == PART_WIRE || P.mode == PART_TYPED || P.mode == PART_KEYED) {
         if (P.variant < 0 || P.variant > 2) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
     } else if (P.mode != PART_AGGREGATE) {
         return fail(ctx, JJS_ERR_ARGUMENT, "bad part kind");
@@ -1508,6 +1663,78 @@ int run_small(jjs_ctx* ctx, const char* what, size_t in_bytes, size_t out_bytes,
     return JJS_SUCCESS;
 }
 
+// ---- registered key sets ----------------------------------------------------------------------------------------
+// cudaMalloc for key-set storage.  A failed allocation also clears the error it leaves behind for cudaGetLastError, which
+// later calls on this context would otherwise report as their own.
+int keyset_malloc(jjs_ctx* ctx, void** p, size_t bytes) {
+    cudaError_t e = cudaMalloc(p, bytes);
+    if (e == cudaSuccess) return JJS_SUCCESS;
+    *p = nullptr;
+    cudaGetLastError();
+    return fail(ctx, e == cudaErrorMemoryAllocation ? JJS_ERR_NOMEM : JJS_ERR_CUDA, "key set: cudaMalloc of %zu bytes failed: %s", bytes,
+                cudaGetErrorString(e));
+}
+
+struct DeviceTemp {   // scratch of one key-set build, freed on every path out
+    void* p = nullptr;
+    ~DeviceTemp() { cudaFree(p); }
+};
+
+// Key set `ks` on device d: copy the wire keys in, decode them with the subgroup test, build the tables (keyset.cuh).
+// key_status (optional) receives 0 / 2 / 3 per key.
+int keyset_build(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, KeySetDev& kd, const uint8_t* pk, uint8_t* key_status) {
+    JJS_CUDA(ctx, cudaSetDevice(d.device));
+    const int nk = keyed_points(ks.variant);
+    const size_t npts = (size_t)nk * ks.n_keys;
+    DeviceTemp wire, bases;
+    int rc = keyset_malloc(ctx, (void**)&kd.u, sizeof(fq) * npts);
+    if (!rc) rc = keyset_malloc(ctx, (void**)&kd.v, sizeof(fq) * npts);
+    if (!rc) rc = keyset_malloc(ctx, (void**)&kd.flags, npts);
+    if (!rc) rc = keyset_malloc(ctx, (void**)&kd.table, sizeof(niels) * npts * KEYED_POINT_ENTRIES);
+    if (!rc) rc = keyset_malloc(ctx, &wire.p, 32 * npts);
+    if (!rc) rc = keyset_malloc(ctx, &bases.p, sizeof(ext) * npts * KEYED_WINDOWS);
+    if (rc) return rc;
+    cudaStream_t st = d.stream;
+    // undecodable keys leave their coordinates unwritten; zero them so that gathering them copies defined values
+    JJS_CUDA(ctx, cudaMemsetAsync(kd.u, 0, sizeof(fq) * npts, st));
+    JJS_CUDA(ctx, cudaMemsetAsync(kd.v, 0, sizeof(fq) * npts, st));
+    JJS_CUDA(ctx, cudaMemcpyAsync(wire.p, pk, 32 * npts, cudaMemcpyHostToDevice, st));
+    const uint8_t* w = static_cast<const uint8_t*>(wire.p);
+    Fields f;
+    f.f[0] = WireField{w, (uint32_t)(32 * nk)};
+    f.f[1] = nk == 2 ? WireField{w + 32, 64} : WireField{nullptr, 0};
+    f.f[2] = f.f[3] = WireField{nullptr, 0};
+    k_decode<<<blocks_for(npts), BLOCK, 0, st>>>(f, nk, 0, ks.n_keys, kd.u, kd.v, kd.flags, d.tables(), 3u);
+    k_keyset_bases<<<blocks_for(npts), BLOCK, 0, st>>>(ks.variant, kd.u, kd.v, kd.flags, ks.n_keys, static_cast<ext*>(bases.p));
+    k_keyset_combine<<<blocks_for(npts * KEYED_WINDOWS * KEYED_GROUPS), BLOCK, 0, st>>>(static_cast<const ext*>(bases.p), npts, kd.table);
+    ctx->launches += 3;
+    JJS_CUDA(ctx, cudaGetLastError());
+    std::vector<uint8_t> flags;
+    if (key_status) {
+        flags.resize(npts);
+        JJS_CUDA(ctx, cudaMemcpyAsync(flags.data(), kd.flags, npts, cudaMemcpyDeviceToHost, st));
+    }
+    JJS_CUDA(ctx, cudaStreamSynchronize(st));
+    for (size_t k = 0; key_status && k < ks.n_keys; k++) key_status[k] = keyed_key_status(ks.variant, flags.data(), ks.n_keys, k);
+    return JJS_SUCCESS;
+}
+
+void keyset_free(jjs_ctx* ctx, KeySet* ks) {
+    for (size_t k = 0; k < ks->dev.size(); k++) {
+        KeySetDev& kd = ks->dev[k];
+        if (!kd.u && !kd.v && !kd.flags && !kd.table) continue;
+        cudaSetDevice(ctx->dev[k].device);
+        cudaDeviceSynchronize();   // work enqueued by the device entry point may still read the tables
+        cudaFree(kd.u); cudaFree(kd.v); cudaFree(kd.flags); cudaFree(kd.table);
+    }
+    delete ks;
+}
+
+KeySet* keyset_lookup(jjs_ctx* ctx, int handle) {
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    return handle >= 0 && (size_t)handle < ctx->keysets.size() ? ctx->keysets[handle] : nullptr;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1541,6 +1768,8 @@ JJS_API int jjs_init(const int* devices, int n_devices, jjs_ctx** out) {
 
 JJS_API void jjs_destroy(jjs_ctx* ctx) {
     if (!ctx) return;
+    for (KeySet* ks : ctx->keysets)
+        if (ks) keyset_free(ctx, ks);
     for (auto& d : ctx->dev) free_device(d);
     delete ctx;
 }
@@ -1757,6 +1986,80 @@ JJS_API int jjs_profile_collect(jjs_ctx* ctx, double* stage_ms, uint64_t* stage_
         stage_ms[r.stage] += ms;
         stage_count[r.stage]++;
     }
+    return rc;
+}
+JJS_API int jjs_keyset_create(jjs_ctx* ctx, int kind, const uint8_t* pk, size_t n_keys, uint8_t* key_status_or_null, int* keyset_out) {
+    JJS_ENTER(ctx);
+    if (kind != JJS_KIND_SINGLE && kind != JJS_KIND_DOUBLE) return fail(ctx, JJS_ERR_ARGUMENT, "key sets hold single or double keys (kind %d)", kind);
+    if (n_keys == 0 || n_keys > 0xffffffffu) return fail(ctx, JJS_ERR_ARGUMENT, "n_keys must be in [1, 2^32)");
+    if (!pk || !keyset_out) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    KeySet* ks = new (std::nothrow) KeySet();
+    if (!ks) return fail(ctx, JJS_ERR_NOMEM, "key set: out of host memory");
+    ks->variant = kind;
+    ks->n_keys = n_keys;
+    ks->dev.resize(ctx->dev.size());
+    for (size_t k = 0; k < ctx->dev.size(); k++) {
+        int rc = keyset_build(ctx, ctx->dev[k], *ks, ks->dev[k], pk, k == 0 ? key_status_or_null : nullptr);
+        if (rc) {
+            keyset_free(ctx, ks);
+            return rc;
+        }
+    }
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    ctx->keysets.push_back(ks);
+    *keyset_out = (int)(ctx->keysets.size() - 1);
+    return JJS_SUCCESS;
+}
+JJS_API int jjs_keyset_destroy(jjs_ctx* ctx, int keyset) {
+    JJS_ENTER(ctx);
+    KeySet* ks = nullptr;
+    {
+        std::lock_guard<std::mutex> lock(ctx->mu);
+        if (keyset >= 0 && (size_t)keyset < ctx->keysets.size()) std::swap(ks, ctx->keysets[keyset]);
+    }
+    if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
+    keyset_free(ctx, ks);
+    return JJS_SUCCESS;
+}
+JJS_API int jjs_verify_keyed(jjs_ctx* ctx, int keyset, const uint32_t* key_index, const uint8_t* sig, const uint8_t* msg32, size_t n,
+                             uint8_t* status_or_null, uint8_t* c32_or_null, uint32_t* accept_bitmap_or_null) {
+    JJS_ENTER(ctx);
+    const KeySet* ks = keyset_lookup(ctx, keyset);
+    if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
+    HostPart P{PART_KEYED, ks->variant, reinterpret_cast<const uint8_t*>(key_index), sig, msg32, nullptr, n, status_or_null, c32_or_null, nullptr,
+               accept_bitmap_or_null, false, ks};
+    return run_parts(ctx, {P});
+}
+JJS_API int jjs_verify_keyed_device(jjs_ctx* ctx, int device_index, int keyset, const uint32_t* d_key_index, const uint8_t* d_sig,
+                                    const uint8_t* d_msg32, size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream) {
+    JJS_ENTER(ctx);
+    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
+    const KeySet* ks = keyset_lookup(ctx, keyset);
+    if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
+    if (n == 0) return JJS_SUCCESS;
+    if (!d_key_index || !d_sig || !d_msg32 || !d_status) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    return run_keyed_device(ctx, ctx->dev[device_index], *ks, ks->dev[device_index], d_key_index, d_sig, d_msg32, n, d_status, d_c32_or_null,
+                            (cudaStream_t)cuda_stream);
+}
+JJS_API int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* entries, size_t n, uint32_t* mismatches) {
+    JJS_ENTER(ctx);
+    const KeySet* ks = keyset_lookup(ctx, keyset);
+    if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
+    if (!mismatches) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    *mismatches = 0;
+    if (n == 0) return JJS_SUCCESS;
+    if (!entries) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    const void* srcs[1] = {entries};
+    const size_t bytes[1] = {4 * n};
+    const KeySetDev& kd = ks->dev[0];
+    uint32_t count = 0;
+    int rc = run_small(ctx, "key-set table check", 4 * n, 4, srcs, bytes, 1, &count, [&](DeviceState& d, uint8_t* in, uint8_t* o) {
+        cudaMemsetAsync(o, 0, 4, d.stream);
+        k_keyset_check<<<blocks_for(n), BLOCK, 0, d.stream>>>(ks->variant, kd.u, kd.v, kd.flags, ks->n_keys, kd.table, reinterpret_cast<const uint32_t*>(in),
+                                                             n, reinterpret_cast<uint32_t*>(o));
+        ctx->launches++;
+    });
+    *mismatches = count;
     return rc;
 }
 JJS_API int jjs_sign_batch(jjs_ctx* ctx, int variant, const uint8_t* sk32, const uint8_t* rnd32, const uint8_t* gen_scalar32_or_null,

@@ -205,10 +205,74 @@ def make_typed_single_batch(bv: BatchVerifier, n: int, invalid_frac: float, seed
     return np.ascontiguousarray(points), np.ascontiguousarray(sig[:, :32]), msg, expected
 
 
+# Invalid keys registered after the valid ones in make_keyed_batch: (class name, encoding of the key's first point)
+KEYED_BAD_KEYS = [("pk_identity", IDENTITY), ("pk_order2", ORDER2), ("pk_order4", ORDER4), ("pk_v_ge_q", V_GE_Q), ("pk_off_curve", OFF_CURVE)] + \
+    [("pk_mixed_order", m) for m in MIXED_ORDER]
+KEYED_CLASSES = CLASSES + [("key_index_out_of_range", 3)]
+
+
+def make_keyed_batch(bv: BatchVerifier, kind: int, n_keys: int, n: int, invalid_frac: float, seed: int = 0xB200, rank: int = 0):
+    """Items under a registered key set (jjs_verify_keyed): n_keys signing keys, each item signed by one drawn uniformly, then a
+    fraction invalidated with the classes of `invalidate` plus an out-of-range key index.  The key classes become indices:
+    the set holds the n_keys signing keys, then one valid key that signs nothing (what `pk_from_next_item` points to when the
+    next item has the same key) and the invalid keys of KEYED_BAD_KEYS (for DOUBLE their second point is a valid pk').
+    Returns (pks[n_keys + 1 + len(KEYED_BAD_KEYS), PK_SIZE], key_index[n], sig, msg, expected_status, class_index)."""
+    rng = np.random.default_rng([seed, rank, kind, 17])
+    sk = random_scalars(rng, n_keys + 1, 251)
+    sk[:, 0] |= 1
+    idx = rng.integers(0, n_keys, size=n, dtype=np.int64).astype(np.uint32)
+    rnd = random_scalars(rng, n_keys + 1 + n, 251)
+    msg = random_scalars(rng, n_keys + 1 + n, 254)
+    pk_all, sig_all = bv.sign_batch(kind, np.concatenate([sk, sk[idx]]), rnd, msg)
+    good, sig, msg = pk_all[:n_keys + 1], sig_all[n_keys + 1:].copy(), msg[n_keys + 1:].copy()
+    bad = np.repeat(good[:1], len(KEYED_BAD_KEYS), axis=0)
+    for b, (_, enc) in enumerate(KEYED_BAD_KEYS):
+        bad[b, :32] = enc
+    pks = np.ascontiguousarray(np.concatenate([good, bad]))
+    bad_of = {}
+    for b, (name, _) in enumerate(KEYED_BAD_KEYS):
+        bad_of.setdefault(name, []).append(n_keys + 1 + b)
+    expected = np.zeros(n, dtype=np.uint8)
+    cls = np.full(n, -1, dtype=np.int16)
+    k = int(round(invalid_frac * n))
+    chosen = np.sort(rng.choice(n, size=k, replace=False)) if k else np.zeros(0, dtype=np.int64)
+    orig_sig, orig_idx = sig.copy(), idx.copy()
+    for j, i in enumerate(chosen):
+        c = j % len(KEYED_CLASSES)
+        name, st = KEYED_CLASSES[c]
+        nxt = (i + 1) % n
+        if name == "u_plus_one":
+            sig[i, :32] = _le((int.from_bytes(sig[i, :32].tobytes(), "little") + 1) % R_INT)
+        elif name == "u_ge_r":
+            sig[i, :32] = U_GE_R
+        elif name == "msg_bit_flip":
+            msg[i, 0] ^= 1
+        elif name == "msg_ge_q":
+            msg[i] = M_GE_Q
+        elif name == "R_from_next_item":
+            sig[i, 32:64] = orig_sig[nxt, 32:64]
+        elif name == "R_sign_flip":
+            sig[i, 63] ^= 0x80
+        elif name == "pk_from_next_item":
+            idx[i] = orig_idx[nxt] if orig_idx[nxt] != orig_idx[i] else n_keys
+        elif name in ("R_identity", "R_order8", "R_v_ge_q", "R_off_curve", "R_mixed_order"):
+            sig[i, 32:64] = {"R_identity": IDENTITY, "R_order8": ORDER8, "R_v_ge_q": V_GE_Q, "R_off_curve": OFF_CURVE,
+                             "R_mixed_order": MIXED_ORDER[j % len(MIXED_ORDER)]}[name]
+        elif name == "key_index_out_of_range":
+            idx[i] = pks.shape[0] + j
+        else:
+            choices = bad_of[name]
+            idx[i] = choices[j % len(choices)]
+        expected[i] = st
+        cls[i] = c
+    return pks, idx, sig, msg, expected, cls
+
+
 def make_batch(bv: BatchVerifier, variant: int, n: int, invalid_frac: float, seed: int = 0xB200, rank: int = 0):
     pk, sig, msg = make_valid(bv, variant, n, seed, rank)
     assert pk.shape == (n, PK_SIZE[variant]) and sig.shape == (n, SIG_SIZE[variant])
     return invalidate(variant, pk, sig, msg, invalid_frac, seed, rank)
 
 
-__all__ = ["make_batch", "make_aggregate_batch", "make_valid", "invalidate", "CLASSES", "AGG_CLASSES", "SINGLE", "DOUBLE", "VARGEN"]
+__all__ = ["make_batch", "make_aggregate_batch", "make_keyed_batch", "make_valid", "invalidate", "CLASSES", "AGG_CLASSES", "KEYED_CLASSES", "SINGLE",
+           "DOUBLE", "VARGEN"]

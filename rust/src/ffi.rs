@@ -81,6 +81,16 @@ extern "C" {
                                        h_offsets: *const u32, d_sig64: *const u8, d_msg32: *const u8, n: usize,
                                        d_status: *mut u8, d_c32_or_null: *mut u8, d_aggpk32_or_null: *mut u8,
                                        cuda_stream: *mut c_void) -> c_int;
+    // registered key sets (single or double keys): decoded, validated and tabulated once, named by an int handle
+    pub fn jjs_keyset_create(ctx: *mut jjs_ctx, kind: c_int, pk: *const u8, n_keys: usize, key_status_or_null: *mut u8,
+                             keyset_out: *mut c_int) -> c_int;
+    pub fn jjs_keyset_destroy(ctx: *mut jjs_ctx, keyset: c_int) -> c_int;
+    pub fn jjs_verify_keyed(ctx: *mut jjs_ctx, keyset: c_int, key_index: *const u32, sig: *const u8, msg32: *const u8, n: usize,
+                            status_or_null: *mut u8, c32_or_null: *mut u8, accept_bitmap_or_null: *mut u32) -> c_int;
+    pub fn jjs_verify_keyed_device(ctx: *mut jjs_ctx, device_index: c_int, keyset: c_int, d_key_index: *const u32, d_sig: *const u8,
+                                   d_msg32: *const u8, n: usize, d_status: *mut u8, d_c32_or_null: *mut u8,
+                                   cuda_stream: *mut c_void) -> c_int;
+    pub fn jjs_keyset_table_check(ctx: *mut jjs_ctx, keyset: c_int, entries: *const u32, n: usize, mismatches: *mut u32) -> c_int;
     // typed inputs: JubJubExtended coordinates, 160 bytes per point (variant 0: PK, R; 1: PK, PK', R, R'; 2: PK, gen, R)
     pub fn jjs_verify_ext(ctx: *mut jjs_ctx, variant: c_int, points_ext160: *const u8, u32_: *const u8, msg32: *const u8,
                           n: usize, status: *mut u8, c32_or_null: *mut u8) -> c_int;
