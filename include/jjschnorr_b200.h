@@ -60,6 +60,23 @@ typedef struct jjs_ctx jjs_ctx;
  * On failure *out still receives a context, for jjs_last_error only: every other entry point returns JJS_ERR_CUDA on
  * it (there is no CPU fallback) and jjs_destroy frees it. */
 int jjs_init(const int* devices, int n_devices, jjs_ctx** out);
+/* A context that never holds more than device_memory_limit bytes of device memory on any of its devices: constant tables,
+ * fixed-base tables, pipeline scratch, staging, aggregate scratch and registered key sets together.  Everything except key
+ * sets is allocated here, so the footprint is known when the call returns.  The library picks the fastest configuration
+ * inside the limit: the capacity C (items per pipeline pass) is the largest power of two in [2^12, 2^20] whose scratch
+ * (about 4.2 KB per item) fits beside the 12-bit fixed-base tables (21 windows of 2^12 points, 8.3 MB per generator, L2
+ * resident); the 21-bit tables of jjs_init (2.4 GB each) are built instead if they fit in what is left.  Every entry point
+ * works on such a context and returns the same bytes as on a jjs_init context; batches of any size stream through C items
+ * per pass (host-buffer calls in windows of the staging reserved here).  A call that needs more (a larger tag table, more
+ * signers in one item than the aggregate key scratch holds, a larger staging window, a key set) grows within the limit or
+ * returns JJS_ERR_NOMEM and leaves the context usable.  A multisig session may have at most C participants.
+ * JJS_ERR_NOMEM if even the smallest configuration (about 40 MB; the message states it) does not fit, with nothing left
+ * allocated and *out an inert context for jjs_last_error, like jjs_init's; JJS_ERR_ARGUMENT for a limit of 0. */
+int jjs_init_limited(const int* devices, int n_devices, size_t device_memory_limit, jjs_ctx** out);
+/* What the context holds on device device_index: bytes of device memory it allocated, the fixed-base window width of its
+ * G / G' tables (21 or 12), and the items per pipeline pass (the largest batch that runs without being cut into passes).
+ * A jjs_init context reports width 21, 2^20 items and what it has allocated so far.  Any pointer may be NULL. */
+int jjs_memory_info(const jjs_ctx* ctx, int device_index, uint64_t* bytes_held, int* fb_window_bits, uint64_t* items_in_flight);
 void jjs_destroy(jjs_ctx* ctx);
 /* Human-readable description of the last failure on this context ("" if none). */
 const char* jjs_last_error(const jjs_ctx* ctx);

@@ -34,14 +34,10 @@ inline BlsScalar bls_scalar_from_u64(uint64_t x) {
 // Owns a jjs_ctx.  One host thread at a time.
 class Gpu {
 public:
-    explicit Gpu(const std::vector<int>& devices = {0}) {
-        int rc = jjs_init(devices.data(), int(devices.size()), &ctx_);
-        if (rc != JJS_SUCCESS) {
-            std::string msg = ctx_ ? jjs_last_error(ctx_) : "allocation failed";
-            if (ctx_) jjs_destroy(ctx_);
-            ctx_ = nullptr;
-            throw std::runtime_error("jjs_init: " + msg);  // no CPU fallback
-        }
+    explicit Gpu(const std::vector<int>& devices = {0}) { init(jjs_init(devices.data(), int(devices.size()), &ctx_), "jjs_init"); }
+    // A context that holds at most device_memory_limit bytes of device memory on each device (jjs_init_limited).
+    Gpu(const std::vector<int>& devices, size_t device_memory_limit) {
+        init(jjs_init_limited(devices.data(), int(devices.size()), device_memory_limit, &ctx_), "jjs_init_limited");
     }
     ~Gpu() { if (ctx_) jjs_destroy(ctx_); }
     Gpu(const Gpu&) = delete;
@@ -52,6 +48,14 @@ public:
     }
 
 private:
+    void init(int rc, const char* what) {
+        if (rc != JJS_SUCCESS) {
+            std::string msg = ctx_ ? jjs_last_error(ctx_) : "allocation failed";
+            if (ctx_) jjs_destroy(ctx_);
+            ctx_ = nullptr;
+            throw std::runtime_error(std::string(what) + ": " + msg);  // no CPU fallback
+        }
+    }
     jjs_ctx* ctx_ = nullptr;
 };
 

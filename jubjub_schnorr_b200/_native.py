@@ -19,6 +19,7 @@ EXPORTS = [
     "jjs_verify_batch", "jjs_status_bitmap_device", "jjs_verify_batch_double", "jjs_verify_batch_vargen", "jjs_verify_batch_aggregate",
     "jjs_verify_mixed",
     "jjs_keyset_create", "jjs_keyset_destroy", "jjs_verify_keyed", "jjs_verify_keyed_device", "jjs_keyset_table_check",
+    "jjs_init_limited", "jjs_memory_info",
 ]
 
 
@@ -47,6 +48,10 @@ def lib():
     vp, sz = C.c_void_p, C.c_size_t
     L.jjs_init.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]
     L.jjs_init.restype = C.c_int
+    L.jjs_init_limited.argtypes = [C.POINTER(C.c_int), C.c_int, sz, C.POINTER(vp)]
+    L.jjs_init_limited.restype = C.c_int
+    L.jjs_memory_info.argtypes = [vp, C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_int), C.POINTER(C.c_uint64)]
+    L.jjs_memory_info.restype = C.c_int
     L.jjs_destroy.argtypes = [vp]
     L.jjs_destroy.restype = None
     L.jjs_last_error.argtypes = [vp]

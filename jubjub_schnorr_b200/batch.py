@@ -35,19 +35,23 @@ def _u8(a, width, name):
 class BatchVerifier:
     """Owns a jjs_ctx over one or more CUDA devices.  One host thread at a time."""
 
-    def __init__(self, devices=None):
+    def __init__(self, devices=None, memory_limit=None):
+        """memory_limit: bytes of device memory the context may hold on each device (jjs_init_limited); None: jjs_init."""
         self._lib = _native.lib()
         self._ctx = C.c_void_p()
         if devices is None:
             devices = [0]
         arr = (C.c_int * len(devices))(*devices)
-        rc = self._lib.jjs_init(arr, len(devices), C.byref(self._ctx))
+        if memory_limit is None:
+            name, rc = "jjs_init", self._lib.jjs_init(arr, len(devices), C.byref(self._ctx))
+        else:
+            name, rc = "jjs_init_limited", self._lib.jjs_init_limited(arr, len(devices), int(memory_limit), C.byref(self._ctx))
         if rc != 0:
             msg = self._lib.jjs_last_error(self._ctx).decode() if self._ctx else "allocation failed"
             if self._ctx:
                 self._lib.jjs_destroy(self._ctx)
                 self._ctx = C.c_void_p()
-            raise JjsError(f"jjs_init failed ({rc}): {msg}")
+            raise JjsError(f"{name} failed ({rc}): {msg}")
         self.devices = list(devices)
 
     def close(self):
@@ -70,6 +74,12 @@ class BatchVerifier:
     def _check(self, rc, what):
         if rc != 0:
             raise JjsError(f"{what} failed ({rc}): {self._lib.jjs_last_error(self._ctx).decode()}")
+
+    def memory_info(self, device_index=0):
+        """{"bytes_held", "fb_window_bits", "items_in_flight"} of the context on one of its devices (jjs_memory_info)."""
+        held, items, bits = C.c_uint64(), C.c_uint64(), C.c_int()
+        self._check(self._lib.jjs_memory_info(self._ctx, device_index, C.byref(held), C.byref(bits), C.byref(items)), "jjs_memory_info")
+        return {"bytes_held": int(held.value), "fb_window_bits": int(bits.value), "items_in_flight": int(items.value)}
 
     @property
     def launch_count(self) -> int:

@@ -575,17 +575,24 @@ JJS_HD void straus_multi32(ext& r, int nb, const fq* tab, size_t stride, const i
     r = acc;
 }
 
+// Window tables of width W bits: fb_windows(W) windows of 2^W entries.  Every kernel that reads the G / G' tables is instantiated
+// at the device default FB_W and at FB_W_SMALL (memory-limited contexts, include/jjschnorr_b200.h jjs_init_limited).
+constexpr int FB_W_SMALL = 12;
+constexpr int fb_windows(int w) { return (252 + w - 1) / w; }
+
 // r = k * B for a fixed base with precomputed window tables: sum over windows of table[w][k_w] (mixed additions)
+template <int W = FB_W>
 JJS_HD void fixedbase_mul(ext& r, const niels* table, const uint32_t* k) {
+    constexpr int WINDOWS = (252 + W - 1) / W, ENTRIES = 1 << W;
     ext acc;
     ext_identity(acc);
 #pragma unroll 1
-    for (int w = 0; w < FB_WINDOWS; w++) {
-        int bit = w * FB_W;
+    for (int w = 0; w < WINDOWS; w++) {
+        int bit = w * W;
         uint32_t lo = k[bit >> 5] >> (bit & 31);
-        if ((bit & 31) + FB_W > 32 && (bit >> 5) + 1 < 8) lo |= k[(bit >> 5) + 1] << (32 - (bit & 31));
-        uint32_t idx = lo & (FB_ENTRIES - 1);
-        niels n = table[(size_t)w * FB_ENTRIES + idx];
+        if ((bit & 31) + W > 32 && (bit >> 5) + 1 < 8) lo |= k[(bit >> 5) + 1] << (32 - (bit & 31));
+        uint32_t idx = lo & (ENTRIES - 1);
+        niels n = table[(size_t)w * ENTRIES + idx];
         ext t;
         ext_add_niels<true>(t, acc, n);
         acc = t;
@@ -595,14 +602,16 @@ JJS_HD void fixedbase_mul(ext& r, const niels* table, const uint32_t* k) {
 
 // acc += k * B (acc.T defined on entry; not on return): the windows are added straight onto a running sum, which saves the
 // separate accumulator of fixedbase_mul and the conversion and addition that would join the two
+template <int W = FB_W>
 JJS_HD void fixedbase_acc(ext& acc, const niels* table, const uint32_t* k) {
+    constexpr int WINDOWS = (252 + W - 1) / W, ENTRIES = 1 << W;
 #pragma unroll 1
-    for (int w = 0; w < FB_WINDOWS; w++) {
-        int bit = w * FB_W;
+    for (int w = 0; w < WINDOWS; w++) {
+        int bit = w * W;
         uint32_t lo = k[bit >> 5] >> (bit & 31);
-        if ((bit & 31) + FB_W > 32 && (bit >> 5) + 1 < 8) lo |= k[(bit >> 5) + 1] << (32 - (bit & 31));
-        uint32_t idx = lo & (FB_ENTRIES - 1);
-        niels n = table[(size_t)w * FB_ENTRIES + idx];
+        if ((bit & 31) + W > 32 && (bit >> 5) + 1 < 8) lo |= k[(bit >> 5) + 1] << (32 - (bit & 31));
+        uint32_t idx = lo & (ENTRIES - 1);
+        niels n = table[(size_t)w * ENTRIES + idx];
         ext_add_niels<true>(acc, acc, n);   // in place
     }
 }
@@ -641,19 +650,20 @@ JJS_HD void niels_from_affine(niels& out, const fq& u, const fq& v) {
     fq_mul(out.t2d, u, v);
     fq_mul(out.t2d, out.t2d, d2);
 }
-// One entry of a fixed-base window table: j * 2^(FB_W w) * B as affine Niels, from scratch (the definition; the device builds
+// One entry of a fixed-base window table: j * 2^(W w) * B as affine Niels, from scratch (the definition; the device builds
 // its tables in two passes, see fb_combine_entries, and the host twin incrementally -- both are checked against this one).
+template <int W = FB_W>
 JJS_HD void fb_table_entry(niels& out, const fq& bu, const fq& bv, int w, int j) {
     fq u, v;
-    fb_affine_multiple(u, v, bu, bv, w * FB_W, j, FB_W);
+    fb_affine_multiple(u, v, bu, bv, w * W, j, W);
     niels_from_affine(out, u, v);
 }
-// Two-pass construction of a window: with j = jh 2^FB_LO + jl the entry is H[jh] + S[jl] for the small tables
-// S[jl] = jl 2^(FB_W w) B (2^FB_LO affine points) and H[jh] = jh 2^(FB_W w + FB_LO) B (2^FB_HI points).  A thread combines
+// Two-pass construction of a window: with j = jh 2^LO + jl the entry is H[jh] + S[jl] for the small tables
+// S[jl] = jl 2^(W w) B (2^LO affine points) and H[jh] = jh 2^(W w + LO) B (2^HI points), LO = (W + 1) / 2, HI = W - LO.  A thread combines
 // FB_BATCH consecutive entries (same jh) and shares one inversion among them (Montgomery's trick): ~50 products per entry
 // instead of the ~1 200 of fb_table_entry, which is what makes 2^21-entry windows cheap to build (12 x 2^21 entries x 2 bases
 // in well under a second).
-constexpr int FB_LO = (FB_W + 1) / 2, FB_HI = FB_W - FB_LO, FB_BATCH = 8;
+constexpr int FB_BATCH = 8;
 JJS_HD void fb_combine_entries(niels* out, const fq* s_u, const fq* s_v, const fq& hu, const fq& hv) {
     ext h, p[FB_BATCH];
     ext_from_affine(h, hu, hv);

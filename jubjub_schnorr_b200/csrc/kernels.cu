@@ -65,8 +65,18 @@ constexpr int BLOCK = JJS_BLOCK;
 #ifndef JJS_EQ_PERSISTENT
 #define JJS_EQ_PERSISTENT 0   // measured (gpurun_out/ab2.log, DESIGN.md section 8): -22 % DRAM reads but +6 % time; off
 #endif
-constexpr size_t CHUNK_ITEMS = size_t(1) << 20;   // items per pipeline pass
+constexpr size_t CHUNK_ITEMS = size_t(1) << 20;   // items per pipeline pass (jjs_init contexts)
 constexpr size_t TAB_THREADS = size_t(1) << 20;   // threads served by the per-thread table scratch (four tables of 1152 B each)
+constexpr size_t SUB_ITEMS = CHUNK_ITEMS / 2;      // items per scratch half
+#ifndef JJS_SUB_CHUNK_LOG2
+#define JJS_SUB_CHUNK_LOG2 19   // 2^18: 20.86 M/s device-resident on 2^20 singles, 2^19: 21.19 (fewer partially filled waves)
+#endif
+#ifndef JJS_FIRST_SLICE_LOG2
+#define JJS_FIRST_SLICE_LOG2 17  // first slice of a host-buffer shard: short, so that compute starts while the rest is still being copied
+#endif
+constexpr size_t SUB_CHUNK = size_t(1) << JJS_SUB_CHUNK_LOG2;      // items per sub-chunk of an overlapped batch (<= SUB_ITEMS)
+constexpr size_t AGG_KEYS_INITIAL = size_t(1) << 21;               // signer keys per scratch half of the aggregate path, first size
+constexpr size_t TAGS_INITIAL = 1024;                              // SAFE tags of the multisig transcripts, first size
 
 struct Fields {
     WireField f[4];
@@ -264,8 +274,9 @@ __global__ void __launch_bounds__(BLOCK) k_subgroup_check(WireField pts, size_t 
 
 // thread T = first + t < neq * *count : equation T % neq of item list[T / neq].  Signature points whose subgroup
 // membership the equation did not establish are appended to `rlist` (indices into the point arrays) for k_rtest.
-// (instantiated per kind of equation: MODE 0 fixed base -- single, double -- and MODE 1 variable base -- var-gen)
-template <int MODE>
+// (instantiated per kind of equation: MODE 0 fixed base -- single, double -- and MODE 1 variable base -- var-gen; MODE 0 also per
+// width W of the fixed-base tables)
+template <int MODE, int W = FB_W>
 __global__ void __launch_bounds__(BLOCK, MODE ? JJS_EQ1_MINBLOCKS : JJS_EQ_MINBLOCKS) k_equation(int variant, const fq* pts_u, const fq* pts_v, uint8_t* pflags, size_t n,
                                                     size_t first, size_t count, const uint32_t* list, const uint32_t* lcount, WireField usc,
                                                     const uint32_t* cwords, uint8_t* eqflags, fq* tab, size_t stride, Tables T,
@@ -288,7 +299,7 @@ __global__ void __launch_bounds__(BLOCK, MODE ? JJS_EQ1_MINBLOCKS : JJS_EQ_MINBL
         int eq = (int)(g % neq);
         size_t item = list[g / neq];
         bool need_r_test;
-        bool ok = stage_equation_item<MODE>(variant, eq, pts_u, pts_v, pflags, n, item, (variant == VAR_DOUBLE && eq == 1) ? T.fb_gn : T.fb_g, usc, cwords,
+        bool ok = stage_equation_item<MODE, W>(variant, eq, pts_u, pts_v, pflags, n, item, (variant == VAR_DOUBLE && eq == 1) ? T.fb_gn : T.fb_g, usc, cwords,
                                             tab + t, tab + 36 * stride + t, stride, &need_r_test);
         if (need_r_test) {
             int pk_slot, r_slot, base_slot;
@@ -371,41 +382,47 @@ __global__ void __launch_bounds__(BLOCK) k_bitmap(const uint8_t* status, size_t 
     if ((threadIdx.x & 31) == 0 && i < n) words[i >> 5] = w;
 }
 
-// Fixed-base tables in two passes (curve.cuh, fb_combine_entries).  Pass 1: the small tables of every window, affine points,
-// small[w][0 .. 2^FB_LO) = jl 2^(FB_W w) B  and  small[w][2^FB_LO .. 2^FB_LO + 2^FB_HI) = jh 2^(FB_W w + FB_LO) B.
-constexpr int FB_SMALL = (1 << FB_LO) + (1 << FB_HI);
+// Fixed-base tables of width W in two passes (curve.cuh, fb_combine_entries), LO = (W + 1) / 2, HI = W - LO.  Pass 1: the small
+// tables of every window, affine points, small[w][0 .. 2^LO) = jl 2^(W w) B  and  small[w][2^LO .. 2^LO + 2^HI) = jh 2^(W w + LO) B.
+template <int W>
 __global__ void __launch_bounds__(BLOCK) k_fb_small(fq* small_u, fq* small_v, int which) {
+    constexpr int LO = (W + 1) / 2, HI = W - LO, WINDOWS = (252 + W - 1) / W, SMALL = (1 << LO) + (1 << HI);
     int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= FB_WINDOWS * FB_SMALL) return;
+    if (t >= WINDOWS * SMALL) return;
     fq bu, bv, u, v;
     fq_load_const(bu, which ? JJS_C(GEN_NUMS_UV)[0] : JJS_C(GEN_UV)[0]);
     fq_load_const(bv, which ? JJS_C(GEN_NUMS_UV)[1] : JJS_C(GEN_UV)[1]);
-    int w = t / FB_SMALL, e = t % FB_SMALL;
-    if (e < (1 << FB_LO)) fb_affine_multiple(u, v, bu, bv, w * FB_W, e, FB_LO);
-    else fb_affine_multiple(u, v, bu, bv, w * FB_W + FB_LO, e - (1 << FB_LO), FB_HI);
+    int w = t / SMALL, e = t % SMALL;
+    if (e < (1 << LO)) fb_affine_multiple(u, v, bu, bv, w * W, e, LO);
+    else fb_affine_multiple(u, v, bu, bv, w * W + LO, e - (1 << LO), HI);
     small_u[t] = u;
     small_v[t] = v;
 }
-// Pass 2: thread t combines entries [FB_BATCH t, FB_BATCH (t + 1)) of the table (FB_BATCH divides 2^FB_LO, so they share jh).
+// Pass 2: thread t combines entries [FB_BATCH t, FB_BATCH (t + 1)) of the table (FB_BATCH divides 2^LO, so they share jh).
+template <int W>
 __global__ void __launch_bounds__(BLOCK) k_fb_combine(niels* out, const fq* small_u, const fq* small_v) {
+    constexpr int LO = (W + 1) / 2, HI = W - LO, WINDOWS = (252 + W - 1) / W, ENTRIES = 1 << W, SMALL = (1 << LO) + (1 << HI);
+    static_assert((1 << LO) % FB_BATCH == 0, "a batch of table entries must share its high half");
     size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (size_t)FB_WINDOWS * FB_ENTRIES / FB_BATCH) return;
+    if (t >= (size_t)WINDOWS * ENTRIES / FB_BATCH) return;
     size_t first = t * FB_BATCH;
-    int w = (int)(first / FB_ENTRIES), j = (int)(first % FB_ENTRIES), jh = j >> FB_LO, jl = j & ((1 << FB_LO) - 1);
-    const fq* su = small_u + (size_t)w * FB_SMALL;
-    const fq* sv = small_v + (size_t)w * FB_SMALL;
-    fb_combine_entries(out + first, su + jl, sv + jl, su[(1 << FB_LO) + jh], sv[(1 << FB_LO) + jh]);
+    int w = (int)(first / ENTRIES), j = (int)(first % ENTRIES), jh = j >> LO, jl = j & ((1 << LO) - 1);
+    const fq* su = small_u + (size_t)w * SMALL;
+    const fq* sv = small_v + (size_t)w * SMALL;
+    fb_combine_entries(out + first, su + jl, sv + jl, su[(1 << LO) + jh], sv[(1 << LO) + jh]);
 }
 // the definition, entry by entry (jjs_fb_table_check compares a sample of the built tables with it)
+template <int W>
 __global__ void __launch_bounds__(BLOCK) k_fb_check(const niels* table, int which, const uint32_t* entries, int n, uint32_t* mismatches) {
+    constexpr int WINDOWS = (252 + W - 1) / W, ENTRIES = 1 << W;
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
     fq u, v;
     fq_load_const(u, which ? JJS_C(GEN_NUMS_UV)[0] : JJS_C(GEN_UV)[0]);
     fq_load_const(v, which ? JJS_C(GEN_NUMS_UV)[1] : JJS_C(GEN_UV)[1]);
     niels e;
-    uint32_t idx = entries[t] % (uint32_t)(FB_WINDOWS * FB_ENTRIES);
-    fb_table_entry(e, u, v, (int)(idx / FB_ENTRIES), (int)(idx % FB_ENTRIES));
+    uint32_t idx = entries[t] % (uint32_t)(WINDOWS * ENTRIES);
+    fb_table_entry<W>(e, u, v, (int)(idx / ENTRIES), (int)(idx % ENTRIES));
     const niels& g = table[idx];
     if (!(fq_eq(e.ypx, g.ypx) && fq_eq(e.ymx, g.ymx) && fq_eq(e.t2d, g.t2d))) atomicAdd(mismatches, 1u);
 }
@@ -462,6 +479,7 @@ __global__ void __launch_bounds__(BLOCK) k_keyed_gather(int variant, const fq* k
 #ifndef JJS_EQK_MINBLOCKS
 #define JJS_EQK_MINBLOCKS 4
 #endif
+template <int W = FB_W>
 __global__ void __launch_bounds__(BLOCK, JJS_EQK_MINBLOCKS) k_equation_keyed(int variant, const fq* pts_u, const fq* pts_v, uint8_t* pflags, size_t n,
                                                                              const uint32_t* list, const uint32_t* lcount, WireField usc,
                                                                              const uint32_t* cwords, uint8_t* eqflags, const niels* ktab,
@@ -475,7 +493,7 @@ __global__ void __launch_bounds__(BLOCK, JJS_EQK_MINBLOCKS) k_equation_keyed(int
     const uint32_t key = key_index[item];   // in range: items under an unknown index never reach the work list
     bool need_r_test = false;
     const bool ok = key < n_keys &&
-                    stage_equation_keyed(variant, eq, pts_u, pts_v, pflags, n, item, eq == 1 ? T.fb_gn : T.fb_g,
+                    stage_equation_keyed<W>(variant, eq, pts_u, pts_v, pflags, n, item, eq == 1 ? T.fb_gn : T.fb_g,
                                          ktab + ((size_t)key * neq + eq) * KEYED_POINT_ENTRIES, usc, cwords, &need_r_test);
     if (need_r_test) {
         int pk_slot, r_slot, base_slot;
@@ -486,8 +504,8 @@ __global__ void __launch_bounds__(BLOCK, JJS_EQK_MINBLOCKS) k_equation_keyed(int
 }
 
 // one thread signs one item; inputs are 32-byte little-endian scalars, outputs the reference's wire bytes.
-// The variant is a template parameter so that every array index below is static.
-template <int VARIANT>
+// The variant is a template parameter so that every array index below is static; W is the width of the fixed-base tables.
+template <int VARIANT, int W = FB_W>
 __global__ void __launch_bounds__(BLOCK) k_sign(const uint8_t* sk, const uint8_t* rnd, const uint8_t* gsc, const uint8_t* msg, size_t n,
                                                 uint8_t* pk_out, uint8_t* sig_out, Tables T) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -498,7 +516,7 @@ __global__ void __launch_bounds__(BLOCK) k_sign(const uint8_t* sk, const uint8_t
     wire_load(wrnd, WireField{rnd, 32}, i);
     wire_load(wm, WireField{msg, 32}, i);
     if (VARIANT == VAR_VARGEN) wire_load(wg, WireField{gsc, 32}, i);
-    bool ok = sign_item(VARIANT, wsk, wrnd, wg, wm, pk, sig, T);
+    bool ok = sign_item<W>(VARIANT, wsk, wrnd, wg, wm, pk, sig, T);
     uint4* po = reinterpret_cast<uint4*>(pk_out + i * PKW * 4);
     uint4* so = reinterpret_cast<uint4*>(sig_out + i * SGW * 4);
 #pragma unroll
@@ -526,13 +544,14 @@ __global__ void __launch_bounds__(BLOCK) k_msig_session(MsigBuffers b, size_t K,
     stage_msig_session(b.pu, b.pv, b.pf, K, b.offsets[s], b.offsets[s + 1], msg, zf, s, b.d_words, b.cd_words, b.a_words, b.rsa_u, b.rsa_v, b.sflags,
                        tab + t, stride, T.safe_tags);
 }
+template <int W = FB_W>
 __global__ void __launch_bounds__(BLOCK, JJS_EQ_MINBLOCKS) k_msig_share(MsigBuffers b, size_t K, WireField zf, fq* tab, size_t stride, Tables T) {
     size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= K) return;
     size_t s = b.owner[j];
     bool ok = false;
     if (b.sflags[s] == (SF_DECODED | SF_NONEMPTY))
-        ok = stage_msig_share(b.pu, b.pv, K, j, zf, b.cd_words, b.a_words + 8 * s, T.fb_g, tab + j, tab + 36 * stride + j, stride);
+        ok = stage_msig_share<W>(b.pu, b.pv, K, j, zf, b.cd_words, b.a_words + 8 * s, T.fb_g, tab + j, tab + 36 * stride + j, stride);
     b.share_ok[j] = ok ? 1 : 0;
 }
 __global__ void __launch_bounds__(BLOCK) k_msig_finalize(MsigBuffers b, size_t n, WireField zf, uint8_t* status, uint32_t* bad, uint8_t* sig64) {
@@ -551,6 +570,7 @@ __global__ void __launch_bounds__(BLOCK) k_msig_finalize(MsigBuffers b, size_t n
 // reference's delinearisation coefficients, and an ordinary hedged signature under it (what a completed SpeedyMuSig
 // session verifies as).  At most JJS_MAX_GEN_SIGNERS signers per item.
 #define JJS_MAX_GEN_SIGNERS 8
+template <int W = FB_W>
 __global__ void __launch_bounds__(BLOCK) k_sign_aggregate(const uint8_t* sk, const uint32_t* offsets, const uint8_t* rnd, const uint8_t* msg, size_t n,
                                                           uint8_t* pks_out, uint8_t* sig_out, Tables T) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -568,7 +588,7 @@ __global__ void __launch_bounds__(BLOCK) k_sign_aggregate(const uint8_t* sk, con
             wire_load(w, WireField{sk, 32}, lo + j);
             ok = ok && fr_wire_is_canonical(w);
             ext P;
-            fixedbase_mul(P, T.fb_g, w);
+            fixedbase_mul<W>(P, T.fb_g, w);
             ext_to_affine(ku[j], kv[j], P);
             uint32_t enc[8];
             point_to_wire(enc, ku[j], kv[j]);
@@ -600,7 +620,7 @@ __global__ void __launch_bounds__(BLOCK) k_sign_aggregate(const uint8_t* sk, con
     uint32_t wr[8], wm[8], pk[16], sig[24];
     wire_load(wr, WireField{rnd, 32}, i);
     wire_load(wm, WireField{msg, 32}, i);
-    ok = ok && sign_item(VAR_SINGLE, agg, wr, wr, wm, pk, sig, T);
+    ok = ok && sign_item<W>(VAR_SINGLE, agg, wr, wr, wm, pk, sig, T);
     uint4* so = reinterpret_cast<uint4*>(sig_out + 64 * i);
 #pragma unroll
     for (int k = 0; k < 4; k++) so[k] = ok ? make_uint4(sig[4 * k], sig[4 * k + 1], sig[4 * k + 2], sig[4 * k + 3]) : make_uint4(0, 0, 0, 0);
@@ -643,34 +663,50 @@ struct DeviceState {
     // staging of the host-buffer entry points: one grow-only device buffer, carved up per call
     uint8_t* stage = nullptr;
     size_t stage_bytes = 0;
+    // Device memory: `held` bytes allocated by the context on this device (key sets included); a memory-limited context
+    // (jjs_init_limited) never lets it exceed `limit` (0: no limit, a jjs_init context).
+    size_t limit = 0, held = 0;
+    // The configuration (pick_config for limited contexts): width of the G / G' tables, items per pipeline pass, per scratch
+    // half, per sub-chunk of an overlapped batch and in the first slice of a host-buffer shard, first size of the aggregate
+    // key scratch and items per aggregate pass the order array serves.
+    int fb_w = FB_W;
+    size_t chunk_items = CHUNK_ITEMS, sub_items = SUB_ITEMS, sub_chunk = SUB_CHUNK, first_slice = size_t(1) << JJS_FIRST_SLICE_LOG2;
+    size_t agg_keys_initial = AGG_KEYS_INITIAL, agg_items = CHUNK_ITEMS;
     Tables tables() const { return Tables{root_tables, dlog_hash, fb_g, fb_gn, safe_tags}; }
 };
 
-// A slice of the pipeline scratch able to hold `cap` items of the widest variant; `tab` serves `cap` threads (the table
-// scratch keeps its global stride TAB_THREADS).
+// Per-thread table scratch of a memory-limited context: TAB_ROWS field elements per item of capacity, the equation kernels'
+// three 36-element tables (tabA, tabB = tabA + 36 stride, and the var-generator's third).
+constexpr int TAB_ROWS = 3 * 36;
+// Stride (threads served at once) in the table scratch of a region of `cap` items for a kernel with `rows` elements per thread.
+// A jjs_init context's scratch holds the aggregation kernel's 4 x 68 rows for TAB_THREADS threads, and every kernel indexes it
+// with that stride.  A limited context gives a region TAB_ROWS x cap elements: the largest power of two <= cap whose rows fit.
+inline size_t tab_threads(const DeviceState& d, size_t cap, int rows) {
+    if (!d.limit) return TAB_THREADS;
+    size_t t = cap;
+    while (t > 1 && t * rows > (size_t)TAB_ROWS * cap) t /= 2;
+    return t;
+}
+
+// A slice of the pipeline scratch able to hold `cap` items of the widest variant; `tab` serves `cap` equation threads with stride
+// `tstride`, or `acap` threads of the aggregation kernel with stride `astride` (tab_threads).
 struct Region {
     fq *pts_u, *pts_v, *tab, *eqtab;
     uint8_t *pflags, *iflags, *eqflags;
     uint32_t *cwords, *rlist, *rcount, *eqlist;   // rcount[0]: deferred subgroup tests, rcount[2]: length of the work list
     size_t cap;
     int half;
+    size_t tstride, astride, acap;
 };
 inline Region region_of(const DeviceState& d, size_t first_item, size_t cap, int half) {
-    return Region{d.pts_u + 4 * first_item, d.pts_v + 4 * first_item, d.tab + first_item,
+    const size_t astride = tab_threads(d, cap, AGG_GROUP * R32_TAB_FQ);
+    return Region{d.pts_u + 4 * first_item, d.pts_v + 4 * first_item, d.tab + (d.limit ? (size_t)TAB_ROWS * first_item : first_item),
                   d.eqtab + (size_t)(half & 1) * d.eqtab_half, d.pflags + 4 * first_item, d.iflags + first_item,
                   d.eqflags + 2 * first_item, d.cwords + 8 * first_item, d.rlist + 2 * first_item, d.rcount + 4 * (half & 1), d.eqlist + 2 * first_item, cap,
-                  half & 1};
+                  half & 1, tab_threads(d, cap, TAB_ROWS), astride, astride < cap ? astride : cap};
 }
-constexpr size_t SUB_ITEMS = CHUNK_ITEMS / 2;      // items per scratch half
-#ifndef JJS_SUB_CHUNK_LOG2
-#define JJS_SUB_CHUNK_LOG2 19   // 2^18: 20.86 M/s device-resident on 2^20 singles, 2^19: 21.19 (fewer partially filled waves)
-#endif
-#ifndef JJS_FIRST_SLICE_LOG2
-#define JJS_FIRST_SLICE_LOG2 17  // first slice of a host-buffer shard: short, so that compute starts while the rest is still being copied
-#endif
-constexpr size_t SUB_CHUNK = size_t(1) << JJS_SUB_CHUNK_LOG2;      // items per sub-chunk of an overlapped batch (<= SUB_ITEMS)
-inline Region region_whole(const DeviceState& d) { return region_of(d, 0, CHUNK_ITEMS, 0); }
-inline Region region_half(const DeviceState& d, size_t j) { return region_of(d, (j & 1) * SUB_ITEMS, SUB_ITEMS, (int)(j & 1)); }
+inline Region region_whole(const DeviceState& d) { return region_of(d, 0, d.chunk_items, 0); }
+inline Region region_half(const DeviceState& d, size_t j) { return region_of(d, (j & 1) * d.sub_items, d.sub_items, (int)(j & 1)); }
 
 // A registered key set (jjs_keyset_create), copied to every device of the context: the decoded key points slot-major as k_decode
 // writes them (point s of key k at s * n_keys + k), their flags, and the window tables key-major (keyset.cuh; the table of point
@@ -758,19 +794,149 @@ struct StageTimer {
 inline unsigned blocks_for(size_t threads) { return (unsigned)((threads + BLOCK - 1) / BLOCK); }
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Allocator of one device of a context: `held` counts every allocation, and a memory-limited context refuses one that would
+// cross its limit.  A dry run only adds the sizes up: the policy of jjs_init_limited (footprint) runs the allocation code of a
+// configuration that way, so what it plans and what a context holds cannot drift apart.
+struct DevAlloc {
+    jjs_ctx* ctx;
+    DeviceState* d;   // nullptr: dry run
+    size_t total = 0;
+    template <typename T>
+    int operator()(T** p, size_t bytes) {
+        total += bytes;
+        if (!d) return JJS_SUCCESS;
+        *p = nullptr;
+        if (d->limit && d->held + bytes > d->limit)
+            return fail(ctx, JJS_ERR_NOMEM, "device %d: %zu more bytes would exceed the context's memory limit of %zu bytes (%zu held)", d->device, bytes,
+                        d->limit, d->held);
+        cudaError_t e = cudaMalloc((void**)p, bytes);
+        if (e != cudaSuccess) {
+            *p = nullptr;
+            cudaGetLastError();
+            return fail(ctx, e == cudaErrorMemoryAllocation ? JJS_ERR_NOMEM : JJS_ERR_CUDA, "cudaMalloc of %zu bytes on device %d failed: %s", bytes,
+                        d->device, cudaGetErrorString(e));
+        }
+        d->held += bytes;
+        return JJS_SUCCESS;
+    }
+};
+inline DevAlloc dev_alloc(jjs_ctx* ctx, DeviceState& d) { return DevAlloc{ctx, &d}; }
+template <typename T>
+void dev_free(DeviceState& d, T*& p, size_t bytes) {
+    if (!p) return;
+    cudaFree(p);
+    p = nullptr;
+    d.held -= bytes;
+}
+// a growth of `more` bytes that frees `less` first: refused up front on a limited context, which then keeps what it has
+int check_growth(jjs_ctx* ctx, const DeviceState& d, size_t less, size_t more, const char* what) {
+    if (d.limit && d.held - less + more > d.limit)
+        return fail(ctx, JJS_ERR_NOMEM, "device %d: growing the %s to %zu bytes would exceed the context's memory limit of %zu bytes (%zu held)", d.device,
+                    what, more, d.limit, d.held);
+    return JJS_SUCCESS;
+}
+
+inline size_t fb_table_bytes(int w) { return sizeof(niels) * (size_t)fb_windows(w) << w; }
+
+// constant tables and the fixed-base tables of width d.fb_w
+int alloc_tables(DevAlloc& A, DeviceState& d) {
+    int rc = A(&d.root_tables, sizeof(tables::ROOT_TABLES));
+    if (!rc) rc = A(&d.dlog_hash, sizeof(tables::DLOG_HASH));
+    if (!rc) rc = A(&d.fb_g, fb_table_bytes(d.fb_w));
+    if (!rc) rc = A(&d.fb_gn, fb_table_bytes(d.fb_w));
+    return rc;
+}
+
+// pipeline scratch for `cap` items of the widest variant (4 points, 2 equations) and `tab_fq` elements of per-thread tables
+int alloc_pipeline(DevAlloc& A, DeviceState& d, size_t cap, size_t tab_fq) {
+    int rc = A(&d.pts_u, sizeof(fq) * 4 * cap);
+    if (!rc) rc = A(&d.pts_v, sizeof(fq) * 4 * cap);
+    if (!rc) rc = A(&d.pflags, 4 * cap);
+    if (!rc) rc = A(&d.iflags, cap);
+    if (!rc) rc = A(&d.eqflags, 2 * cap);
+    if (!rc) rc = A(&d.cwords, 32 * cap);
+    if (!rc) rc = A(&d.rlist, sizeof(uint32_t) * 2 * cap);
+    if (!rc) rc = A(&d.rcount, 8 * sizeof(uint32_t));
+    if (!rc) rc = A(&d.eqlist, sizeof(uint32_t) * 2 * cap);
+    if (!rc) rc = A(&d.tab, sizeof(fq) * tab_fq);
+    return rc;
+}
+
+// one half of the aggregate path's scratch: `keys` signer keys; the order and sort state are allocated once
+inline size_t agg_key_bytes(size_t keys) { return keys * (2 * sizeof(fq) + 1 + 32 + 2 * sizeof(uint32_t)); }
+int alloc_agg_half(DevAlloc& A, const DeviceState& d, AggScratch& a, size_t keys) {
+    int rc = A(&a.keys_u, sizeof(fq) * keys);
+    if (!rc) rc = A(&a.keys_v, sizeof(fq) * keys);
+    if (!rc) rc = A(&a.kflags, keys);
+    if (!rc) rc = A(&a.kcoef, 32 * keys);
+    if (!rc) rc = A(&a.kmap, sizeof(uint32_t) * keys);
+    if (!rc) rc = A(&a.kitem, sizeof(uint32_t) * keys);
+    if (!rc && !a.order) rc = A(&a.order, sizeof(uint32_t) * d.agg_items);
+    if (!rc && !a.sort) rc = A(&a.sort, sizeof(AggSort));
+    if (!rc) a.cap_keys = keys;
+    return rc;
+}
+void free_agg_keys(DeviceState& d, AggScratch& a) {
+    const size_t k = a.cap_keys;
+    dev_free(d, a.keys_u, sizeof(fq) * k); dev_free(d, a.keys_v, sizeof(fq) * k); dev_free(d, a.kflags, k); dev_free(d, a.kcoef, 32 * k);
+    dev_free(d, a.kmap, sizeof(uint32_t) * k); dev_free(d, a.kitem, sizeof(uint32_t) * k);
+    a.cap_keys = 0;
+}
+
+// ---- memory-limited contexts (jjs_init_limited) -------------------------------------------------------------------------------
+// A configuration is the width W of the G / G' tables and the capacity C, the items per pipeline pass.  From C follow the
+// scratch halves (C / 2 items), the sub-chunks of an overlapped batch (C / 2), the first host slice (at most 2^17), the table
+// scratch (TAB_ROWS x C elements: the equation kernels' three tables; aggregate and multisig passes are cut to the items whose
+// 4 x 68-element tables fit, tab_threads), the aggregate passes (C / 8 items per half) and their key scratch (4 keys per item),
+// and the staging of the host-buffer entry points (LIMITED_STAGE_PER_ITEM bytes per item of capacity: a window of C double
+// items with challenges, or a signing chunk of C items).  No persistent-equation scratch (eqtab).
+constexpr size_t LIMITED_MIN_ITEMS = size_t(1) << 12, LIMITED_STAGE_PER_ITEM = 320;
+void configure_limited(DeviceState& d, int w, size_t cap) {
+    d.fb_w = w;
+    d.chunk_items = cap;
+    d.sub_items = cap / 2;
+    d.sub_chunk = cap / 2;
+    d.first_slice = d.sub_chunk < d.first_slice ? d.sub_chunk : d.first_slice;
+    d.agg_items = tab_threads(d, d.sub_items, AGG_GROUP * R32_TAB_FQ);
+    d.agg_keys_initial = 4 * d.agg_items;
+}
+// what a limited context allocates on a device at init besides alloc_tables and the first SAFE tag table (ensure_tags)
+int alloc_limited_scratch(DevAlloc& A, DeviceState& d) {
+    int rc = alloc_pipeline(A, d, d.chunk_items, (size_t)TAB_ROWS * d.chunk_items);
+    for (int h = 0; h < 2 && !rc; h++) rc = alloc_agg_half(A, d, d.agg[h], d.agg_keys_initial);
+    if (!rc) rc = A(&d.stage, LIMITED_STAGE_PER_ITEM * d.chunk_items);
+    if (!rc) d.stage_bytes = LIMITED_STAGE_PER_ITEM * d.chunk_items;
+    return rc;
+}
+// bytes a limited context of width w and capacity cap holds on a device after init: a dry run of its allocations
+size_t footprint(int w, size_t cap) {
+    DeviceState d;
+    d.limit = 1;   // tab_threads of a limited context
+    configure_limited(d, w, cap);
+    DevAlloc A{nullptr, nullptr};
+    alloc_tables(A, d);
+    alloc_limited_scratch(A, d);
+    return A.total + sizeof(fq) * TAGS_INITIAL;
+}
+// The policy: the largest capacity in [2^12, 2^20] whose scratch fits in `limit` beside the 12-bit tables, then the device's
+// default width instead if its tables fit as well.  The fastest configuration inside the limit: the capacity decides whether one
+// pass fills the GPU, the width costs about 2 % (DESIGN.md section 11).  False if not even the smallest one fits.
+bool pick_config(size_t limit, int* w, size_t* cap) {
+    for (size_t c = CHUNK_ITEMS; c >= LIMITED_MIN_ITEMS; c /= 2) {
+        if (footprint(FB_W_SMALL, c) > limit) continue;
+        *cap = c;
+        *w = footprint(FB_W, c) <= limit ? FB_W : FB_W_SMALL;
+        return true;
+    }
+    return false;
+}
+
 int ensure_scratch(jjs_ctx* ctx, DeviceState& d) {
     if (d.pts_u) return JJS_SUCCESS;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
-    JJS_CUDA(ctx, cudaMalloc(&d.pts_u, sizeof(fq) * 4 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.pts_v, sizeof(fq) * 4 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.pflags, 4 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.iflags, CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.eqflags, 2 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.cwords, 32 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.rlist, sizeof(uint32_t) * 2 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.rcount, 8 * sizeof(uint32_t)));
-    JJS_CUDA(ctx, cudaMalloc(&d.eqlist, sizeof(uint32_t) * 2 * CHUNK_ITEMS));
-    JJS_CUDA(ctx, cudaMalloc(&d.tab, sizeof(fq) * AGG_GROUP * R32_TAB_FQ * TAB_THREADS));   // the key-aggregation kernel's four tables per thread
+    DevAlloc A = dev_alloc(ctx, d);
+    int rc = alloc_pipeline(A, d, CHUNK_ITEMS, (size_t)AGG_GROUP * R32_TAB_FQ * TAB_THREADS);   // the key-aggregation kernel's four tables per thread
+    if (rc) return rc;
     {
         cudaDeviceProp prop;
         JJS_CUDA(ctx, cudaGetDeviceProperties(&prop, d.device));
@@ -788,7 +954,8 @@ int ensure_scratch(jjs_ctx* ctx, DeviceState& d) {
         if (per_sm < 1) return fail(ctx, JJS_ERR_CUDA, "the equation kernel does not fit on an SM of device %d", d.device);
         d.eq_grid = per_sm * prop.multiProcessorCount;
         d.eqtab_half = per_thread * (size_t)d.eq_grid * block;
-        JJS_CUDA(ctx, cudaMalloc(&d.eqtab, sizeof(fq) * 2 * d.eqtab_half));
+        rc = A(&d.eqtab, sizeof(fq) * 2 * d.eqtab_half);
+        if (rc) return rc;
     }
     return JJS_SUCCESS;
 }
@@ -797,12 +964,15 @@ int ensure_scratch(jjs_ctx* ctx, DeviceState& d) {
 // flight at that point: the host entry points are synchronous)
 int ensure_stage(jjs_ctx* ctx, DeviceState& d, size_t bytes) {
     if (bytes <= d.stage_bytes) return JJS_SUCCESS;
+    int rc = check_growth(ctx, d, d.stage_bytes, bytes, "staging buffer");
+    if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     JJS_CUDA(ctx, cudaDeviceSynchronize());
-    cudaFree(d.stage);
-    d.stage = nullptr;
+    dev_free(d, d.stage, d.stage_bytes);
     d.stage_bytes = 0;
-    JJS_CUDA(ctx, cudaMalloc(&d.stage, bytes));
+    DevAlloc A = dev_alloc(ctx, d);
+    rc = A(&d.stage, bytes);
+    if (rc) return rc;
     d.stage_bytes = bytes;
     return JJS_SUCCESS;
 }
@@ -812,8 +982,10 @@ int ensure_stage(jjs_ctx* ctx, DeviceState& d, size_t bytes) {
 // waits for the device once.
 int ensure_tags(jjs_ctx* ctx, DeviceState& d, size_t n_absorb) {
     if (n_absorb < d.n_tags) return JJS_SUCCESS;
-    size_t want = d.n_tags ? d.n_tags : 1024;
+    size_t want = d.n_tags ? d.n_tags : TAGS_INITIAL;
     while (want <= n_absorb) want *= 2;
+    int rc = check_growth(ctx, d, sizeof(fq) * d.n_tags, sizeof(fq) * want, "SAFE tag table");
+    if (rc) return rc;
     {
         std::lock_guard<std::mutex> lock(ctx->mu);
         while (ctx->tags.size() < want) {
@@ -824,36 +996,33 @@ int ensure_tags(jjs_ctx* ctx, DeviceState& d, size_t n_absorb) {
     }
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     JJS_CUDA(ctx, cudaDeviceSynchronize());
-    cudaFree(d.safe_tags);
-    d.safe_tags = nullptr;
+    dev_free(d, d.safe_tags, sizeof(fq) * d.n_tags);
     d.n_tags = 0;
-    JJS_CUDA(ctx, cudaMalloc(&d.safe_tags, sizeof(fq) * want));
+    DevAlloc A = dev_alloc(ctx, d);
+    rc = A(&d.safe_tags, sizeof(fq) * want);
+    if (rc) return rc;
     JJS_CUDA(ctx, cudaMemcpy(d.safe_tags, ctx->tags.data(), sizeof(fq) * want, cudaMemcpyHostToDevice));
     d.n_tags = want;
     return JJS_SUCCESS;
 }
 
 // key scratch of the aggregate path, both halves; growing waits for the device
-constexpr size_t AGG_KEYS_INITIAL = size_t(1) << 21;
 int ensure_agg_scratch(jjs_ctx* ctx, DeviceState& d, size_t keys) {
     if (keys <= d.agg[0].cap_keys) return JJS_SUCCESS;
-    size_t want = d.agg[0].cap_keys ? d.agg[0].cap_keys : AGG_KEYS_INITIAL;
+    size_t want = d.agg[0].cap_keys ? d.agg[0].cap_keys : d.agg_keys_initial;
     while (want < keys) want *= 2;
+    int rc = check_growth(ctx, d, 2 * agg_key_bytes(d.agg[0].cap_keys), 2 * agg_key_bytes(want), "aggregate key scratch");
+    if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     JJS_CUDA(ctx, cudaDeviceSynchronize());
+    for (int h = 0; h < 2; h++) free_agg_keys(d, d.agg[h]);
+    DevAlloc A = dev_alloc(ctx, d);
     for (int h = 0; h < 2; h++) {
-        AggScratch& a = d.agg[h];
-        cudaFree(a.keys_u); cudaFree(a.keys_v); cudaFree(a.kflags); cudaFree(a.kcoef); cudaFree(a.kmap); cudaFree(a.kitem);
-        a.keys_u = a.keys_v = nullptr; a.kflags = nullptr; a.kcoef = a.kmap = a.kitem = nullptr; a.cap_keys = 0;
-        JJS_CUDA(ctx, cudaMalloc(&a.keys_u, sizeof(fq) * want));
-        JJS_CUDA(ctx, cudaMalloc(&a.keys_v, sizeof(fq) * want));
-        JJS_CUDA(ctx, cudaMalloc(&a.kflags, want));
-        JJS_CUDA(ctx, cudaMalloc(&a.kcoef, 32 * want));
-        JJS_CUDA(ctx, cudaMalloc(&a.kmap, sizeof(uint32_t) * want));
-        JJS_CUDA(ctx, cudaMalloc(&a.kitem, sizeof(uint32_t) * want));
-        if (!a.order) JJS_CUDA(ctx, cudaMalloc(&a.order, sizeof(uint32_t) * CHUNK_ITEMS));
-        if (!a.sort) JJS_CUDA(ctx, cudaMalloc(&a.sort, sizeof(AggSort)));
-        a.cap_keys = want;
+        rc = alloc_agg_half(A, d, d.agg[h], want);
+        if (rc) {
+            for (int k = 0; k <= h; k++) free_agg_keys(d, d.agg[k]);
+            return rc;
+        }
     }
     return JJS_SUCCESS;
 }
@@ -923,11 +1092,11 @@ int enqueue_equations(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant
         ctx->launches++;
     }
 #else
+    const auto keq = variant == VAR_VARGEN ? k_equation<1> : (d.fb_w == FB_W_SMALL ? k_equation<0, FB_W_SMALL> : k_equation<0>);
     for (size_t first = 0; first < neq * m; first += R.cap) {
         size_t cnt = neq * m - first < R.cap ? neq * m - first : R.cap;
-        (variant == VAR_VARGEN ? k_equation<1> : k_equation<0>)<<<blocks_for(cnt), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, first, cnt, R.eqlist,
-                                                                                                       R.rcount + 2, fu, R.cwords, R.eqflags, R.tab, TAB_THREADS, T, R.rlist,
-                                                                                                       R.rcount);
+        keq<<<blocks_for(cnt), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, first, cnt, R.eqlist, R.rcount + 2, fu, R.cwords, R.eqflags, R.tab,
+                                                   R.tstride, T, R.rlist, R.rcount);
         ctx->launches++;
     }
 #endif
@@ -983,7 +1152,7 @@ int run_chunk_ext(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, co
     return JJS_SUCCESS;
 }
 
-// aggregate_pk(..).verify(..) for one chunk of m <= R.cap items with K <= cap_keys signer keys; everything on `stream`,
+// aggregate_pk(..).verify(..) for one chunk of m <= R.acap items with K <= cap_keys signer keys; everything on `stream`,
 // nothing on the host.  d_keys: the chunk's first key; d_offsets: the chunk's m + 1 offsets (absolute, first = key_lo).
 int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uint8_t* d_keys, const uint32_t* d_offsets, uint32_t key_lo, size_t K,
                         const uint8_t* d_sig, const uint8_t* d_msg, size_t m, uint8_t* d_status, uint8_t* d_c, uint8_t* d_agg, cudaStream_t stream) {
@@ -1005,7 +1174,7 @@ int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uin
     k_agg_scatter<<<blocks_for(m), BLOCK, 0, stream>>>(d_offsets, key_lo, m, A.sort, A.order, A.kmap, A.kitem);
     if (K) k_agg_coeffs<<<blocks_for(K), BLOCK, 0, stream>>>(A.keys_u, A.keys_v, A.kflags, d_offsets, A.kmap, A.kitem, key_lo, K, A.kcoef, T);
     k_aggregate<<<blocks_for(m), BLOCK, 0, stream>>>(A.keys_u, A.keys_v, A.kflags, d_offsets, A.order, key_lo, m, R.pts_u, R.pts_v, R.pflags, d_agg, R.tab,
-                                                    TAB_THREADS, A.kcoef, T);
+                                                    R.astride, A.kcoef, T);
     t2.stop(stream);
     ctx->launches += 7;
     int rc = enqueue_challenges(ctx, d, R, VAR_SINGLE, m, fmsg, fu, stream, true);
@@ -1040,7 +1209,7 @@ int run_chunk_keyed(jjs_ctx* ctx, DeviceState& d, const Region& R, const KeySet&
     if (rc) return rc;
     StageTimer t3(ctx, d.device, 3, stream);
     JJS_CUDA(ctx, cudaMemsetAsync(R.rcount, 0, sizeof(uint32_t), stream));
-    k_equation_keyed<<<blocks_for(nk * m), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, R.eqlist, R.rcount + 2, fu, R.cwords, R.eqflags,
+    (d.fb_w == FB_W_SMALL ? k_equation_keyed<FB_W_SMALL> : k_equation_keyed<>)<<<blocks_for(nk * m), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, R.eqlist, R.rcount + 2, fu, R.cwords, R.eqflags,
                                                               kd.table, key_index, ks.n_keys, T, R.rlist, R.rcount);
     t3.stop(stream);
     StageTimer t5(ctx, d.device, 5, stream);
@@ -1090,10 +1259,10 @@ int run_device(jjs_ctx* ctx, DeviceState& d, int variant, const uint8_t* pk, con
     int rc = ensure_scratch(ctx, d);
     if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > SUB_CHUNK);
+    Overlap ov(ctx, d, stream, n > d.sub_chunk);
     rc = ov.begin();
     if (rc) return rc;
-    const size_t step = ov.on ? SUB_CHUNK : CHUNK_ITEMS;
+    const size_t step = ov.on ? d.sub_chunk : d.chunk_items;
     for (size_t off = 0; off < n; off += step, ov.advance()) {
         size_t m = n - off < step ? n - off : step;
         rc = run_chunk(ctx, d, ov.next_region(), variant, pk + off * pk_size(variant), sig + off * sig_size(variant), msg + off * 32, m,
@@ -1112,10 +1281,10 @@ int run_keyed_device(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, const KeySe
     int rc = ensure_scratch(ctx, d);
     if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > SUB_CHUNK);
+    Overlap ov(ctx, d, stream, n > d.sub_chunk);
     rc = ov.begin();
     if (rc) return rc;
-    const size_t step = ov.on ? SUB_CHUNK : CHUNK_ITEMS;
+    const size_t step = ov.on ? d.sub_chunk : d.chunk_items;
     for (size_t off = 0; off < n; off += step, ov.advance()) {
         size_t m = n - off < step ? n - off : step;
         rc = run_chunk_keyed(ctx, d, ov.next_region(), ks, kd, key_index + off, sig + off * sig_size(ks.variant), msg + off * 32, m, status + off,
@@ -1153,19 +1322,19 @@ int run_aggregate_device(jjs_ctx* ctx, DeviceState& d, const uint8_t* d_pks, con
     int rc = ensure_scratch(ctx, d);
     const size_t max_cnt = agg_max_item_keys(h_offsets, n);
     if (!rc) rc = ensure_tags(ctx, d, 2 + 2 * max_cnt);
-    if (!rc) rc = ensure_agg_scratch(ctx, d, max_cnt > AGG_KEYS_INITIAL ? max_cnt : AGG_KEYS_INITIAL);
+    if (!rc) rc = ensure_agg_scratch(ctx, d, max_cnt > d.agg_keys_initial ? max_cnt : d.agg_keys_initial);
     if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > SUB_CHUNK);
+    Overlap ov(ctx, d, stream, n > d.sub_chunk);
     rc = ov.begin();
     if (rc) return rc;
-    const size_t step = ov.on ? SUB_CHUNK : SUB_ITEMS;
+    const size_t step = ov.on ? d.sub_chunk : d.sub_items;
     for (size_t off = 0; off < n; ov.advance()) {
-        size_t end = agg_chunk_end(h_offsets, off, n, step, d.agg[0].cap_keys);
+        Region R = ov.on ? ov.next_region() : region_half(d, 0);
+        size_t end = agg_chunk_end(h_offsets, off, n, step < R.acap ? step : R.acap, d.agg[0].cap_keys);
         size_t m = end - off;
         uint32_t key_lo = h_offsets[off];
         size_t K = h_offsets[end] - key_lo;
-        Region R = ov.on ? ov.next_region() : region_half(d, 0);
         rc = run_chunk_aggregate(ctx, d, R, d_pks + 32 * (size_t)key_lo, d_offsets + off, key_lo, K, d_sig + 64 * off, d_msg + 32 * off, m, d_status + off,
                                  d_c ? d_c + 32 * off : nullptr, d_agg ? d_agg + 32 * off : nullptr, ov.next_stream());
         if (rc) return rc;
@@ -1289,7 +1458,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
             o_off[p] = total; total += align_up(4 * (m + 1), 256);
             size_t mc = agg_max_item_keys(P.offsets + lo, m);
             if (mc > max_cnt) max_cnt = mc;
-            rc = ensure_agg_scratch(ctx, d, mc > AGG_KEYS_INITIAL ? mc : AGG_KEYS_INITIAL);
+            rc = ensure_agg_scratch(ctx, d, mc > d.agg_keys_initial ? mc : d.agg_keys_initial);
             if (rc) return rc;
         }
     }
@@ -1319,13 +1488,13 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         // Pipeline slices: slice j + 1 is copied in on the copy stream while slice j is being verified (the kernels of one
         // slice run far longer than its copy); the first slice of a device is short so that compute starts early.
         for (size_t off = 0; off < m; j++) {
-            const size_t want = j == 0 ? (size_t(1) << JJS_FIRST_SLICE_LOG2) : SUB_CHUNK;
+            const size_t want = j == 0 ? d.first_slice : d.sub_chunk;
             size_t cnt = m - off < want ? m - off : want;
             cudaStream_t cs = serial ? d.stream : d.sub[j & 1];
             Region R = region_half(d, j);
             if (P.mode == PART_AGGREGATE) {
                 const uint32_t* ho = P.offsets + lo;   // host offsets of this shard
-                size_t end = agg_chunk_end(ho, off, m, want, d.agg[0].cap_keys);
+                size_t end = agg_chunk_end(ho, off, m, want < R.acap ? want : R.acap, d.agg[0].cap_keys);
                 cnt = end - off;
                 const uint32_t key0 = ho[0], key_lo = ho[off];
                 const size_t K = ho[end] - key_lo;
@@ -1380,10 +1549,49 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
     return JJS_SUCCESS;
 }
 
+// Device staging that device_job lays out for items [lo, hi) of part P.
+inline size_t part_stage_bytes(const HostPart& P, size_t lo, size_t hi) {
+    const size_t m = hi - lo;
+    size_t pkb, sgb;
+    part_in_bytes(P, lo, hi, &pkb, &sgb);
+    size_t b = align_up(pkb, 256) + align_up(sgb, 256) + 2 * align_up(32 * m, 256) + align_up(m, 256) + align_up(4 * ((m + 31) / 32), 256);
+    if (P.mode == PART_AGGREGATE) b += align_up(32 * m, 256) + align_up(4 * (m + 1), 256);
+    return b;
+}
+// The largest window [lo, end) of part P whose staging fits `budget` bytes, ending on a bitmap word (or at hi); at least one word.
+size_t window_end(const HostPart& P, size_t lo, size_t hi, size_t budget) {
+    size_t good = 1, bad = (hi - lo + 31) / 32 + 1;   // in bitmap words
+    while (bad - good > 1) {
+        const size_t mid = (good + bad) / 2, end = lo + 32 * mid < hi ? lo + 32 * mid : hi;
+        if (part_stage_bytes(P, lo, end) <= budget) good = mid;
+        else bad = mid;
+    }
+    return lo + 32 * good < hi ? lo + 32 * good : hi;
+}
+// A memory-limited context cannot stage a whole shard: it runs device_job window by window, each window as large as the staging
+// buffer it reserved at init allows (or grows within its limit for a window of one bitmap word), so batches of any size stream
+// through it.  Each window is verified and copied back before the next is staged.
+int device_job_windows(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const std::vector<std::vector<Shard>>& shards) {
+    DeviceState& d = ctx->dev[k];
+    std::vector<std::vector<Shard>> win(parts.size(), std::vector<Shard>(ctx->dev.size(), Shard{0, 0}));
+    for (size_t p = 0; p < parts.size(); p++) {
+        const size_t hi = shards[p][k].hi;
+        for (size_t off = shards[p][k].lo; off < hi;) {
+            const size_t end = window_end(parts[p], off, hi, d.stage_bytes);
+            win[p][k] = Shard{off, end};
+            int rc = device_job(ctx, k, parts, win);
+            if (rc) return rc;
+            off = end;
+        }
+        win[p][k] = Shard{0, 0};
+    }
+    return JJS_SUCCESS;
+}
+
 // device_job, and on failure a drain of the device: nothing may still be reading or writing the caller's buffers when the
 // call returns
 int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const std::vector<std::vector<Shard>>& shards) {
-    int rc = device_job(ctx, k, parts, shards);
+    int rc = ctx->dev[k].limit ? device_job_windows(ctx, k, parts, shards) : device_job(ctx, k, parts, shards);
     if (rc) {
         cudaSetDevice(ctx->dev[k].device);
         cudaDeviceSynchronize();
@@ -1449,7 +1657,8 @@ HostPart aggregate_part(const uint8_t* pks, const uint32_t* offsets, const uint8
     return HostPart{PART_AGGREGATE, VAR_SINGLE, pks, sig, msg, offsets, n, status, c_out, agg_out, bitmap, false};
 }
 
-// multisig::combine for n ragged sessions (host buffers, device 0); chunks hold at most 2^20 participants
+// multisig::combine for n ragged sessions (host buffers, device 0); a chunk holds as many sessions as the table scratch serves
+// threads of k_msig_session and as many participants as it serves threads of k_msig_share (2^20 each on a jjs_init context)
 int run_msig(jjs_ctx* ctx, const uint8_t* pks, const uint8_t* Rs, const uint8_t* Ss, const uint8_t* zs, const uint32_t* offsets, const uint8_t* msg,
              size_t n, uint8_t* share_ok, uint8_t* status, uint32_t* bad, uint8_t* sig) {
     JJS_ENTER(ctx);
@@ -1465,11 +1674,13 @@ int run_msig(jjs_ctx* ctx, const uint8_t* pks, const uint8_t* Rs, const uint8_t*
     if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     Tables T = d.tables();
+    const size_t sess_stride = tab_threads(d, d.chunk_items, AGG_GROUP * R32_TAB_FQ), share_stride = tab_threads(d, d.chunk_items, 2 * 36);
+    const size_t max_sessions = sess_stride < d.chunk_items ? sess_stride : d.chunk_items;
     std::vector<uint32_t> rel, owner, order;
     for (size_t s0 = 0; s0 < n;) {
         size_t s1 = s0;
-        while (s1 < n && s1 - s0 < CHUNK_ITEMS && offsets[s1 + 1] - offsets[s0] <= TAB_THREADS) s1++;
-        if (s1 == s0) return fail(ctx, JJS_ERR_ARGUMENT, "a session has more than 2^20 participants");
+        while (s1 < n && s1 - s0 < max_sessions && offsets[s1 + 1] - offsets[s0] <= share_stride) s1++;
+        if (s1 == s0) return fail(ctx, JJS_ERR_ARGUMENT, "a session has more than %zu participants", share_stride);
         const size_t m = s1 - s0, K = offsets[s1] - offsets[s0], k0 = offsets[s0];
         rel.resize(m + 1);
         owner.resize(K ? K : 1);
@@ -1510,8 +1721,8 @@ int run_msig(jjs_ctx* ctx, const uint8_t* pks, const uint8_t* Rs, const uint8_t*
         f.f[0] = WireField{B + o_pk, 32}; f.f[1] = WireField{B + o_R, 32}; f.f[2] = WireField{B + o_S, 32}; f.f[3] = WireField{nullptr, 0};
         WireField fmsg{B + o_msg, 32}, fz{B + o_z, 32};
         if (K) k_decode<<<blocks_for(3 * K), BLOCK, 0, st>>>(f, 3, 0, K, b.pu, b.pv, b.pf, T, 0u);
-        k_msig_session<<<blocks_for(m), BLOCK, 0, st>>>(b, K, m, fmsg, fz, d.tab, TAB_THREADS, T);
-        if (K) k_msig_share<<<blocks_for(K), BLOCK, 0, st>>>(b, K, fz, d.tab, TAB_THREADS, T);
+        k_msig_session<<<blocks_for(m), BLOCK, 0, st>>>(b, K, m, fmsg, fz, d.tab, sess_stride, T);
+        if (K) (d.fb_w == FB_W_SMALL ? k_msig_share<FB_W_SMALL> : k_msig_share<>)<<<blocks_for(K), BLOCK, 0, st>>>(b, K, fz, d.tab, share_stride, T);
         k_msig_finalize<<<blocks_for(m), BLOCK, 0, st>>>(b, m, fz, B + o_st, reinterpret_cast<uint32_t*>(B + o_bad), B + o_sig);
         ctx->launches += 4;
         auto down = [&](void* dst, size_t at, size_t bytes) { if (ce == cudaSuccess && bytes) ce = cudaMemcpyAsync(dst, B + at, bytes, cudaMemcpyDeviceToHost, st); };
@@ -1536,7 +1747,7 @@ int run_sign(jjs_ctx* ctx, int variant, const uint8_t* sk, const uint8_t* rnd, c
     DeviceState& d = ctx->dev[0];
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     const size_t pks = pk_size(variant), sgs = sig_size(variant);
-    const size_t chunk = n < CHUNK_ITEMS ? n : CHUNK_ITEMS;
+    const size_t chunk = n < d.chunk_items ? n : d.chunk_items;
     int rc = ensure_stage(ctx, d, chunk * (4 * 32 + pks + sgs));
     if (rc) return rc;
     uint8_t* buf = d.stage;
@@ -1549,9 +1760,11 @@ int run_sign(jjs_ctx* ctx, int variant, const uint8_t* sk, const uint8_t* rnd, c
         if (ce == cudaSuccess && variant == VAR_VARGEN) ce = cudaMemcpyAsync(d_g, gsc + 32 * off, 32 * m, cudaMemcpyHostToDevice, d.stream);
         if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_msg, msg + 32 * off, 32 * m, cudaMemcpyHostToDevice, d.stream);
         if (ce == cudaSuccess) {
-            if (variant == VAR_SINGLE) k_sign<VAR_SINGLE><<<blocks_for(m), BLOCK, 0, d.stream>>>(d_sk, d_rnd, d_g, d_msg, m, d_pk, d_sig, d.tables());
-            else if (variant == VAR_DOUBLE) k_sign<VAR_DOUBLE><<<blocks_for(m), BLOCK, 0, d.stream>>>(d_sk, d_rnd, d_g, d_msg, m, d_pk, d_sig, d.tables());
-            else k_sign<VAR_VARGEN><<<blocks_for(m), BLOCK, 0, d.stream>>>(d_sk, d_rnd, d_g, d_msg, m, d_pk, d_sig, d.tables());
+            const bool small = d.fb_w == FB_W_SMALL;
+            const auto ks = variant == VAR_SINGLE ? (small ? k_sign<VAR_SINGLE, FB_W_SMALL> : k_sign<VAR_SINGLE>)
+                            : variant == VAR_DOUBLE ? (small ? k_sign<VAR_DOUBLE, FB_W_SMALL> : k_sign<VAR_DOUBLE>)
+                                                    : (small ? k_sign<VAR_VARGEN, FB_W_SMALL> : k_sign<VAR_VARGEN>);
+            ks<<<blocks_for(m), BLOCK, 0, d.stream>>>(d_sk, d_rnd, d_g, d_msg, m, d_pk, d_sig, d.tables());
             ctx->launches++;
             ce = cudaMemcpyAsync(pk_out + pks * off, d_pk, pks * m, cudaMemcpyDeviceToHost, d.stream);
         }
@@ -1563,6 +1776,33 @@ int run_sign(jjs_ctx* ctx, int variant, const uint8_t* sk, const uint8_t* rnd, c
     return JJS_SUCCESS;
 }
 
+// G / G' tables of width W in two passes (k_fb_small, k_fb_combine)
+template <int W>
+int build_fb_tables(jjs_ctx* ctx, DeviceState& d) {
+    constexpr int LO = (W + 1) / 2, HI = W - LO, WINDOWS = (252 + W - 1) / W, SMALL = (1 << LO) + (1 << HI);
+    const size_t small_bytes = sizeof(fq) * WINDOWS * SMALL;
+    fq *small_u = nullptr, *small_v = nullptr;
+    DevAlloc A = dev_alloc(ctx, d);
+    int rc = A(&small_u, small_bytes);
+    if (!rc) rc = A(&small_v, small_bytes);
+    if (!rc) {
+        for (int which = 0; which < 2; which++) {
+            k_fb_small<W><<<blocks_for(WINDOWS * SMALL), BLOCK, 0, d.stream>>>(small_u, small_v, which);
+            k_fb_combine<W><<<blocks_for((size_t)WINDOWS * ((size_t)1 << W) / FB_BATCH), BLOCK, 0, d.stream>>>(which ? d.fb_gn : d.fb_g, small_u, small_v);
+        }
+        ctx->launches += 4;
+    }
+    cudaError_t e1 = cudaGetLastError(), e2 = cudaStreamSynchronize(d.stream);
+    dev_free(d, small_u, small_bytes);
+    dev_free(d, small_v, small_bytes);
+    if (rc) return rc;
+    JJS_CUDA(ctx, e1);
+    JJS_CUDA(ctx, e2);
+    return JJS_SUCCESS;
+}
+
+// Constant tables, fixed-base tables and SAFE tags of one device; a memory-limited context (d.limit set, configure_limited
+// applied) also allocates all its scratch here.
 int init_device(jjs_ctx* ctx, DeviceState& d) {
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     cudaDeviceProp prop;
@@ -1576,34 +1816,15 @@ int init_device(jjs_ctx* ctx, DeviceState& d) {
         JJS_CUDA(ctx, cudaStreamCreateWithFlags(&d.sub[k], cudaStreamNonBlocking));
         JJS_CUDA(ctx, cudaEventCreateWithFlags(&d.join[k], cudaEventDisableTiming));
     }
-    JJS_CUDA(ctx, cudaMalloc(&d.root_tables, sizeof(tables::ROOT_TABLES)));
+    DevAlloc A = dev_alloc(ctx, d);
+    int rc = alloc_tables(A, d);
+    if (rc) return rc;
     JJS_CUDA(ctx, cudaMemcpy(d.root_tables, tables::ROOT_TABLES, sizeof(tables::ROOT_TABLES), cudaMemcpyHostToDevice));
-    JJS_CUDA(ctx, cudaMalloc(&d.dlog_hash, sizeof(tables::DLOG_HASH)));
     JJS_CUDA(ctx, cudaMemcpy(d.dlog_hash, tables::DLOG_HASH, sizeof(tables::DLOG_HASH), cudaMemcpyHostToDevice));
-    const size_t fb_bytes = sizeof(niels) * FB_WINDOWS * FB_ENTRIES;
-    JJS_CUDA(ctx, cudaMalloc(&d.fb_g, fb_bytes));
-    JJS_CUDA(ctx, cudaMalloc(&d.fb_gn, fb_bytes));
-    {
-        static_assert((1 << FB_LO) % FB_BATCH == 0, "a batch of table entries must share its high half");
-        fq *small_u = nullptr, *small_v = nullptr;
-        JJS_CUDA(ctx, cudaMalloc(&small_u, sizeof(fq) * FB_WINDOWS * FB_SMALL));
-        {
-            cudaError_t em = cudaMalloc(&small_v, sizeof(fq) * FB_WINDOWS * FB_SMALL);
-            if (em != cudaSuccess) cudaFree(small_u);
-            JJS_CUDA(ctx, em);
-        }
-        for (int which = 0; which < 2; which++) {
-            k_fb_small<<<blocks_for(FB_WINDOWS * FB_SMALL), BLOCK, 0, d.stream>>>(small_u, small_v, which);
-            k_fb_combine<<<blocks_for((size_t)FB_WINDOWS * FB_ENTRIES / FB_BATCH), BLOCK, 0, d.stream>>>(which ? d.fb_gn : d.fb_g, small_u, small_v);
-        }
-        ctx->launches += 4;
-        cudaError_t e1 = cudaGetLastError(), e2 = cudaStreamSynchronize(d.stream);
-        cudaFree(small_u);
-        cudaFree(small_v);
-        JJS_CUDA(ctx, e1);
-        JJS_CUDA(ctx, e2);
-    }
-    return ensure_tags(ctx, d, 1023);
+    rc = d.fb_w == FB_W_SMALL ? build_fb_tables<FB_W_SMALL>(ctx, d) : build_fb_tables<FB_W>(ctx, d);
+    if (!rc) rc = ensure_tags(ctx, d, TAGS_INITIAL - 1);
+    if (!rc && d.limit) rc = alloc_limited_scratch(A, d);
+    return rc;
 }
 
 void free_device(DeviceState& d) {
@@ -1664,20 +1885,15 @@ int run_small(jjs_ctx* ctx, const char* what, size_t in_bytes, size_t out_bytes,
 }
 
 // ---- registered key sets ----------------------------------------------------------------------------------------
-// cudaMalloc for key-set storage.  A failed allocation also clears the error it leaves behind for cudaGetLastError, which
-// later calls on this context would otherwise report as their own.
-int keyset_malloc(jjs_ctx* ctx, void** p, size_t bytes) {
-    cudaError_t e = cudaMalloc(p, bytes);
-    if (e == cudaSuccess) return JJS_SUCCESS;
-    *p = nullptr;
-    cudaGetLastError();
-    return fail(ctx, e == cudaErrorMemoryAllocation ? JJS_ERR_NOMEM : JJS_ERR_CUDA, "key set: cudaMalloc of %zu bytes failed: %s", bytes,
-                cudaGetErrorString(e));
-}
+// Device memory of a key set of npts key points: decoded points and flags, and the tables.
+inline size_t keyset_point_bytes(size_t npts) { return npts * (2 * sizeof(fq) + 1); }
+inline size_t keyset_table_bytes(size_t npts) { return sizeof(niels) * npts * KEYED_POINT_ENTRIES; }
 
 struct DeviceTemp {   // scratch of one key-set build, freed on every path out
-    void* p = nullptr;
-    ~DeviceTemp() { cudaFree(p); }
+    DeviceState& d;
+    size_t bytes;
+    uint8_t* p = nullptr;
+    ~DeviceTemp() { dev_free(d, p, bytes); }
 };
 
 // Key set `ks` on device d: copy the wire keys in, decode them with the subgroup test, build the tables (keyset.cuh).
@@ -1686,27 +1902,33 @@ int keyset_build(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, KeySetDev& kd, 
     JJS_CUDA(ctx, cudaSetDevice(d.device));
     const int nk = keyed_points(ks.variant);
     const size_t npts = (size_t)nk * ks.n_keys;
-    DeviceTemp wire, bases;
-    int rc = keyset_malloc(ctx, (void**)&kd.u, sizeof(fq) * npts);
-    if (!rc) rc = keyset_malloc(ctx, (void**)&kd.v, sizeof(fq) * npts);
-    if (!rc) rc = keyset_malloc(ctx, (void**)&kd.flags, npts);
-    if (!rc) rc = keyset_malloc(ctx, (void**)&kd.table, sizeof(niels) * npts * KEYED_POINT_ENTRIES);
-    if (!rc) rc = keyset_malloc(ctx, &wire.p, 32 * npts);
-    if (!rc) rc = keyset_malloc(ctx, &bases.p, sizeof(ext) * npts * KEYED_WINDOWS);
+    DeviceTemp wire{d, 32 * npts}, bases{d, sizeof(ext) * npts * KEYED_WINDOWS};
+    // a limited context refuses a key set that would cross its limit before allocating any of it
+    const size_t need = keyset_point_bytes(npts) + keyset_table_bytes(npts) + wire.bytes + bases.bytes;
+    if (d.limit && d.held + need > d.limit)
+        return fail(ctx, JJS_ERR_NOMEM, "key set: %zu bytes on device %d would exceed the context's memory limit of %zu bytes (%zu held)", need, d.device,
+                    d.limit, d.held);
+    DevAlloc A = dev_alloc(ctx, d);
+    int rc = A(&kd.u, sizeof(fq) * npts);
+    if (!rc) rc = A(&kd.v, sizeof(fq) * npts);
+    if (!rc) rc = A(&kd.flags, npts);
+    if (!rc) rc = A(&kd.table, keyset_table_bytes(npts));
+    if (!rc) rc = A(&wire.p, wire.bytes);
+    if (!rc) rc = A(&bases.p, bases.bytes);
     if (rc) return rc;
     cudaStream_t st = d.stream;
     // undecodable keys leave their coordinates unwritten; zero them so that gathering them copies defined values
     JJS_CUDA(ctx, cudaMemsetAsync(kd.u, 0, sizeof(fq) * npts, st));
     JJS_CUDA(ctx, cudaMemsetAsync(kd.v, 0, sizeof(fq) * npts, st));
     JJS_CUDA(ctx, cudaMemcpyAsync(wire.p, pk, 32 * npts, cudaMemcpyHostToDevice, st));
-    const uint8_t* w = static_cast<const uint8_t*>(wire.p);
+    const uint8_t* w = wire.p;
     Fields f;
     f.f[0] = WireField{w, (uint32_t)(32 * nk)};
     f.f[1] = nk == 2 ? WireField{w + 32, 64} : WireField{nullptr, 0};
     f.f[2] = f.f[3] = WireField{nullptr, 0};
     k_decode<<<blocks_for(npts), BLOCK, 0, st>>>(f, nk, 0, ks.n_keys, kd.u, kd.v, kd.flags, d.tables(), 3u);
-    k_keyset_bases<<<blocks_for(npts), BLOCK, 0, st>>>(ks.variant, kd.u, kd.v, kd.flags, ks.n_keys, static_cast<ext*>(bases.p));
-    k_keyset_combine<<<blocks_for(npts * KEYED_WINDOWS * KEYED_GROUPS), BLOCK, 0, st>>>(static_cast<const ext*>(bases.p), npts, kd.table);
+    k_keyset_bases<<<blocks_for(npts), BLOCK, 0, st>>>(ks.variant, kd.u, kd.v, kd.flags, ks.n_keys, reinterpret_cast<ext*>(bases.p));
+    k_keyset_combine<<<blocks_for(npts * KEYED_WINDOWS * KEYED_GROUPS), BLOCK, 0, st>>>(reinterpret_cast<const ext*>(bases.p), npts, kd.table);
     ctx->launches += 3;
     JJS_CUDA(ctx, cudaGetLastError());
     std::vector<uint8_t> flags;
@@ -1720,12 +1942,15 @@ int keyset_build(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, KeySetDev& kd, 
 }
 
 void keyset_free(jjs_ctx* ctx, KeySet* ks) {
+    const size_t npts = (size_t)keyed_points(ks->variant) * ks->n_keys;
     for (size_t k = 0; k < ks->dev.size(); k++) {
         KeySetDev& kd = ks->dev[k];
         if (!kd.u && !kd.v && !kd.flags && !kd.table) continue;
-        cudaSetDevice(ctx->dev[k].device);
+        DeviceState& d = ctx->dev[k];
+        cudaSetDevice(d.device);
         cudaDeviceSynchronize();   // work enqueued by the device entry point may still read the tables
-        cudaFree(kd.u); cudaFree(kd.v); cudaFree(kd.flags); cudaFree(kd.table);
+        dev_free(d, kd.u, sizeof(fq) * npts); dev_free(d, kd.v, sizeof(fq) * npts); dev_free(d, kd.flags, npts);
+        dev_free(d, kd.table, keyset_table_bytes(npts));
     }
     delete ks;
 }
@@ -1741,7 +1966,11 @@ extern "C" {
 
 #define JJS_API __attribute__((visibility("default")))
 
-JJS_API int jjs_init(const int* devices, int n_devices, jjs_ctx** out) {
+}  // extern "C"
+
+namespace {
+// jjs_init and jjs_init_limited; limit 0: no limit
+int init_context(const int* devices, int n_devices, size_t limit, jjs_ctx** out) {
     if (!out || n_devices < 1 || n_devices > 64) return JJS_ERR_ARGUMENT;
     *out = nullptr;
     jjs_ctx* ctx = new (std::nothrow) jjs_ctx();
@@ -1752,17 +1981,62 @@ JJS_API int jjs_init(const int* devices, int n_devices, jjs_ctx** out) {
     cudaError_t e = cudaGetDeviceCount(&count);
     if (e != cudaSuccess || count < 1)
         return fail(ctx, JJS_ERR_CUDA, "no CUDA device available: %s", e != cudaSuccess ? cudaGetErrorString(e) : "device count is 0");
+    int w = FB_W;
+    size_t cap = CHUNK_ITEMS;
+    if (limit) {
+#if JJS_EQ_V2 || JJS_EQ_PERSISTENT
+        return fail(ctx, JJS_ERR_ARGUMENT, "memory-limited contexts are not available in a build with the persistent equation kernel");
+#endif
+        if (!pick_config(limit, &w, &cap))
+            return fail(ctx, JJS_ERR_NOMEM, "a device memory limit of %zu bytes is below the smallest configuration, %zu bytes (%d-bit tables, %zu items per pass)",
+                        limit, footprint(FB_W_SMALL, LIMITED_MIN_ITEMS), FB_W_SMALL, LIMITED_MIN_ITEMS);
+    }
     ctx->dev.resize(n_devices);
     for (int i = 0; i < n_devices; i++) {
         int ord = devices ? devices[i] : i;
         if (ord < 0 || ord >= count) return fail(ctx, JJS_ERR_ARGUMENT, "device ordinal %d not present (%d devices)", ord, count);
         for (int k = 0; k < i; k++)
             if (ctx->dev[k].device == ord) return fail(ctx, JJS_ERR_ARGUMENT, "device ordinal %d listed twice", ord);
-        ctx->dev[i].device = ord;
-        int rc = init_device(ctx, ctx->dev[i]);
-        if (rc) return rc;
+        DeviceState& d = ctx->dev[i];
+        d.device = ord;
+        if (limit) {
+            d.limit = limit;
+            configure_limited(d, w, cap);
+        }
+        int rc = init_device(ctx, d);
+        if (rc) {
+            if (limit) {   // nothing is left allocated
+                for (auto& dv : ctx->dev) free_device(dv);
+                ctx->dev.clear();
+            }
+            return rc;
+        }
     }
     ctx->ready = true;
+    return JJS_SUCCESS;
+}
+}  // namespace
+
+extern "C" {
+
+JJS_API int jjs_init(const int* devices, int n_devices, jjs_ctx** out) { return init_context(devices, n_devices, 0, out); }
+
+JJS_API int jjs_init_limited(const int* devices, int n_devices, size_t device_memory_limit, jjs_ctx** out) {
+    if (device_memory_limit == 0) {
+        if (out) *out = nullptr;
+        return JJS_ERR_ARGUMENT;
+    }
+    return init_context(devices, n_devices, device_memory_limit, out);
+}
+
+JJS_API int jjs_memory_info(const jjs_ctx* ctx, int device_index, uint64_t* bytes_held, int* fb_window_bits, uint64_t* items_in_flight) {
+    if (!ctx) return JJS_ERR_ARGUMENT;
+    if (!ctx->ready || ctx->dev.empty()) return JJS_ERR_CUDA;
+    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(const_cast<jjs_ctx*>(ctx), JJS_ERR_ARGUMENT, "device_index out of range");
+    const DeviceState& d = ctx->dev[device_index];
+    if (bytes_held) *bytes_held = d.held;
+    if (fb_window_bits) *fb_window_bits = d.fb_w;
+    if (items_in_flight) *items_in_flight = d.chunk_items;
     return JJS_SUCCESS;
 }
 
@@ -1879,9 +2153,10 @@ JJS_API int jjs_subgroup_check(jjs_ctx* ctx, const uint8_t* points32, size_t n, 
     const void* srcs[1] = {points32};
     const size_t bytes[1] = {32 * n};
     return run_small(ctx, "subgroup check", 32 * n, n, srcs, bytes, 1, out, [&](DeviceState& d, uint8_t* in, uint8_t* o) {
-        for (size_t first = 0; first < n; first += TAB_THREADS) {
-            size_t cnt = n - first < TAB_THREADS ? n - first : TAB_THREADS;
-            k_subgroup_check<<<blocks_for(cnt), BLOCK, 0, d.stream>>>(WireField{in, 32}, first, cnt, method, o, d.tab, TAB_THREADS, d.tables());
+        const size_t stride = tab_threads(d, d.chunk_items, 36);
+        for (size_t first = 0; first < n; first += stride) {
+            size_t cnt = n - first < stride ? n - first : stride;
+            k_subgroup_check<<<blocks_for(cnt), BLOCK, 0, d.stream>>>(WireField{in, 32}, first, cnt, method, o, d.tab, stride, d.tables());
             ctx->launches++;
         }
     });
@@ -1898,7 +2173,7 @@ JJS_API int jjs_fb_table_check(jjs_ctx* ctx, int which, const uint32_t* entries,
     uint32_t count = 0;
     int rc = run_small(ctx, "fixed-base table check", 4 * n, 4, srcs, bytes, 1, &count, [&](DeviceState& d, uint8_t* in, uint8_t* o) {
         cudaMemsetAsync(o, 0, 4, d.stream);
-        k_fb_check<<<blocks_for(n), BLOCK, 0, d.stream>>>(which ? d.fb_gn : d.fb_g, which, reinterpret_cast<const uint32_t*>(in), (int)n,
+        (d.fb_w == FB_W_SMALL ? k_fb_check<FB_W_SMALL> : k_fb_check<FB_W>)<<<blocks_for(n), BLOCK, 0, d.stream>>>(which ? d.fb_gn : d.fb_g, which, reinterpret_cast<const uint32_t*>(in), (int)n,
                                                          reinterpret_cast<uint32_t*>(o));
         ctx->launches++;
     });
@@ -1932,7 +2207,7 @@ JJS_API int jjs_sign_aggregate_batch(jjs_ctx* ctx, const uint8_t* sk32, const ui
     }
     uint8_t *b = d.stage, *o_pks = d.stage + align_up(in_bytes, 256), *o_sig = o_pks + 32 * K;
     if (ce == cudaSuccess) {
-        k_sign_aggregate<<<blocks_for(n), BLOCK, 0, d.stream>>>(b, reinterpret_cast<uint32_t*>(b + bytes[0]), b + bytes[0] + bytes[1],
+        (d.fb_w == FB_W_SMALL ? k_sign_aggregate<FB_W_SMALL> : k_sign_aggregate<>)<<<blocks_for(n), BLOCK, 0, d.stream>>>(b, reinterpret_cast<uint32_t*>(b + bytes[0]), b + bytes[0] + bytes[1],
                                                               b + bytes[0] + bytes[1] + bytes[2], n, o_pks, o_sig, d.tables());
         ctx->launches++;
         ce = cudaGetLastError();

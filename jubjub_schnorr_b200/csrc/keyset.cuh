@@ -148,7 +148,8 @@ JJS_HD void stage_keyed_gather(int variant, const fq* keys_u, const fq* keys_v, 
 
 // Equation `eq` of an item under a registered key: u*B + c*PK == R with both products from tables (`fb` for B = G or G',
 // `ktab` the key point's table).  Updates R's flags like stage_equation_item: PF_TORSION_FREE when the equation holds,
-// otherwise `*need_r_test` if R's subgroup test is still pending.
+// otherwise `*need_r_test` if R's subgroup test is still pending.  W: window width of `fb`.
+template <int W = FB_W>
 JJS_HD bool stage_equation_keyed(int variant, int eq, const fq* pts_u, const fq* pts_v, uint8_t* pflags, size_t n, size_t item, const niels* fb,
                                  const niels* ktab, const WireField& usc, const uint32_t* c_words, bool* need_r_test) {
     int pk_slot, r_slot, base_slot;
@@ -162,7 +163,7 @@ JJS_HD bool stage_equation_keyed(int variant, int eq, const fq* pts_u, const fq*
     ext acc;
     ext_identity(acc);
     keyed_acc(acc, ktab, c);
-    fixedbase_acc(acc, fb, u);
+    fixedbase_acc<W>(acc, fb, u);
     const bool ok = ext_eq_affine(acc, pts_u[r_slot * n + item], pts_v[r_slot * n + item]);
     uint8_t rf = pflags[r_slot * n + item];
     if (rf & PF_TORSION_PENDING) {

@@ -122,7 +122,8 @@ JJS_HD void stage_msig_session(const fq* pu, const fq* pv, const uint8_t* pf, si
     }
 }
 
-// z_j G + (c d_j) pk_j - a S_j == R_j
+// z_j G + (c d_j) pk_j - a S_j == R_j  (W: window width of fb_g)
+template <int W = FB_W>
 JJS_HD bool stage_msig_share(const fq* pu, const fq* pv, size_t K, size_t j, const WireField& zf, const uint32_t* cd_words, const uint32_t* a_session,
                              const niels* fb_g, fq* tabA, fq* tabB, size_t stride) {
     uint32_t z[8], cd[8], a[8];
@@ -136,7 +137,7 @@ JJS_HD bool stage_msig_share(const fq* pu, const fq* pv, size_t K, size_t j, con
     varbase_table_build(tabB, stride, pu[2 * K + j], pv[2 * K + j]);
     ext acc, zg, sum;
     straus2<64>(acc, tabA, tabB, stride, dA, dB);
-    fixedbase_mul(zg, fb_g, z);
+    fixedbase_mul<W>(zg, fb_g, z);
     pniels nz;
     ext_to_pniels(nz, zg);
     ext_add_pniels<false>(sum, acc, nz);

@@ -34,7 +34,8 @@ JJS_HD void words_to_fq(fq& r, const uint32_t* w) {  // canonical words (< q) ->
 
 // variant: 0 single, 1 double, 2 var-generator.  sk, rnd (and gsc for var-gen: generator = gsc * G) are
 // JubJub scalars < r as 8 words, msg a BlsScalar < q.  Returns false if an input is out of range.
-// Outputs: pk (32 or 64 bytes as words), sig (64 or 96 bytes as words).
+// Outputs: pk (32 or 64 bytes as words), sig (64 or 96 bytes as words).  W: window width of T's fixed-base tables.
+template <int W = FB_W>
 JJS_HD bool sign_item(int variant, const uint32_t* sk, const uint32_t* rnd, const uint32_t* gsc, const uint32_t* msg, uint32_t* pk_out,
                       uint32_t* sig_out, const Tables& T) {
     if (!fr_wire_is_canonical(sk) || !fr_wire_is_canonical(rnd) || ge_q(msg)) return false;
@@ -48,7 +49,7 @@ JJS_HD bool sign_item(int variant, const uint32_t* sk, const uint32_t* rnd, cons
     words_to_fq(in[0], rnd);
     words_to_fq(in[1], sk);
     if (variant == VAR_VARGEN) {
-        fixedbase_mul(P, T.fb_g, gsc);
+        fixedbase_mul<W>(P, T.fb_g, gsc);
         ext_to_affine(gu, gv, P);
         in[2] = gu; in[3] = gv; in[4] = m;
         hash_truncated(r, in, 5);
@@ -61,10 +62,10 @@ JJS_HD bool sign_item(int variant, const uint32_t* sk, const uint32_t* rnd, cons
     fq pu, pv, ru, rv, pu2, pv2, ru2, rv2;
     if (variant == VAR_VARGEN) {
         fr_mul(t, sk, gsc);
-        fixedbase_mul(P, T.fb_g, t);
+        fixedbase_mul<W>(P, T.fb_g, t);
         ext_to_affine(pu, pv, P);
         fr_mul(t, r, gsc);
-        fixedbase_mul(P, T.fb_g, t);
+        fixedbase_mul<W>(P, T.fb_g, t);
         ext_to_affine(ru, rv, P);
         in[0] = ru; in[1] = rv; in[2] = pu; in[3] = pv; in[4] = gu; in[5] = gv; in[6] = m;
         hash_truncated(c, in, 7);
@@ -72,9 +73,9 @@ JJS_HD bool sign_item(int variant, const uint32_t* sk, const uint32_t* rnd, cons
         point_to_wire(pk_out + 8, gu, gv);
         point_to_wire(sig_out + 8, ru, rv);
     } else {
-        fixedbase_mul(P, T.fb_g, sk);
+        fixedbase_mul<W>(P, T.fb_g, sk);
         ext_to_affine(pu, pv, P);
-        fixedbase_mul(P, T.fb_g, r);
+        fixedbase_mul<W>(P, T.fb_g, r);
         ext_to_affine(ru, rv, P);
         point_to_wire(pk_out, pu, pv);
         point_to_wire(sig_out + 8, ru, rv);
@@ -82,9 +83,9 @@ JJS_HD bool sign_item(int variant, const uint32_t* sk, const uint32_t* rnd, cons
             in[0] = ru; in[1] = rv; in[2] = pu; in[3] = pv; in[4] = m;
             hash_truncated(c, in, 5);
         } else {
-            fixedbase_mul(P, T.fb_gn, sk);
+            fixedbase_mul<W>(P, T.fb_gn, sk);
             ext_to_affine(pu2, pv2, P);
-            fixedbase_mul(P, T.fb_gn, r);
+            fixedbase_mul<W>(P, T.fb_gn, r);
             ext_to_affine(ru2, rv2, P);
             point_to_wire(pk_out + 8, pu2, pv2);
             point_to_wire(sig_out + 16, ru2, rv2);

@@ -224,8 +224,8 @@ JJS_HD uint8_t subgroup_check(const WireField& f, size_t i, int method, fq* tab,
 // interleave, compared projectively with R (equality with Gen, PK in the subgroup puts R there too).
 // tabA must be followed by two more per-thread tables at tabA + 36 stride (== tabB) and tabA + 72 stride.
 // MODE: -1 either kind (decided by base_slot at run time), 0 fixed base only, 1 variable base only -- the kernels instantiate the
-// two kinds separately so that neither carries the other's code and registers.
-template <int MODE = -1>
+// two kinds separately so that neither carries the other's code and registers.  W: window width of the fixed-base table `fb`.
+template <int MODE = -1, int W = FB_W>
 JJS_HD bool stage_equation(const fq* pts_u, const fq* pts_v, size_t n, size_t item, int pk_slot, int r_slot, int base_slot,
                            const niels* fb, const WireField& usc, const uint32_t* c_words, fq* tabA, fq* tabB, size_t stride,
                            bool* r_implied = nullptr) {
@@ -248,7 +248,7 @@ JJS_HD bool stage_equation(const fq* pts_u, const fq* pts_v, size_t n, size_t it
         straus2<33>(acc, tabA, tabB, stride, dT, dR);
         uint32_t ru[8];
         fr_mul_short(ru, rho, u);  // |rho| * u mod r,  |rho| < 2^126
-        fixedbase_acc(acc, fb, ru);
+        fixedbase_acc<W>(acc, fb, ru);
         bool ok = ext_is_identity(acc);
         if (r_implied) *r_implied = ok && rho_odd;
         return ok;
@@ -297,7 +297,7 @@ JJS_HD void equation_slots(int variant, int eq, int& pk_slot, int& r_slot, int& 
     else if (variant == VAR_DOUBLE) { pk_slot = eq; r_slot = 2 + eq; base_slot = -1; }
     else { pk_slot = 0; r_slot = 2; base_slot = 1; }
 }
-template <int MODE = -1>
+template <int MODE = -1, int W = FB_W>
 JJS_HD bool stage_equation_item(int variant, int eq, const fq* pts_u, const fq* pts_v, uint8_t* pflags, size_t n, size_t item, const niels* fb,
                                 const WireField& usc, const uint32_t* c_words, fq* tabA, fq* tabB, size_t stride, bool* need_r_test) {
     int pk_slot, r_slot, base_slot;
@@ -306,7 +306,7 @@ JJS_HD bool stage_equation_item(int variant, int eq, const fq* pts_u, const fq* 
     if (!point_flags_valid(pflags[pk_slot * n + item])) return false;
     if (base_slot >= 0 && !point_flags_valid(pflags[base_slot * n + item])) return false;
     bool implied = false;
-    bool ok = stage_equation<MODE>(pts_u, pts_v, n, item, pk_slot, r_slot, base_slot, fb, usc, c_words, tabA, tabB, stride, &implied);
+    bool ok = stage_equation<MODE, W>(pts_u, pts_v, n, item, pk_slot, r_slot, base_slot, fb, usc, c_words, tabA, tabB, stride, &implied);
     uint8_t rf = pflags[r_slot * n + item];
     if (rf & PF_TORSION_PENDING) {
         if (implied) pflags[r_slot * n + item] = (uint8_t)((rf & ~PF_TORSION_PENDING) | PF_TORSION_FREE);

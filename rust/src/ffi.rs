@@ -38,6 +38,10 @@ pub struct jjs_part {
 
 extern "C" {
     pub fn jjs_init(devices: *const c_int, n_devices: c_int, out: *mut *mut jjs_ctx) -> c_int;
+    // a context that never holds more than device_memory_limit bytes on any of its devices
+    pub fn jjs_init_limited(devices: *const c_int, n_devices: c_int, device_memory_limit: usize, out: *mut *mut jjs_ctx) -> c_int;
+    pub fn jjs_memory_info(ctx: *const jjs_ctx, device_index: c_int, bytes_held: *mut u64, fb_window_bits: *mut c_int,
+                           items_in_flight: *mut u64) -> c_int;
     pub fn jjs_destroy(ctx: *mut jjs_ctx);
     pub fn jjs_last_error(ctx: *const jjs_ctx) -> *const c_char;
     pub fn jjs_device_count(ctx: *const jjs_ctx) -> c_int;

@@ -76,6 +76,18 @@ impl GpuVerifier {
     pub fn new(devices: &[i32]) -> Result<Self, String> {
         let mut ctx = ptr::null_mut();
         let rc = unsafe { ffi::jjs_init(devices.as_ptr(), devices.len() as i32, &mut ctx) };
+        Self::from_init(rc, ctx)
+    }
+
+    /// A verifier that holds at most `device_memory_limit` bytes of device memory on each of `devices` (jjs_init_limited): the
+    /// library picks the fastest configuration that fits.  Fails when even the smallest one (about 40 MB) does not.
+    pub fn with_memory_limit(devices: &[i32], device_memory_limit: usize) -> Result<Self, String> {
+        let mut ctx = ptr::null_mut();
+        let rc = unsafe { ffi::jjs_init_limited(devices.as_ptr(), devices.len() as i32, device_memory_limit, &mut ctx) };
+        Self::from_init(rc, ctx)
+    }
+
+    fn from_init(rc: i32, ctx: *mut ffi::jjs_ctx) -> Result<Self, String> {
         if rc != 0 {
             let msg = if ctx.is_null() {
                 String::from("jjs_init: allocation failed")
@@ -276,13 +288,21 @@ impl Drop for GpuVerifier {
 static GLOBAL: OnceLock<Mutex<GpuVerifier>> = OnceLock::new();
 
 /// The verifier the scalar methods use: created on first use over the devices named by `JJS_B200_DEVICES` ("0,1,2,..",
-/// default "0").  There is no CPU fallback: without a usable sm_100a device this panics with the library's message.
+/// default "0"), holding at most `JJS_B200_MEMORY_LIMIT` bytes of device memory on each when that is set (else the full-size
+/// context of `GpuVerifier::new`).  There is no CPU fallback: without a usable sm_100a device this panics with the library's message.
 pub fn global() -> MutexGuard<'static, GpuVerifier> {
     GLOBAL
         .get_or_init(|| {
             let spec = std::env::var("JJS_B200_DEVICES").unwrap_or_else(|_| String::from("0"));
             let devices: Vec<i32> = spec.split(',').filter_map(|d| d.trim().parse().ok()).collect();
-            Mutex::new(GpuVerifier::new(&devices).expect("jubjub-schnorr gpu feature: no usable B200"))
+            let verifier = match std::env::var("JJS_B200_MEMORY_LIMIT") {
+                Ok(limit) => {
+                    let bytes: usize = limit.trim().parse().expect("JJS_B200_MEMORY_LIMIT: a number of bytes");
+                    GpuVerifier::with_memory_limit(&devices, bytes)
+                }
+                Err(_) => GpuVerifier::new(&devices),
+            };
+            Mutex::new(verifier.expect("jubjub-schnorr gpu feature: no usable B200"))
         })
         .lock()
         .expect("gpu verifier poisoned")
