@@ -230,6 +230,23 @@ int jjs_multisig_combine(jjs_ctx* ctx, const uint8_t* pks32, const uint8_t* R32,
                          const uint32_t* offsets, const uint8_t* msg32, size_t n, uint8_t* share_ok_or_null, uint8_t* status,
                          uint32_t* bad_index_or_null, uint8_t* sig64_or_null);
 
+/* All-or-nothing verification of n single (kind JJS_KIND_SINGLE: pk32, sig64) or double (JJS_KIND_DOUBLE: pk64, sig96)
+ * items.  *all_valid = 1 iff every item would get JJS_OK from jjs_verify_single / jjs_verify_double, except that a batch
+ * containing an item whose equation fails is accepted with probability at most 2^-128; an all-valid batch is never
+ * rejected.  n == 0 gives 1.  No per-item results: to find the failing items, call jjs_verify_single / _double.
+ * One random linear combination of all the equations with secret 128-bit weights, evaluated as a multi-scalar
+ * multiplication (DESIGN.md section 12); every point is subgroup-tested.
+ * seed32_or_null: NULL draws a fresh 32-byte secret seed from the operating system for every call (what production must
+ * do); a caller-given seed makes the call deterministic and is for tests only -- whoever knows the seed can forge a
+ * batch that passes.  Other kinds: JJS_ERR_ARGUMENT.  Host buffers, sharded over the context's devices. */
+int jjs_verify_all(jjs_ctx* ctx, int kind, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg32, size_t n,
+                   const uint8_t* seed32_or_null, int* all_valid);
+/* The same on device buffers of device `device_index`; *d_all_valid (device memory, one 32-bit int) is written on cuda_stream,
+ * enqueue-only like the other device-buffer entry points; seed32_or_null is host memory, read during the call. */
+int jjs_verify_all_device(jjs_ctx* ctx, int device_index, int kind, const uint8_t* d_pk, const uint8_t* d_sig,
+                          const uint8_t* d_msg32, size_t n, const uint8_t* seed32_or_null, int* d_all_valid,
+                          void* cuda_stream);
+
 /* Challenge hash only (hash parity hook): c = challenge_hash(..) for already-valid encodings, no curve
  * check.  variant: 0 single, 1 double, 2 var-generator.  Host buffers. */
 int jjs_challenge_only(jjs_ctx* ctx, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg32,

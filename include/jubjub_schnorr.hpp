@@ -46,6 +46,14 @@ public:
     void check(int rc, const char* what) const {
         if (rc != JJS_SUCCESS) throw std::runtime_error(std::string(what) + ": " + jjs_last_error(ctx_));
     }
+    // NEW: whether all n single (JJS_KIND_SINGLE) or double (JJS_KIND_DOUBLE) items verify, by one random linear combination
+    // (jjs_verify_all; a batch with a failing item passes with probability at most 2^-128).  Wire buffers as in the C ABI;
+    // seed32: nullptr draws fresh secret weights for every call, 32 given bytes are for tests only.
+    bool verify_all(int kind, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg32, size_t n, const uint8_t* seed32 = nullptr) const {
+        int ok = 0;
+        check(jjs_verify_all(ctx_, kind, pk, sig, msg32, n, seed32, &ok), "jjs_verify_all");
+        return ok == 1;
+    }
 
 private:
     void init(int rc, const char* what) {

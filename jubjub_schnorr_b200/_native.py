@@ -20,6 +20,7 @@ EXPORTS = [
     "jjs_verify_mixed",
     "jjs_keyset_create", "jjs_keyset_destroy", "jjs_verify_keyed", "jjs_verify_keyed_device", "jjs_keyset_table_check",
     "jjs_init_limited", "jjs_memory_info",
+    "jjs_verify_all", "jjs_verify_all_device",
 ]
 
 
@@ -114,5 +115,9 @@ def lib():
     L.jjs_verify_keyed_device.restype = C.c_int
     L.jjs_keyset_table_check.argtypes = [vp, C.c_int, vp, sz, vp]
     L.jjs_keyset_table_check.restype = C.c_int
+    L.jjs_verify_all.argtypes = [vp, C.c_int, vp, vp, vp, sz, vp, C.POINTER(C.c_int)]
+    L.jjs_verify_all.restype = C.c_int
+    L.jjs_verify_all_device.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, sz, vp, vp, vp]
+    L.jjs_verify_all_device.restype = C.c_int
     _lib = L
     return L

@@ -352,6 +352,37 @@ class BatchVerifier:
         self._check(self._lib.jjs_keyset_table_check(self._ctx, ks.handle, idx.ctypes.data, idx.shape[0], bad.ctypes.data), "jjs_keyset_table_check")
         return int(bad[0])
 
+    # ---- whole-batch verification ----------------------------------------------------------------
+    @staticmethod
+    def _seed_ptr(seed):
+        if seed is None:
+            return None, None
+        s = np.ascontiguousarray(np.frombuffer(bytes(seed), dtype=np.uint8))
+        if s.size != 32:
+            raise ValueError("seed must be 32 bytes")
+        return s, s.ctypes.data
+
+    def verify_all(self, kind, pk, sig, msg32, seed=None) -> bool:
+        """True iff every item (kind SINGLE or DOUBLE) would verify, by one random linear combination of all the equations
+        (jjs_verify_all): a batch with a failing equation passes with probability at most 2^-128.  seed: None draws a fresh
+        secret seed from the operating system for every call; 32 given bytes make the call deterministic (tests only)."""
+        if kind not in (SINGLE, DOUBLE):
+            raise ValueError("verify_all takes SINGLE or DOUBLE items")
+        pk, sig, msg = _u8(pk, PK_SIZE[kind], "pk"), _u8(sig, SIG_SIZE[kind], "sig"), _u8(msg32, 32, "msg")
+        n = msg.shape[0]
+        if pk.shape[0] != n or sig.shape[0] != n:
+            raise ValueError("pk, sig and msg must describe the same number of items")
+        keep, sp = self._seed_ptr(seed)
+        ok = C.c_int(0)
+        self._check(self._lib.jjs_verify_all(self._ctx, kind, pk.ctypes.data, sig.ctypes.data, msg.ctypes.data, n, sp, C.byref(ok)), "jjs_verify_all")
+        return bool(ok.value)
+
+    def verify_all_device(self, kind, d_pk, d_sig, d_msg, n, d_all_valid, seed=None, stream=None, device_index=0):
+        """jjs_verify_all_device on raw device pointers: the int32 verdict is written to d_all_valid on `stream`."""
+        keep, sp = self._seed_ptr(seed)
+        self._check(self._lib.jjs_verify_all_device(self._ctx, device_index, kind, d_pk, d_sig, d_msg, n, sp, d_all_valid, stream),
+                    "jjs_verify_all_device")
+
     # ---- raw host / device pointers (pinned torch tensors, device tensors: pass .data_ptr()) ----------
     def verify_host_ptr(self, variant, pk_ptr, sig_ptr, msg_ptr, n, status_ptr, c_ptr=None):
         fn = {SINGLE: self._lib.jjs_verify_single, DOUBLE: self._lib.jjs_verify_double, VARGEN: self._lib.jjs_verify_vargen}[variant]

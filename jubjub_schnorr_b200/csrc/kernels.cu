@@ -4,6 +4,8 @@
 // u*B + c*PK); intermediates travel between the stages as SoA arrays of 32-byte field elements in HBM,
 // so every warp access is a run of 128-bit vector loads.  There is deliberately no CPU path.
 #include <cuda_runtime.h>
+#include <cub/device/device_radix_sort.cuh>
+#include <sys/random.h>
 
 #include <atomic>
 #include <cstdarg>
@@ -17,6 +19,7 @@
 #include "../../include/jjschnorr_b200.h"
 #include "keyset.cuh"
 #include "multisig_core.cuh"
+#include "rlc.cuh"
 #include "sign_core.cuh"
 #include "verify_core.cuh"
 #include "safe_tag.h"
@@ -380,6 +383,117 @@ __global__ void __launch_bounds__(BLOCK) k_bitmap(const uint8_t* status, size_t 
     bool ok = i < n && status[i] == 0;
     uint32_t w = __ballot_sync(0xffffffffu, ok);
     if ((threadIdx.x & 31) == 0 && i < n) words[i >> 5] = w;
+}
+
+// ---- whole-batch verification (rlc.cuh): one random linear combination per call --------------------------------------------
+__global__ void k_rlc_init(RlcAcc* acc) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) rlc_acc_init(*acc);
+}
+// thread = item: validity by the reference's precedence (every point decoded and valid, scalars in range), weights from the
+// call-wide index base + item, sort entries and the G scalars
+__global__ void __launch_bounds__(BLOCK) k_rlc_digits(int variant, const uint8_t* pflags, const uint8_t* iflags, const uint32_t* cwords, WireField usc, size_t m,
+                                                      RlcShape s, RlcSeed seed, uint64_t base, uint32_t* keys, uint32_t* vals, uint32_t* zu, RlcAcc* acc) {
+    const size_t item = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (item >= m) return;
+    const bool dbl = variant == VAR_DOUBLE;
+    const bool valid = stage_status(variant, pflags, (uint8_t)(iflags[item] | IF_EQ0_OK | IF_EQ1_OK), m, item) == 0;
+    if (!valid) acc->valid = 0;
+    uint32_t u[8], c[8];
+    wire_load(u, usc, item);
+#pragma unroll
+    for (int i = 0; i < 8; i++) c[i] = cwords[item * 8 + i];
+    rlc_item_entries(keys + item * s.per_item, vals + item * s.per_item, zu + item * 8, zu + (m + item) * 8, dbl, valid, c, u, seed, base + item, m, item, s);
+}
+__global__ void __launch_bounds__(BLOCK) k_rlc_bucket_init(ext* buckets, size_t nb) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < nb) ext_identity(buckets[i]);
+}
+constexpr int RLC_SEG = 32;      // sorted entries per thread of a segment pass
+constexpr int RLC_SLICE = 32;    // buckets per thread of the bucket reduction
+__global__ void __launch_bounds__(BLOCK) k_rlc_segments0(const uint32_t* keys, const uint32_t* vals, const fq* pts_u, const fq* pts_v, size_t len, uint32_t sentinel,
+                                                         ext* buckets, uint32_t* ckeys, ext* cpts, bool final_level) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    rlc_segment(keys, RlcAffineSrc{pts_u, pts_v, vals}, len, t, RLC_SEG, sentinel, buckets, ckeys, cpts, final_level);
+}
+__global__ void __launch_bounds__(BLOCK) k_rlc_segments(const uint32_t* keys, const ext* pts, size_t len, uint32_t sentinel, ext* buckets, uint32_t* ckeys,
+                                                        ext* cpts, bool final_level) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    rlc_segment(keys, RlcExtSrc{pts}, len, t, RLC_SEG, sentinel, buckets, ckeys, cpts, final_level);
+}
+// thread = slice of RLC_SLICE buckets of one window
+__global__ void __launch_bounds__(BLOCK) k_rlc_slices(const ext* buckets, int nw, uint32_t per_window, ext* partial) {
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t slices = per_window / RLC_SLICE;
+    if (t >= (size_t)nw * slices) return;
+    const uint32_t w = (uint32_t)(t / slices), sl = (uint32_t)(t % slices);
+    rlc_bucket_slice(partial[t], buckets + (size_t)w * per_window, sl * RLC_SLICE, (sl + 1) * RLC_SLICE);
+}
+// block = window, 32 threads: the window's slice sums
+__global__ void __launch_bounds__(32) k_rlc_window_sums(const ext* partial, uint32_t slices, ext* W) {
+    __shared__ ext part[32];
+    ext acc;
+    ext_identity(acc);
+    for (uint32_t i = threadIdx.x; i < slices; i += 32) rlc_add(acc, partial[(size_t)blockIdx.x * slices + i]);
+    part[threadIdx.x] = acc;
+    __syncwarp();
+    if (threadIdx.x == 0) {
+        for (int k = 1; k < 32; k++) rlc_add(acc, part[k]);
+        W[blockIdx.x] = acc;
+    }
+}
+// one thread: Horner over the windows, added to the half's accumulator
+__global__ void k_rlc_horner(const ext* W, int nw, int c, RlcAcc* acc) {
+    if (blockIdx.x || threadIdx.x) return;
+    ext P;
+    rlc_horner(P, W, nw, c);
+    rlc_add(acc->P, P);
+}
+// one block: the pass's G (and G') scalar sums into the accumulator, mod r.  Sums of up to 2^24 values below 2^252 fit in nine
+// words, so the block adds exactly and reduces once.
+constexpr int RLC_SUM_THREADS = 256;
+__global__ void __launch_bounds__(RLC_SUM_THREADS) k_rlc_scalars(const uint32_t* zu, size_t m, int neq, RlcAcc* acc) {
+    __shared__ uint32_t part[RLC_SUM_THREADS][9];
+    for (int eq = 0; eq < neq; eq++) {
+        uint32_t s[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+        for (size_t i = threadIdx.x; i < m; i += RLC_SUM_THREADS) {
+            s[8] += add8c(s, s, zu + ((size_t)eq * m + i) * 8, 0u);
+        }
+        for (int k = 0; k < 9; k++) part[threadIdx.x][k] = s[k];
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int t = 1; t < RLC_SUM_THREADS; t++) s[8] += part[t][8] + add8c(s, s, part[t], 0u);
+            uint32_t wide[16] = {0}, red[8];
+            for (int k = 0; k < 9; k++) wide[k] = s[k];
+            fr_reduce_wide(red, wide, 9 * 32);
+            fr_add(acc->su[eq], acc->su[eq], red);
+        }
+        __syncthreads();
+    }
+}
+struct RlcOut {
+    ext P;
+    uint32_t valid;
+};
+// one thread: the halves' accumulators summed, the G terms added; writes the device's partial point (host entry point, summed
+// over devices on the host) and / or the verdict (device entry point)
+template <int W>
+__global__ void k_rlc_finish(const RlcAcc* acc0, const RlcAcc* acc1_or_null, int variant, Tables T, RlcOut* out, int* all_valid) {
+    if (blockIdx.x || threadIdx.x) return;
+    ext P = acc0->P;
+    uint32_t su[2][8], valid = acc0->valid;
+    for (int i = 0; i < 8; i++) { su[0][i] = acc0->su[0][i]; su[1][i] = acc0->su[1][i]; }
+    if (acc1_or_null) {
+        rlc_add(P, acc1_or_null->P);
+        fr_add(su[0], su[0], acc1_or_null->su[0]);
+        fr_add(su[1], su[1], acc1_or_null->su[1]);
+        valid &= acc1_or_null->valid;
+    }
+    rlc_fixed_terms<W>(P, su, variant == VAR_DOUBLE, T.fb_g, T.fb_gn);
+    if (out) {
+        out->P = P;
+        out->valid = valid;
+    }
+    if (all_valid) *all_valid = (valid && ext_is_identity(P)) ? 1 : 0;
 }
 
 // Fixed-base tables of width W in two passes (curve.cuh, fb_combine_entries), LO = (W + 1) / 2, HI = W - LO.  Pass 1: the small
@@ -1222,6 +1336,118 @@ int run_chunk_keyed(jjs_ctx* ctx, DeviceState& d, const Region& R, const KeySet&
     return JJS_SUCCESS;
 }
 
+// ---- whole-batch verification: one pass of the combination ----------------------------------------------------------------
+// No per-item equation runs on this path, so its scratch is the region's equation-table scratch: TAB_ROWS field elements
+// (3 456 bytes) per item of capacity, contiguous from rlc_base.  On a limited context that is R.tab itself; a jjs_init
+// context's table scratch is laid out by row for the equation kernels (column = thread), so each half takes a contiguous
+// half of the whole allocation instead (4 352 bytes per item of a half).  The half's accumulator sits at the start.
+constexpr size_t RLC_ROW_BYTES = sizeof(fq) * TAB_ROWS;
+inline uint8_t* rlc_base(const DeviceState& d, const Region& R) {
+    if (d.limit) return reinterpret_cast<uint8_t*>(R.tab);
+    return reinterpret_cast<uint8_t*>(d.tab) + (size_t)R.half * (sizeof(fq) * AGG_GROUP * R32_TAB_FQ * TAB_THREADS / 2);
+}
+inline RlcAcc* rlc_acc(const DeviceState& d, const Region& R) { return reinterpret_cast<RlcAcc*>(rlc_base(d, R)); }
+
+// Where the buffers of a pass of m items with window width c go, in bytes from rlc_base; `total` is what it needs.
+struct RlcPlan {
+    RlcShape s;
+    size_t entries, n1, n2, cub_bytes;
+    size_t o_zu, o_keys[2], o_vals[2], o_cub, o_buckets, o_ck[2], o_cp[2], o_partial, o_W, total;
+};
+inline int rlc_plan(RlcPlan& p, int variant, size_t m, int c) {
+    p.s = rlc_shape(variant == VAR_DOUBLE, c);
+    p.entries = m * (size_t)p.s.per_item;
+    p.n1 = 2 * rlc_segments(p.entries, RLC_SEG);
+    p.n2 = 2 * rlc_segments(p.n1, RLC_SEG);
+    cub::DoubleBuffer<uint32_t> kb(nullptr, nullptr), vb(nullptr, nullptr);
+    p.cub_bytes = 0;
+    if (cub::DeviceRadixSort::SortPairs(nullptr, p.cub_bytes, kb, vb, (int)p.entries, 0, p.s.end_bit) != cudaSuccess) return JJS_ERR_CUDA;
+    const size_t neq = variant == VAR_DOUBLE ? 2 : 1, nb = p.s.sentinel, slices = nb / RLC_SLICE;
+    size_t o = align_up(sizeof(RlcAcc), 256);
+    auto take = [&](size_t bytes) { size_t at = o; o += align_up(bytes, 256); return at; };
+    p.o_zu = take(32 * neq * m);
+    for (int k = 0; k < 2; k++) { p.o_keys[k] = take(4 * p.entries); p.o_vals[k] = take(4 * p.entries); }
+    p.o_cub = take(p.cub_bytes);
+    p.o_buckets = take(sizeof(ext) * nb);
+    p.o_ck[0] = take(4 * p.n1); p.o_cp[0] = take(sizeof(ext) * p.n1);
+    p.o_ck[1] = take(4 * p.n2); p.o_cp[1] = take(sizeof(ext) * p.n2);
+    p.o_partial = take(sizeof(ext) * slices);
+    p.o_W = take(sizeof(ext) * p.s.nw_big);
+    p.total = o;
+    return JJS_SUCCESS;
+}
+// The window width of a pass: the cheapest c whose buffers fit the region's scratch, by a count of point additions (one per
+// sort entry, about 2.3 mixed-addition equivalents per bucket for the running sums).  It follows from the point count alone.
+inline int rlc_choose(jjs_ctx* ctx, RlcPlan& best, int variant, size_t m, size_t budget) {
+    double best_cost = 0;
+    bool found = false;
+    for (int c = RLC_C_MIN; c <= RLC_C_MAX; c++) {
+        RlcPlan p;
+        if (rlc_plan(p, variant, m, c)) return fail(ctx, JJS_ERR_CUDA, "radix sort: temporary storage query failed");
+        if (p.total > budget) continue;
+        const double cost = (double)p.entries + 2.3 * (double)p.s.sentinel;
+        if (!found || cost < best_cost) { best = p; best_cost = cost; found = true; }
+    }
+    if (!found) return fail(ctx, JJS_ERR_NOMEM, "whole-batch verification: %zu items do not fit the pass scratch of %zu bytes", m, budget);
+    return JJS_SUCCESS;
+}
+
+// One pass of m <= R.cap items (device pointers): decode with every point subgroup-tested, work list and challenges, then the
+// combination of the pass added into the half's accumulator.  `base`: position of the pass's first item in the whole call.
+int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t m,
+                  uint64_t base, const RlcSeed& seed, cudaStream_t stream) {
+    const int slots = variant_slots(variant), neq = variant == VAR_DOUBLE ? 2 : 1;
+    Tables T = d.tables();
+    Fields pts;
+    WireField fmsg, fu;
+    variant_fields(variant, pk, sig, msg, pts, fmsg, fu);
+    RlcPlan p;
+    int rc = rlc_choose(ctx, p, variant, m, RLC_ROW_BYTES * R.cap);
+    if (rc) return rc;
+    StageTimer t0(ctx, d.device, 0, stream);
+    k_decode<<<blocks_for(slots * m), BLOCK, 0, stream>>>(pts, slots, 0, m, R.pts_u, R.pts_v, R.pflags, T, (1u << slots) - 1u);
+    t0.stop(stream);
+    ctx->launches++;
+    rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
+    if (rc) return rc;
+    uint8_t* B = rlc_base(d, R);
+    RlcAcc* acc = rlc_acc(d, R);
+    uint32_t* zu = reinterpret_cast<uint32_t*>(B + p.o_zu);
+    StageTimer t3(ctx, d.device, 3, stream);
+    k_rlc_digits<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.cwords, fu, m, p.s, seed, base,
+                                                       reinterpret_cast<uint32_t*>(B + p.o_keys[0]), reinterpret_cast<uint32_t*>(B + p.o_vals[0]), zu, acc);
+    cub::DoubleBuffer<uint32_t> kb(reinterpret_cast<uint32_t*>(B + p.o_keys[0]), reinterpret_cast<uint32_t*>(B + p.o_keys[1]));
+    cub::DoubleBuffer<uint32_t> vb(reinterpret_cast<uint32_t*>(B + p.o_vals[0]), reinterpret_cast<uint32_t*>(B + p.o_vals[1]));
+    size_t cub_bytes = p.cub_bytes;
+    JJS_CUDA(ctx, cub::DeviceRadixSort::SortPairs(B + p.o_cub, cub_bytes, kb, vb, (int)p.entries, 0, p.s.end_bit, stream));
+    ext* buckets = reinterpret_cast<ext*>(B + p.o_buckets);
+    k_rlc_bucket_init<<<blocks_for(p.s.sentinel), BLOCK, 0, stream>>>(buckets, p.s.sentinel);
+    // level 0 on the sorted pairs, then the merge levels on the carries until one segment is left
+    size_t len = p.entries;
+    size_t segs = rlc_segments(len, RLC_SEG);
+    k_rlc_segments0<<<blocks_for(segs), BLOCK, 0, stream>>>(kb.Current(), vb.Current(), R.pts_u, R.pts_v, len, p.s.sentinel, buckets,
+                                                            reinterpret_cast<uint32_t*>(B + p.o_ck[0]), reinterpret_cast<ext*>(B + p.o_cp[0]), segs == 1);
+    ctx->launches += 4;
+    for (int lv = 0; segs > 1; lv ^= 1) {
+        len = 2 * segs;
+        segs = rlc_segments(len, RLC_SEG);
+        k_rlc_segments<<<blocks_for(segs), BLOCK, 0, stream>>>(reinterpret_cast<const uint32_t*>(B + p.o_ck[lv]), reinterpret_cast<const ext*>(B + p.o_cp[lv]), len,
+                                                               p.s.sentinel, buckets, reinterpret_cast<uint32_t*>(B + p.o_ck[lv ^ 1]),
+                                                               reinterpret_cast<ext*>(B + p.o_cp[lv ^ 1]), segs == 1);
+        ctx->launches++;
+    }
+    const uint32_t slices = p.s.buckets_per_window / RLC_SLICE;
+    ext* partial = reinterpret_cast<ext*>(B + p.o_partial);
+    ext* W = reinterpret_cast<ext*>(B + p.o_W);
+    k_rlc_slices<<<blocks_for((size_t)p.s.nw_big * slices), BLOCK, 0, stream>>>(buckets, p.s.nw_big, p.s.buckets_per_window, partial);
+    k_rlc_window_sums<<<p.s.nw_big, 32, 0, stream>>>(partial, slices, W);
+    k_rlc_horner<<<1, 1, 0, stream>>>(W, p.s.nw_big, p.s.c, acc);
+    k_rlc_scalars<<<1, RLC_SUM_THREADS, 0, stream>>>(zu, m, neq, acc);
+    t3.stop(stream);
+    ctx->launches += 4;
+    return JJS_SUCCESS;
+}
+
 // Sub-chunks of an overlapped batch alternate between the two internal streams and scratch halves: kernels of neighbouring
 // sub-chunks overlap, which hides the partially filled last wave of every launch (per-thread work is uniform, so a launch
 // ends with SMs idling for up to one block duration).  With per-stage profiling on, everything stays on `stream` so that
@@ -1297,6 +1523,36 @@ int run_keyed_device(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, const KeySe
     return JJS_SUCCESS;
 }
 
+// jjs_verify_all_device: the passes of n items through the sub-chunks of run_device, then the verdict written on `stream`
+int run_rlc_device(jjs_ctx* ctx, DeviceState& d, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t n, const RlcSeed& seed,
+                   int* all_valid, cudaStream_t stream) {
+    int rc = ensure_scratch(ctx, d);
+    if (rc) return rc;
+    JJS_CUDA(ctx, cudaSetDevice(d.device));
+    Overlap ov(ctx, d, stream, n > d.sub_chunk);
+    rc = ov.begin();
+    if (rc) return rc;
+    const int nacc = ov.on ? 2 : 1;
+    for (int h = 0; h < nacc; h++) {
+        k_rlc_init<<<1, 1, 0, ov.on ? d.sub[h] : stream>>>(rlc_acc(d, ov.on ? region_half(d, h) : region_whole(d)));
+        ctx->launches++;
+    }
+    const size_t step = ov.on ? d.sub_chunk : d.chunk_items;
+    for (size_t off = 0; off < n; off += step, ov.advance()) {
+        size_t m = n - off < step ? n - off : step;
+        rc = run_chunk_rlc(ctx, d, ov.next_region(), variant, pk + off * pk_size(variant), sig + off * sig_size(variant), msg + off * 32, m, off, seed,
+                           ov.next_stream());
+        if (rc) return rc;
+    }
+    rc = ov.end();
+    if (rc) return rc;
+    (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, stream>>>(
+        rlc_acc(d, region_half(d, 0)), nacc == 2 ? rlc_acc(d, region_half(d, 1)) : nullptr, variant, d.tables(), nullptr, all_valid);
+    ctx->launches++;
+    JJS_CUDA(ctx, cudaGetLastError());
+    return JJS_SUCCESS;
+}
+
 // Chunks of an aggregate-key batch: at most `max_items` items and `max_keys` signer keys each (an item with more keys than
 // that forms a chunk of its own, for which the caller grows the key scratch first).
 inline size_t agg_chunk_end(const uint32_t* offsets, size_t first, size_t n, size_t max_items, size_t max_keys) {
@@ -1352,7 +1608,19 @@ int run_aggregate_device(jjs_ctx* ctx, DeviceState& d, const uint8_t* d_pks, con
 // loaded device), and every device is driven by its own host thread: copies in on the copy stream, pipeline slices alternating
 // between the two compute streams, results copied out at the end, one synchronisation.  A single host thread would serialise
 // the devices whenever the caller's memory is pageable (cudaMemcpyAsync from pageable memory returns only after staging).
-enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2, PART_KEYED = 3 };
+enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2, PART_KEYED = 3, PART_ALL = 4 };
+// whole-batch verification: the devices' partial points and validity flags, summed on the host as the devices finish
+struct RlcSink {
+    std::mutex mu;
+    ext P;
+    bool valid = true;
+    RlcSink() { ext_identity(P); }
+    void add(const RlcOut& o) {
+        std::lock_guard<std::mutex> lock(mu);
+        rlc_add(P, o.P);
+        valid = valid && o.valid;
+    }
+};
 struct HostPart {
     int mode, variant;
     const uint8_t *pk, *sig, *msg;    // typed: pk = points_ext160, sig = u32;  keyed: pk = the uint32 key indices
@@ -1362,6 +1630,8 @@ struct HostPart {
     uint32_t* bitmap;
     bool challenge_only;
     const KeySet* keys = nullptr;     // keyed only
+    const RlcSeed* seed = nullptr;    // whole-batch only: the weights' seed and where the devices' results go
+    RlcSink* sink = nullptr;
 };
 struct Shard {
     size_t lo, hi;
@@ -1469,6 +1739,14 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
     rc = ensure_stage(ctx, d, total);
     if (rc) return rc;
     const bool serial = ctx->profile;   // stage timers must not overlap
+    int p_all = -1;                     // the whole-batch part, if any: its accumulators start out empty on both halves
+    for (size_t p = 0; p < parts.size(); p++)
+        if (parts[p].mode == PART_ALL && shards[p][k].hi > shards[p][k].lo) p_all = (int)p;
+    if (p_all >= 0)
+        for (int h = 0; h < 2; h++) {
+            k_rlc_init<<<1, 1, 0, serial ? d.stream : d.sub[h]>>>(rlc_acc(d, region_half(d, h)));
+            ctx->launches++;
+        }
     size_t j = 0;                       // slice counter of this device: slices alternate between the compute streams / scratch halves
     for (size_t p = 0; p < parts.size(); p++) {
         const HostPart& P = parts[p];
@@ -1514,6 +1792,8 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
                 if (P.mode == PART_TYPED)
                     rc = run_chunk_ext(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * 32, S.msg + off * 32, cnt, S.status + off,
                                        want_c ? S.c + off * 32 : nullptr, cs);
+                else if (P.mode == PART_ALL)
+                    rc = run_chunk_rlc(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * sgs, S.msg + off * 32, cnt, lo + off, *P.seed, cs);
                 else if (P.mode == PART_KEYED)
                     rc = run_chunk_keyed(ctx, d, R, *P.keys, P.keys->dev[k], reinterpret_cast<const uint32_t*>(S.pk + off * pks), S.sig + off * sgs,
                                          S.msg + off * 32, cnt, S.status + off, want_c ? S.c + off * 32 : nullptr, cs);
@@ -1544,8 +1824,17 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
             JJS_CUDA(ctx, cudaMemcpyAsync(P.bitmap + lo / 32, S.bitmap, 4 * ((m + 31) / 32), cudaMemcpyDeviceToHost, d.stream));
         }
     }
+    RlcOut out;
+    if (p_all >= 0) {   // the device's partial point: both halves' accumulators and the G terms, staged in the part's challenge slot
+        RlcOut* d_out = reinterpret_cast<RlcOut*>(st[p_all].c);
+        (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, d.stream>>>(
+            rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), parts[p_all].variant, d.tables(), d_out, nullptr);
+        ctx->launches++;
+        JJS_CUDA(ctx, cudaMemcpyAsync(&out, d_out, sizeof(RlcOut), cudaMemcpyDeviceToHost, d.stream));
+    }
     JJS_CUDA(ctx, cudaGetLastError());
     JJS_CUDA(ctx, cudaStreamSynchronize(d.stream));
+    if (p_all >= 0) parts[p_all].sink->add(out);
     return JJS_SUCCESS;
 }
 
@@ -1602,6 +1891,10 @@ int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& part
 int validate_part(jjs_ctx* ctx, const HostPart& P) {
     if (P.mode == PART_WIRE || P.mode == PART_TYPED || P.mode == PART_KEYED) {
         if (P.variant < 0 || P.variant > 2) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
+    } else if (P.mode == PART_ALL) {
+        if (P.variant != VAR_SINGLE && P.variant != VAR_DOUBLE) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
+        if (P.n && (!P.pk || !P.sig || !P.msg)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+        return JJS_SUCCESS;
     } else if (P.mode != PART_AGGREGATE) {
         return fail(ctx, JJS_ERR_ARGUMENT, "bad part kind");
     }
@@ -1953,6 +2246,31 @@ void keyset_free(jjs_ctx* ctx, KeySet* ks) {
         dev_free(d, kd.table, keyset_table_bytes(npts));
     }
     delete ks;
+}
+
+// The weights' seed: the caller's 32 bytes, or 32 fresh bytes from the operating system
+int rlc_seed(jjs_ctx* ctx, const uint8_t* seed32_or_null, RlcSeed& seed) {
+    uint8_t b[32];
+    if (seed32_or_null) {
+        memcpy(b, seed32_or_null, 32);
+    } else {
+        for (size_t got = 0; got < 32;) {
+            ssize_t r = getrandom(b + got, 32 - got, 0);
+            if (r < 0) {
+                if (errno == EINTR) continue;
+                return fail(ctx, JJS_ERR_ARGUMENT, "getrandom failed: %s", strerror(errno));
+            }
+            got += (size_t)r;
+        }
+    }
+    for (int i = 0; i < 8; i++) seed.w[i] = (uint32_t)b[4 * i] | (uint32_t)b[4 * i + 1] << 8 | (uint32_t)b[4 * i + 2] << 16 | (uint32_t)b[4 * i + 3] << 24;
+    return JJS_SUCCESS;
+}
+// kinds of the whole-batch entry points; on a context whose jjs_init failed the refusal keeps the reason of the failure
+int rlc_check_kind(jjs_ctx* ctx, int kind) {
+    if (kind == JJS_KIND_SINGLE || kind == JJS_KIND_DOUBLE) return JJS_SUCCESS;
+    if (ctx && ctx->ready) return fail(ctx, JJS_ERR_ARGUMENT, "whole-batch verification takes single or double items (kind %d)", kind);
+    return JJS_ERR_ARGUMENT;
 }
 
 KeySet* keyset_lookup(jjs_ctx* ctx, int handle) {
@@ -2336,6 +2654,38 @@ JJS_API int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* ent
     });
     *mismatches = count;
     return rc;
+}
+JJS_API int jjs_verify_all(jjs_ctx* ctx, int kind, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg32, size_t n, const uint8_t* seed32_or_null,
+                           int* all_valid) {
+    int rc = rlc_check_kind(ctx, kind);
+    if (rc) return rc;
+    JJS_ENTER(ctx);
+    if (!all_valid) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    *all_valid = 0;
+    RlcSeed seed;
+    rc = rlc_seed(ctx, seed32_or_null, seed);
+    if (rc) return rc;
+    RlcSink sink;
+    HostPart P = wire_part(kind, pk, sig, msg32, n, nullptr, nullptr, nullptr);
+    P.mode = PART_ALL;
+    P.seed = &seed;
+    P.sink = &sink;
+    rc = run_parts(ctx, {P});
+    if (rc) return rc;
+    *all_valid = sink.valid && ext_is_identity(sink.P) ? 1 : 0;
+    return JJS_SUCCESS;
+}
+JJS_API int jjs_verify_all_device(jjs_ctx* ctx, int device_index, int kind, const uint8_t* d_pk, const uint8_t* d_sig, const uint8_t* d_msg32, size_t n,
+                                  const uint8_t* seed32_or_null, int* d_all_valid, void* cuda_stream) {
+    int rc = rlc_check_kind(ctx, kind);
+    if (rc) return rc;
+    JJS_ENTER(ctx);
+    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
+    if (!d_all_valid || (n && (!d_pk || !d_sig || !d_msg32))) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    RlcSeed seed;
+    rc = rlc_seed(ctx, seed32_or_null, seed);
+    if (rc) return rc;
+    return run_rlc_device(ctx, ctx->dev[device_index], kind, d_pk, d_sig, d_msg32, n, seed, d_all_valid, (cudaStream_t)cuda_stream);
 }
 JJS_API int jjs_sign_batch(jjs_ctx* ctx, int variant, const uint8_t* sk32, const uint8_t* rnd32, const uint8_t* gen_scalar32_or_null,
                            const uint8_t* msg32, size_t n, uint8_t* pk_out, uint8_t* sig_out) {

@@ -95,6 +95,12 @@ extern "C" {
                                    d_msg32: *const u8, n: usize, d_status: *mut u8, d_c32_or_null: *mut u8,
                                    cuda_stream: *mut c_void) -> c_int;
     pub fn jjs_keyset_table_check(ctx: *mut jjs_ctx, keyset: c_int, entries: *const u32, n: usize, mismatches: *mut u32) -> c_int;
+    // NEW all-or-nothing verification of single / double items by one random linear combination (DESIGN.md section 12)
+    pub fn jjs_verify_all(ctx: *mut jjs_ctx, kind: c_int, pk: *const u8, sig: *const u8, msg32: *const u8, n: usize,
+                          seed32_or_null: *const u8, all_valid: *mut c_int) -> c_int;
+    pub fn jjs_verify_all_device(ctx: *mut jjs_ctx, device_index: c_int, kind: c_int, d_pk: *const u8, d_sig: *const u8,
+                                 d_msg32: *const u8, n: usize, seed32_or_null: *const u8, d_all_valid: *mut c_int,
+                                 cuda_stream: *mut c_void) -> c_int;
     // typed inputs: JubJubExtended coordinates, 160 bytes per point (variant 0: PK, R; 1: PK, PK', R, R'; 2: PK, gen, R)
     pub fn jjs_verify_ext(ctx: *mut jjs_ctx, variant: c_int, points_ext160: *const u8, u32_: *const u8, msg32: *const u8,
                           n: usize, status: *mut u8, c32_or_null: *mut u8) -> c_int;

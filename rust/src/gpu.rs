@@ -11,6 +11,7 @@
 
 extern crate std;
 
+use core::ffi::c_int;
 use std::ffi::CStr;
 use std::ptr;
 use std::string::String;
@@ -127,6 +128,28 @@ impl GpuVerifier {
         let rc = unsafe { ffi::jjs_verify_single(self.ctx, pk.as_ptr(), sig.as_ptr(), msg.as_ptr(), n, status.as_mut_ptr(), ptr::null_mut()) };
         self.check(rc, "jjs_verify_single");
         status.into_iter().map(status_to_result).collect()
+    }
+
+    /// NEW: `items.iter().all(|(pk, sig, m)| pk.verify(sig, *m).is_ok())` by one random linear combination of all the equations
+    /// (jjs_verify_all, fresh secret weights from the operating system): a batch with a failing item passes with probability at
+    /// most 2^-128.  No per-item answer: call verify_batch to find the failing items.
+    pub fn verify_all(&mut self, items: &[(PublicKey, Signature, BlsScalar)]) -> bool {
+        let n = items.len();
+        let (pk, sig, msg) = wire::<_, _, 32, 64>(items);
+        let mut ok: c_int = 0;
+        let rc = unsafe { ffi::jjs_verify_all(self.ctx, ffi::JJS_KIND_SINGLE, pk.as_ptr(), sig.as_ptr(), msg.as_ptr(), n, ptr::null(), &mut ok) };
+        self.check(rc, "jjs_verify_all");
+        ok == 1
+    }
+
+    /// The same for double items.
+    pub fn verify_all_double(&mut self, items: &[(PublicKeyDouble, SignatureDouble, BlsScalar)]) -> bool {
+        let n = items.len();
+        let (pk, sig, msg) = wire::<_, _, 64, 96>(items);
+        let mut ok: c_int = 0;
+        let rc = unsafe { ffi::jjs_verify_all(self.ctx, ffi::JJS_KIND_DOUBLE, pk.as_ptr(), sig.as_ptr(), msg.as_ptr(), n, ptr::null(), &mut ok) };
+        self.check(rc, "jjs_verify_all");
+        ok == 1
     }
 
     // ---- double: PublicKeyDouble::verify (src/keys/public/double.rs:86-117) --------------------------------------------
