@@ -246,6 +246,23 @@ int jjs_verify_all(jjs_ctx* ctx, int kind, const uint8_t* pk, const uint8_t* sig
 int jjs_verify_all_device(jjs_ctx* ctx, int device_index, int kind, const uint8_t* d_pk, const uint8_t* d_sig,
                           const uint8_t* d_msg32, size_t n, const uint8_t* seed32_or_null, int* d_all_valid,
                           void* cuda_stream);
+/* All-or-nothing verification of every item of every part (jjs_part as for jjs_verify_mixed; any of the four kinds).
+ * *all_valid = 1 iff every item would get JJS_OK from jjs_verify_mixed, except that a batch holding an item whose
+ * equation fails is accepted with probability at most 2^-128; an all-valid batch is never rejected.  One random linear
+ * combination over all parts (DESIGN.md section 13): the weights of an item are those of its position in the whole call
+ * (the sizes of the preceding parts plus its index in its part), so a one-part call gives jjs_verify_all's combination for
+ * the same seed.  The output fields of every part (status, c32, aggpk32, accept_bitmap) must be NULL.  n_parts == 0 or all
+ * parts empty gives 1.  Seed: as jjs_verify_all.  Host buffers, each part sharded over the devices as jjs_verify_mixed
+ * shards it.  JJS_ERR_ARGUMENT for an unknown kind, an aggregate part without offsets, a non-NULL output field or a NULL
+ * all_valid. */
+int jjs_verify_all_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null, int* all_valid);
+/* The same on device buffers of device `device_index`.  The parts' pointers are device memory.  h_offsets_or_null[p] is
+ * the host copy of aggregate part p's offsets (the same rule as jjs_verify_aggregate_device), and NULL for other kinds.
+ * The whole array may be NULL when no part is aggregate.  Enqueue-only on cuda_stream, with the growth exception of
+ * jjs_verify_aggregate_device.  *d_all_valid is device memory. */
+int jjs_verify_all_mixed_device(jjs_ctx* ctx, int device_index, const jjs_part* parts, size_t n_parts,
+                                const uint32_t* const* h_offsets_or_null, const uint8_t* seed32_or_null,
+                                int* d_all_valid, void* cuda_stream);
 
 /* Challenge hash only (hash parity hook): c = challenge_hash(..) for already-valid encodings, no curve
  * check.  variant: 0 single, 1 double, 2 var-generator.  Host buffers. */

@@ -54,6 +54,13 @@ public:
         check(jjs_verify_all(ctx_, kind, pk, sig, msg32, n, seed32, &ok), "jjs_verify_all");
         return ok == 1;
     }
+    // NEW: whether every item of every part (any kind, jjs_part as for jjs_verify_mixed with every output field NULL) verifies,
+    // by one random linear combination over all parts (jjs_verify_all_mixed); seed32 as for verify_all.
+    bool verify_all_mixed(const jjs_part* parts, size_t n_parts, const uint8_t* seed32 = nullptr) const {
+        int ok = 0;
+        check(jjs_verify_all_mixed(ctx_, parts, n_parts, seed32, &ok), "jjs_verify_all_mixed");
+        return ok == 1;
+    }
 
 private:
     void init(int rc, const char* what) {

@@ -383,6 +383,52 @@ class BatchVerifier:
         self._check(self._lib.jjs_verify_all_device(self._ctx, device_index, kind, d_pk, d_sig, d_msg, n, sp, d_all_valid, stream),
                     "jjs_verify_all_device")
 
+    def verify_all_mixed(self, parts, seed=None) -> bool:
+        """True iff every item of every part would verify (jjs_verify_mixed status 0), by one random linear combination over all
+        the parts (jjs_verify_all_mixed).  parts: as for verify_mixed, (kind, pk, sig, msg) or, for AGGREGATE, (kind, pks, sig,
+        msg, offsets), any of the four kinds.  seed: as for verify_all."""
+        structs, keep = [], []
+        for part in parts:
+            kind, pk, sig, msg = part[0], part[1], part[2], part[3]
+            if kind not in PK_SIZE:
+                raise ValueError("unknown kind %r" % (kind,))
+            pk, sig, msg = _u8(pk, PK_SIZE[kind], "pk"), _u8(sig, SIG_SIZE[kind], "sig"), _u8(msg, 32, "msg")
+            n = msg.shape[0]
+            off = None
+            if kind == AGGREGATE:
+                off = np.ascontiguousarray(part[4], dtype=np.uint32)
+                if off.shape[0] != n + 1 or int(off[-1]) != pk.shape[0] or int(off[0]) != 0:
+                    raise ValueError("offsets must have n + 1 entries covering pks32 exactly")
+            elif pk.shape[0] != n:
+                raise ValueError("pk, sig and msg must describe the same number of items")
+            if sig.shape[0] != n:
+                raise ValueError("pk, sig and msg must describe the same number of items")
+            structs.append(_native.Part(kind, pk.ctypes.data, off.ctypes.data if off is not None else None, sig.ctypes.data, msg.ctypes.data, n,
+                                        None, None, None, None))
+            keep.append((pk, sig, msg, off))
+        arr = (_native.Part * max(len(structs), 1))(*structs)
+        keep_seed, sp = self._seed_ptr(seed)
+        ok = C.c_int(0)
+        self._check(self._lib.jjs_verify_all_mixed(self._ctx, arr, len(structs), sp, C.byref(ok)), "jjs_verify_all_mixed")
+        return bool(ok.value)
+
+    def verify_all_mixed_device(self, parts, d_all_valid, seed=None, stream=None, device_index=0):
+        """jjs_verify_all_mixed_device on raw device pointers: parts = iterable of (kind, pk_ptr, sig_ptr, msg_ptr, n) or, for
+        AGGREGATE, (kind, pks_ptr, sig_ptr, msg_ptr, n, d_offsets_ptr, h_offsets) with h_offsets the host copy of the offsets.
+        The int32 verdict is written to d_all_valid on `stream`."""
+        structs, hosts, keep = [], [], []
+        for part in parts:
+            kind, pk, sig, msg, n = part[:5]
+            d_off, h_off = (part[5], np.ascontiguousarray(part[6], dtype=np.uint32)) if kind == AGGREGATE else (None, None)
+            structs.append(_native.Part(kind, pk, d_off, sig, msg, n, None, None, None, None))
+            hosts.append(h_off.ctypes.data if h_off is not None else None)
+            keep.append(h_off)
+        arr = (_native.Part * max(len(structs), 1))(*structs)
+        harr = (C.c_void_p * max(len(hosts), 1))(*hosts)
+        keep_seed, sp = self._seed_ptr(seed)
+        self._check(self._lib.jjs_verify_all_mixed_device(self._ctx, device_index, arr, len(structs), harr, sp, d_all_valid, stream),
+                    "jjs_verify_all_mixed_device")
+
     # ---- raw host / device pointers (pinned torch tensors, device tensors: pass .data_ptr()) ----------
     def verify_host_ptr(self, variant, pk_ptr, sig_ptr, msg_ptr, n, status_ptr, c_ptr=None):
         fn = {SINGLE: self._lib.jjs_verify_single, DOUBLE: self._lib.jjs_verify_double, VARGEN: self._lib.jjs_verify_vargen}[variant]

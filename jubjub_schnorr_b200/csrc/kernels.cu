@@ -395,14 +395,14 @@ __global__ void __launch_bounds__(BLOCK) k_rlc_digits(int variant, const uint8_t
                                                       RlcShape s, RlcSeed seed, uint64_t base, uint32_t* keys, uint32_t* vals, uint32_t* zu, RlcAcc* acc) {
     const size_t item = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (item >= m) return;
-    const bool dbl = variant == VAR_DOUBLE;
     const bool valid = stage_status(variant, pflags, (uint8_t)(iflags[item] | IF_EQ0_OK | IF_EQ1_OK), m, item) == 0;
     if (!valid) acc->valid = 0;
     uint32_t u[8], c[8];
     wire_load(u, usc, item);
 #pragma unroll
     for (int i = 0; i < 8; i++) c[i] = cwords[item * 8 + i];
-    rlc_item_entries(keys + item * s.per_item, vals + item * s.per_item, zu + item * 8, zu + (m + item) * 8, dbl, valid, c, u, seed, base + item, m, item, s);
+    rlc_item_entries(keys + item * s.per_item, vals + item * s.per_item, zu + item * 8, zu + (m + item) * 8, variant, valid, c, u, seed, base + item, m, item,
+                     s);
 }
 __global__ void __launch_bounds__(BLOCK) k_rlc_bucket_init(ext* buckets, size_t nb) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -474,21 +474,20 @@ struct RlcOut {
     ext P;
     uint32_t valid;
 };
-// one thread: the halves' accumulators summed, the G terms added; writes the device's partial point (host entry point, summed
-// over devices on the host) and / or the verdict (device entry point)
+// one thread: the halves' accumulators summed, the G and G' terms added (a call may mix kinds, and a zero scalar sum adds the
+// identity); writes the device's partial point (host entry point, summed over devices on the host) and / or the verdict
+// (device entry point)
 template <int W>
-__global__ void k_rlc_finish(const RlcAcc* acc0, const RlcAcc* acc1_or_null, int variant, Tables T, RlcOut* out, int* all_valid) {
+__global__ void k_rlc_finish(const RlcAcc* acc0, const RlcAcc* acc1, Tables T, RlcOut* out, int* all_valid) {
     if (blockIdx.x || threadIdx.x) return;
     ext P = acc0->P;
     uint32_t su[2][8], valid = acc0->valid;
     for (int i = 0; i < 8; i++) { su[0][i] = acc0->su[0][i]; su[1][i] = acc0->su[1][i]; }
-    if (acc1_or_null) {
-        rlc_add(P, acc1_or_null->P);
-        fr_add(su[0], su[0], acc1_or_null->su[0]);
-        fr_add(su[1], su[1], acc1_or_null->su[1]);
-        valid &= acc1_or_null->valid;
-    }
-    rlc_fixed_terms<W>(P, su, variant == VAR_DOUBLE, T.fb_g, T.fb_gn);
+    rlc_add(P, acc1->P);
+    fr_add(su[0], su[0], acc1->su[0]);
+    fr_add(su[1], su[1], acc1->su[1]);
+    valid &= acc1->valid;
+    rlc_fixed_terms<W>(P, su, true, T.fb_g, T.fb_gn);
     if (out) {
         out->P = P;
         out->valid = valid;
@@ -1266,10 +1265,13 @@ int run_chunk_ext(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, co
     return JJS_SUCCESS;
 }
 
-// aggregate_pk(..).verify(..) for one chunk of m <= R.acap items with K <= cap_keys signer keys; everything on `stream`,
-// nothing on the host.  d_keys: the chunk's first key; d_offsets: the chunk's m + 1 offsets (absolute, first = key_lo).
-int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uint8_t* d_keys, const uint32_t* d_offsets, uint32_t key_lo, size_t K,
-                        const uint8_t* d_sig, const uint8_t* d_msg, size_t m, uint8_t* d_status, uint8_t* d_c, uint8_t* d_agg, cudaStream_t stream) {
+// The front of an aggregate-key chunk of m items with K <= cap_keys signer keys, on `stream`: signer keys and R decoded, the
+// ordering by signer count, the coefficients, the aggregate keys into slot 0 (the aggregation kernel's tables at `tab`,
+// serving `stride` >= m threads), then the work list and challenges.  R's subgroup test runs at decode when `r_test`, else it
+// is left to the equation.  d_keys: the chunk's first key; d_offsets: the chunk's m + 1 offsets (absolute, first = key_lo).
+int enqueue_aggregate_front(jjs_ctx* ctx, DeviceState& d, const Region& R, const uint8_t* d_keys, const uint32_t* d_offsets, uint32_t key_lo, size_t K,
+                            const uint8_t* d_sig, const uint8_t* d_msg, size_t m, uint8_t* d_agg, fq* tab, size_t stride, bool r_test,
+                            cudaStream_t stream) {
     AggScratch& A = d.agg[R.half];
     Tables T = d.tables();
     Fields fk, fr;
@@ -1279,7 +1281,7 @@ int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uin
     WireField fmsg{d_msg, 32}, fu{d_sig, 64};
     StageTimer t0(ctx, d.device, 0, stream);
     if (K) k_decode<<<blocks_for(K), BLOCK, 0, stream>>>(fk, 1, 0, K, A.keys_u, A.keys_v, A.kflags, T, 0u);
-    k_decode<<<blocks_for(m), BLOCK, 0, stream>>>(fr, 1, 1, m, R.pts_u, R.pts_v, R.pflags, T, 0u);
+    k_decode<<<blocks_for(m), BLOCK, 0, stream>>>(fr, 1, 1, m, R.pts_u, R.pts_v, R.pflags, T, r_test ? 1u : 0u);
     t0.stop(stream);
     StageTimer t2(ctx, d.device, 2, stream);
     JJS_CUDA(ctx, cudaMemsetAsync(A.sort, 0, sizeof(AggSort), stream));
@@ -1287,11 +1289,19 @@ int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uin
     k_agg_scan<<<1, 32, 0, stream>>>(A.sort);
     k_agg_scatter<<<blocks_for(m), BLOCK, 0, stream>>>(d_offsets, key_lo, m, A.sort, A.order, A.kmap, A.kitem);
     if (K) k_agg_coeffs<<<blocks_for(K), BLOCK, 0, stream>>>(A.keys_u, A.keys_v, A.kflags, d_offsets, A.kmap, A.kitem, key_lo, K, A.kcoef, T);
-    k_aggregate<<<blocks_for(m), BLOCK, 0, stream>>>(A.keys_u, A.keys_v, A.kflags, d_offsets, A.order, key_lo, m, R.pts_u, R.pts_v, R.pflags, d_agg, R.tab,
-                                                    R.astride, A.kcoef, T);
+    k_aggregate<<<blocks_for(m), BLOCK, 0, stream>>>(A.keys_u, A.keys_v, A.kflags, d_offsets, A.order, key_lo, m, R.pts_u, R.pts_v, R.pflags, d_agg, tab,
+                                                    stride, A.kcoef, T);
     t2.stop(stream);
     ctx->launches += 7;
-    int rc = enqueue_challenges(ctx, d, R, VAR_SINGLE, m, fmsg, fu, stream, true);
+    return enqueue_challenges(ctx, d, R, VAR_SINGLE, m, fmsg, fu, stream, true);
+}
+
+// aggregate_pk(..).verify(..) for one chunk of m <= R.acap items with K <= cap_keys signer keys; everything on `stream`,
+// nothing on the host.  Arguments as enqueue_aggregate_front.
+int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uint8_t* d_keys, const uint32_t* d_offsets, uint32_t key_lo, size_t K,
+                        const uint8_t* d_sig, const uint8_t* d_msg, size_t m, uint8_t* d_status, uint8_t* d_c, uint8_t* d_agg, cudaStream_t stream) {
+    WireField fu{d_sig, 64};
+    int rc = enqueue_aggregate_front(ctx, d, R, d_keys, d_offsets, key_lo, K, d_sig, d_msg, m, d_agg, R.tab, R.astride, false, stream);
     if (!rc) rc = enqueue_equations(ctx, d, R, VAR_SINGLE, m, fu, stream);
     if (rc) return rc;
     StageTimer t4(ctx, d.device, 4, stream);
@@ -1340,13 +1350,25 @@ int run_chunk_keyed(jjs_ctx* ctx, DeviceState& d, const Region& R, const KeySet&
 // No per-item equation runs on this path, so its scratch is the region's equation-table scratch: TAB_ROWS field elements
 // (3 456 bytes) per item of capacity, contiguous from rlc_base.  On a limited context that is R.tab itself; a jjs_init
 // context's table scratch is laid out by row for the equation kernels (column = thread), so each half takes a contiguous
-// half of the whole allocation instead (4 352 bytes per item of a half).  The half's accumulator sits at the start.
-constexpr size_t RLC_ROW_BYTES = sizeof(fq) * TAB_ROWS;
+// half of the whole allocation instead (4 352 bytes per item of a half).  The half's accumulator takes the last RLC_ACC_BYTES
+// of those 3 456 per item: the pass buffers (rlc_plan) and the aggregation tables of an aggregate pass (rlc_agg_items) stay
+// below it, so no pass of the call overwrites what earlier passes on the half accumulated, and the two halves stay disjoint.
+constexpr size_t RLC_ROW_BYTES = sizeof(fq) * TAB_ROWS, RLC_ACC_BYTES = 256;
+static_assert(sizeof(RlcAcc) <= RLC_ACC_BYTES, "the accumulator must fit its slot");
 inline uint8_t* rlc_base(const DeviceState& d, const Region& R) {
     if (d.limit) return reinterpret_cast<uint8_t*>(R.tab);
     return reinterpret_cast<uint8_t*>(d.tab) + (size_t)R.half * (sizeof(fq) * AGG_GROUP * R32_TAB_FQ * TAB_THREADS / 2);
 }
-inline RlcAcc* rlc_acc(const DeviceState& d, const Region& R) { return reinterpret_cast<RlcAcc*>(rlc_base(d, R)); }
+inline size_t rlc_pass_bytes(const Region& R) { return RLC_ROW_BYTES * R.cap - RLC_ACC_BYTES; }
+inline RlcAcc* rlc_acc(const DeviceState& d, const Region& R) { return reinterpret_cast<RlcAcc*>(rlc_base(d, R) + rlc_pass_bytes(R)); }
+// Items of an aggregate pass: as many as the aggregation kernel's per-thread tables (stride = this count) fit below the
+// accumulator, and the order array serves.
+constexpr size_t AGG_TAB_BYTES = sizeof(fq) * AGG_GROUP * R32_TAB_FQ;
+inline size_t rlc_agg_items(const DeviceState& d, const Region& R) {
+    size_t t = rlc_pass_bytes(R) / AGG_TAB_BYTES;
+    if (t > R.cap) t = R.cap;
+    return t < d.agg_items ? t : d.agg_items;
+}
 
 // Where the buffers of a pass of m items with window width c go, in bytes from rlc_base; `total` is what it needs.
 struct RlcPlan {
@@ -1355,7 +1377,7 @@ struct RlcPlan {
     size_t o_zu, o_keys[2], o_vals[2], o_cub, o_buckets, o_ck[2], o_cp[2], o_partial, o_W, total;
 };
 inline int rlc_plan(RlcPlan& p, int variant, size_t m, int c) {
-    p.s = rlc_shape(variant == VAR_DOUBLE, c);
+    p.s = rlc_shape(variant, c);
     p.entries = m * (size_t)p.s.per_item;
     p.n1 = 2 * rlc_segments(p.entries, RLC_SEG);
     p.n2 = 2 * rlc_segments(p.n1, RLC_SEG);
@@ -1363,7 +1385,7 @@ inline int rlc_plan(RlcPlan& p, int variant, size_t m, int c) {
     p.cub_bytes = 0;
     if (cub::DeviceRadixSort::SortPairs(nullptr, p.cub_bytes, kb, vb, (int)p.entries, 0, p.s.end_bit) != cudaSuccess) return JJS_ERR_CUDA;
     const size_t neq = variant == VAR_DOUBLE ? 2 : 1, nb = p.s.sentinel, slices = nb / RLC_SLICE;
-    size_t o = align_up(sizeof(RlcAcc), 256);
+    size_t o = 0;
     auto take = [&](size_t bytes) { size_t at = o; o += align_up(bytes, 256); return at; };
     p.o_zu = take(32 * neq * m);
     for (int k = 0; k < 2; k++) { p.o_keys[k] = take(4 * p.entries); p.o_vals[k] = take(4 * p.entries); }
@@ -1392,25 +1414,35 @@ inline int rlc_choose(jjs_ctx* ctx, RlcPlan& best, int variant, size_t m, size_t
     return JJS_SUCCESS;
 }
 
-// One pass of m <= R.cap items (device pointers): decode with every point subgroup-tested, work list and challenges, then the
-// combination of the pass added into the half's accumulator.  `base`: position of the pass's first item in the whole call.
-int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t m,
-                  uint64_t base, const RlcSeed& seed, cudaStream_t stream) {
-    const int slots = variant_slots(variant), neq = variant == VAR_DOUBLE ? 2 : 1;
-    Tables T = d.tables();
-    Fields pts;
-    WireField fmsg, fu;
-    variant_fields(variant, pk, sig, msg, pts, fmsg, fu);
+// One pass of m <= R.cap items of kind `kind` (JJS_KIND_*, device pointers), with every point subgroup-tested before it enters:
+// single, double and var-generator items decode every slot with its test, then work list and challenges; aggregate items
+// (m <= rlc_agg_items; pk = the pass's first signer key, offsets, key_lo and K as run_chunk_aggregate) run the front of the
+// aggregate path with R's test on, its aggregation tables in the pass scratch.  Then the combination of the pass is added into
+// the half's accumulator.  `base`: position of the pass's first item in the whole call.
+int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int kind, const uint8_t* pk, const uint32_t* offsets, uint32_t key_lo, size_t K,
+                  const uint8_t* sig, const uint8_t* msg, size_t m, uint64_t base, const RlcSeed& seed, cudaStream_t stream) {
+    const bool agg = kind == JJS_KIND_AGGREGATE;
+    const int variant = agg ? VAR_SINGLE : kind, neq = variant == VAR_DOUBLE ? 2 : 1;
     RlcPlan p;
-    int rc = rlc_choose(ctx, p, variant, m, RLC_ROW_BYTES * R.cap);
-    if (rc) return rc;
-    StageTimer t0(ctx, d.device, 0, stream);
-    k_decode<<<blocks_for(slots * m), BLOCK, 0, stream>>>(pts, slots, 0, m, R.pts_u, R.pts_v, R.pflags, T, (1u << slots) - 1u);
-    t0.stop(stream);
-    ctx->launches++;
-    rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
+    int rc = rlc_choose(ctx, p, variant, m, rlc_pass_bytes(R));
     if (rc) return rc;
     uint8_t* B = rlc_base(d, R);
+    WireField fu;
+    if (agg) {
+        fu = WireField{sig, 64};
+        rc = enqueue_aggregate_front(ctx, d, R, pk, offsets, key_lo, K, sig, msg, m, nullptr, reinterpret_cast<fq*>(B), rlc_agg_items(d, R), true, stream);
+    } else {
+        const int slots = variant_slots(variant);
+        Fields pts;
+        WireField fmsg;
+        variant_fields(variant, pk, sig, msg, pts, fmsg, fu);
+        StageTimer t0(ctx, d.device, 0, stream);
+        k_decode<<<blocks_for(slots * m), BLOCK, 0, stream>>>(pts, slots, 0, m, R.pts_u, R.pts_v, R.pflags, d.tables(), (1u << slots) - 1u);
+        t0.stop(stream);
+        ctx->launches++;
+        rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
+    }
+    if (rc) return rc;
     RlcAcc* acc = rlc_acc(d, R);
     uint32_t* zu = reinterpret_cast<uint32_t*>(B + p.o_zu);
     StageTimer t3(ctx, d.device, 3, stream);
@@ -1523,36 +1555,6 @@ int run_keyed_device(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, const KeySe
     return JJS_SUCCESS;
 }
 
-// jjs_verify_all_device: the passes of n items through the sub-chunks of run_device, then the verdict written on `stream`
-int run_rlc_device(jjs_ctx* ctx, DeviceState& d, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t n, const RlcSeed& seed,
-                   int* all_valid, cudaStream_t stream) {
-    int rc = ensure_scratch(ctx, d);
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > d.sub_chunk);
-    rc = ov.begin();
-    if (rc) return rc;
-    const int nacc = ov.on ? 2 : 1;
-    for (int h = 0; h < nacc; h++) {
-        k_rlc_init<<<1, 1, 0, ov.on ? d.sub[h] : stream>>>(rlc_acc(d, ov.on ? region_half(d, h) : region_whole(d)));
-        ctx->launches++;
-    }
-    const size_t step = ov.on ? d.sub_chunk : d.chunk_items;
-    for (size_t off = 0; off < n; off += step, ov.advance()) {
-        size_t m = n - off < step ? n - off : step;
-        rc = run_chunk_rlc(ctx, d, ov.next_region(), variant, pk + off * pk_size(variant), sig + off * sig_size(variant), msg + off * 32, m, off, seed,
-                           ov.next_stream());
-        if (rc) return rc;
-    }
-    rc = ov.end();
-    if (rc) return rc;
-    (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, stream>>>(
-        rlc_acc(d, region_half(d, 0)), nacc == 2 ? rlc_acc(d, region_half(d, 1)) : nullptr, variant, d.tables(), nullptr, all_valid);
-    ctx->launches++;
-    JJS_CUDA(ctx, cudaGetLastError());
-    return JJS_SUCCESS;
-}
-
 // Chunks of an aggregate-key batch: at most `max_items` items and `max_keys` signer keys each (an item with more keys than
 // that forms a chunk of its own, for which the caller grows the key scratch first).
 inline size_t agg_chunk_end(const uint32_t* offsets, size_t first, size_t n, size_t max_items, size_t max_keys) {
@@ -1602,6 +1604,72 @@ int run_aggregate_device(jjs_ctx* ctx, DeviceState& d, const uint8_t* d_pks, con
     return JJS_SUCCESS;
 }
 
+// One part of a device-buffer whole-batch call (jjs_verify_all_device, jjs_verify_all_mixed_device): kind JJS_KIND_*,
+// device pointers; aggregate parts also carry the host copy of their offsets, which plans the passes.
+struct RlcDevPart {
+    int kind;
+    const uint8_t *pk, *sig, *msg;
+    const uint32_t *d_offsets, *h_offsets;
+    size_t n;
+};
+// The passes of every part through the sub-chunks of run_device (aggregate parts cut by agg_chunk_end), alternating between
+// the scratch halves and their accumulators, then the verdict written on `stream`.  Enqueue-only unless the aggregate key
+// scratch or the tag table has to grow, as run_aggregate_device.
+int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& parts, const RlcSeed& seed, int* all_valid, cudaStream_t stream) {
+    int rc = ensure_scratch(ctx, d);
+    size_t n = 0, max_cnt = 0;
+    bool any_agg = false;
+    for (const RlcDevPart& P : parts) {
+        n += P.n;
+        if (P.kind != JJS_KIND_AGGREGATE || !P.n) continue;
+        any_agg = true;
+        const size_t mc = agg_max_item_keys(P.h_offsets, P.n);
+        if (mc > max_cnt) max_cnt = mc;
+    }
+    if (!rc && any_agg) rc = ensure_tags(ctx, d, 2 + 2 * max_cnt);
+    if (!rc && any_agg) rc = ensure_agg_scratch(ctx, d, max_cnt > d.agg_keys_initial ? max_cnt : d.agg_keys_initial);
+    if (rc) return rc;
+    JJS_CUDA(ctx, cudaSetDevice(d.device));
+    Overlap ov(ctx, d, stream, n > d.sub_chunk);
+    rc = ov.begin();
+    if (rc) return rc;
+    for (int h = 0; h < 2; h++) {
+        k_rlc_init<<<1, 1, 0, ov.on ? d.sub[h] : stream>>>(rlc_acc(d, region_half(d, h)));
+        ctx->launches++;
+    }
+    uint64_t base = 0;
+    for (const RlcDevPart& P : parts) {
+        for (size_t off = 0; off < P.n; ov.advance()) {
+            const Region R = region_half(d, ov.i);
+            size_t end = off + (P.n - off < d.sub_chunk ? P.n - off : d.sub_chunk);
+            uint32_t key_lo = 0;
+            size_t K = 0;
+            if (P.kind == JJS_KIND_AGGREGATE) {
+                const size_t most = rlc_agg_items(d, R);
+                end = agg_chunk_end(P.h_offsets, off, P.n, d.sub_chunk < most ? d.sub_chunk : most, d.agg[0].cap_keys);
+                key_lo = P.h_offsets[off];
+                K = P.h_offsets[end] - key_lo;
+            }
+            const size_t m = end - off;
+            rc = P.kind == JJS_KIND_AGGREGATE
+                     ? run_chunk_rlc(ctx, d, R, P.kind, P.pk + 32 * (size_t)key_lo, P.d_offsets + off, key_lo, K, P.sig + 64 * off, P.msg + 32 * off, m,
+                                     base + off, seed, ov.next_stream())
+                     : run_chunk_rlc(ctx, d, R, P.kind, P.pk + off * pk_size(P.kind), nullptr, 0, 0, P.sig + off * sig_size(P.kind), P.msg + off * 32, m,
+                                     base + off, seed, ov.next_stream());
+            if (rc) return rc;
+            off = end;
+        }
+        base += P.n;
+    }
+    rc = ov.end();
+    if (rc) return rc;
+    (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, stream>>>(
+        rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), d.tables(), nullptr, all_valid);
+    ctx->launches++;
+    JJS_CUDA(ctx, cudaGetLastError());
+    return JJS_SUCCESS;
+}
+
 // ---- host-buffer entry points ---------------------------------------------------------------------------------------------
 // A call verifies one or more PARTS (each a homogeneous batch: one of the three wire variants, aggregate-key items, or typed
 // items).  Every part is cut into contiguous shards, one per device of the context (small parts go whole to the least
@@ -1630,15 +1698,17 @@ struct HostPart {
     uint32_t* bitmap;
     bool challenge_only;
     const KeySet* keys = nullptr;     // keyed only
-    const RlcSeed* seed = nullptr;    // whole-batch only: the weights' seed and where the devices' results go
-    RlcSink* sink = nullptr;
+    const RlcSeed* seed = nullptr;    // whole-batch only (variant: the JJS_KIND_* of the part): the weights' seed, where the devices'
+    RlcSink* sink = nullptr;          // results go (one sink per call) and the position of the part's first item in the call
+    uint64_t base = 0;
 };
+inline bool part_aggregate(const HostPart& p) { return p.mode == PART_AGGREGATE || (p.mode == PART_ALL && p.variant == JJS_KIND_AGGREGATE); }
 struct Shard {
     size_t lo, hi;
 };
 
 inline double part_weight(const HostPart& p) {   // relative cost of one item (executed multiplies, single = 1)
-    if (p.mode == PART_AGGREGATE) {
+    if (part_aggregate(p)) {
         double avg = p.n ? (double)(p.offsets[p.n] - p.offsets[0]) / (double)p.n : 0.0;
         return 1.0 + 0.75 * avg;
     }
@@ -1680,7 +1750,7 @@ struct StagedPart {   // device staging of one part's shard
 
 inline size_t part_in_bytes(const HostPart& p, size_t lo, size_t hi, size_t* pk_bytes, size_t* sig_bytes) {
     const size_t m = hi - lo;
-    if (p.mode == PART_AGGREGATE) {
+    if (part_aggregate(p)) {
         *pk_bytes = 32 * (size_t)(p.offsets[hi] - p.offsets[lo]);
         *sig_bytes = 64 * m;
     } else if (p.mode == PART_TYPED) {
@@ -1723,7 +1793,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         o_st[p] = total; total += align_up(m, 256);
         o_c[p] = total; total += align_up(32 * m, 256);
         o_bm[p] = total; total += align_up(4 * ((m + 31) / 32), 256);
-        if (P.mode == PART_AGGREGATE) {
+        if (part_aggregate(P)) {
             o_agg[p] = total; total += align_up(32 * m, 256);
             o_off[p] = total; total += align_up(4 * (m + 1), 256);
             size_t mc = agg_max_item_keys(P.offsets + lo, m);
@@ -1739,8 +1809,8 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
     rc = ensure_stage(ctx, d, total);
     if (rc) return rc;
     const bool serial = ctx->profile;   // stage timers must not overlap
-    int p_all = -1;                     // the whole-batch part, if any: its accumulators start out empty on both halves
-    for (size_t p = 0; p < parts.size(); p++)
+    int p_all = -1;                     // the first whole-batch part with items here, if any: all of them add into the accumulators of
+    for (size_t p = 0; p < parts.size() && p_all < 0; p++)   // both halves, which start out empty
         if (parts[p].mode == PART_ALL && shards[p][k].hi > shards[p][k].lo) p_all = (int)p;
     if (p_all >= 0)
         for (int h = 0; h < 2; h++) {
@@ -1755,7 +1825,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         StagedPart& S = st[p];
         S.pk = d.stage + o_pk[p]; S.sig = d.stage + o_sig[p]; S.msg = d.stage + o_msg[p]; S.status = d.stage + o_st[p]; S.c = d.stage + o_c[p];
         S.bitmap = reinterpret_cast<uint32_t*>(d.stage + o_bm[p]);
-        if (P.mode == PART_AGGREGATE) {
+        if (part_aggregate(P)) {
             S.agg = d.stage + o_agg[p];
             S.offsets = reinterpret_cast<uint32_t*>(d.stage + o_off[p]);
             JJS_CUDA(ctx, cudaMemcpyAsync(S.offsets, P.offsets + lo, 4 * (m + 1), cudaMemcpyHostToDevice, d.copy_stream));
@@ -1770,9 +1840,10 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
             size_t cnt = m - off < want ? m - off : want;
             cudaStream_t cs = serial ? d.stream : d.sub[j & 1];
             Region R = region_half(d, j);
-            if (P.mode == PART_AGGREGATE) {
+            if (part_aggregate(P)) {
                 const uint32_t* ho = P.offsets + lo;   // host offsets of this shard
-                size_t end = agg_chunk_end(ho, off, m, want < R.acap ? want : R.acap, d.agg[0].cap_keys);
+                const size_t most = P.mode == PART_ALL ? rlc_agg_items(d, R) : R.acap;
+                size_t end = agg_chunk_end(ho, off, m, want < most ? want : most, d.agg[0].cap_keys);
                 cnt = end - off;
                 const uint32_t key0 = ho[0], key_lo = ho[off];
                 const size_t K = ho[end] - key_lo;
@@ -1781,8 +1852,12 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
                 JJS_CUDA(ctx, cudaMemcpyAsync(S.msg + 32 * off, P.msg + 32 * (lo + off), 32 * cnt, cudaMemcpyHostToDevice, d.copy_stream));
                 JJS_CUDA(ctx, cudaEventRecord(d.copied, d.copy_stream));
                 JJS_CUDA(ctx, cudaStreamWaitEvent(cs, d.copied, 0));
-                rc = run_chunk_aggregate(ctx, d, R, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off, S.msg + 32 * off, cnt,
-                                         S.status + off, want_c ? S.c + 32 * off : nullptr, P.agg_out ? S.agg + 32 * off : nullptr, cs);
+                if (P.mode == PART_ALL)
+                    rc = run_chunk_rlc(ctx, d, R, JJS_KIND_AGGREGATE, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off,
+                                       S.msg + 32 * off, cnt, P.base + lo + off, *P.seed, cs);
+                else
+                    rc = run_chunk_aggregate(ctx, d, R, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off, S.msg + 32 * off,
+                                             cnt, S.status + off, want_c ? S.c + 32 * off : nullptr, P.agg_out ? S.agg + 32 * off : nullptr, cs);
             } else {
                 JJS_CUDA(ctx, cudaMemcpyAsync(S.pk + off * pks, P.pk + (lo + off) * pks, cnt * pks, cudaMemcpyHostToDevice, d.copy_stream));
                 JJS_CUDA(ctx, cudaMemcpyAsync(S.sig + off * sgs, P.sig + (lo + off) * sgs, cnt * sgs, cudaMemcpyHostToDevice, d.copy_stream));
@@ -1793,7 +1868,8 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
                     rc = run_chunk_ext(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * 32, S.msg + off * 32, cnt, S.status + off,
                                        want_c ? S.c + off * 32 : nullptr, cs);
                 else if (P.mode == PART_ALL)
-                    rc = run_chunk_rlc(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * sgs, S.msg + off * 32, cnt, lo + off, *P.seed, cs);
+                    rc = run_chunk_rlc(ctx, d, R, P.variant, S.pk + off * pks, nullptr, 0, 0, S.sig + off * sgs, S.msg + off * 32, cnt, P.base + lo + off,
+                                       *P.seed, cs);
                 else if (P.mode == PART_KEYED)
                     rc = run_chunk_keyed(ctx, d, R, *P.keys, P.keys->dev[k], reinterpret_cast<const uint32_t*>(S.pk + off * pks), S.sig + off * sgs,
                                          S.msg + off * 32, cnt, S.status + off, want_c ? S.c + off * 32 : nullptr, cs);
@@ -1828,7 +1904,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
     if (p_all >= 0) {   // the device's partial point: both halves' accumulators and the G terms, staged in the part's challenge slot
         RlcOut* d_out = reinterpret_cast<RlcOut*>(st[p_all].c);
         (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, d.stream>>>(
-            rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), parts[p_all].variant, d.tables(), d_out, nullptr);
+            rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), d.tables(), d_out, nullptr);
         ctx->launches++;
         JJS_CUDA(ctx, cudaMemcpyAsync(&out, d_out, sizeof(RlcOut), cudaMemcpyDeviceToHost, d.stream));
     }
@@ -1844,7 +1920,7 @@ inline size_t part_stage_bytes(const HostPart& P, size_t lo, size_t hi) {
     size_t pkb, sgb;
     part_in_bytes(P, lo, hi, &pkb, &sgb);
     size_t b = align_up(pkb, 256) + align_up(sgb, 256) + 2 * align_up(32 * m, 256) + align_up(m, 256) + align_up(4 * ((m + 31) / 32), 256);
-    if (P.mode == PART_AGGREGATE) b += align_up(32 * m, 256) + align_up(4 * (m + 1), 256);
+    if (part_aggregate(P)) b += align_up(32 * m, 256) + align_up(4 * (m + 1), 256);
     return b;
 }
 // The largest window [lo, end) of part P whose staging fits `budget` bytes, ending on a bitmap word (or at hi); at least one word.
@@ -1892,9 +1968,10 @@ int validate_part(jjs_ctx* ctx, const HostPart& P) {
     if (P.mode == PART_WIRE || P.mode == PART_TYPED || P.mode == PART_KEYED) {
         if (P.variant < 0 || P.variant > 2) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
     } else if (P.mode == PART_ALL) {
-        if (P.variant != VAR_SINGLE && P.variant != VAR_DOUBLE) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
-        if (P.n && (!P.pk || !P.sig || !P.msg)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-        return JJS_SUCCESS;
+        if (P.variant < JJS_KIND_SINGLE || P.variant > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "bad kind");
+        if (P.variant == JJS_KIND_AGGREGATE && !P.offsets) return fail(ctx, JJS_ERR_ARGUMENT, "an aggregate part needs its offsets");
+        if (P.n && (!P.sig || !P.msg)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+        if (P.variant != JJS_KIND_AGGREGATE) return P.n && !P.pk ? fail(ctx, JJS_ERR_ARGUMENT, "null buffer") : JJS_SUCCESS;
     } else if (P.mode != PART_AGGREGATE) {
         return fail(ctx, JJS_ERR_ARGUMENT, "bad part kind");
     }
@@ -1903,8 +1980,8 @@ int validate_part(jjs_ctx* ctx, const HostPart& P) {
         if (!P.pk || !P.sig || !P.msg || !P.c_out) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
         return JJS_SUCCESS;
     }
-    if (!P.sig || !P.msg || (!P.status && !P.bitmap)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    if (P.mode == PART_AGGREGATE) {
+    if (P.mode != PART_ALL && (!P.sig || !P.msg || (!P.status && !P.bitmap))) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    if (part_aggregate(P)) {
         if (!P.offsets) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
         for (size_t i = 0; i < P.n; i++)
             if (P.offsets[i + 1] < P.offsets[i]) return fail(ctx, JJS_ERR_ARGUMENT, "offsets must be non-decreasing");
@@ -2685,7 +2762,65 @@ JJS_API int jjs_verify_all_device(jjs_ctx* ctx, int device_index, int kind, cons
     RlcSeed seed;
     rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
-    return run_rlc_device(ctx, ctx->dev[device_index], kind, d_pk, d_sig, d_msg32, n, seed, d_all_valid, (cudaStream_t)cuda_stream);
+    return run_rlc_device(ctx, ctx->dev[device_index], {RlcDevPart{kind, d_pk, d_sig, d_msg32, nullptr, nullptr, n}}, seed, d_all_valid,
+                          (cudaStream_t)cuda_stream);
+}
+JJS_API int jjs_verify_all_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null, int* all_valid) {
+    JJS_ENTER(ctx);
+    if (!all_valid || (n_parts && !parts)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    *all_valid = 0;
+    RlcSeed seed;
+    RlcSink sink;
+    std::vector<HostPart> hp;
+    hp.reserve(n_parts);
+    uint64_t base = 0;
+    for (size_t i = 0; i < n_parts; i++) {
+        const jjs_part& p = parts[i];
+        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
+        if (p.status || p.c32 || p.aggpk32 || p.accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: whole-batch verification has no per-item outputs", i);
+        HostPart P = wire_part(p.kind, p.pk, p.sig, p.msg32, p.n, nullptr, nullptr, nullptr);
+        P.mode = PART_ALL;
+        P.offsets = p.kind == JJS_KIND_AGGREGATE ? p.offsets : nullptr;
+        P.seed = &seed;
+        P.sink = &sink;
+        P.base = base;
+        base += p.n;
+        hp.push_back(P);
+    }
+    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    if (!rc) rc = run_parts(ctx, hp);
+    if (rc) return rc;
+    *all_valid = sink.valid && ext_is_identity(sink.P) ? 1 : 0;
+    return JJS_SUCCESS;
+}
+JJS_API int jjs_verify_all_mixed_device(jjs_ctx* ctx, int device_index, const jjs_part* parts, size_t n_parts, const uint32_t* const* h_offsets_or_null,
+                                        const uint8_t* seed32_or_null, int* d_all_valid, void* cuda_stream) {
+    JJS_ENTER(ctx);
+    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
+    if (!d_all_valid || (n_parts && !parts)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    std::vector<RlcDevPart> dp;
+    dp.reserve(n_parts);
+    for (size_t i = 0; i < n_parts; i++) {
+        const jjs_part& p = parts[i];
+        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
+        if (p.status || p.c32 || p.aggpk32 || p.accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: whole-batch verification has no per-item outputs", i);
+        const uint32_t* ho = nullptr;
+        if (p.kind == JJS_KIND_AGGREGATE) {
+            ho = h_offsets_or_null ? h_offsets_or_null[i] : nullptr;
+            if (!p.offsets || !ho) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: an aggregate part needs its offsets on the device and on the host", i);
+            for (size_t j = 0; j < p.n; j++)
+                if (ho[j + 1] < ho[j]) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: offsets must be non-decreasing", i);
+            if (p.n && ho[p.n] > ho[0] && !p.pk) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null key buffer", i);
+        } else if (p.n && !p.pk) {
+            return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer", i);
+        }
+        if (p.n && (!p.sig || !p.msg32)) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer", i);
+        dp.push_back(RlcDevPart{p.kind, p.pk, p.sig, p.msg32, p.kind == JJS_KIND_AGGREGATE ? p.offsets : nullptr, ho, p.n});
+    }
+    RlcSeed seed;
+    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    if (rc) return rc;
+    return run_rlc_device(ctx, ctx->dev[device_index], dp, seed, d_all_valid, (cudaStream_t)cuda_stream);
 }
 JJS_API int jjs_sign_batch(jjs_ctx* ctx, int variant, const uint8_t* sk32, const uint8_t* rnd32, const uint8_t* gen_scalar32_or_null,
                            const uint8_t* msg32, size_t n, uint8_t* pk_out, uint8_t* sig_out) {

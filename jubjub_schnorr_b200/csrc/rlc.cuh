@@ -3,6 +3,8 @@
 //
 // A batch of n valid-point items is accepted iff
 //     (sum z_i u_i) G + sum (z_i c_i) PK_i - sum z_i R_i == O        (double items: the same with z'_i, G', PK'_i, R'_i added)
+// A var-generator item contributes (z_i u_i) Gen_i to the multi-scalar multiplication instead of a G term, and an aggregate-key
+// item enters as a single item on its aggregate key (DESIGN.md section 13).
 // for secret 128-bit weights z_i drawn from a ChaCha20 stream keyed by a 32-byte seed.  The G terms are fixed-base products;
 // the rest is one multi-scalar multiplication by buckets (Pippenger): every scalar is cut into signed c-bit digits, each
 // digit becomes a (window, bucket) key with a reference to its point, the pairs are radix-sorted by key, the sorted array is
@@ -63,12 +65,13 @@ struct RlcShape {
     int end_bit;
 };
 JJS_HD int rlc_windows(int bits, int c) { return bits / c + 1; }   // the top window absorbs the last carry
-JJS_HD RlcShape rlc_shape(int variant_double, int c) {
+// variant: VAR_SINGLE (also aggregate-key items), VAR_DOUBLE or VAR_VARGEN
+JJS_HD RlcShape rlc_shape(int variant, int c) {
     RlcShape s;
     s.c = c;
     s.nw_big = rlc_windows(RLC_SCALAR_BITS, c);
     s.nw_small = rlc_windows(RLC_WEIGHT_BITS, c);
-    s.per_item = (variant_double ? 2 : 1) * (s.nw_big + s.nw_small);
+    s.per_item = variant == VAR_DOUBLE ? 2 * (s.nw_big + s.nw_small) : (variant == VAR_VARGEN ? 2 * s.nw_big + s.nw_small : s.nw_big + s.nw_small);
     s.buckets_per_window = 1u << (c - 1);
     s.sentinel = (uint32_t)s.nw_big * s.buckets_per_window;
     s.end_bit = 0;
@@ -99,11 +102,15 @@ JJS_HD void rlc_scalar_entries(uint32_t* keys, uint32_t* vals, const uint32_t* k
     }
 }
 // Everything one item contributes: weights, z c (and z' c) mod r as the PK scalars, the weights themselves as the (negated)
-// R scalars, and z u (z' u) mod r for the G (G') sums.  `valid`: the item would get status 0 from its equation alone; an item
+// R scalars, and z u (z' u) mod r for the G (G') sums.  A var-generator item has no fixed base: z u mod r is a full-size scalar
+// on its generator (slot 1) and its G scalar is zero.  `valid`: the item would get status 0 from its equation alone; an item
 // that is not valid contributes nothing (sentinel keys, zero G scalars) and the caller clears the batch's validity flag.
-// Point references: slot * m + item, the layout of the decoded-point arrays.  Entries: [PK | R | PK' | R'] windows.
-JJS_HD void rlc_item_entries(uint32_t* keys, uint32_t* vals, uint32_t* zu, uint32_t* zu2, bool is_double, bool valid, const uint32_t* c8,
+// Point references: slot * m + item, the layout of the decoded-point arrays.  Entries: [PK | R | PK' | R'] windows for single
+// and double items (aggregate items: the single layout on the aggregate key), [PK | Gen | R] for var-generator items.
+// `zu2` is written for double items only.  variant: as rlc_shape.
+JJS_HD void rlc_item_entries(uint32_t* keys, uint32_t* vals, uint32_t* zu, uint32_t* zu2, int variant, bool valid, const uint32_t* c8,
                              const uint32_t* u8, const RlcSeed& seed, uint64_t index, size_t m, size_t item, const RlcShape& s) {
+    const bool is_double = variant == VAR_DOUBLE;
     if (!valid) {
         for (int e = 0; e < s.per_item; e++) { keys[e] = s.sentinel; vals[e] = 0; }
         for (int i = 0; i < 8; i++) { zu[i] = 0; if (is_double) zu2[i] = 0; }
@@ -111,6 +118,15 @@ JJS_HD void rlc_item_entries(uint32_t* keys, uint32_t* vals, uint32_t* zu, uint3
     }
     uint32_t z[8] = {0, 0, 0, 0, 0, 0, 0, 0}, z2[8] = {0, 0, 0, 0, 0, 0, 0, 0}, zc[8];
     rlc_weights(z, z2, seed, index);
+    if (variant == VAR_VARGEN) {
+        fr_mul_short(zc, z, c8);
+        rlc_scalar_entries(keys, vals, zc, s.nw_big, s, (uint32_t)item, false);
+        fr_mul_short(zc, z, u8);
+        rlc_scalar_entries(keys + s.nw_big, vals + s.nw_big, zc, s.nw_big, s, (uint32_t)(m + item), false);
+        rlc_scalar_entries(keys + 2 * s.nw_big, vals + 2 * s.nw_big, z, s.nw_small, s, (uint32_t)(2 * m + item), true);
+        for (int i = 0; i < 8; i++) zu[i] = 0;
+        return;
+    }
     const int eqs = is_double ? 2 : 1;
     for (int eq = 0; eq < eqs; eq++) {
         const uint32_t* w = eq ? z2 : z;
@@ -261,13 +277,13 @@ JJS_HD void rlc_acc_init(RlcAcc& a) {
     for (int i = 0; i < 8; i++) { a.su[0][i] = 0; a.su[1][i] = 0; }
     a.valid = 1;
 }
-// The G terms, added to the point sum: P + su0 G (+ su1 G' for double items)
+// The G terms, added to the point sum: P + su0 G (+ su1 G' when `with_gn`; a zero su1 adds the identity)
 template <int W>
-JJS_HD void rlc_fixed_terms(ext& P, const uint32_t (*su)[8], bool is_double, const niels* fb_g, const niels* fb_gn) {
+JJS_HD void rlc_fixed_terms(ext& P, const uint32_t (*su)[8], bool with_gn, const niels* fb_g, const niels* fb_gn) {
     ext t;
     fixedbase_mul<W>(t, fb_g, su[0]);
     rlc_add(P, t);
-    if (is_double) {
+    if (with_gn) {
         fixedbase_mul<W>(t, fb_gn, su[1]);
         rlc_add(P, t);
     }

@@ -101,6 +101,12 @@ extern "C" {
     pub fn jjs_verify_all_device(ctx: *mut jjs_ctx, device_index: c_int, kind: c_int, d_pk: *const u8, d_sig: *const u8,
                                  d_msg32: *const u8, n: usize, seed32_or_null: *const u8, d_all_valid: *mut c_int,
                                  cuda_stream: *mut c_void) -> c_int;
+    // NEW all-or-nothing verification of the items of every part, any kind, by one combination (DESIGN.md section 13)
+    pub fn jjs_verify_all_mixed(ctx: *mut jjs_ctx, parts: *const jjs_part, n_parts: usize, seed32_or_null: *const u8,
+                                all_valid: *mut c_int) -> c_int;
+    pub fn jjs_verify_all_mixed_device(ctx: *mut jjs_ctx, device_index: c_int, parts: *const jjs_part, n_parts: usize,
+                                       h_offsets_or_null: *const *const u32, seed32_or_null: *const u8, d_all_valid: *mut c_int,
+                                       cuda_stream: *mut c_void) -> c_int;
     // typed inputs: JubJubExtended coordinates, 160 bytes per point (variant 0: PK, R; 1: PK, PK', R, R'; 2: PK, gen, R)
     pub fn jjs_verify_ext(ctx: *mut jjs_ctx, variant: c_int, points_ext160: *const u8, u32_: *const u8, msg32: *const u8,
                           n: usize, status: *mut u8, c32_or_null: *mut u8) -> c_int;

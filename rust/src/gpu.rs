@@ -299,6 +299,23 @@ impl GpuVerifier {
         self.check(rc, "jjs_verify_mixed");
         (unpack(&wa, na), unpack(&wb, nb), unpack(&wc, nc))
     }
+
+    /// NEW: whether every item of the three lists verifies, by one random linear combination over all of them
+    /// (jjs_verify_all_mixed, fresh secret weights): a batch with a failing item passes with probability at most 2^-128.
+    pub fn verify_all_mixed(&mut self, singles: &[(PublicKey, Signature, BlsScalar)], doubles: &[(PublicKeyDouble, SignatureDouble, BlsScalar)],
+                            var_gens: &[(PublicKeyVarGen, SignatureVarGen, BlsScalar)]) -> bool {
+        let (a, b, c) = (wire::<_, _, 32, 64>(singles), wire::<_, _, 64, 96>(doubles), wire::<_, _, 64, 64>(var_gens));
+        let part = |kind, w: &(Vec<u8>, Vec<u8>, Vec<u8>), n| ffi::jjs_part {
+            kind, pk: w.0.as_ptr(), offsets: ptr::null(), sig: w.1.as_ptr(), msg32: w.2.as_ptr(), n,
+            status: ptr::null_mut(), c32: ptr::null_mut(), aggpk32: ptr::null_mut(), accept_bitmap: ptr::null_mut(),
+        };
+        let parts = [part(ffi::JJS_KIND_SINGLE, &a, singles.len()), part(ffi::JJS_KIND_DOUBLE, &b, doubles.len()),
+                     part(ffi::JJS_KIND_VARGEN, &c, var_gens.len())];
+        let mut ok: c_int = 0;
+        let rc = unsafe { ffi::jjs_verify_all_mixed(self.ctx, parts.as_ptr(), parts.len(), ptr::null(), &mut ok) };
+        self.check(rc, "jjs_verify_all_mixed");
+        ok == 1
+    }
 }
 
 impl Drop for GpuVerifier {
