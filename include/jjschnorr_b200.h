@@ -263,6 +263,27 @@ int jjs_verify_all_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, co
 int jjs_verify_all_mixed_device(jjs_ctx* ctx, int device_index, const jjs_part* parts, size_t n_parts,
                                 const uint32_t* const* h_offsets_or_null, const uint8_t* seed32_or_null,
                                 int* d_all_valid, void* cuda_stream);
+/* Per-item verification of every item of every part (jjs_part as for jjs_verify_mixed, any of the four kinds, output fields
+ * as there: status / c32 / aggpk32 / accept_bitmap, status and accept_bitmap not both NULL).  The outputs are what
+ * jjs_verify_mixed writes for the same parts, except that an item whose verification equation fails is reported JJS_OK (and
+ * its accept bit set) with probability at most 2^-128.  An item whose equation holds is never misreported, and decoding and
+ * point-validity results are exact.  Every item that passes decoding and validity enters a random linear combination of its
+ * GROUP: at most 2^16 consecutive items of one pass (DESIGN.md section 14).  Only the items of groups whose combination fails
+ * are then verified one by one.  A batch in which few items fail therefore costs about one whole-batch call.  A batch in which
+ * most groups hold a failing item costs more than jjs_verify_mixed.
+ * *fallback_items_or_null receives the number of items verified one by one (0 for an all-valid batch).
+ * Seed: as jjs_verify_all (NULL in production).  Host buffers, parts sharded over the devices as jjs_verify_mixed shards them.
+ * JJS_ERR_ARGUMENT for an unknown kind, an aggregate part without offsets, a part with neither status nor accept_bitmap, or
+ * NULL parts with n_parts > 0. */
+int jjs_verify_grouped(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null,
+                       uint64_t* fallback_items_or_null);
+/* The same on device buffers of device `device_index`.  Parts and h_offsets_or_null are as for
+ * jjs_verify_all_mixed_device, and the output fields of the parts are device memory; here every non-empty part needs its
+ * status (accept_bitmap, if given, is computed from it).  *d_fallback_items_or_null (device memory) is written on cuda_stream.
+ * The call only enqueues work, with the growth exception of jjs_verify_aggregate_device. */
+int jjs_verify_grouped_device(jjs_ctx* ctx, int device_index, const jjs_part* parts, size_t n_parts,
+                              const uint32_t* const* h_offsets_or_null, const uint8_t* seed32_or_null,
+                              uint64_t* d_fallback_items_or_null, void* cuda_stream);
 
 /* Challenge hash only (hash parity hook): c = challenge_hash(..) for already-valid encodings, no curve
  * check.  variant: 0 single, 1 double, 2 var-generator.  Host buffers. */

@@ -61,6 +61,14 @@ public:
         check(jjs_verify_all_mixed(ctx_, parts, n_parts, seed32, &ok), "jjs_verify_all_mixed");
         return ok == 1;
     }
+    // NEW: per-item results of every part (jjs_part as for jjs_verify_mixed, outputs included) by one random linear combination
+    // per group of consecutive items, the per-item equations only in failing groups (jjs_verify_grouped); seed32 as for
+    // verify_all.  Returns the number of items verified one by one.
+    uint64_t verify_grouped(const jjs_part* parts, size_t n_parts, const uint8_t* seed32 = nullptr) const {
+        uint64_t fallback = 0;
+        check(jjs_verify_grouped(ctx_, parts, n_parts, seed32, &fallback), "jjs_verify_grouped");
+        return fallback;
+    }
 
 private:
     void init(int rc, const char* what) {

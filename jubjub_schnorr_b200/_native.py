@@ -21,6 +21,7 @@ EXPORTS = [
     "jjs_keyset_create", "jjs_keyset_destroy", "jjs_verify_keyed", "jjs_verify_keyed_device", "jjs_keyset_table_check",
     "jjs_init_limited", "jjs_memory_info",
     "jjs_verify_all", "jjs_verify_all_device", "jjs_verify_all_mixed", "jjs_verify_all_mixed_device",
+    "jjs_verify_grouped", "jjs_verify_grouped_device",
 ]
 
 
@@ -123,5 +124,9 @@ def lib():
     L.jjs_verify_all_mixed.restype = C.c_int
     L.jjs_verify_all_mixed_device.argtypes = [vp, C.c_int, C.POINTER(Part), sz, vp, vp, vp, vp]
     L.jjs_verify_all_mixed_device.restype = C.c_int
+    L.jjs_verify_grouped.argtypes = [vp, C.POINTER(Part), sz, vp, C.POINTER(C.c_uint64)]
+    L.jjs_verify_grouped.restype = C.c_int
+    L.jjs_verify_grouped_device.argtypes = [vp, C.c_int, C.POINTER(Part), sz, vp, vp, vp, vp]
+    L.jjs_verify_grouped_device.restype = C.c_int
     _lib = L
     return L

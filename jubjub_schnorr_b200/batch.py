@@ -152,6 +152,41 @@ class BatchVerifier:
     def verify_mixed(self, parts, want_challenge=False, want_bitmap=False):
         """Several batches of different kinds in one call (jjs_verify_mixed).  parts: iterable of (kind, pk, sig, msg) or, for
         AGGREGATE, (kind, pks, sig, msg, offsets).  Returns one dict per part: status, and c / aggpk / bitmap when asked for."""
+        arr, keep, out = self._mixed_parts(parts, want_challenge, want_bitmap)
+        self._check(self._lib.jjs_verify_mixed(self._ctx, arr, len(out)), "jjs_verify_mixed")
+        return out
+
+    def verify_grouped(self, parts, seed=None, want_challenge=False, want_bitmap=False):
+        """Per-item results as verify_mixed returns them, by one random linear combination per group of consecutive items and
+        the per-item equations only in groups whose combination fails (jjs_verify_grouped): an item whose equation fails is
+        reported valid with probability at most 2^-128.  Returns (results, fallback_items), fallback_items = the items verified
+        one by one.  seed: as for verify_all."""
+        arr, keep, out = self._mixed_parts(parts, want_challenge, want_bitmap)
+        keep_seed, sp = self._seed_ptr(seed)
+        fb = C.c_uint64(0)
+        self._check(self._lib.jjs_verify_grouped(self._ctx, arr, len(out), sp, C.byref(fb)), "jjs_verify_grouped")
+        return out, int(fb.value)
+
+    def verify_grouped_device(self, parts, d_fallback=None, seed=None, stream=None, device_index=0):
+        """jjs_verify_grouped_device on raw device pointers: parts = iterable of (kind, pk_ptr, sig_ptr, msg_ptr, n, status_ptr,
+        c_ptr_or_None, aggpk_ptr_or_None, bitmap_ptr_or_None) or, for AGGREGATE, the same followed by d_offsets_ptr and h_offsets
+        (the host copy of the offsets).  The uint64 fallback count is written to d_fallback (if given) on `stream`."""
+        structs, hosts, keep = [], [], []
+        for part in parts:
+            kind, pk, sig, msg, n, st, c, agg, bm = part[:9]
+            d_off, h_off = (part[9], np.ascontiguousarray(part[10], dtype=np.uint32)) if kind == AGGREGATE else (None, None)
+            structs.append(_native.Part(kind, pk, d_off, sig, msg, n, st, c, agg, bm))
+            hosts.append(h_off.ctypes.data if h_off is not None else None)
+            keep.append(h_off)
+        arr = (_native.Part * max(len(structs), 1))(*structs)
+        harr = (C.c_void_p * max(len(hosts), 1))(*hosts)
+        keep_seed, sp = self._seed_ptr(seed)
+        self._check(self._lib.jjs_verify_grouped_device(self._ctx, device_index, arr, len(structs), harr, sp, d_fallback, stream),
+                    "jjs_verify_grouped_device")
+
+    @staticmethod
+    def _mixed_parts(parts, want_challenge, want_bitmap):
+        """jjs_part array and output arrays of verify_mixed / verify_grouped"""
         structs, keep, out = [], [], []
         for part in parts:
             kind, pk, sig, msg = part[0], part[1], part[2], part[3]
@@ -178,9 +213,8 @@ class BatchVerifier:
                                         ptr(res.get("bitmap"))))
             keep.append((pk, sig, msg, off))
             out.append(res)
-        arr = (_native.Part * len(structs))(*structs)
-        self._check(self._lib.jjs_verify_mixed(self._ctx, arr, len(structs)), "jjs_verify_mixed")
-        return out
+        arr = (_native.Part * max(len(structs), 1))(*structs)
+        return arr, keep, out
 
     def verify_mixed_ptr(self, parts):
         """jjs_verify_mixed on raw host pointers (e.g. pinned torch tensors): parts = iterable of

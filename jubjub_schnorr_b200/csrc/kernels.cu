@@ -389,20 +389,27 @@ __global__ void __launch_bounds__(BLOCK) k_bitmap(const uint8_t* status, size_t 
 __global__ void k_rlc_init(RlcAcc* acc) {
     if (blockIdx.x == 0 && threadIdx.x == 0) rlc_acc_init(*acc);
 }
-// thread = item: validity by the reference's precedence (every point decoded and valid, scalars in range), weights from the
-// call-wide index base + item, sort entries and the G scalars
+// Whether item `item` of a pass of m enters the combination: status 0 by the reference's precedence (every point decoded and
+// valid, scalars in range) with the equation bits assumed
+__device__ __forceinline__ bool rlc_item_valid(int variant, const uint8_t* pflags, const uint8_t* iflags, size_t m, size_t item) {
+    return stage_status(variant, pflags, (uint8_t)(iflags[item] | IF_EQ0_OK | IF_EQ1_OK), m, item) == 0;
+}
+// thread = item: validity (rlc_item_valid), weights from the call-wide index base + item, sort entries of the item's group
+// (item >> gshift; a whole-batch pass has one group) and the G scalars.  acc: the whole-batch accumulator, whose validity flag an
+// invalid item clears (nullptr for a grouped pass, whose invalid items keep the status their flags give)
 __global__ void __launch_bounds__(BLOCK) k_rlc_digits(int variant, const uint8_t* pflags, const uint8_t* iflags, const uint32_t* cwords, WireField usc, size_t m,
-                                                      RlcShape s, RlcSeed seed, uint64_t base, uint32_t* keys, uint32_t* vals, uint32_t* zu, RlcAcc* acc) {
+                                                      int gshift, RlcShape s, RlcSeed seed, uint64_t base, uint32_t* keys, uint32_t* vals, uint32_t* zu,
+                                                      RlcAcc* acc) {
     const size_t item = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (item >= m) return;
-    const bool valid = stage_status(variant, pflags, (uint8_t)(iflags[item] | IF_EQ0_OK | IF_EQ1_OK), m, item) == 0;
-    if (!valid) acc->valid = 0;
+    const bool valid = rlc_item_valid(variant, pflags, iflags, m, item);
+    if (!valid && acc) acc->valid = 0;
     uint32_t u[8], c[8];
     wire_load(u, usc, item);
 #pragma unroll
     for (int i = 0; i < 8; i++) c[i] = cwords[item * 8 + i];
     rlc_item_entries(keys + item * s.per_item, vals + item * s.per_item, zu + item * 8, zu + (m + item) * 8, variant, valid, c, u, seed, base + item, m, item,
-                     s);
+                     s, (uint32_t)(item >> gshift));
 }
 __global__ void __launch_bounds__(BLOCK) k_rlc_bucket_init(ext* buckets, size_t nb) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -420,7 +427,7 @@ __global__ void __launch_bounds__(BLOCK) k_rlc_segments(const uint32_t* keys, co
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     rlc_segment(keys, RlcExtSrc{pts}, len, t, RLC_SEG, sentinel, buckets, ckeys, cpts, final_level);
 }
-// thread = slice of RLC_SLICE buckets of one window
+// thread = slice of RLC_SLICE buckets of one window (of every group's windows, nw = groups x nw_big)
 __global__ void __launch_bounds__(BLOCK) k_rlc_slices(const ext* buckets, int nw, uint32_t per_window, ext* partial) {
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t slices = per_window / RLC_SLICE;
@@ -448,16 +455,32 @@ __global__ void k_rlc_horner(const ext* W, int nw, int c, RlcAcc* acc) {
     rlc_horner(P, W, nw, c);
     rlc_add(acc->P, P);
 }
-// one block: the pass's G (and G') scalar sums into the accumulator, mod r.  Sums of up to 2^24 values below 2^252 fit in nine
-// words, so the block adds exactly and reduces once.
+// block = group of g items: the group's G (and G') scalar sums added into su[group], mod r (a whole-batch pass: one block, su =
+// the accumulator's, g >= m).  Sums of up to 2^24 values below 2^252 fit in nine words, so the block adds exactly and reduces once.
 constexpr int RLC_SUM_THREADS = 256;
-__global__ void __launch_bounds__(RLC_SUM_THREADS) k_rlc_scalars(const uint32_t* zu, size_t m, int neq, RlcAcc* acc) {
+__global__ void __launch_bounds__(RLC_SUM_THREADS) k_rlc_scalars(const uint32_t* zu, size_t m, size_t g, int neq, uint32_t (*su)[2][8]) {
     __shared__ uint32_t part[RLC_SUM_THREADS][9];
+    const size_t lo = (size_t)blockIdx.x * g, hi = lo + g < m ? lo + g : m;
     for (int eq = 0; eq < neq; eq++) {
         uint32_t s[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-        for (size_t i = threadIdx.x; i < m; i += RLC_SUM_THREADS) {
-            s[8] += add8c(s, s, zu + ((size_t)eq * m + i) * 8, 0u);
+        // One block reads a whole pass of a whole-batch call, so the loads of four values are issued before their additions.
+        const uint4* z = reinterpret_cast<const uint4*>(zu + (size_t)eq * m * 8);
+        constexpr int AHEAD = 4;
+        size_t i = lo + threadIdx.x;
+        for (; i + (AHEAD - 1) * RLC_SUM_THREADS < hi; i += AHEAD * RLC_SUM_THREADS) {
+            uint4 v[2 * AHEAD];
+#pragma unroll
+            for (int k = 0; k < AHEAD; k++) {
+                v[2 * k] = z[2 * (i + k * RLC_SUM_THREADS)];
+                v[2 * k + 1] = z[2 * (i + k * RLC_SUM_THREADS) + 1];
+            }
+#pragma unroll
+            for (int k = 0; k < AHEAD; k++) {
+                const uint32_t w[8] = {v[2 * k].x, v[2 * k].y, v[2 * k].z, v[2 * k].w, v[2 * k + 1].x, v[2 * k + 1].y, v[2 * k + 1].z, v[2 * k + 1].w};
+                s[8] += add8c(s, s, w, 0u);
+            }
         }
+        for (; i < hi; i += RLC_SUM_THREADS) s[8] += add8c(s, s, zu + ((size_t)eq * m + i) * 8, 0u);
         for (int k = 0; k < 9; k++) part[threadIdx.x][k] = s[k];
         __syncthreads();
         if (threadIdx.x == 0) {
@@ -465,10 +488,48 @@ __global__ void __launch_bounds__(RLC_SUM_THREADS) k_rlc_scalars(const uint32_t*
             uint32_t wide[16] = {0}, red[8];
             for (int k = 0; k < 9; k++) wide[k] = s[k];
             fr_reduce_wide(red, wide, 9 * 32);
-            fr_add(acc->su[eq], acc->su[eq], red);
+            fr_add(su[blockIdx.x][eq], su[blockIdx.x][eq], red);
         }
         __syncthreads();
     }
+}
+// thread = group: Horner over the group's windows, its G and G' terms added; verdict[group] = 1 iff the group's combination
+// is the identity
+template <int W>
+__global__ void __launch_bounds__(BLOCK) k_rlc_verdicts(const ext* Wsum, int nw, int c, size_t groups, const uint32_t (*su)[2][8], Tables T,
+                                                         uint8_t* verdict) {
+    const size_t grp = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (grp >= groups) return;
+    ext P;
+    rlc_horner(P, Wsum + grp * (size_t)nw, nw, c);
+    rlc_fixed_terms<W>(P, su[grp], true, T.fb_g, T.fb_gn);
+    verdict[grp] = ext_is_identity(P) ? 1 : 0;
+}
+// thread = item of a grouped pass: an item that entered a group whose combination holds gets its equation bits; one that entered
+// a failing group goes on the equation work list (the list and count of k_work_list, reset by the caller) and into *fallback.
+// Items that did not enter keep cleared equation bits: their status comes from their flags.
+__global__ void __launch_bounds__(BLOCK) k_rlc_gate(int variant, const uint8_t* pflags, const uint8_t* iflags, size_t m, int gshift, const uint8_t* verdict,
+                                                    uint8_t* eqflags, uint32_t* list, uint32_t* count, unsigned long long* fallback) {
+    const size_t item = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool redo = false;
+    if (item < m && rlc_item_valid(variant, pflags, iflags, m, item)) {
+        if (verdict[item >> gshift]) {
+            eqflags[item] = 1;
+            if (variant == VAR_DOUBLE) eqflags[m + item] = 1;
+        } else {
+            redo = true;
+        }
+    }
+    const uint32_t mask = __ballot_sync(0xffffffffu, redo);
+    if (mask == 0) return;
+    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
+    uint32_t at = 0;
+    if (lane == leader) {
+        at = atomicAdd(count, (uint32_t)__popc(mask));
+        if (fallback) atomicAdd(fallback, (unsigned long long)__popc(mask));
+    }
+    at = __shfl_sync(0xffffffffu, at, leader);
+    if (redo) list[at + __popc(mask & ((1u << lane) - 1u))] = (uint32_t)item;
 }
 struct RlcOut {
     ext P;
@@ -1370,14 +1431,16 @@ inline size_t rlc_agg_items(const DeviceState& d, const Region& R) {
     return t < d.agg_items ? t : d.agg_items;
 }
 
-// Where the buffers of a pass of m items with window width c go, in bytes from rlc_base; `total` is what it needs.
+// Where the buffers of a pass of m items in G groups with window width c go, in bytes from rlc_base; `total` is what it needs.
+// A grouped pass (jjs_verify_grouped) also keeps each group's scalar sums and verdict; a whole-batch pass (G = 1) keeps its sums
+// in the half's accumulator and has neither.
 struct RlcPlan {
     RlcShape s;
     size_t entries, n1, n2, cub_bytes;
-    size_t o_zu, o_keys[2], o_vals[2], o_cub, o_buckets, o_ck[2], o_cp[2], o_partial, o_W, total;
+    size_t o_zu, o_keys[2], o_vals[2], o_cub, o_buckets, o_ck[2], o_cp[2], o_partial, o_W, o_su, o_verdict, total;
 };
-inline int rlc_plan(RlcPlan& p, int variant, size_t m, int c) {
-    p.s = rlc_shape(variant, c);
+inline int rlc_plan(RlcPlan& p, int variant, size_t m, int c, size_t groups, bool grouped) {
+    p.s = rlc_shape(variant, c, groups);
     p.entries = m * (size_t)p.s.per_item;
     p.n1 = 2 * rlc_segments(p.entries, RLC_SEG);
     p.n2 = 2 * rlc_segments(p.n1, RLC_SEG);
@@ -1394,18 +1457,21 @@ inline int rlc_plan(RlcPlan& p, int variant, size_t m, int c) {
     p.o_ck[0] = take(4 * p.n1); p.o_cp[0] = take(sizeof(ext) * p.n1);
     p.o_ck[1] = take(4 * p.n2); p.o_cp[1] = take(sizeof(ext) * p.n2);
     p.o_partial = take(sizeof(ext) * slices);
-    p.o_W = take(sizeof(ext) * p.s.nw_big);
+    p.o_W = take(sizeof(ext) * groups * p.s.nw_big);
+    p.o_su = grouped ? take(sizeof(uint32_t) * 16 * groups) : 0;
+    p.o_verdict = grouped ? take(groups) : 0;
     p.total = o;
     return JJS_SUCCESS;
 }
 // The window width of a pass: the cheapest c whose buffers fit the region's scratch, by a count of point additions (one per
-// sort entry, about 2.3 mixed-addition equivalents per bucket for the running sums).  It follows from the point count alone.
-inline int rlc_choose(jjs_ctx* ctx, RlcPlan& best, int variant, size_t m, size_t budget) {
+// sort entry, about 2.3 mixed-addition equivalents per bucket of every group for the running sums).  It follows from the point
+// and group counts alone.
+inline int rlc_choose(jjs_ctx* ctx, RlcPlan& best, int variant, size_t m, size_t groups, bool grouped, size_t budget) {
     double best_cost = 0;
     bool found = false;
     for (int c = RLC_C_MIN; c <= RLC_C_MAX; c++) {
         RlcPlan p;
-        if (rlc_plan(p, variant, m, c)) return fail(ctx, JJS_ERR_CUDA, "radix sort: temporary storage query failed");
+        if (rlc_plan(p, variant, m, c, groups, grouped)) return fail(ctx, JJS_ERR_CUDA, "radix sort: temporary storage query failed");
         if (p.total > budget) continue;
         const double cost = (double)p.entries + 2.3 * (double)p.s.sentinel;
         if (!found || cost < best_cost) { best = p; best_cost = cost; found = true; }
@@ -1414,23 +1480,45 @@ inline int rlc_choose(jjs_ctx* ctx, RlcPlan& best, int variant, size_t m, size_t
     return JJS_SUCCESS;
 }
 
+// log2 of the items per group of a grouped pass (jjs_verify_grouped; DESIGN.md section 14 has the sweep that chose it).  0: one
+// group per pass.  A build-time define for A/B measurements only; the header promises groups of at most 2^16 items.
+#ifndef JJS_GROUP_LOG2
+#define JJS_GROUP_LOG2 12
+#endif
+static_assert(JJS_GROUP_LOG2 >= 0 && JJS_GROUP_LOG2 <= 16, "groups hold at most 2^16 items");
+constexpr int RLC_ONE_GROUP = 31;   // the group shift of a pass that is one group (passes hold fewer than 2^31 items)
+
+// The per-item outputs of a grouped pass (device pointers at the pass's first item; c and agg may be null) and the call's
+// count of items verified one by one (may be null).
+struct GroupedOut {
+    uint8_t *status, *c, *agg;
+    unsigned long long* fallback;
+};
+
 // One pass of m <= R.cap items of kind `kind` (JJS_KIND_*, device pointers), with every point subgroup-tested before it enters:
 // single, double and var-generator items decode every slot with its test, then work list and challenges; aggregate items
 // (m <= rlc_agg_items; pk = the pass's first signer key, offsets, key_lo and K as run_chunk_aggregate) run the front of the
-// aggregate path with R's test on, its aggregation tables in the pass scratch.  Then the combination of the pass is added into
-// the half's accumulator.  `base`: position of the pass's first item in the whole call.
+// aggregate path with R's test on, its aggregation tables in the pass scratch.  `base`: position of the pass's first item in
+// the whole call.
+// Whole-batch (out == nullptr): the combination of the pass is added into the half's accumulator.  Grouped: every group of
+// 2^JJS_GROUP_LOG2 consecutive items gets its own combination and verdict, the items of failing groups run the per-item equations
+// (their tables in the half's own pass scratch), and the pass's statuses are written to `out`.
 int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int kind, const uint8_t* pk, const uint32_t* offsets, uint32_t key_lo, size_t K,
-                  const uint8_t* sig, const uint8_t* msg, size_t m, uint64_t base, const RlcSeed& seed, cudaStream_t stream) {
+                  const uint8_t* sig, const uint8_t* msg, size_t m, uint64_t base, const RlcSeed& seed, cudaStream_t stream,
+                  const GroupedOut* out = nullptr) {
     const bool agg = kind == JJS_KIND_AGGREGATE;
     const int variant = agg ? VAR_SINGLE : kind, neq = variant == VAR_DOUBLE ? 2 : 1;
+    const int gshift = out && JJS_GROUP_LOG2 ? JJS_GROUP_LOG2 : RLC_ONE_GROUP;
+    const size_t g = size_t(1) << gshift, groups = (m + g - 1) >> gshift;
     RlcPlan p;
-    int rc = rlc_choose(ctx, p, variant, m, rlc_pass_bytes(R));
+    int rc = rlc_choose(ctx, p, variant, m, groups, out != nullptr, rlc_pass_bytes(R));
     if (rc) return rc;
     uint8_t* B = rlc_base(d, R);
     WireField fu;
     if (agg) {
         fu = WireField{sig, 64};
-        rc = enqueue_aggregate_front(ctx, d, R, pk, offsets, key_lo, K, sig, msg, m, nullptr, reinterpret_cast<fq*>(B), rlc_agg_items(d, R), true, stream);
+        rc = enqueue_aggregate_front(ctx, d, R, pk, offsets, key_lo, K, sig, msg, m, out ? out->agg : nullptr, reinterpret_cast<fq*>(B), rlc_agg_items(d, R),
+                                     true, stream);
     } else {
         const int slots = variant_slots(variant);
         Fields pts;
@@ -1443,10 +1531,10 @@ int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int kind, const
         rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
     }
     if (rc) return rc;
-    RlcAcc* acc = rlc_acc(d, R);
+    RlcAcc* acc = out ? nullptr : rlc_acc(d, R);
     uint32_t* zu = reinterpret_cast<uint32_t*>(B + p.o_zu);
     StageTimer t3(ctx, d.device, 3, stream);
-    k_rlc_digits<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.cwords, fu, m, p.s, seed, base,
+    k_rlc_digits<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.cwords, fu, m, gshift, p.s, seed, base,
                                                        reinterpret_cast<uint32_t*>(B + p.o_keys[0]), reinterpret_cast<uint32_t*>(B + p.o_vals[0]), zu, acc);
     cub::DoubleBuffer<uint32_t> kb(reinterpret_cast<uint32_t*>(B + p.o_keys[0]), reinterpret_cast<uint32_t*>(B + p.o_keys[1]));
     cub::DoubleBuffer<uint32_t> vb(reinterpret_cast<uint32_t*>(B + p.o_vals[0]), reinterpret_cast<uint32_t*>(B + p.o_vals[1]));
@@ -1469,14 +1557,41 @@ int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int kind, const
         ctx->launches++;
     }
     const uint32_t slices = p.s.buckets_per_window / RLC_SLICE;
+    const int nwin = (int)(groups * p.s.nw_big);   // every group's windows
     ext* partial = reinterpret_cast<ext*>(B + p.o_partial);
     ext* W = reinterpret_cast<ext*>(B + p.o_W);
-    k_rlc_slices<<<blocks_for((size_t)p.s.nw_big * slices), BLOCK, 0, stream>>>(buckets, p.s.nw_big, p.s.buckets_per_window, partial);
-    k_rlc_window_sums<<<p.s.nw_big, 32, 0, stream>>>(partial, slices, W);
-    k_rlc_horner<<<1, 1, 0, stream>>>(W, p.s.nw_big, p.s.c, acc);
-    k_rlc_scalars<<<1, RLC_SUM_THREADS, 0, stream>>>(zu, m, neq, acc);
+    k_rlc_slices<<<blocks_for((size_t)nwin * slices), BLOCK, 0, stream>>>(buckets, nwin, p.s.buckets_per_window, partial);
+    k_rlc_window_sums<<<nwin, 32, 0, stream>>>(partial, slices, W);
+    ctx->launches += 2;
+    if (!out) {
+        k_rlc_horner<<<1, 1, 0, stream>>>(W, p.s.nw_big, p.s.c, acc);
+        k_rlc_scalars<<<1, RLC_SUM_THREADS, 0, stream>>>(zu, m, g, neq, &acc->su);
+        t3.stop(stream);
+        ctx->launches += 2;
+        return JJS_SUCCESS;
+    }
+    // grouped: the verdicts are consumed into the equation bits and the work list before any equation runs, so the fallback
+    // equations may take the whole pass scratch for their tables.  Not R.tab with R.tstride: on a jjs_init context those rows
+    // span both halves' pass scratch, and the other half's pass may be running.
+    auto* su = reinterpret_cast<uint32_t(*)[2][8]>(B + p.o_su);
+    uint8_t* verdict = B + p.o_verdict;
+    JJS_CUDA(ctx, cudaMemsetAsync(su, 0, sizeof(uint32_t) * 16 * groups, stream));
+    k_rlc_scalars<<<(unsigned)groups, RLC_SUM_THREADS, 0, stream>>>(zu, m, g, neq, su);
+    (d.fb_w == FB_W_SMALL ? k_rlc_verdicts<FB_W_SMALL> : k_rlc_verdicts<FB_W>)<<<blocks_for(groups), BLOCK, 0, stream>>>(W, p.s.nw_big, p.s.c, groups, su,
+                                                                                                                      d.tables(), verdict);
+    JJS_CUDA(ctx, cudaMemsetAsync(R.rcount + 2, 0, sizeof(uint32_t), stream));
+    k_rlc_gate<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, m, gshift, verdict, R.eqflags, R.eqlist, R.rcount + 2, out->fallback);
     t3.stop(stream);
-    ctx->launches += 4;
+    ctx->launches += 3;
+    Region F = R;
+    F.tab = reinterpret_cast<fq*>(B);
+    F.tstride = R.cap;
+    rc = enqueue_equations(ctx, d, F, variant, m, fu, stream);
+    if (rc) return rc;
+    StageTimer t4(ctx, d.device, 4, stream);
+    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.eqflags, R.cwords, m, out->status, out->c);
+    t4.stop(stream);
+    ctx->launches++;
     return JJS_SUCCESS;
 }
 
@@ -1604,18 +1719,24 @@ int run_aggregate_device(jjs_ctx* ctx, DeviceState& d, const uint8_t* d_pks, con
     return JJS_SUCCESS;
 }
 
-// One part of a device-buffer whole-batch call (jjs_verify_all_device, jjs_verify_all_mixed_device): kind JJS_KIND_*,
-// device pointers; aggregate parts also carry the host copy of their offsets, which plans the passes.
+// One part of a device-buffer whole-batch or grouped call (jjs_verify_all_device, jjs_verify_all_mixed_device,
+// jjs_verify_grouped_device): kind JJS_KIND_*, device pointers; aggregate parts also carry the host copy of their offsets, which
+// plans the passes.  The per-item outputs are those of a grouped call.
 struct RlcDevPart {
     int kind;
     const uint8_t *pk, *sig, *msg;
     const uint32_t *d_offsets, *h_offsets;
     size_t n;
+    uint8_t *status = nullptr, *c = nullptr, *agg = nullptr;
+    uint32_t* bitmap = nullptr;
 };
 // The passes of every part through the sub-chunks of run_device (aggregate parts cut by agg_chunk_end), alternating between
-// the scratch halves and their accumulators, then the verdict written on `stream`.  Enqueue-only unless the aggregate key
-// scratch or the tag table has to grow, as run_aggregate_device.
-int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& parts, const RlcSeed& seed, int* all_valid, cudaStream_t stream) {
+// the scratch halves.  Whole-batch (fallback == nullptr): the passes add into the halves' accumulators, then the verdict is
+// written to *all_valid on `stream`.  Grouped (all_valid == nullptr): every pass is self-contained and writes its items'
+// outputs; *fallback (may be null when all_valid is) counts the items verified one by one.  Enqueue-only unless the aggregate
+// key scratch or the tag table has to grow, as run_aggregate_device.
+int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& parts, const RlcSeed& seed, int* all_valid, unsigned long long* fallback,
+                   cudaStream_t stream) {
     int rc = ensure_scratch(ctx, d);
     size_t n = 0, max_cnt = 0;
     bool any_agg = false;
@@ -1630,10 +1751,12 @@ int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& 
     if (!rc && any_agg) rc = ensure_agg_scratch(ctx, d, max_cnt > d.agg_keys_initial ? max_cnt : d.agg_keys_initial);
     if (rc) return rc;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
+    const bool grouped = all_valid == nullptr;
+    if (fallback) JJS_CUDA(ctx, cudaMemsetAsync(fallback, 0, sizeof(unsigned long long), stream));
     Overlap ov(ctx, d, stream, n > d.sub_chunk);
     rc = ov.begin();
     if (rc) return rc;
-    for (int h = 0; h < 2; h++) {
+    for (int h = 0; h < 2 && !grouped; h++) {
         k_rlc_init<<<1, 1, 0, ov.on ? d.sub[h] : stream>>>(rlc_acc(d, region_half(d, h)));
         ctx->launches++;
     }
@@ -1651,11 +1774,12 @@ int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& 
                 K = P.h_offsets[end] - key_lo;
             }
             const size_t m = end - off;
+            const GroupedOut go{grouped ? P.status + off : nullptr, P.c ? P.c + 32 * off : nullptr, P.agg ? P.agg + 32 * off : nullptr, fallback};
             rc = P.kind == JJS_KIND_AGGREGATE
                      ? run_chunk_rlc(ctx, d, R, P.kind, P.pk + 32 * (size_t)key_lo, P.d_offsets + off, key_lo, K, P.sig + 64 * off, P.msg + 32 * off, m,
-                                     base + off, seed, ov.next_stream())
+                                     base + off, seed, ov.next_stream(), grouped ? &go : nullptr)
                      : run_chunk_rlc(ctx, d, R, P.kind, P.pk + off * pk_size(P.kind), nullptr, 0, 0, P.sig + off * sig_size(P.kind), P.msg + off * 32, m,
-                                     base + off, seed, ov.next_stream());
+                                     base + off, seed, ov.next_stream(), grouped ? &go : nullptr);
             if (rc) return rc;
             off = end;
         }
@@ -1663,6 +1787,15 @@ int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& 
     }
     rc = ov.end();
     if (rc) return rc;
+    if (grouped) {
+        for (const RlcDevPart& P : parts) {
+            if (!P.bitmap || !P.n) continue;
+            k_bitmap<<<blocks_for(P.n), BLOCK, 0, stream>>>(P.status, P.n, P.bitmap);
+            ctx->launches++;
+        }
+        JJS_CUDA(ctx, cudaGetLastError());
+        return JJS_SUCCESS;
+    }
     (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, stream>>>(
         rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), d.tables(), nullptr, all_valid);
     ctx->launches++;
@@ -1676,17 +1809,23 @@ int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& 
 // loaded device), and every device is driven by its own host thread: copies in on the copy stream, pipeline slices alternating
 // between the two compute streams, results copied out at the end, one synchronisation.  A single host thread would serialise
 // the devices whenever the caller's memory is pageable (cudaMemcpyAsync from pageable memory returns only after staging).
-enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2, PART_KEYED = 3, PART_ALL = 4 };
-// whole-batch verification: the devices' partial points and validity flags, summed on the host as the devices finish
+enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2, PART_KEYED = 3, PART_ALL = 4, PART_GROUPED = 5 };
+// whole-batch verification: the devices' partial points and validity flags, summed on the host as the devices finish;
+// grouped verification: the items the devices verified one by one
 struct RlcSink {
     std::mutex mu;
     ext P;
     bool valid = true;
+    uint64_t fallback = 0;
     RlcSink() { ext_identity(P); }
     void add(const RlcOut& o) {
         std::lock_guard<std::mutex> lock(mu);
         rlc_add(P, o.P);
         valid = valid && o.valid;
+    }
+    void add_fallback(uint64_t items) {
+        std::lock_guard<std::mutex> lock(mu);
+        fallback += items;
     }
 };
 struct HostPart {
@@ -1698,11 +1837,12 @@ struct HostPart {
     uint32_t* bitmap;
     bool challenge_only;
     const KeySet* keys = nullptr;     // keyed only
-    const RlcSeed* seed = nullptr;    // whole-batch only (variant: the JJS_KIND_* of the part): the weights' seed, where the devices'
-    RlcSink* sink = nullptr;          // results go (one sink per call) and the position of the part's first item in the call
-    uint64_t base = 0;
+    const RlcSeed* seed = nullptr;    // whole-batch and grouped only (variant: the JJS_KIND_* of the part): the weights' seed, where
+    RlcSink* sink = nullptr;          // the devices' results go (one sink per call) and the position of the part's first item in the
+    uint64_t base = 0;                // call
 };
-inline bool part_aggregate(const HostPart& p) { return p.mode == PART_AGGREGATE || (p.mode == PART_ALL && p.variant == JJS_KIND_AGGREGATE); }
+inline bool part_rlc(const HostPart& p) { return p.mode == PART_ALL || p.mode == PART_GROUPED; }
+inline bool part_aggregate(const HostPart& p) { return p.mode == PART_AGGREGATE || (part_rlc(p) && p.variant == JJS_KIND_AGGREGATE); }
 struct Shard {
     size_t lo, hi;
 };
@@ -1806,8 +1946,15 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         rc = ensure_tags(ctx, d, 2 + 2 * max_cnt);
         if (rc) return rc;
     }
+    int p_grp = -1;                     // the first grouped part with items here, if any: its sink gets the device's fallback count,
+    for (size_t p = 0; p < parts.size() && p_grp < 0; p++)   // which is staged after the parts
+        if (parts[p].mode == PART_GROUPED && shards[p][k].hi > shards[p][k].lo) p_grp = (int)p;
+    const size_t o_fb = total;
+    if (p_grp >= 0) total += 256;
     rc = ensure_stage(ctx, d, total);
     if (rc) return rc;
+    unsigned long long* d_fb = p_grp >= 0 ? reinterpret_cast<unsigned long long*>(d.stage + o_fb) : nullptr;
+    if (d_fb) JJS_CUDA(ctx, cudaMemsetAsync(d_fb, 0, sizeof(unsigned long long), d.copy_stream));   // before every slice's copies
     const bool serial = ctx->profile;   // stage timers must not overlap
     int p_all = -1;                     // the first whole-batch part with items here, if any: all of them add into the accumulators of
     for (size_t p = 0; p < parts.size() && p_all < 0; p++)   // both halves, which start out empty
@@ -1842,7 +1989,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
             Region R = region_half(d, j);
             if (part_aggregate(P)) {
                 const uint32_t* ho = P.offsets + lo;   // host offsets of this shard
-                const size_t most = P.mode == PART_ALL ? rlc_agg_items(d, R) : R.acap;
+                const size_t most = part_rlc(P) ? rlc_agg_items(d, R) : R.acap;
                 size_t end = agg_chunk_end(ho, off, m, want < most ? want : most, d.agg[0].cap_keys);
                 cnt = end - off;
                 const uint32_t key0 = ho[0], key_lo = ho[off];
@@ -1852,9 +1999,10 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
                 JJS_CUDA(ctx, cudaMemcpyAsync(S.msg + 32 * off, P.msg + 32 * (lo + off), 32 * cnt, cudaMemcpyHostToDevice, d.copy_stream));
                 JJS_CUDA(ctx, cudaEventRecord(d.copied, d.copy_stream));
                 JJS_CUDA(ctx, cudaStreamWaitEvent(cs, d.copied, 0));
-                if (P.mode == PART_ALL)
+                const GroupedOut go{S.status + off, want_c ? S.c + 32 * off : nullptr, P.agg_out ? S.agg + 32 * off : nullptr, d_fb};
+                if (part_rlc(P))
                     rc = run_chunk_rlc(ctx, d, R, JJS_KIND_AGGREGATE, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off,
-                                       S.msg + 32 * off, cnt, P.base + lo + off, *P.seed, cs);
+                                       S.msg + 32 * off, cnt, P.base + lo + off, *P.seed, cs, P.mode == PART_GROUPED ? &go : nullptr);
                 else
                     rc = run_chunk_aggregate(ctx, d, R, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off, S.msg + 32 * off,
                                              cnt, S.status + off, want_c ? S.c + 32 * off : nullptr, P.agg_out ? S.agg + 32 * off : nullptr, cs);
@@ -1867,9 +2015,11 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
                 if (P.mode == PART_TYPED)
                     rc = run_chunk_ext(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * 32, S.msg + off * 32, cnt, S.status + off,
                                        want_c ? S.c + off * 32 : nullptr, cs);
-                else if (P.mode == PART_ALL)
+                else if (part_rlc(P)) {
+                    const GroupedOut go{S.status + off, want_c ? S.c + off * 32 : nullptr, nullptr, d_fb};
                     rc = run_chunk_rlc(ctx, d, R, P.variant, S.pk + off * pks, nullptr, 0, 0, S.sig + off * sgs, S.msg + off * 32, cnt, P.base + lo + off,
-                                       *P.seed, cs);
+                                       *P.seed, cs, P.mode == PART_GROUPED ? &go : nullptr);
+                }
                 else if (P.mode == PART_KEYED)
                     rc = run_chunk_keyed(ctx, d, R, *P.keys, P.keys->dev[k], reinterpret_cast<const uint32_t*>(S.pk + off * pks), S.sig + off * sgs,
                                          S.msg + off * 32, cnt, S.status + off, want_c ? S.c + off * 32 : nullptr, cs);
@@ -1908,9 +2058,12 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         ctx->launches++;
         JJS_CUDA(ctx, cudaMemcpyAsync(&out, d_out, sizeof(RlcOut), cudaMemcpyDeviceToHost, d.stream));
     }
+    unsigned long long fb = 0;
+    if (d_fb) JJS_CUDA(ctx, cudaMemcpyAsync(&fb, d_fb, sizeof(fb), cudaMemcpyDeviceToHost, d.stream));
     JJS_CUDA(ctx, cudaGetLastError());
     JJS_CUDA(ctx, cudaStreamSynchronize(d.stream));
     if (p_all >= 0) parts[p_all].sink->add(out);
+    if (p_grp >= 0) parts[p_grp].sink->add_fallback(fb);
     return JJS_SUCCESS;
 }
 
@@ -1939,10 +2092,13 @@ size_t window_end(const HostPart& P, size_t lo, size_t hi, size_t budget) {
 int device_job_windows(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const std::vector<std::vector<Shard>>& shards) {
     DeviceState& d = ctx->dev[k];
     std::vector<std::vector<Shard>> win(parts.size(), std::vector<Shard>(ctx->dev.size(), Shard{0, 0}));
+    bool grouped = false;   // device_job stages a grouped call's fallback count after the parts
+    for (const HostPart& P : parts) grouped = grouped || P.mode == PART_GROUPED;
+    const size_t budget = d.stage_bytes - (grouped ? 256 : 0);
     for (size_t p = 0; p < parts.size(); p++) {
         const size_t hi = shards[p][k].hi;
         for (size_t off = shards[p][k].lo; off < hi;) {
-            const size_t end = window_end(parts[p], off, hi, d.stage_bytes);
+            const size_t end = window_end(parts[p], off, hi, budget);
             win[p][k] = Shard{off, end};
             int rc = device_job(ctx, k, parts, win);
             if (rc) return rc;
@@ -1967,9 +2123,10 @@ int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& part
 int validate_part(jjs_ctx* ctx, const HostPart& P) {
     if (P.mode == PART_WIRE || P.mode == PART_TYPED || P.mode == PART_KEYED) {
         if (P.variant < 0 || P.variant > 2) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
-    } else if (P.mode == PART_ALL) {
+    } else if (part_rlc(P)) {
         if (P.variant < JJS_KIND_SINGLE || P.variant > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "bad kind");
         if (P.variant == JJS_KIND_AGGREGATE && !P.offsets) return fail(ctx, JJS_ERR_ARGUMENT, "an aggregate part needs its offsets");
+        if (P.mode == PART_GROUPED && !P.status && !P.bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "a part needs a status or a bitmap output");
         if (P.n && (!P.sig || !P.msg)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
         if (P.variant != JJS_KIND_AGGREGATE) return P.n && !P.pk ? fail(ctx, JJS_ERR_ARGUMENT, "null buffer") : JJS_SUCCESS;
     } else if (P.mode != PART_AGGREGATE) {
@@ -2763,7 +2920,7 @@ JJS_API int jjs_verify_all_device(jjs_ctx* ctx, int device_index, int kind, cons
     rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
     return run_rlc_device(ctx, ctx->dev[device_index], {RlcDevPart{kind, d_pk, d_sig, d_msg32, nullptr, nullptr, n}}, seed, d_all_valid,
-                          (cudaStream_t)cuda_stream);
+                          nullptr, (cudaStream_t)cuda_stream);
 }
 JJS_API int jjs_verify_all_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null, int* all_valid) {
     JJS_ENTER(ctx);
@@ -2820,7 +2977,70 @@ JJS_API int jjs_verify_all_mixed_device(jjs_ctx* ctx, int device_index, const jj
     RlcSeed seed;
     int rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
-    return run_rlc_device(ctx, ctx->dev[device_index], dp, seed, d_all_valid, (cudaStream_t)cuda_stream);
+    return run_rlc_device(ctx, ctx->dev[device_index], dp, seed, d_all_valid, nullptr, (cudaStream_t)cuda_stream);
+}
+JJS_API int jjs_verify_grouped(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null, uint64_t* fallback_items_or_null) {
+    JJS_ENTER(ctx);
+    if (n_parts && !parts) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    if (fallback_items_or_null) *fallback_items_or_null = 0;
+    RlcSeed seed;
+    RlcSink sink;
+    std::vector<HostPart> hp;
+    hp.reserve(n_parts);
+    uint64_t base = 0;
+    for (size_t i = 0; i < n_parts; i++) {
+        const jjs_part& p = parts[i];
+        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
+        HostPart P = p.kind == JJS_KIND_AGGREGATE ? aggregate_part(p.pk, p.offsets, p.sig, p.msg32, p.n, p.status, p.c32, p.aggpk32, p.accept_bitmap)
+                                                  : wire_part(p.kind, p.pk, p.sig, p.msg32, p.n, p.status, p.c32, p.accept_bitmap);
+        P.mode = PART_GROUPED;
+        P.variant = p.kind;
+        P.seed = &seed;
+        P.sink = &sink;
+        P.base = base;
+        base += p.n;
+        hp.push_back(P);
+    }
+    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    if (!rc) rc = run_parts(ctx, hp);
+    if (rc) return rc;
+    if (fallback_items_or_null) *fallback_items_or_null = sink.fallback;
+    return JJS_SUCCESS;
+}
+JJS_API int jjs_verify_grouped_device(jjs_ctx* ctx, int device_index, const jjs_part* parts, size_t n_parts, const uint32_t* const* h_offsets_or_null,
+                                      const uint8_t* seed32_or_null, uint64_t* d_fallback_items_or_null, void* cuda_stream) {
+    JJS_ENTER(ctx);
+    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
+    if (n_parts && !parts) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    std::vector<RlcDevPart> dp;
+    dp.reserve(n_parts);
+    for (size_t i = 0; i < n_parts; i++) {
+        const jjs_part& p = parts[i];
+        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
+        if (!p.status && !p.accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: a part needs a status or a bitmap output", i);
+        const uint32_t* ho = nullptr;
+        if (p.kind == JJS_KIND_AGGREGATE) {
+            ho = h_offsets_or_null ? h_offsets_or_null[i] : nullptr;
+            if (!p.offsets || !ho) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: an aggregate part needs its offsets on the device and on the host", i);
+            for (size_t j = 0; j < p.n; j++)
+                if (ho[j + 1] < ho[j]) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: offsets must be non-decreasing", i);
+            if (p.n && ho[p.n] > ho[0] && !p.pk) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null key buffer", i);
+        } else if (p.n && !p.pk) {
+            return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer", i);
+        }
+        if (p.n && (!p.sig || !p.msg32 || !p.status)) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer (the device entry needs a status buffer)", i);
+        RlcDevPart P{p.kind, p.pk, p.sig, p.msg32, p.kind == JJS_KIND_AGGREGATE ? p.offsets : nullptr, ho, p.n};
+        P.status = p.status;
+        P.c = p.c32;
+        P.agg = p.kind == JJS_KIND_AGGREGATE ? p.aggpk32 : nullptr;
+        P.bitmap = p.accept_bitmap;
+        dp.push_back(P);
+    }
+    RlcSeed seed;
+    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    if (rc) return rc;
+    return run_rlc_device(ctx, ctx->dev[device_index], dp, seed, nullptr, reinterpret_cast<unsigned long long*>(d_fallback_items_or_null),
+                          (cudaStream_t)cuda_stream);
 }
 JJS_API int jjs_sign_batch(jjs_ctx* ctx, int variant, const uint8_t* sk32, const uint8_t* rnd32, const uint8_t* gen_scalar32_or_null,
                            const uint8_t* msg32, size_t n, uint8_t* pk_out, uint8_t* sig_out) {

@@ -57,6 +57,9 @@ JJS_HD void rlc_weights(uint32_t* z, uint32_t* z2, const RlcSeed& seed, uint64_t
 // Shape of the combination of one pass: window width c, windows of a full-size scalar (z c mod r < 2^252) and of a weight
 // (< 2^128), sort entries per item, the key of an empty entry (zero digit, or an item that is not valid) and the key bits.
 // Digits are signed, d in (-2^(c-1), 2^(c-1)]; key = window * 2^(c-1) + |d| - 1, so every key below `sentinel` is a bucket.
+// Grouped verification (jjs_verify_grouped, DESIGN.md section 14) cuts a pass into G groups of consecutive items, each with a
+// combination of its own: key = (group * nw_big + window) * 2^(c-1) + |d| - 1, so a group's buckets are nw_big more "windows"
+// and sorted runs never mix groups.  G = 1 is the whole-batch combination, key for key.
 constexpr int RLC_SCALAR_BITS = 252, RLC_WEIGHT_BITS = 128;
 constexpr int RLC_C_MIN = 6, RLC_C_MAX = 16;   // at least one 32-bucket slice per window (kernels.cu, RLC_SLICE)
 struct RlcShape {
@@ -66,14 +69,14 @@ struct RlcShape {
 };
 JJS_HD int rlc_windows(int bits, int c) { return bits / c + 1; }   // the top window absorbs the last carry
 // variant: VAR_SINGLE (also aggregate-key items), VAR_DOUBLE or VAR_VARGEN
-JJS_HD RlcShape rlc_shape(int variant, int c) {
+JJS_HD RlcShape rlc_shape(int variant, int c, size_t groups = 1) {
     RlcShape s;
     s.c = c;
     s.nw_big = rlc_windows(RLC_SCALAR_BITS, c);
     s.nw_small = rlc_windows(RLC_WEIGHT_BITS, c);
     s.per_item = variant == VAR_DOUBLE ? 2 * (s.nw_big + s.nw_small) : (variant == VAR_VARGEN ? 2 * s.nw_big + s.nw_small : s.nw_big + s.nw_small);
     s.buckets_per_window = 1u << (c - 1);
-    s.sentinel = (uint32_t)s.nw_big * s.buckets_per_window;
+    s.sentinel = (uint32_t)(groups * (size_t)s.nw_big) * s.buckets_per_window;
     s.end_bit = 0;
     while ((1u << s.end_bit) <= s.sentinel) s.end_bit++;
     return s;
@@ -87,8 +90,9 @@ JJS_HD uint32_t rlc_bits(const uint32_t* k, int pos, int c) {
     return x & ((1u << c) - 1u);
 }
 // The entries of one scalar k (nw windows) on point `ref` (index into the point arrays), negated if `neg`: key / value pairs
-// keys[w], vals[w] for w < nw; value = ref * 2 + sign.
-JJS_HD void rlc_scalar_entries(uint32_t* keys, uint32_t* vals, const uint32_t* k, int nw, const RlcShape& s, uint32_t ref, bool neg) {
+// keys[w], vals[w] for w < nw; value = ref * 2 + sign.  key0: the first key of the item's group.
+JJS_HD void rlc_scalar_entries(uint32_t* keys, uint32_t* vals, const uint32_t* k, int nw, const RlcShape& s, uint32_t ref, bool neg,
+                               uint32_t key0 = 0) {
     const uint32_t half = s.buckets_per_window, full = half * 2;
     uint32_t carry = 0;
 #pragma unroll 1
@@ -97,7 +101,7 @@ JJS_HD void rlc_scalar_entries(uint32_t* keys, uint32_t* vals, const uint32_t* k
         bool dneg = x > half;
         uint32_t mag = dneg ? full - x : x;
         carry = dneg ? 1u : 0u;
-        keys[w] = mag ? (uint32_t)w * half + mag - 1 : s.sentinel;
+        keys[w] = mag ? key0 + (uint32_t)w * half + mag - 1 : s.sentinel;
         vals[w] = ref * 2u + ((dneg != neg) ? 1u : 0u);
     }
 }
@@ -107,9 +111,10 @@ JJS_HD void rlc_scalar_entries(uint32_t* keys, uint32_t* vals, const uint32_t* k
 // that is not valid contributes nothing (sentinel keys, zero G scalars) and the caller clears the batch's validity flag.
 // Point references: slot * m + item, the layout of the decoded-point arrays.  Entries: [PK | R | PK' | R'] windows for single
 // and double items (aggregate items: the single layout on the aggregate key), [PK | Gen | R] for var-generator items.
-// `zu2` is written for double items only.  variant: as rlc_shape.
+// `zu2` is written for double items only.  variant: as rlc_shape.  group: the item's group (0 for a whole-batch pass).
 JJS_HD void rlc_item_entries(uint32_t* keys, uint32_t* vals, uint32_t* zu, uint32_t* zu2, int variant, bool valid, const uint32_t* c8,
-                             const uint32_t* u8, const RlcSeed& seed, uint64_t index, size_t m, size_t item, const RlcShape& s) {
+                             const uint32_t* u8, const RlcSeed& seed, uint64_t index, size_t m, size_t item, const RlcShape& s,
+                             uint32_t group = 0) {
     const bool is_double = variant == VAR_DOUBLE;
     if (!valid) {
         for (int e = 0; e < s.per_item; e++) { keys[e] = s.sentinel; vals[e] = 0; }
@@ -118,12 +123,13 @@ JJS_HD void rlc_item_entries(uint32_t* keys, uint32_t* vals, uint32_t* zu, uint3
     }
     uint32_t z[8] = {0, 0, 0, 0, 0, 0, 0, 0}, z2[8] = {0, 0, 0, 0, 0, 0, 0, 0}, zc[8];
     rlc_weights(z, z2, seed, index);
+    const uint32_t key0 = group * (uint32_t)s.nw_big * s.buckets_per_window;
     if (variant == VAR_VARGEN) {
         fr_mul_short(zc, z, c8);
-        rlc_scalar_entries(keys, vals, zc, s.nw_big, s, (uint32_t)item, false);
+        rlc_scalar_entries(keys, vals, zc, s.nw_big, s, (uint32_t)item, false, key0);
         fr_mul_short(zc, z, u8);
-        rlc_scalar_entries(keys + s.nw_big, vals + s.nw_big, zc, s.nw_big, s, (uint32_t)(m + item), false);
-        rlc_scalar_entries(keys + 2 * s.nw_big, vals + 2 * s.nw_big, z, s.nw_small, s, (uint32_t)(2 * m + item), true);
+        rlc_scalar_entries(keys + s.nw_big, vals + s.nw_big, zc, s.nw_big, s, (uint32_t)(m + item), false, key0);
+        rlc_scalar_entries(keys + 2 * s.nw_big, vals + 2 * s.nw_big, z, s.nw_small, s, (uint32_t)(2 * m + item), true, key0);
         for (int i = 0; i < 8; i++) zu[i] = 0;
         return;
     }
@@ -134,8 +140,8 @@ JJS_HD void rlc_item_entries(uint32_t* keys, uint32_t* vals, uint32_t* zu, uint3
         fr_mul_short(zc, w, c8);
         uint32_t* k = keys + eq * (s.nw_big + s.nw_small);
         uint32_t* v = vals + eq * (s.nw_big + s.nw_small);
-        rlc_scalar_entries(k, v, zc, s.nw_big, s, pk_ref, false);
-        rlc_scalar_entries(k + s.nw_big, v + s.nw_big, w, s.nw_small, s, r_ref, true);
+        rlc_scalar_entries(k, v, zc, s.nw_big, s, pk_ref, false, key0);
+        rlc_scalar_entries(k + s.nw_big, v + s.nw_big, w, s.nw_small, s, r_ref, true, key0);
         fr_mul_short(eq ? zu2 : zu, w, u8);
     }
 }

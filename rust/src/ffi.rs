@@ -107,6 +107,11 @@ extern "C" {
     pub fn jjs_verify_all_mixed_device(ctx: *mut jjs_ctx, device_index: c_int, parts: *const jjs_part, n_parts: usize,
                                        h_offsets_or_null: *const *const u32, seed32_or_null: *const u8, d_all_valid: *mut c_int,
                                        cuda_stream: *mut c_void) -> c_int;
+    pub fn jjs_verify_grouped(ctx: *mut jjs_ctx, parts: *const jjs_part, n_parts: usize, seed32_or_null: *const u8,
+                              fallback_items_or_null: *mut u64) -> c_int;
+    pub fn jjs_verify_grouped_device(ctx: *mut jjs_ctx, device_index: c_int, parts: *const jjs_part, n_parts: usize,
+                                     h_offsets_or_null: *const *const u32, seed32_or_null: *const u8,
+                                     d_fallback_items_or_null: *mut u64, cuda_stream: *mut c_void) -> c_int;
     // typed inputs: JubJubExtended coordinates, 160 bytes per point (variant 0: PK, R; 1: PK, PK', R, R'; 2: PK, gen, R)
     pub fn jjs_verify_ext(ctx: *mut jjs_ctx, variant: c_int, points_ext160: *const u8, u32_: *const u8, msg32: *const u8,
                           n: usize, status: *mut u8, c32_or_null: *mut u8) -> c_int;

@@ -316,6 +316,25 @@ impl GpuVerifier {
         self.check(rc, "jjs_verify_all_mixed");
         ok == 1
     }
+
+    /// NEW: verify_mixed's per-item answers by one random linear combination per group of consecutive items, the per-item
+    /// equations running only in groups whose combination fails (jjs_verify_grouped, fresh secret weights): a failing item is
+    /// reported valid with probability at most 2^-128.
+    pub fn verify_grouped(&mut self, singles: &[(PublicKey, Signature, BlsScalar)], doubles: &[(PublicKeyDouble, SignatureDouble, BlsScalar)],
+                          var_gens: &[(PublicKeyVarGen, SignatureVarGen, BlsScalar)]) -> (Vec<bool>, Vec<bool>, Vec<bool>) {
+        let (a, b, c) = (wire::<_, _, 32, 64>(singles), wire::<_, _, 64, 96>(doubles), wire::<_, _, 64, 64>(var_gens));
+        let (na, nb, nc) = (singles.len(), doubles.len(), var_gens.len());
+        let (mut wa, mut wb, mut wc) = (vec![0u32; (na + 31) / 32], vec![0u32; (nb + 31) / 32], vec![0u32; (nc + 31) / 32]);
+        let part = |kind, w: &(Vec<u8>, Vec<u8>, Vec<u8>), n, words: &mut Vec<u32>| ffi::jjs_part {
+            kind, pk: w.0.as_ptr(), offsets: ptr::null(), sig: w.1.as_ptr(), msg32: w.2.as_ptr(), n,
+            status: ptr::null_mut(), c32: ptr::null_mut(), aggpk32: ptr::null_mut(), accept_bitmap: words.as_mut_ptr(),
+        };
+        let parts = [part(ffi::JJS_KIND_SINGLE, &a, na, &mut wa), part(ffi::JJS_KIND_DOUBLE, &b, nb, &mut wb),
+                     part(ffi::JJS_KIND_VARGEN, &c, nc, &mut wc)];
+        let rc = unsafe { ffi::jjs_verify_grouped(self.ctx, parts.as_ptr(), parts.len(), ptr::null(), ptr::null_mut()) };
+        self.check(rc, "jjs_verify_grouped");
+        (unpack(&wa, na), unpack(&wb, nb), unpack(&wc, nc))
+    }
 }
 
 impl Drop for GpuVerifier {
