@@ -1282,6 +1282,18 @@ int enqueue_equations(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant
     return JJS_SUCCESS;
 }
 
+// The tail of a chunk of m items: enqueue_equations, then the statuses (and challenges, c_out may be null).
+int finish_chunk(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, size_t m, const WireField& fu, uint8_t* status, uint8_t* c_out,
+                 cudaStream_t stream) {
+    int rc = enqueue_equations(ctx, d, R, variant, m, fu, stream);
+    if (rc) return rc;
+    StageTimer t4(ctx, d.device, 4, stream);
+    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.eqflags, R.cwords, m, status, c_out);
+    t4.stop(stream);
+    ctx->launches++;
+    return JJS_SUCCESS;
+}
+
 // The whole pipeline for one chunk of m <= R.cap items (device pointers) on `stream`.
 int run_chunk(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t m,
               uint8_t* status, uint8_t* c_out, cudaStream_t stream, bool challenge_only) {
@@ -1300,13 +1312,7 @@ int run_chunk(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, const 
         JJS_CUDA(ctx, cudaMemcpyAsync(c_out, R.cwords, 32 * m, cudaMemcpyDeviceToDevice, stream));
         return JJS_SUCCESS;
     }
-    rc = enqueue_equations(ctx, d, R, variant, m, fu, stream);
-    if (rc) return rc;
-    StageTimer t4(ctx, d.device, 4, stream);
-    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.eqflags, R.cwords, m, status, c_out);
-    t4.stop(stream);
-    ctx->launches++;
-    return JJS_SUCCESS;
+    return finish_chunk(ctx, d, R, variant, m, fu, status, c_out, stream);
 }
 
 // Typed inputs: the same pipeline behind k_decode_ext (points as JubJubExtended coordinates, 160 bytes each, item-major).
@@ -1319,11 +1325,7 @@ int run_chunk_ext(jjs_ctx* ctx, DeviceState& d, const Region& R, int variant, co
     t0.stop(stream);
     ctx->launches++;
     int rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
-    if (!rc) rc = enqueue_equations(ctx, d, R, variant, m, fu, stream);
-    if (rc) return rc;
-    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.eqflags, R.cwords, m, status, c_out);
-    ctx->launches++;
-    return JJS_SUCCESS;
+    return rc ? rc : finish_chunk(ctx, d, R, variant, m, fu, status, c_out, stream);
 }
 
 // The front of an aggregate-key chunk of m items with K <= cap_keys signer keys, on `stream`: signer keys and R decoded, the
@@ -1363,13 +1365,7 @@ int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uin
                         const uint8_t* d_sig, const uint8_t* d_msg, size_t m, uint8_t* d_status, uint8_t* d_c, uint8_t* d_agg, cudaStream_t stream) {
     WireField fu{d_sig, 64};
     int rc = enqueue_aggregate_front(ctx, d, R, d_keys, d_offsets, key_lo, K, d_sig, d_msg, m, d_agg, R.tab, R.astride, false, stream);
-    if (!rc) rc = enqueue_equations(ctx, d, R, VAR_SINGLE, m, fu, stream);
-    if (rc) return rc;
-    StageTimer t4(ctx, d.device, 4, stream);
-    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(VAR_SINGLE, R.pflags, R.iflags, R.eqflags, R.cwords, m, d_status, d_c);
-    t4.stop(stream);
-    ctx->launches++;
-    return JJS_SUCCESS;
+    return rc ? rc : finish_chunk(ctx, d, R, VAR_SINGLE, m, fu, d_status, d_c, stream);
 }
 
 // The pipeline for one chunk of m <= R.cap items under a registered key set (device pointers, key_index: the chunk's first
@@ -1586,13 +1582,7 @@ int run_chunk_rlc(jjs_ctx* ctx, DeviceState& d, const Region& R, int kind, const
     Region F = R;
     F.tab = reinterpret_cast<fq*>(B);
     F.tstride = R.cap;
-    rc = enqueue_equations(ctx, d, F, variant, m, fu, stream);
-    if (rc) return rc;
-    StageTimer t4(ctx, d.device, 4, stream);
-    k_finalize<<<blocks_for(m), BLOCK, 0, stream>>>(variant, R.pflags, R.iflags, R.eqflags, R.cwords, m, out->status, out->c);
-    t4.stop(stream);
-    ctx->launches++;
-    return JJS_SUCCESS;
+    return finish_chunk(ctx, d, F, variant, m, fu, out->status, out->c, stream);
 }
 
 // Sub-chunks of an overlapped batch alternate between the two internal streams and scratch halves: kernels of neighbouring
@@ -1613,7 +1603,6 @@ struct Overlap {
         return JJS_SUCCESS;
     }
     cudaStream_t next_stream() const { return on ? d.sub[i & 1] : stream; }
-    Region next_region() const { return on ? region_half(d, i) : region_whole(d); }
     void advance() { i++; }
     int end() {
         if (!on) return JJS_SUCCESS;
@@ -1624,51 +1613,6 @@ struct Overlap {
         return JJS_SUCCESS;
     }
 };
-
-// Enqueue the whole pipeline for n items (device pointers); the work is ordered after what `stream` holds now and
-// `stream` waits for it.
-int run_device(jjs_ctx* ctx, DeviceState& d, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t n,
-               uint8_t* status, uint8_t* c_out, cudaStream_t stream, bool challenge_only = false) {
-    int rc = ensure_scratch(ctx, d);
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > d.sub_chunk);
-    rc = ov.begin();
-    if (rc) return rc;
-    const size_t step = ov.on ? d.sub_chunk : d.chunk_items;
-    for (size_t off = 0; off < n; off += step, ov.advance()) {
-        size_t m = n - off < step ? n - off : step;
-        rc = run_chunk(ctx, d, ov.next_region(), variant, pk + off * pk_size(variant), sig + off * sig_size(variant), msg + off * 32, m,
-                       status ? status + off : nullptr, c_out ? c_out + off * 32 : nullptr, ov.next_stream(), challenge_only);
-        if (rc) return rc;
-    }
-    rc = ov.end();
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaGetLastError());
-    return JJS_SUCCESS;
-}
-
-// run_device for items under a registered key set
-int run_keyed_device(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, const KeySetDev& kd, const uint32_t* key_index, const uint8_t* sig,
-                     const uint8_t* msg, size_t n, uint8_t* status, uint8_t* c_out, cudaStream_t stream) {
-    int rc = ensure_scratch(ctx, d);
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > d.sub_chunk);
-    rc = ov.begin();
-    if (rc) return rc;
-    const size_t step = ov.on ? d.sub_chunk : d.chunk_items;
-    for (size_t off = 0; off < n; off += step, ov.advance()) {
-        size_t m = n - off < step ? n - off : step;
-        rc = run_chunk_keyed(ctx, d, ov.next_region(), ks, kd, key_index + off, sig + off * sig_size(ks.variant), msg + off * 32, m, status + off,
-                             c_out ? c_out + off * 32 : nullptr, ov.next_stream());
-        if (rc) return rc;
-    }
-    rc = ov.end();
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaGetLastError());
-    return JJS_SUCCESS;
-}
 
 // Chunks of an aggregate-key batch: at most `max_items` items and `max_keys` signer keys each (an item with more keys than
 // that forms a chunk of its own, for which the caller grows the key scratch first).
@@ -1686,129 +1630,14 @@ inline size_t agg_max_item_keys(const uint32_t* offsets, size_t n) {
     return mx;
 }
 
-// aggregate_pk(..).verify(..) for n items whose wire data already sits on the device.  `h_offsets` is the host copy of
-// the n + 1 offsets (it plans the chunks and sizes the tag table; it is read during the call only); d_offsets the same
-// array on the device.  Enqueue-only unless a scratch has to grow (first call, or more keys / signers than ever before).
-int run_aggregate_device(jjs_ctx* ctx, DeviceState& d, const uint8_t* d_pks, const uint32_t* d_offsets, const uint32_t* h_offsets,
-                         const uint8_t* d_sig, const uint8_t* d_msg, size_t n, uint8_t* d_status, uint8_t* d_c, uint8_t* d_agg,
-                         cudaStream_t stream) {
-    int rc = ensure_scratch(ctx, d);
-    const size_t max_cnt = agg_max_item_keys(h_offsets, n);
-    if (!rc) rc = ensure_tags(ctx, d, 2 + 2 * max_cnt);
-    if (!rc) rc = ensure_agg_scratch(ctx, d, max_cnt > d.agg_keys_initial ? max_cnt : d.agg_keys_initial);
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaSetDevice(d.device));
-    Overlap ov(ctx, d, stream, n > d.sub_chunk);
-    rc = ov.begin();
-    if (rc) return rc;
-    const size_t step = ov.on ? d.sub_chunk : d.sub_items;
-    for (size_t off = 0; off < n; ov.advance()) {
-        Region R = ov.on ? ov.next_region() : region_half(d, 0);
-        size_t end = agg_chunk_end(h_offsets, off, n, step < R.acap ? step : R.acap, d.agg[0].cap_keys);
-        size_t m = end - off;
-        uint32_t key_lo = h_offsets[off];
-        size_t K = h_offsets[end] - key_lo;
-        rc = run_chunk_aggregate(ctx, d, R, d_pks + 32 * (size_t)key_lo, d_offsets + off, key_lo, K, d_sig + 64 * off, d_msg + 32 * off, m, d_status + off,
-                                 d_c ? d_c + 32 * off : nullptr, d_agg ? d_agg + 32 * off : nullptr, ov.next_stream());
-        if (rc) return rc;
-        off = end;
-    }
-    rc = ov.end();
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaGetLastError());
-    return JJS_SUCCESS;
-}
-
-// One part of a device-buffer whole-batch or grouped call (jjs_verify_all_device, jjs_verify_all_mixed_device,
-// jjs_verify_grouped_device): kind JJS_KIND_*, device pointers; aggregate parts also carry the host copy of their offsets, which
-// plans the passes.  The per-item outputs are those of a grouped call.
-struct RlcDevPart {
-    int kind;
-    const uint8_t *pk, *sig, *msg;
-    const uint32_t *d_offsets, *h_offsets;
-    size_t n;
-    uint8_t *status = nullptr, *c = nullptr, *agg = nullptr;
-    uint32_t* bitmap = nullptr;
-};
-// The passes of every part through the sub-chunks of run_device (aggregate parts cut by agg_chunk_end), alternating between
-// the scratch halves.  Whole-batch (fallback == nullptr): the passes add into the halves' accumulators, then the verdict is
-// written to *all_valid on `stream`.  Grouped (all_valid == nullptr): every pass is self-contained and writes its items'
-// outputs; *fallback (may be null when all_valid is) counts the items verified one by one.  Enqueue-only unless the aggregate
-// key scratch or the tag table has to grow, as run_aggregate_device.
-int run_rlc_device(jjs_ctx* ctx, DeviceState& d, const std::vector<RlcDevPart>& parts, const RlcSeed& seed, int* all_valid, unsigned long long* fallback,
-                   cudaStream_t stream) {
-    int rc = ensure_scratch(ctx, d);
-    size_t n = 0, max_cnt = 0;
-    bool any_agg = false;
-    for (const RlcDevPart& P : parts) {
-        n += P.n;
-        if (P.kind != JJS_KIND_AGGREGATE || !P.n) continue;
-        any_agg = true;
-        const size_t mc = agg_max_item_keys(P.h_offsets, P.n);
-        if (mc > max_cnt) max_cnt = mc;
-    }
-    if (!rc && any_agg) rc = ensure_tags(ctx, d, 2 + 2 * max_cnt);
-    if (!rc && any_agg) rc = ensure_agg_scratch(ctx, d, max_cnt > d.agg_keys_initial ? max_cnt : d.agg_keys_initial);
-    if (rc) return rc;
-    JJS_CUDA(ctx, cudaSetDevice(d.device));
-    const bool grouped = all_valid == nullptr;
-    if (fallback) JJS_CUDA(ctx, cudaMemsetAsync(fallback, 0, sizeof(unsigned long long), stream));
-    Overlap ov(ctx, d, stream, n > d.sub_chunk);
-    rc = ov.begin();
-    if (rc) return rc;
-    for (int h = 0; h < 2 && !grouped; h++) {
-        k_rlc_init<<<1, 1, 0, ov.on ? d.sub[h] : stream>>>(rlc_acc(d, region_half(d, h)));
-        ctx->launches++;
-    }
-    uint64_t base = 0;
-    for (const RlcDevPart& P : parts) {
-        for (size_t off = 0; off < P.n; ov.advance()) {
-            const Region R = region_half(d, ov.i);
-            size_t end = off + (P.n - off < d.sub_chunk ? P.n - off : d.sub_chunk);
-            uint32_t key_lo = 0;
-            size_t K = 0;
-            if (P.kind == JJS_KIND_AGGREGATE) {
-                const size_t most = rlc_agg_items(d, R);
-                end = agg_chunk_end(P.h_offsets, off, P.n, d.sub_chunk < most ? d.sub_chunk : most, d.agg[0].cap_keys);
-                key_lo = P.h_offsets[off];
-                K = P.h_offsets[end] - key_lo;
-            }
-            const size_t m = end - off;
-            const GroupedOut go{grouped ? P.status + off : nullptr, P.c ? P.c + 32 * off : nullptr, P.agg ? P.agg + 32 * off : nullptr, fallback};
-            rc = P.kind == JJS_KIND_AGGREGATE
-                     ? run_chunk_rlc(ctx, d, R, P.kind, P.pk + 32 * (size_t)key_lo, P.d_offsets + off, key_lo, K, P.sig + 64 * off, P.msg + 32 * off, m,
-                                     base + off, seed, ov.next_stream(), grouped ? &go : nullptr)
-                     : run_chunk_rlc(ctx, d, R, P.kind, P.pk + off * pk_size(P.kind), nullptr, 0, 0, P.sig + off * sig_size(P.kind), P.msg + off * 32, m,
-                                     base + off, seed, ov.next_stream(), grouped ? &go : nullptr);
-            if (rc) return rc;
-            off = end;
-        }
-        base += P.n;
-    }
-    rc = ov.end();
-    if (rc) return rc;
-    if (grouped) {
-        for (const RlcDevPart& P : parts) {
-            if (!P.bitmap || !P.n) continue;
-            k_bitmap<<<blocks_for(P.n), BLOCK, 0, stream>>>(P.status, P.n, P.bitmap);
-            ctx->launches++;
-        }
-        JJS_CUDA(ctx, cudaGetLastError());
-        return JJS_SUCCESS;
-    }
-    (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, stream>>>(
-        rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), d.tables(), nullptr, all_valid);
-    ctx->launches++;
-    JJS_CUDA(ctx, cudaGetLastError());
-    return JJS_SUCCESS;
-}
-
-// ---- host-buffer entry points ---------------------------------------------------------------------------------------------
-// A call verifies one or more PARTS (each a homogeneous batch: one of the three wire variants, aggregate-key items, or typed
-// items).  Every part is cut into contiguous shards, one per device of the context (small parts go whole to the least
-// loaded device), and every device is driven by its own host thread: copies in on the copy stream, pipeline slices alternating
-// between the two compute streams, results copied out at the end, one synchronisation.  A single host thread would serialise
-// the devices whenever the caller's memory is pageable (cudaMemcpyAsync from pageable memory returns only after staging).
+// ---- parts and passes -----------------------------------------------------------------------------------------------------
+// A call verifies one or more PARTS (each a homogeneous batch: one of the three wire variants, aggregate-key items, typed items,
+// items under a registered key set, or the whole-batch or grouped items of one kind).  A host-buffer call cuts every part into
+// shards, one per device of the context (small parts go whole to the least loaded device), and every device is driven by its
+// own host thread: copies in on the copy stream, pipeline slices alternating between the two compute streams, results copied
+// out at the end, one synchronisation.  A single host thread would serialise the devices whenever the caller's memory is
+// pageable (cudaMemcpyAsync from pageable memory returns only after staging).  A device-buffer call runs its parts on one device
+// and the caller's stream (run_device_parts).  Both cut a part into passes with pass_end and run every pass through run_pass.
 enum PartMode : int { PART_WIRE = 0, PART_AGGREGATE = 1, PART_TYPED = 2, PART_KEYED = 3, PART_ALL = 4, PART_GROUPED = 5 };
 // whole-batch verification: the devices' partial points and validity flags, summed on the host as the devices finish;
 // grouped verification: the items the devices verified one by one
@@ -1828,28 +1657,42 @@ struct RlcSink {
         fallback += items;
     }
 };
-struct HostPart {
-    int mode, variant;
-    const uint8_t *pk, *sig, *msg;    // typed: pk = points_ext160, sig = u32;  keyed: pk = the uint32 key indices
-    const uint32_t* offsets;          // aggregate only
-    size_t n;
-    uint8_t *status, *c_out, *agg_out;
-    uint32_t* bitmap;
-    bool challenge_only;
-    const KeySet* keys = nullptr;     // keyed only
-    const RlcSeed* seed = nullptr;    // whole-batch and grouped only (variant: the JJS_KIND_* of the part): the weights' seed, where
-    RlcSink* sink = nullptr;          // the devices' results go (one sink per call) and the position of the part's first item in the
-    uint64_t base = 0;                // call
+// One part of a call; its buffers are the host's (host-buffer calls) or the device's (device-buffer calls).
+struct Part {
+    int mode = PART_WIRE;
+    int variant = VAR_SINGLE;                  // wire, typed and keyed parts: VAR_*; the others: the part's JJS_KIND_*
+    const uint8_t *pk = nullptr, *sig = nullptr, *msg = nullptr;   // typed: pk = points_ext160, sig = u32;  keyed: pk = the uint32
+                                                                   // key indices;  aggregate: pk = the signer keys
+    const uint32_t* offsets = nullptr;         // aggregate only: the n + 1 offsets beside the other buffers,
+    const uint32_t* h_offsets = nullptr;       // and their host copy, which plans the passes (the same array in a host-buffer call)
+    size_t n = 0;
+    uint8_t *status = nullptr, *c_out = nullptr, *agg_out = nullptr;
+    uint32_t* bitmap = nullptr;
+    bool challenge_only = false;
+    const KeySet* keys = nullptr;              // keyed only
+    const RlcSeed* seed = nullptr;             // whole-batch and grouped only: the weights' seed, where the devices' results go (one
+    RlcSink* sink = nullptr;                   // sink per host-buffer call) and the position of the part's first item in the call
+    uint64_t base = 0;
 };
-inline bool part_rlc(const HostPart& p) { return p.mode == PART_ALL || p.mode == PART_GROUPED; }
-inline bool part_aggregate(const HostPart& p) { return p.mode == PART_AGGREGATE || (part_rlc(p) && p.variant == JJS_KIND_AGGREGATE); }
+inline bool part_rlc(const Part& p) { return p.mode == PART_ALL || p.mode == PART_GROUPED; }
+inline bool part_aggregate(const Part& p) { return p.mode == PART_AGGREGATE || (part_rlc(p) && p.variant == JJS_KIND_AGGREGATE); }
+// Bytes per item of a part's pk and sig buffers; pk of an aggregate part: per signer key.
+struct Strides {
+    size_t pk, sig;
+};
+inline Strides part_strides(const Part& p) {
+    if (part_aggregate(p)) return {32, 64};
+    if (p.mode == PART_TYPED) return {160 * (size_t)variant_slots(p.variant), 32};
+    if (p.mode == PART_KEYED) return {sizeof(uint32_t), sig_size(p.variant)};
+    return {pk_size(p.variant), sig_size(p.variant)};
+}
 struct Shard {
     size_t lo, hi;
 };
 
-inline double part_weight(const HostPart& p) {   // relative cost of one item (executed multiplies, single = 1)
+inline double part_weight(const Part& p) {   // relative cost of one item (executed multiplies, single = 1)
     if (part_aggregate(p)) {
-        double avg = p.n ? (double)(p.offsets[p.n] - p.offsets[0]) / (double)p.n : 0.0;
+        double avg = p.n ? (double)(p.h_offsets[p.n] - p.h_offsets[0]) / (double)p.n : 0.0;
         return 1.0 + 0.75 * avg;
     }
     return p.variant == VAR_DOUBLE ? 1.9 : (p.variant == VAR_VARGEN ? 1.4 : 1.0);
@@ -1858,7 +1701,7 @@ inline double part_weight(const HostPart& p) {   // relative cost of one item (e
 // shards[part][device].  Large parts are split evenly (every device then carries the same share of every kind, so the
 // devices finish together whatever the mix); parts too small to be worth splitting go whole to the least loaded device.
 constexpr size_t MIN_SPLIT_ITEMS = 8192;
-void plan_shards(const std::vector<HostPart>& parts, size_t g, std::vector<std::vector<Shard>>& shards) {
+void plan_shards(const std::vector<Part>& parts, size_t g, std::vector<std::vector<Shard>>& shards) {
     shards.assign(parts.size(), std::vector<Shard>(g, Shard{0, 0}));
     std::vector<double> load(g, 0.0);
     for (size_t p = 0; p < parts.size(); p++) {
@@ -1883,52 +1726,183 @@ void plan_shards(const std::vector<HostPart>& parts, size_t g, std::vector<std::
     }
 }
 
+// Checks part P of a host-buffer call, or of a device-buffer call (on_device), which also needs the host copy of an aggregate
+// part's offsets and a status buffer (a host-buffer call may take a bitmap instead).  `part` >= 0: the message names the part.
+int validate_part(jjs_ctx* ctx, const Part& P, bool on_device, long part = -1) {
+    const bool agg = part_aggregate(P), offsets = P.offsets && (P.h_offsets || !on_device);
+    const char* why = [&]() -> const char* {
+        if (P.mode != PART_AGGREGATE && (P.variant < 0 || P.variant > (part_rlc(P) ? JJS_KIND_AGGREGATE : VAR_VARGEN)))
+            return part_rlc(P) ? "bad kind" : "bad variant";
+        if (part_rlc(P) && agg && !offsets)   // whole-batch and grouped parts are checked for these even when empty
+            return on_device ? "an aggregate part needs its offsets on the device and on the host" : "an aggregate part needs its offsets";
+        if (P.mode == PART_GROUPED && !P.status && !P.bitmap) return "a part needs a status or a bitmap output";
+        if (P.n == 0) return nullptr;
+        if (P.challenge_only) return !P.pk || !P.sig || !P.msg || !P.c_out ? "null buffer" : nullptr;
+        if (!P.sig || !P.msg) return "null buffer";
+        if (P.mode != PART_ALL && !P.status && (on_device || !P.bitmap)) return on_device ? "null buffer (a device call needs a status buffer)" : "null buffer";
+        if (!agg) return P.pk ? nullptr : "null buffer";
+        if (!offsets) return "null buffer";
+        for (size_t i = 0; i < P.n; i++)
+            if (P.h_offsets[i + 1] < P.h_offsets[i]) return "offsets must be non-decreasing";
+        return P.h_offsets[P.n] > P.h_offsets[0] && !P.pk ? "null key buffer" : nullptr;
+    }();
+    if (!why) return JJS_SUCCESS;
+    return part < 0 ? fail(ctx, JJS_ERR_ARGUMENT, "%s", why) : fail(ctx, JJS_ERR_ARGUMENT, "part %ld: %s", part, why);
+}
+
+// End of the pass of part P that starts at item `off` of n and takes at most `want` items.  An aggregate pass also holds no more
+// items than the aggregation tables of region R serve (in the pass scratch for whole-batch and grouped parts) and no more signer
+// keys than the key scratch (agg_chunk_end on h_offsets, the host offsets of the n items).
+inline size_t pass_end(const DeviceState& d, const Region& R, const Part& P, const uint32_t* h_offsets, size_t off, size_t n, size_t want) {
+    if (!part_aggregate(P)) return off + (n - off < want ? n - off : want);
+    const size_t most = part_rlc(P) ? rlc_agg_items(d, R) : R.acap;
+    return agg_chunk_end(h_offsets, off, n, want < most ? want : most, d.agg[0].cap_keys);
+}
+
+// Scratch on device d for items [ranges[p].lo, ranges[p].hi) of every part p: the pipeline scratch, then the SAFE tags and the
+// aggregate key scratch for the most signer keys of one item.  Growing either waits for the device.
+int prepare_parts(jjs_ctx* ctx, DeviceState& d, const std::vector<Part>& parts, const std::vector<Shard>& ranges) {
+    int rc = ensure_scratch(ctx, d);
+    bool agg = false;
+    size_t most = 0;
+    for (size_t p = 0; p < parts.size(); p++) {
+        if (!part_aggregate(parts[p]) || ranges[p].hi == ranges[p].lo) continue;
+        agg = true;
+        const size_t mc = agg_max_item_keys(parts[p].h_offsets + ranges[p].lo, ranges[p].hi - ranges[p].lo);
+        if (mc > most) most = mc;
+    }
+    if (!rc && agg) rc = ensure_tags(ctx, d, 2 + 2 * most);
+    if (!rc && agg) rc = ensure_agg_scratch(ctx, d, most > d.agg_keys_initial ? most : d.agg_keys_initial);
+    return rc;
+}
+
+// Device buffers of a part from its item `first` on: the caller's (device-buffer calls, first = 0) or the staging of device_job.
+// pk of an aggregate part is at signer key `key0`; status, c and agg may be null.
+struct PartPtrs {
+    const uint8_t *pk, *sig, *msg;
+    const uint32_t* offsets;
+    uint8_t *status, *c, *agg;
+    size_t first;
+    uint32_t key0;
+};
+
+// One pass of items [off, off + cnt) after b.first of part P, on device k in region R on `stream`: the run_chunk* of the part's
+// mode.  fallback: a grouped call's count of the items verified one by one.
+int run_pass(jjs_ctx* ctx, size_t k, const Region& R, const Part& P, const PartPtrs& b, size_t off, size_t cnt, cudaStream_t stream,
+             unsigned long long* fallback) {
+    DeviceState& d = ctx->dev[k];
+    const Strides s = part_strides(P);
+    const uint8_t *sig = b.sig + s.sig * off, *msg = b.msg + 32 * off;
+    uint8_t* status = b.status ? b.status + off : nullptr;
+    uint8_t* c = b.c ? b.c + 32 * off : nullptr;
+    uint8_t* agg = b.agg ? b.agg + 32 * off : nullptr;
+    const GroupedOut go{status, c, agg, fallback};
+    const GroupedOut* out = P.mode == PART_GROUPED ? &go : nullptr;
+    const uint64_t base = P.base + b.first + off;
+    if (part_aggregate(P)) {
+        const uint32_t key_lo = P.h_offsets[b.first + off];
+        const size_t K = P.h_offsets[b.first + off + cnt] - key_lo;
+        const uint8_t* keys = b.pk + s.pk * (size_t)(key_lo - b.key0);
+        if (P.mode == PART_AGGREGATE) return run_chunk_aggregate(ctx, d, R, keys, b.offsets + off, key_lo, K, sig, msg, cnt, status, c, agg, stream);
+        return run_chunk_rlc(ctx, d, R, JJS_KIND_AGGREGATE, keys, b.offsets + off, key_lo, K, sig, msg, cnt, base, *P.seed, stream, out);
+    }
+    const uint8_t* pk = b.pk + s.pk * off;
+    switch (P.mode) {
+    case PART_WIRE: return run_chunk(ctx, d, R, P.variant, pk, sig, msg, cnt, status, c, stream, P.challenge_only);
+    case PART_TYPED: return run_chunk_ext(ctx, d, R, P.variant, pk, sig, msg, cnt, status, c, stream);
+    case PART_KEYED:
+        return run_chunk_keyed(ctx, d, R, *P.keys, P.keys->dev[k], reinterpret_cast<const uint32_t*>(pk), sig, msg, cnt, status, c, stream);
+    default: return run_chunk_rlc(ctx, d, R, P.variant, pk, nullptr, 0, 0, sig, msg, cnt, base, *P.seed, stream, out);
+    }
+}
+
+// Enqueue `parts` (device pointers, checked) on device k: the work is ordered after what `stream` holds now and `stream` waits
+// for it.  Per-item wire and keyed parts that do not overlap run passes of chunk_items in the whole region (twice a half's
+// capacity, so a double pass launches its equations once instead of twice); every other pass takes up to sub_chunk items in the
+// next scratch half.  Whole-batch parts (all_valid set) add into the halves' accumulators and the verdict is written to
+// *all_valid, also when there are no items.  Grouped parts write their items' outputs, and *fallback (may be null) counts the
+// items verified one by one.  Enqueue-only unless a scratch has to grow (prepare_parts).
+int run_device_parts(jjs_ctx* ctx, size_t k, const std::vector<Part>& parts, cudaStream_t stream, int* all_valid, unsigned long long* fallback) {
+    DeviceState& d = ctx->dev[k];
+    JJS_CUDA(ctx, cudaSetDevice(d.device));
+    size_t n = 0;
+    std::vector<Shard> ranges;
+    for (const Part& P : parts) {
+        ranges.push_back(Shard{0, P.n});
+        n += P.n;
+    }
+    int rc = prepare_parts(ctx, d, parts, ranges);
+    if (rc) return rc;
+    if (fallback) JJS_CUDA(ctx, cudaMemsetAsync(fallback, 0, sizeof(unsigned long long), stream));
+    Overlap ov(ctx, d, stream, n > d.sub_chunk);
+    rc = ov.begin();
+    if (rc) return rc;
+    for (int h = 0; h < 2 && all_valid; h++) {
+        k_rlc_init<<<1, 1, 0, ov.on ? d.sub[h] : stream>>>(rlc_acc(d, region_half(d, h)));
+        ctx->launches++;
+    }
+    for (const Part& P : parts) {
+        const bool whole = !ov.on && (P.mode == PART_WIRE || P.mode == PART_KEYED);
+        const PartPtrs b{P.pk, P.sig, P.msg, P.offsets, P.status, P.c_out, P.agg_out, 0, 0};
+        for (size_t off = 0; off < P.n; ov.advance()) {
+            const Region R = whole ? region_whole(d) : region_half(d, ov.i);
+            const size_t end = pass_end(d, R, P, P.h_offsets, off, P.n, whole ? d.chunk_items : d.sub_chunk);
+            rc = run_pass(ctx, k, R, P, b, off, end - off, ov.next_stream(), fallback);
+            if (rc) return rc;
+            off = end;
+        }
+    }
+    rc = ov.end();
+    if (rc) return rc;
+    for (const Part& P : parts) {
+        if (!P.bitmap || !P.n) continue;
+        k_bitmap<<<blocks_for(P.n), BLOCK, 0, stream>>>(P.status, P.n, P.bitmap);
+        ctx->launches++;
+    }
+    if (all_valid) {
+        (d.fb_w == FB_W_SMALL ? k_rlc_finish<FB_W_SMALL> : k_rlc_finish<FB_W>)<<<1, 1, 0, stream>>>(
+            rlc_acc(d, region_half(d, 0)), rlc_acc(d, region_half(d, 1)), d.tables(), nullptr, all_valid);
+        ctx->launches++;
+    }
+    JJS_CUDA(ctx, cudaGetLastError());
+    return JJS_SUCCESS;
+}
+
+// ---- host-buffer calls ------------------------------------------------------------------------------------------------------
 struct StagedPart {   // device staging of one part's shard
     uint8_t *pk = nullptr, *sig = nullptr, *msg = nullptr, *status = nullptr, *c = nullptr, *agg = nullptr;
     uint32_t *offsets = nullptr, *bitmap = nullptr;
 };
 
-inline size_t part_in_bytes(const HostPart& p, size_t lo, size_t hi, size_t* pk_bytes, size_t* sig_bytes) {
-    const size_t m = hi - lo;
-    if (part_aggregate(p)) {
-        *pk_bytes = 32 * (size_t)(p.offsets[hi] - p.offsets[lo]);
-        *sig_bytes = 64 * m;
-    } else if (p.mode == PART_TYPED) {
-        *pk_bytes = 160 * (size_t)variant_slots(p.variant) * m;
-        *sig_bytes = 32 * m;
-    } else if (p.mode == PART_KEYED) {
-        *pk_bytes = sizeof(uint32_t) * m;
-        *sig_bytes = sig_size(p.variant) * m;
-    } else {
-        *pk_bytes = pk_size(p.variant) * m;
-        *sig_bytes = sig_size(p.variant) * m;
-    }
-    return *pk_bytes + *sig_bytes + 32 * m;
+// bytes of the pk buffer of items [lo, hi) of part P (aggregate parts: of their signer keys)
+inline size_t part_pk_bytes(const Part& P, size_t lo, size_t hi) {
+    return part_strides(P).pk * (part_aggregate(P) ? (size_t)(P.h_offsets[hi] - P.h_offsets[lo]) : hi - lo);
 }
 
 // Everything device k does for one call.  Runs on its own host thread when the context has several devices.
-int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const std::vector<std::vector<Shard>>& shards) {
+int device_job(jjs_ctx* ctx, size_t k, const std::vector<Part>& parts, const std::vector<std::vector<Shard>>& shards) {
     DeviceState& d = ctx->dev[k];
+    std::vector<Shard> mine(parts.size());
     bool any = false;
-    for (size_t p = 0; p < parts.size(); p++) any = any || shards[p][k].hi > shards[p][k].lo;
+    for (size_t p = 0; p < parts.size(); p++) {
+        mine[p] = shards[p][k];
+        any = any || mine[p].hi > mine[p].lo;
+    }
     if (!any) return JJS_SUCCESS;
     JJS_CUDA(ctx, cudaSetDevice(d.device));
-    int rc = ensure_scratch(ctx, d);
+    int rc = prepare_parts(ctx, d, parts, mine);
     if (rc) return rc;
     // staging layout
     std::vector<StagedPart> st(parts.size());
     std::vector<size_t> o_pk(parts.size()), o_sig(parts.size()), o_msg(parts.size()), o_st(parts.size()), o_c(parts.size()), o_agg(parts.size()),
         o_off(parts.size()), o_bm(parts.size());
     size_t total = 0;
-    size_t max_cnt = 0;
     for (size_t p = 0; p < parts.size(); p++) {
-        const HostPart& P = parts[p];
-        const size_t lo = shards[p][k].lo, hi = shards[p][k].hi, m = hi - lo;
+        const Part& P = parts[p];
+        const size_t lo = mine[p].lo, hi = mine[p].hi, m = hi - lo;
         if (!m) continue;
-        size_t pkb, sgb;
-        part_in_bytes(P, lo, hi, &pkb, &sgb);
-        o_pk[p] = total; total += align_up(pkb, 256);
-        o_sig[p] = total; total += align_up(sgb, 256);
+        o_pk[p] = total; total += align_up(part_pk_bytes(P, lo, hi), 256);
+        o_sig[p] = total; total += align_up(part_strides(P).sig * m, 256);
         o_msg[p] = total; total += align_up(32 * m, 256);
         o_st[p] = total; total += align_up(m, 256);
         o_c[p] = total; total += align_up(32 * m, 256);
@@ -1936,19 +1910,11 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         if (part_aggregate(P)) {
             o_agg[p] = total; total += align_up(32 * m, 256);
             o_off[p] = total; total += align_up(4 * (m + 1), 256);
-            size_t mc = agg_max_item_keys(P.offsets + lo, m);
-            if (mc > max_cnt) max_cnt = mc;
-            rc = ensure_agg_scratch(ctx, d, mc > d.agg_keys_initial ? mc : d.agg_keys_initial);
-            if (rc) return rc;
         }
-    }
-    if (max_cnt) {
-        rc = ensure_tags(ctx, d, 2 + 2 * max_cnt);
-        if (rc) return rc;
     }
     int p_grp = -1;                     // the first grouped part with items here, if any: its sink gets the device's fallback count,
     for (size_t p = 0; p < parts.size() && p_grp < 0; p++)   // which is staged after the parts
-        if (parts[p].mode == PART_GROUPED && shards[p][k].hi > shards[p][k].lo) p_grp = (int)p;
+        if (parts[p].mode == PART_GROUPED && mine[p].hi > mine[p].lo) p_grp = (int)p;
     const size_t o_fb = total;
     if (p_grp >= 0) total += 256;
     rc = ensure_stage(ctx, d, total);
@@ -1958,7 +1924,7 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
     const bool serial = ctx->profile;   // stage timers must not overlap
     int p_all = -1;                     // the first whole-batch part with items here, if any: all of them add into the accumulators of
     for (size_t p = 0; p < parts.size() && p_all < 0; p++)   // both halves, which start out empty
-        if (parts[p].mode == PART_ALL && shards[p][k].hi > shards[p][k].lo) p_all = (int)p;
+        if (parts[p].mode == PART_ALL && mine[p].hi > mine[p].lo) p_all = (int)p;
     if (p_all >= 0)
         for (int h = 0; h < 2; h++) {
             k_rlc_init<<<1, 1, 0, serial ? d.stream : d.sub[h]>>>(rlc_acc(d, region_half(d, h)));
@@ -1966,69 +1932,40 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
         }
     size_t j = 0;                       // slice counter of this device: slices alternate between the compute streams / scratch halves
     for (size_t p = 0; p < parts.size(); p++) {
-        const HostPart& P = parts[p];
-        const size_t lo = shards[p][k].lo, hi = shards[p][k].hi, m = hi - lo;
+        const Part& P = parts[p];
+        const size_t lo = mine[p].lo, hi = mine[p].hi, m = hi - lo;
         if (!m) continue;
         StagedPart& S = st[p];
         S.pk = d.stage + o_pk[p]; S.sig = d.stage + o_sig[p]; S.msg = d.stage + o_msg[p]; S.status = d.stage + o_st[p]; S.c = d.stage + o_c[p];
         S.bitmap = reinterpret_cast<uint32_t*>(d.stage + o_bm[p]);
-        if (part_aggregate(P)) {
+        const uint32_t* ho = part_aggregate(P) ? P.h_offsets + lo : nullptr;   // host offsets of this shard
+        if (ho) {
             S.agg = d.stage + o_agg[p];
             S.offsets = reinterpret_cast<uint32_t*>(d.stage + o_off[p]);
-            JJS_CUDA(ctx, cudaMemcpyAsync(S.offsets, P.offsets + lo, 4 * (m + 1), cudaMemcpyHostToDevice, d.copy_stream));
+            JJS_CUDA(ctx, cudaMemcpyAsync(S.offsets, ho, 4 * (m + 1), cudaMemcpyHostToDevice, d.copy_stream));
         }
+        const Strides s = part_strides(P);
         const bool want_c = P.c_out != nullptr || P.challenge_only;
-        const size_t pks = P.mode == PART_TYPED ? 160 * (size_t)variant_slots(P.variant) : (P.mode == PART_KEYED ? sizeof(uint32_t) : pk_size(P.variant));
-        const size_t sgs = P.mode == PART_TYPED ? 32 : (P.mode == PART_AGGREGATE ? 64 : sig_size(P.variant));
+        const PartPtrs b{S.pk, S.sig, S.msg, S.offsets, S.status, want_c ? S.c : nullptr, P.agg_out ? S.agg : nullptr, lo, ho ? ho[0] : 0u};
         // Pipeline slices: slice j + 1 is copied in on the copy stream while slice j is being verified (the kernels of one
         // slice run far longer than its copy); the first slice of a device is short so that compute starts early.
         for (size_t off = 0; off < m; j++) {
-            const size_t want = j == 0 ? d.first_slice : d.sub_chunk;
-            size_t cnt = m - off < want ? m - off : want;
             cudaStream_t cs = serial ? d.stream : d.sub[j & 1];
-            Region R = region_half(d, j);
-            if (part_aggregate(P)) {
-                const uint32_t* ho = P.offsets + lo;   // host offsets of this shard
-                const size_t most = part_rlc(P) ? rlc_agg_items(d, R) : R.acap;
-                size_t end = agg_chunk_end(ho, off, m, want < most ? want : most, d.agg[0].cap_keys);
-                cnt = end - off;
-                const uint32_t key0 = ho[0], key_lo = ho[off];
-                const size_t K = ho[end] - key_lo;
-                if (K) JJS_CUDA(ctx, cudaMemcpyAsync(S.pk + 32 * (size_t)(key_lo - key0), P.pk + 32 * (size_t)key_lo, 32 * K, cudaMemcpyHostToDevice, d.copy_stream));
-                JJS_CUDA(ctx, cudaMemcpyAsync(S.sig + 64 * off, P.sig + 64 * (lo + off), 64 * cnt, cudaMemcpyHostToDevice, d.copy_stream));
-                JJS_CUDA(ctx, cudaMemcpyAsync(S.msg + 32 * off, P.msg + 32 * (lo + off), 32 * cnt, cudaMemcpyHostToDevice, d.copy_stream));
-                JJS_CUDA(ctx, cudaEventRecord(d.copied, d.copy_stream));
-                JJS_CUDA(ctx, cudaStreamWaitEvent(cs, d.copied, 0));
-                const GroupedOut go{S.status + off, want_c ? S.c + 32 * off : nullptr, P.agg_out ? S.agg + 32 * off : nullptr, d_fb};
-                if (part_rlc(P))
-                    rc = run_chunk_rlc(ctx, d, R, JJS_KIND_AGGREGATE, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off,
-                                       S.msg + 32 * off, cnt, P.base + lo + off, *P.seed, cs, P.mode == PART_GROUPED ? &go : nullptr);
-                else
-                    rc = run_chunk_aggregate(ctx, d, R, S.pk + 32 * (size_t)(key_lo - key0), S.offsets + off, key_lo, K, S.sig + 64 * off, S.msg + 32 * off,
-                                             cnt, S.status + off, want_c ? S.c + 32 * off : nullptr, P.agg_out ? S.agg + 32 * off : nullptr, cs);
+            const Region R = region_half(d, j);
+            const size_t end = pass_end(d, R, P, ho, off, m, j == 0 ? d.first_slice : d.sub_chunk), cnt = end - off;
+            if (ho) {
+                const size_t K = ho[end] - ho[off];
+                if (K) JJS_CUDA(ctx, cudaMemcpyAsync(S.pk + s.pk * (ho[off] - ho[0]), P.pk + s.pk * ho[off], s.pk * K, cudaMemcpyHostToDevice, d.copy_stream));
             } else {
-                JJS_CUDA(ctx, cudaMemcpyAsync(S.pk + off * pks, P.pk + (lo + off) * pks, cnt * pks, cudaMemcpyHostToDevice, d.copy_stream));
-                JJS_CUDA(ctx, cudaMemcpyAsync(S.sig + off * sgs, P.sig + (lo + off) * sgs, cnt * sgs, cudaMemcpyHostToDevice, d.copy_stream));
-                JJS_CUDA(ctx, cudaMemcpyAsync(S.msg + off * 32, P.msg + (lo + off) * 32, cnt * 32, cudaMemcpyHostToDevice, d.copy_stream));
-                JJS_CUDA(ctx, cudaEventRecord(d.copied, d.copy_stream));
-                JJS_CUDA(ctx, cudaStreamWaitEvent(cs, d.copied, 0));
-                if (P.mode == PART_TYPED)
-                    rc = run_chunk_ext(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * 32, S.msg + off * 32, cnt, S.status + off,
-                                       want_c ? S.c + off * 32 : nullptr, cs);
-                else if (part_rlc(P)) {
-                    const GroupedOut go{S.status + off, want_c ? S.c + off * 32 : nullptr, nullptr, d_fb};
-                    rc = run_chunk_rlc(ctx, d, R, P.variant, S.pk + off * pks, nullptr, 0, 0, S.sig + off * sgs, S.msg + off * 32, cnt, P.base + lo + off,
-                                       *P.seed, cs, P.mode == PART_GROUPED ? &go : nullptr);
-                }
-                else if (P.mode == PART_KEYED)
-                    rc = run_chunk_keyed(ctx, d, R, *P.keys, P.keys->dev[k], reinterpret_cast<const uint32_t*>(S.pk + off * pks), S.sig + off * sgs,
-                                         S.msg + off * 32, cnt, S.status + off, want_c ? S.c + off * 32 : nullptr, cs);
-                else
-                    rc = run_chunk(ctx, d, R, P.variant, S.pk + off * pks, S.sig + off * sgs, S.msg + off * 32, cnt, S.status + off,
-                                   want_c ? S.c + off * 32 : nullptr, cs, P.challenge_only);
+                JJS_CUDA(ctx, cudaMemcpyAsync(S.pk + off * s.pk, P.pk + (lo + off) * s.pk, cnt * s.pk, cudaMemcpyHostToDevice, d.copy_stream));
             }
+            JJS_CUDA(ctx, cudaMemcpyAsync(S.sig + off * s.sig, P.sig + (lo + off) * s.sig, cnt * s.sig, cudaMemcpyHostToDevice, d.copy_stream));
+            JJS_CUDA(ctx, cudaMemcpyAsync(S.msg + off * 32, P.msg + (lo + off) * 32, cnt * 32, cudaMemcpyHostToDevice, d.copy_stream));
+            JJS_CUDA(ctx, cudaEventRecord(d.copied, d.copy_stream));
+            JJS_CUDA(ctx, cudaStreamWaitEvent(cs, d.copied, 0));
+            rc = run_pass(ctx, k, R, P, b, off, cnt, cs, d_fb);
             if (rc) return rc;
-            off += cnt;
+            off = end;
         }
     }
     if (!serial)
@@ -2037,8 +1974,8 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
             JJS_CUDA(ctx, cudaStreamWaitEvent(d.stream, d.join[q], 0));
         }
     for (size_t p = 0; p < parts.size(); p++) {
-        const HostPart& P = parts[p];
-        const size_t lo = shards[p][k].lo, hi = shards[p][k].hi, m = hi - lo;
+        const Part& P = parts[p];
+        const size_t lo = mine[p].lo, hi = mine[p].hi, m = hi - lo;
         if (!m) continue;
         const StagedPart& S = st[p];
         if (!P.challenge_only && P.status) JJS_CUDA(ctx, cudaMemcpyAsync(P.status + lo, S.status, m, cudaMemcpyDeviceToHost, d.stream));
@@ -2068,16 +2005,15 @@ int device_job(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const
 }
 
 // Device staging that device_job lays out for items [lo, hi) of part P.
-inline size_t part_stage_bytes(const HostPart& P, size_t lo, size_t hi) {
+inline size_t part_stage_bytes(const Part& P, size_t lo, size_t hi) {
     const size_t m = hi - lo;
-    size_t pkb, sgb;
-    part_in_bytes(P, lo, hi, &pkb, &sgb);
-    size_t b = align_up(pkb, 256) + align_up(sgb, 256) + 2 * align_up(32 * m, 256) + align_up(m, 256) + align_up(4 * ((m + 31) / 32), 256);
+    size_t b = align_up(part_pk_bytes(P, lo, hi), 256) + align_up(part_strides(P).sig * m, 256) + 2 * align_up(32 * m, 256) + align_up(m, 256) +
+               align_up(4 * ((m + 31) / 32), 256);
     if (part_aggregate(P)) b += align_up(32 * m, 256) + align_up(4 * (m + 1), 256);
     return b;
 }
 // The largest window [lo, end) of part P whose staging fits `budget` bytes, ending on a bitmap word (or at hi); at least one word.
-size_t window_end(const HostPart& P, size_t lo, size_t hi, size_t budget) {
+size_t window_end(const Part& P, size_t lo, size_t hi, size_t budget) {
     size_t good = 1, bad = (hi - lo + 31) / 32 + 1;   // in bitmap words
     while (bad - good > 1) {
         const size_t mid = (good + bad) / 2, end = lo + 32 * mid < hi ? lo + 32 * mid : hi;
@@ -2089,11 +2025,11 @@ size_t window_end(const HostPart& P, size_t lo, size_t hi, size_t budget) {
 // A memory-limited context cannot stage a whole shard: it runs device_job window by window, each window as large as the staging
 // buffer it reserved at init allows (or grows within its limit for a window of one bitmap word), so batches of any size stream
 // through it.  Each window is verified and copied back before the next is staged.
-int device_job_windows(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const std::vector<std::vector<Shard>>& shards) {
+int device_job_windows(jjs_ctx* ctx, size_t k, const std::vector<Part>& parts, const std::vector<std::vector<Shard>>& shards) {
     DeviceState& d = ctx->dev[k];
     std::vector<std::vector<Shard>> win(parts.size(), std::vector<Shard>(ctx->dev.size(), Shard{0, 0}));
     bool grouped = false;   // device_job stages a grouped call's fallback count after the parts
-    for (const HostPart& P : parts) grouped = grouped || P.mode == PART_GROUPED;
+    for (const Part& P : parts) grouped = grouped || P.mode == PART_GROUPED;
     const size_t budget = d.stage_bytes - (grouped ? 256 : 0);
     for (size_t p = 0; p < parts.size(); p++) {
         const size_t hi = shards[p][k].hi;
@@ -2111,7 +2047,7 @@ int device_job_windows(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& part
 
 // device_job, and on failure a drain of the device: nothing may still be reading or writing the caller's buffers when the
 // call returns
-int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& parts, const std::vector<std::vector<Shard>>& shards) {
+int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<Part>& parts, const std::vector<std::vector<Shard>>& shards) {
     int rc = ctx->dev[k].limit ? device_job_windows(ctx, k, parts, shards) : device_job(ctx, k, parts, shards);
     if (rc) {
         cudaSetDevice(ctx->dev[k].device);
@@ -2120,43 +2056,10 @@ int device_job_drained(jjs_ctx* ctx, size_t k, const std::vector<HostPart>& part
     return rc;
 }
 
-int validate_part(jjs_ctx* ctx, const HostPart& P) {
-    if (P.mode == PART_WIRE || P.mode == PART_TYPED || P.mode == PART_KEYED) {
-        if (P.variant < 0 || P.variant > 2) return fail(ctx, JJS_ERR_ARGUMENT, "bad variant");
-    } else if (part_rlc(P)) {
-        if (P.variant < JJS_KIND_SINGLE || P.variant > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "bad kind");
-        if (P.variant == JJS_KIND_AGGREGATE && !P.offsets) return fail(ctx, JJS_ERR_ARGUMENT, "an aggregate part needs its offsets");
-        if (P.mode == PART_GROUPED && !P.status && !P.bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "a part needs a status or a bitmap output");
-        if (P.n && (!P.sig || !P.msg)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-        if (P.variant != JJS_KIND_AGGREGATE) return P.n && !P.pk ? fail(ctx, JJS_ERR_ARGUMENT, "null buffer") : JJS_SUCCESS;
-    } else if (P.mode != PART_AGGREGATE) {
-        return fail(ctx, JJS_ERR_ARGUMENT, "bad part kind");
-    }
-    if (P.n == 0) return JJS_SUCCESS;
-    if (P.challenge_only) {
-        if (!P.pk || !P.sig || !P.msg || !P.c_out) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-        return JJS_SUCCESS;
-    }
-    if (P.mode != PART_ALL && (!P.sig || !P.msg || (!P.status && !P.bitmap))) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    if (part_aggregate(P)) {
-        if (!P.offsets) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-        for (size_t i = 0; i < P.n; i++)
-            if (P.offsets[i + 1] < P.offsets[i]) return fail(ctx, JJS_ERR_ARGUMENT, "offsets must be non-decreasing");
-        if (P.offsets[P.n] > P.offsets[0] && !P.pk) return fail(ctx, JJS_ERR_ARGUMENT, "null key buffer");
-    } else if (!P.pk) {
-        return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    }
-    return JJS_SUCCESS;
-}
-
-int run_parts(jjs_ctx* ctx, const std::vector<HostPart>& parts) {
-    JJS_ENTER(ctx);
+// A host-buffer call of checked parts.
+int run_parts(jjs_ctx* ctx, const std::vector<Part>& parts) {
     bool any = false;
-    for (const HostPart& P : parts) {
-        int rc = validate_part(ctx, P);
-        if (rc) return rc;
-        any = any || P.n > 0;
-    }
+    for (const Part& P : parts) any = any || P.n > 0;
     if (!any) return JJS_SUCCESS;
     const size_t g = ctx->dev.size();
     std::vector<std::vector<Shard>> shards;
@@ -2174,14 +2077,46 @@ int run_parts(jjs_ctx* ctx, const std::vector<HostPart>& parts) {
         if (rcs[k]) return rcs[k];
     return JJS_SUCCESS;
 }
-
-HostPart wire_part(int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t n, uint8_t* status, uint8_t* c_out, uint32_t* bitmap,
-                   bool challenge_only = false) {
-    return HostPart{PART_WIRE, variant, pk, sig, msg, nullptr, n, status, c_out, nullptr, bitmap, challenge_only};
+// A host-buffer call of one part.
+int run_part(jjs_ctx* ctx, const Part& P) {
+    JJS_ENTER(ctx);
+    int rc = validate_part(ctx, P, false);
+    return rc ? rc : run_parts(ctx, {P});
 }
-HostPart aggregate_part(const uint8_t* pks, const uint32_t* offsets, const uint8_t* sig, const uint8_t* msg, size_t n, uint8_t* status, uint8_t* c_out,
-                        uint8_t* agg_out, uint32_t* bitmap) {
-    return HostPart{PART_AGGREGATE, VAR_SINGLE, pks, sig, msg, offsets, n, status, c_out, agg_out, bitmap, false};
+
+Part wire_part(int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t n, uint8_t* status, uint8_t* c_out, uint32_t* bitmap) {
+    return Part{PART_WIRE, variant, pk, sig, msg, nullptr, nullptr, n, status, c_out, nullptr, bitmap};
+}
+Part aggregate_part(const uint8_t* pks, const uint32_t* offsets, const uint32_t* h_offsets, const uint8_t* sig, const uint8_t* msg, size_t n,
+                    uint8_t* status, uint8_t* c_out, uint8_t* agg_out, uint32_t* bitmap) {
+    return Part{PART_AGGREGATE, JJS_KIND_AGGREGATE, pks, sig, msg, offsets, h_offsets, n, status, c_out, agg_out, bitmap};
+}
+
+// The checked parts of a jjs_part array: per-item parts (mode PART_WIRE: wire or aggregate parts by kind), or the whole-batch
+// (PART_ALL: no per-item outputs) or grouped (PART_GROUPED) parts of one call, whose items are weighted by their position in the
+// call.  The parts of a device-buffer call (on_device) take the host copies of the aggregate parts' offsets from h_offsets.
+int parts_from_jjs(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, int mode, bool on_device, const uint32_t* const* h_offsets,
+                   const RlcSeed* seed, RlcSink* sink, std::vector<Part>& out) {
+    out.reserve(n_parts);
+    uint64_t base = 0;
+    for (size_t i = 0; i < n_parts; i++) {
+        const jjs_part& p = parts[i];
+        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
+        if (mode == PART_ALL && (p.status || p.c32 || p.aggpk32 || p.accept_bitmap))
+            return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: whole-batch verification has no per-item outputs", i);
+        const bool agg = p.kind == JJS_KIND_AGGREGATE;
+        const uint32_t* ho = !agg ? nullptr : !on_device ? p.offsets : h_offsets ? h_offsets[i] : nullptr;
+        Part P{mode == PART_WIRE && agg ? (int)PART_AGGREGATE : mode, p.kind, p.pk, p.sig, p.msg32, agg ? p.offsets : nullptr, ho, p.n, p.status,
+               p.c32, agg ? p.aggpk32 : nullptr, p.accept_bitmap};
+        P.seed = seed;
+        P.sink = sink;
+        P.base = base;
+        base += p.n;
+        int rc = validate_part(ctx, P, on_device, (long)i);
+        if (rc) return rc;
+        out.push_back(P);
+    }
+    return JJS_SUCCESS;
 }
 
 // multisig::combine for n ragged sessions (host buffers, device 0); a chunk holds as many sessions as the table scratch serves
@@ -2375,14 +2310,13 @@ void free_device(DeviceState& d) {
     }
 }
 
-int device_entry(jjs_ctx* ctx, int variant, int device_index, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg, size_t n,
-                 uint8_t* status, uint8_t* c_out, void* stream) {
+// a per-item device-buffer call of one part on the caller's stream
+int device_entry(jjs_ctx* ctx, int device_index, const Part& P, void* stream) {
     JJS_ENTER(ctx);
     if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
-    if (n == 0) return JJS_SUCCESS;
-    if (!pk || !sig || !msg || !status) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    DeviceState& d = ctx->dev[device_index];
-    return run_device(ctx, d, variant, pk, sig, msg, n, status, c_out, (cudaStream_t)stream);
+    int rc = validate_part(ctx, P, true);
+    if (rc || P.n == 0) return rc;
+    return run_device_parts(ctx, (size_t)device_index, {P}, (cudaStream_t)stream, nullptr, nullptr);
 }
 
 // small synchronous utilities on device 0: copy in, one kernel, copy out
@@ -2606,50 +2540,44 @@ JJS_API uint64_t jjs_launch_count(const jjs_ctx* ctx) { return ctx ? ctx->launch
 
 JJS_API int jjs_verify_single(jjs_ctx* ctx, const uint8_t* pk32, const uint8_t* sig64, const uint8_t* msg32, size_t n, uint8_t* status,
                               uint8_t* c32_or_null) {
-    return run_parts(ctx, {wire_part(VAR_SINGLE, pk32, sig64, msg32, n, status, c32_or_null, nullptr)});
+    return run_part(ctx, wire_part(VAR_SINGLE, pk32, sig64, msg32, n, status, c32_or_null, nullptr));
 }
 JJS_API int jjs_verify_double(jjs_ctx* ctx, const uint8_t* pk64, const uint8_t* sig96, const uint8_t* msg32, size_t n, uint8_t* status,
                               uint8_t* c32_or_null) {
-    return run_parts(ctx, {wire_part(VAR_DOUBLE, pk64, sig96, msg32, n, status, c32_or_null, nullptr)});
+    return run_part(ctx, wire_part(VAR_DOUBLE, pk64, sig96, msg32, n, status, c32_or_null, nullptr));
 }
 JJS_API int jjs_verify_vargen(jjs_ctx* ctx, const uint8_t* pk64, const uint8_t* sig64, const uint8_t* msg32, size_t n, uint8_t* status,
                               uint8_t* c32_or_null) {
-    return run_parts(ctx, {wire_part(VAR_VARGEN, pk64, sig64, msg32, n, status, c32_or_null, nullptr)});
+    return run_part(ctx, wire_part(VAR_VARGEN, pk64, sig64, msg32, n, status, c32_or_null, nullptr));
 }
 JJS_API int jjs_verify_aggregate(jjs_ctx* ctx, const uint8_t* pks32, const uint32_t* offsets, const uint8_t* sig64, const uint8_t* msg32, size_t n,
                                  uint8_t* status, uint8_t* c32_or_null, uint8_t* aggpk32_or_null) {
     if (ctx && ctx->ready && n && !status) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_parts(ctx, {aggregate_part(pks32, offsets, sig64, msg32, n, status, c32_or_null, aggpk32_or_null, nullptr)});
+    return run_part(ctx, aggregate_part(pks32, offsets, offsets, sig64, msg32, n, status, c32_or_null, aggpk32_or_null, nullptr));
 }
 JJS_API int jjs_verify_batch(jjs_ctx* ctx, const uint8_t* pk32, const uint8_t* sig64, const uint8_t* msg32, size_t n, uint32_t* accept_bitmap) {
     if (ctx && ctx->ready && n && !accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_parts(ctx, {wire_part(VAR_SINGLE, pk32, sig64, msg32, n, nullptr, nullptr, accept_bitmap)});
+    return run_part(ctx, wire_part(VAR_SINGLE, pk32, sig64, msg32, n, nullptr, nullptr, accept_bitmap));
 }
 JJS_API int jjs_verify_batch_double(jjs_ctx* ctx, const uint8_t* pk64, const uint8_t* sig96, const uint8_t* msg32, size_t n, uint32_t* accept_bitmap) {
     if (ctx && ctx->ready && n && !accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_parts(ctx, {wire_part(VAR_DOUBLE, pk64, sig96, msg32, n, nullptr, nullptr, accept_bitmap)});
+    return run_part(ctx, wire_part(VAR_DOUBLE, pk64, sig96, msg32, n, nullptr, nullptr, accept_bitmap));
 }
 JJS_API int jjs_verify_batch_vargen(jjs_ctx* ctx, const uint8_t* pk64, const uint8_t* sig64, const uint8_t* msg32, size_t n, uint32_t* accept_bitmap) {
     if (ctx && ctx->ready && n && !accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_parts(ctx, {wire_part(VAR_VARGEN, pk64, sig64, msg32, n, nullptr, nullptr, accept_bitmap)});
+    return run_part(ctx, wire_part(VAR_VARGEN, pk64, sig64, msg32, n, nullptr, nullptr, accept_bitmap));
 }
 JJS_API int jjs_verify_batch_aggregate(jjs_ctx* ctx, const uint8_t* pks32, const uint32_t* offsets, const uint8_t* sig64, const uint8_t* msg32, size_t n,
                                        uint32_t* accept_bitmap) {
     if (ctx && ctx->ready && n && !accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_parts(ctx, {aggregate_part(pks32, offsets, sig64, msg32, n, nullptr, nullptr, nullptr, accept_bitmap)});
+    return run_part(ctx, aggregate_part(pks32, offsets, offsets, sig64, msg32, n, nullptr, nullptr, nullptr, accept_bitmap));
 }
 JJS_API int jjs_verify_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts) {
     JJS_ENTER(ctx);
     if (n_parts && !parts) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    std::vector<HostPart> hp;
-    hp.reserve(n_parts);
-    for (size_t i = 0; i < n_parts; i++) {
-        const jjs_part& p = parts[i];
-        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
-        if (p.kind == JJS_KIND_AGGREGATE) hp.push_back(aggregate_part(p.pk, p.offsets, p.sig, p.msg32, p.n, p.status, p.c32, p.aggpk32, p.accept_bitmap));
-        else hp.push_back(wire_part(p.kind, p.pk, p.sig, p.msg32, p.n, p.status, p.c32, p.accept_bitmap));
-    }
-    return run_parts(ctx, hp);
+    std::vector<Part> hp;
+    int rc = parts_from_jjs(ctx, parts, n_parts, PART_WIRE, false, nullptr, nullptr, nullptr, hp);
+    return rc ? rc : run_parts(ctx, hp);
 }
 JJS_API int jjs_status_bitmap_device(jjs_ctx* ctx, int device_index, const uint8_t* d_status, size_t n, uint32_t* d_accept_bitmap, void* cuda_stream) {
     JJS_ENTER(ctx);
@@ -2664,36 +2592,31 @@ JJS_API int jjs_status_bitmap_device(jjs_ctx* ctx, int device_index, const uint8
 }
 JJS_API int jjs_verify_single_device(jjs_ctx* ctx, int device_index, const uint8_t* d_pk32, const uint8_t* d_sig64, const uint8_t* d_msg32,
                                      size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream) {
-    return device_entry(ctx, VAR_SINGLE, device_index, d_pk32, d_sig64, d_msg32, n, d_status, d_c32_or_null, cuda_stream);
+    return device_entry(ctx, device_index, wire_part(VAR_SINGLE, d_pk32, d_sig64, d_msg32, n, d_status, d_c32_or_null, nullptr), cuda_stream);
 }
 JJS_API int jjs_verify_double_device(jjs_ctx* ctx, int device_index, const uint8_t* d_pk64, const uint8_t* d_sig96, const uint8_t* d_msg32,
                                      size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream) {
-    return device_entry(ctx, VAR_DOUBLE, device_index, d_pk64, d_sig96, d_msg32, n, d_status, d_c32_or_null, cuda_stream);
+    return device_entry(ctx, device_index, wire_part(VAR_DOUBLE, d_pk64, d_sig96, d_msg32, n, d_status, d_c32_or_null, nullptr), cuda_stream);
 }
 JJS_API int jjs_verify_vargen_device(jjs_ctx* ctx, int device_index, const uint8_t* d_pk64, const uint8_t* d_sig64, const uint8_t* d_msg32,
                                      size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream) {
-    return device_entry(ctx, VAR_VARGEN, device_index, d_pk64, d_sig64, d_msg32, n, d_status, d_c32_or_null, cuda_stream);
+    return device_entry(ctx, device_index, wire_part(VAR_VARGEN, d_pk64, d_sig64, d_msg32, n, d_status, d_c32_or_null, nullptr), cuda_stream);
 }
 JJS_API int jjs_verify_aggregate_device(jjs_ctx* ctx, int device_index, const uint8_t* d_pks32, const uint32_t* d_offsets, const uint32_t* h_offsets,
                                         const uint8_t* d_sig64, const uint8_t* d_msg32, size_t n, uint8_t* d_status, uint8_t* d_c32_or_null,
                                         uint8_t* d_aggpk32_or_null, void* cuda_stream) {
-    JJS_ENTER(ctx);
-    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
-    if (n == 0) return JJS_SUCCESS;
-    if (!d_offsets || !h_offsets || !d_sig64 || !d_msg32 || !d_status) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    for (size_t i = 0; i < n; i++)
-        if (h_offsets[i + 1] < h_offsets[i]) return fail(ctx, JJS_ERR_ARGUMENT, "offsets must be non-decreasing");
-    if (h_offsets[n] > h_offsets[0] && !d_pks32) return fail(ctx, JJS_ERR_ARGUMENT, "null key buffer");
-    return run_aggregate_device(ctx, ctx->dev[device_index], d_pks32, d_offsets, h_offsets, d_sig64, d_msg32, n, d_status, d_c32_or_null,
-                                d_aggpk32_or_null, (cudaStream_t)cuda_stream);
+    return device_entry(ctx, device_index,
+                        aggregate_part(d_pks32, d_offsets, h_offsets, d_sig64, d_msg32, n, d_status, d_c32_or_null, d_aggpk32_or_null, nullptr), cuda_stream);
 }
 JJS_API int jjs_verify_ext(jjs_ctx* ctx, int variant, const uint8_t* points_ext160, const uint8_t* u32, const uint8_t* msg32, size_t n,
                            uint8_t* status, uint8_t* c32_or_null) {
     if (ctx && ctx->ready && n && !status) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_parts(ctx, {HostPart{PART_TYPED, variant, points_ext160, u32, msg32, nullptr, n, status, c32_or_null, nullptr, nullptr, false}});
+    return run_part(ctx, Part{PART_TYPED, variant, points_ext160, u32, msg32, nullptr, nullptr, n, status, c32_or_null});
 }
 JJS_API int jjs_challenge_only(jjs_ctx* ctx, int variant, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg32, size_t n, uint8_t* c32) {
-    return run_parts(ctx, {wire_part(variant, pk, sig, msg32, n, nullptr, c32, nullptr, true)});
+    Part P = wire_part(variant, pk, sig, msg32, n, nullptr, c32, nullptr);
+    P.challenge_only = true;
+    return run_part(ctx, P);
 }
 JJS_API int jjs_subgroup_check(jjs_ctx* ctx, const uint8_t* points32, size_t n, int method, uint8_t* out) {
     JJS_ENTER(ctx);
@@ -2853,20 +2776,17 @@ JJS_API int jjs_verify_keyed(jjs_ctx* ctx, int keyset, const uint32_t* key_index
     JJS_ENTER(ctx);
     const KeySet* ks = keyset_lookup(ctx, keyset);
     if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
-    HostPart P{PART_KEYED, ks->variant, reinterpret_cast<const uint8_t*>(key_index), sig, msg32, nullptr, n, status_or_null, c32_or_null, nullptr,
-               accept_bitmap_or_null, false, ks};
-    return run_parts(ctx, {P});
+    return run_part(ctx, Part{PART_KEYED, ks->variant, reinterpret_cast<const uint8_t*>(key_index), sig, msg32, nullptr, nullptr, n, status_or_null,
+                              c32_or_null, nullptr, accept_bitmap_or_null, false, ks});
 }
 JJS_API int jjs_verify_keyed_device(jjs_ctx* ctx, int device_index, int keyset, const uint32_t* d_key_index, const uint8_t* d_sig,
                                     const uint8_t* d_msg32, size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream) {
     JJS_ENTER(ctx);
-    if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
     const KeySet* ks = keyset_lookup(ctx, keyset);
     if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
-    if (n == 0) return JJS_SUCCESS;
-    if (!d_key_index || !d_sig || !d_msg32 || !d_status) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    return run_keyed_device(ctx, ctx->dev[device_index], *ks, ks->dev[device_index], d_key_index, d_sig, d_msg32, n, d_status, d_c32_or_null,
-                            (cudaStream_t)cuda_stream);
+    return device_entry(ctx, device_index, Part{PART_KEYED, ks->variant, reinterpret_cast<const uint8_t*>(d_key_index), d_sig, d_msg32, nullptr, nullptr, n,
+                                                d_status, d_c32_or_null, nullptr, nullptr, false, ks},
+                        cuda_stream);
 }
 JJS_API int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* entries, size_t n, uint32_t* mismatches) {
     JJS_ENTER(ctx);
@@ -2900,11 +2820,10 @@ JJS_API int jjs_verify_all(jjs_ctx* ctx, int kind, const uint8_t* pk, const uint
     rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
     RlcSink sink;
-    HostPart P = wire_part(kind, pk, sig, msg32, n, nullptr, nullptr, nullptr);
-    P.mode = PART_ALL;
+    Part P{PART_ALL, kind, pk, sig, msg32, nullptr, nullptr, n};
     P.seed = &seed;
     P.sink = &sink;
-    rc = run_parts(ctx, {P});
+    rc = run_part(ctx, P);
     if (rc) return rc;
     *all_valid = sink.valid && ext_is_identity(sink.P) ? 1 : 0;
     return JJS_SUCCESS;
@@ -2915,12 +2834,14 @@ JJS_API int jjs_verify_all_device(jjs_ctx* ctx, int device_index, int kind, cons
     if (rc) return rc;
     JJS_ENTER(ctx);
     if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
-    if (!d_all_valid || (n && (!d_pk || !d_sig || !d_msg32))) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    if (!d_all_valid) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
     RlcSeed seed;
-    rc = rlc_seed(ctx, seed32_or_null, seed);
+    Part P{PART_ALL, kind, d_pk, d_sig, d_msg32, nullptr, nullptr, n};
+    P.seed = &seed;
+    rc = validate_part(ctx, P, true);
+    if (!rc) rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
-    return run_rlc_device(ctx, ctx->dev[device_index], {RlcDevPart{kind, d_pk, d_sig, d_msg32, nullptr, nullptr, n}}, seed, d_all_valid,
-                          nullptr, (cudaStream_t)cuda_stream);
+    return run_device_parts(ctx, (size_t)device_index, {P}, (cudaStream_t)cuda_stream, d_all_valid, nullptr);
 }
 JJS_API int jjs_verify_all_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null, int* all_valid) {
     JJS_ENTER(ctx);
@@ -2928,23 +2849,9 @@ JJS_API int jjs_verify_all_mixed(jjs_ctx* ctx, const jjs_part* parts, size_t n_p
     *all_valid = 0;
     RlcSeed seed;
     RlcSink sink;
-    std::vector<HostPart> hp;
-    hp.reserve(n_parts);
-    uint64_t base = 0;
-    for (size_t i = 0; i < n_parts; i++) {
-        const jjs_part& p = parts[i];
-        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
-        if (p.status || p.c32 || p.aggpk32 || p.accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: whole-batch verification has no per-item outputs", i);
-        HostPart P = wire_part(p.kind, p.pk, p.sig, p.msg32, p.n, nullptr, nullptr, nullptr);
-        P.mode = PART_ALL;
-        P.offsets = p.kind == JJS_KIND_AGGREGATE ? p.offsets : nullptr;
-        P.seed = &seed;
-        P.sink = &sink;
-        P.base = base;
-        base += p.n;
-        hp.push_back(P);
-    }
-    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    std::vector<Part> hp;
+    int rc = parts_from_jjs(ctx, parts, n_parts, PART_ALL, false, nullptr, &seed, &sink, hp);
+    if (!rc) rc = rlc_seed(ctx, seed32_or_null, seed);
     if (!rc) rc = run_parts(ctx, hp);
     if (rc) return rc;
     *all_valid = sink.valid && ext_is_identity(sink.P) ? 1 : 0;
@@ -2955,29 +2862,12 @@ JJS_API int jjs_verify_all_mixed_device(jjs_ctx* ctx, int device_index, const jj
     JJS_ENTER(ctx);
     if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
     if (!d_all_valid || (n_parts && !parts)) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    std::vector<RlcDevPart> dp;
-    dp.reserve(n_parts);
-    for (size_t i = 0; i < n_parts; i++) {
-        const jjs_part& p = parts[i];
-        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
-        if (p.status || p.c32 || p.aggpk32 || p.accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: whole-batch verification has no per-item outputs", i);
-        const uint32_t* ho = nullptr;
-        if (p.kind == JJS_KIND_AGGREGATE) {
-            ho = h_offsets_or_null ? h_offsets_or_null[i] : nullptr;
-            if (!p.offsets || !ho) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: an aggregate part needs its offsets on the device and on the host", i);
-            for (size_t j = 0; j < p.n; j++)
-                if (ho[j + 1] < ho[j]) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: offsets must be non-decreasing", i);
-            if (p.n && ho[p.n] > ho[0] && !p.pk) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null key buffer", i);
-        } else if (p.n && !p.pk) {
-            return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer", i);
-        }
-        if (p.n && (!p.sig || !p.msg32)) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer", i);
-        dp.push_back(RlcDevPart{p.kind, p.pk, p.sig, p.msg32, p.kind == JJS_KIND_AGGREGATE ? p.offsets : nullptr, ho, p.n});
-    }
     RlcSeed seed;
-    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    std::vector<Part> dp;
+    int rc = parts_from_jjs(ctx, parts, n_parts, PART_ALL, true, h_offsets_or_null, &seed, nullptr, dp);
+    if (!rc) rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
-    return run_rlc_device(ctx, ctx->dev[device_index], dp, seed, d_all_valid, nullptr, (cudaStream_t)cuda_stream);
+    return run_device_parts(ctx, (size_t)device_index, dp, (cudaStream_t)cuda_stream, d_all_valid, nullptr);
 }
 JJS_API int jjs_verify_grouped(jjs_ctx* ctx, const jjs_part* parts, size_t n_parts, const uint8_t* seed32_or_null, uint64_t* fallback_items_or_null) {
     JJS_ENTER(ctx);
@@ -2985,23 +2875,9 @@ JJS_API int jjs_verify_grouped(jjs_ctx* ctx, const jjs_part* parts, size_t n_par
     if (fallback_items_or_null) *fallback_items_or_null = 0;
     RlcSeed seed;
     RlcSink sink;
-    std::vector<HostPart> hp;
-    hp.reserve(n_parts);
-    uint64_t base = 0;
-    for (size_t i = 0; i < n_parts; i++) {
-        const jjs_part& p = parts[i];
-        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
-        HostPart P = p.kind == JJS_KIND_AGGREGATE ? aggregate_part(p.pk, p.offsets, p.sig, p.msg32, p.n, p.status, p.c32, p.aggpk32, p.accept_bitmap)
-                                                  : wire_part(p.kind, p.pk, p.sig, p.msg32, p.n, p.status, p.c32, p.accept_bitmap);
-        P.mode = PART_GROUPED;
-        P.variant = p.kind;
-        P.seed = &seed;
-        P.sink = &sink;
-        P.base = base;
-        base += p.n;
-        hp.push_back(P);
-    }
-    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    std::vector<Part> hp;
+    int rc = parts_from_jjs(ctx, parts, n_parts, PART_GROUPED, false, nullptr, &seed, &sink, hp);
+    if (!rc) rc = rlc_seed(ctx, seed32_or_null, seed);
     if (!rc) rc = run_parts(ctx, hp);
     if (rc) return rc;
     if (fallback_items_or_null) *fallback_items_or_null = sink.fallback;
@@ -3012,35 +2888,13 @@ JJS_API int jjs_verify_grouped_device(jjs_ctx* ctx, int device_index, const jjs_
     JJS_ENTER(ctx);
     if (device_index < 0 || (size_t)device_index >= ctx->dev.size()) return fail(ctx, JJS_ERR_ARGUMENT, "device_index out of range");
     if (n_parts && !parts) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    std::vector<RlcDevPart> dp;
-    dp.reserve(n_parts);
-    for (size_t i = 0; i < n_parts; i++) {
-        const jjs_part& p = parts[i];
-        if (p.kind < JJS_KIND_SINGLE || p.kind > JJS_KIND_AGGREGATE) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: bad kind", i);
-        if (!p.status && !p.accept_bitmap) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: a part needs a status or a bitmap output", i);
-        const uint32_t* ho = nullptr;
-        if (p.kind == JJS_KIND_AGGREGATE) {
-            ho = h_offsets_or_null ? h_offsets_or_null[i] : nullptr;
-            if (!p.offsets || !ho) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: an aggregate part needs its offsets on the device and on the host", i);
-            for (size_t j = 0; j < p.n; j++)
-                if (ho[j + 1] < ho[j]) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: offsets must be non-decreasing", i);
-            if (p.n && ho[p.n] > ho[0] && !p.pk) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null key buffer", i);
-        } else if (p.n && !p.pk) {
-            return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer", i);
-        }
-        if (p.n && (!p.sig || !p.msg32 || !p.status)) return fail(ctx, JJS_ERR_ARGUMENT, "part %zu: null buffer (the device entry needs a status buffer)", i);
-        RlcDevPart P{p.kind, p.pk, p.sig, p.msg32, p.kind == JJS_KIND_AGGREGATE ? p.offsets : nullptr, ho, p.n};
-        P.status = p.status;
-        P.c = p.c32;
-        P.agg = p.kind == JJS_KIND_AGGREGATE ? p.aggpk32 : nullptr;
-        P.bitmap = p.accept_bitmap;
-        dp.push_back(P);
-    }
     RlcSeed seed;
-    int rc = rlc_seed(ctx, seed32_or_null, seed);
+    std::vector<Part> dp;
+    int rc = parts_from_jjs(ctx, parts, n_parts, PART_GROUPED, true, h_offsets_or_null, &seed, nullptr, dp);
+    if (!rc) rc = rlc_seed(ctx, seed32_or_null, seed);
     if (rc) return rc;
-    return run_rlc_device(ctx, ctx->dev[device_index], dp, seed, nullptr, reinterpret_cast<unsigned long long*>(d_fallback_items_or_null),
-                          (cudaStream_t)cuda_stream);
+    return run_device_parts(ctx, (size_t)device_index, dp, (cudaStream_t)cuda_stream, nullptr,
+                            reinterpret_cast<unsigned long long*>(d_fallback_items_or_null));
 }
 JJS_API int jjs_sign_batch(jjs_ctx* ctx, int variant, const uint8_t* sk32, const uint8_t* rnd32, const uint8_t* gen_scalar32_or_null,
                            const uint8_t* msg32, size_t n, uint8_t* pk_out, uint8_t* sig_out) {
