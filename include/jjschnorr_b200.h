@@ -172,13 +172,14 @@ int jjs_verify_aggregate_device(jjs_ctx* ctx, int device_index, const uint8_t* d
                                 const uint32_t* h_offsets, const uint8_t* d_sig64, const uint8_t* d_msg32, size_t n,
                                 uint8_t* d_status, uint8_t* d_c32_or_null, uint8_t* d_aggpk32_or_null, void* cuda_stream);
 
-/* ---- registered key sets: many signatures under a small, stable set of keys (validators, frequent senders, a
- *      service's registered devices).  A key set is decoded and validated once, and every key point gets a table of
- *      32 windows x 128 points j 2^(8 w) PK in affine Niels form, 96 B each: 393 216 B per single key, 786 432 B per
- *      double key (pk with G, pk' with G'), on every device of the context.  Verification against it then evaluates
+/* ---- registered key sets: many signatures under a stable set of keys (validators, frequent senders, a service's
+ *      registered devices).  A key set is decoded and validated once, and with jjs_keyset_create every key point gets a
+ *      table of 32 windows x 128 points j 2^(8 w) PK in affine Niels form, 96 B each: 393 216 B per single key, 786 432 B
+ *      per double key (pk with G, pk' with G'), on every device of the context.  Verification against it then evaluates
  *      u G + c PK == R from precomputed tables only, and returns exactly what jjs_verify_single (single key sets) or
- *      jjs_verify_double (double key sets) returns for the same items with the keys written out.  A key set is named by
- *      an int handle owned by the context; jjs_destroy frees the key sets still registered. --- */
+ *      jjs_verify_double (double key sets) returns for the same items with the keys written out.  jjs_keyset_create_limited
+ *      builds narrower tables, or none, within a byte budget.  A key set is named by an int handle owned by the context;
+ *      jjs_destroy frees the key sets still registered. --- */
 
 /* Register n_keys >= 1 keys of kind JJS_KIND_SINGLE (pk: n_keys x 32 B, PublicKey) or JJS_KIND_DOUBLE (pk: n_keys x 64 B,
  * PublicKeyDouble) on every device of the context.  Keys that do not decode or fail is_valid() are registered too, so that
@@ -198,10 +199,27 @@ int jjs_verify_keyed(jjs_ctx* ctx, int keyset, const uint32_t* key_index, const 
 int jjs_verify_keyed_device(jjs_ctx* ctx, int device_index, int keyset, const uint32_t* d_key_index, const uint8_t* d_sig,
                             const uint8_t* d_msg32, size_t n, uint8_t* d_status, uint8_t* d_c32_or_null, void* cuda_stream);
 /* Key-set table self-check (a cross-check hook for the tests, like jjs_fb_table_check): recompute the n entries named by
- * `entries` from their definition j 2^(8 w) PK by plain double-and-add on device 0 and count those that differ.  Flat index
- * (key * points_per_key + point) * 4096 + w * 128 + j - 1, reduced modulo the table size; points_per_key is 1 (single) or
- * 2 (double: pk, then pk').  The table of a key that failed is_valid() is that of the identity.  Host buffers. */
+ * `entries` from their definition j 2^(KW w) PK by plain double-and-add on device 0 and count those that differ, KW being the
+ * set's key-window width (jjs_keyset_info).  Flat index (key * points_per_key + point) * E + w * 2^(KW-1) + j - 1, with
+ * E = ceil(251 / KW) * 2^(KW-1) entries per key point (4096 at KW = 8: 32 windows x 128), reduced modulo the table size;
+ * points_per_key is 1 (single) or 2 (double: pk, then pk').  The table of a key that failed is_valid() is that of the
+ * identity.  JJS_ERR_ARGUMENT on a points-only set, which has no table.  Host buffers. */
 int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* entries, size_t n, uint32_t* mismatches);
+/* As jjs_keyset_create, holding at most bytes_per_device bytes of device memory per device (and, on a jjs_init_limited
+ * context, no more than its limit leaves): the widest key-window width 8..4 that fits, else decoded points only (65 B per key
+ * point).  The bound covers the peak of the build, which also holds 32 B of wire key and ceil(251 / KW) x 128 B of window
+ * bases per key point until it returns.  Per key point the tables take ceil(251 / KW) x 2^(KW-1) x 96 B: 393 216 B at KW = 8,
+ * 221 184 at 7, 129 024 at 6, 78 336 at 5, 48 384 at 4.  A narrower width costs a few additions per equation (12 + 32
+ * at 8, 12 + 63 at 4); a points-only set skips decoding the keys and their subgroup tests but evaluates each item's equation as
+ * jjs_verify_single does.  Same items, same statuses and challenges as jjs_keyset_create.  JJS_ERR_ARGUMENT for
+ * bytes_per_device == 0 and the arguments jjs_keyset_create refuses; JJS_ERR_NOMEM, nothing held, when not even the points
+ * fit (the message states what they need).  Synchronous. */
+int jjs_keyset_create_limited(jjs_ctx* ctx, int kind, const uint8_t* pk, size_t n_keys, size_t bytes_per_device,
+                              uint8_t* key_status_or_null, int* keyset_out);
+/* What a key set holds: key-window width (8..4, 0 = points only) and bytes per device (points, flags and tables: what
+ * jjs_memory_info's bytes_held grew by on each device, and what jjs_keyset_destroy returns); any pointer may be NULL.
+ * JJS_ERR_ARGUMENT for an unknown handle. */
+int jjs_keyset_info(const jjs_ctx* ctx, int keyset, int* key_window_bits, uint64_t* bytes_per_device);
 
 /* Typed inputs (what a Rust caller holds before any to_bytes()): every point is given by its JubJubExtended
  * coordinates (u, v, z, t1, t2), each the in-memory BlsScalar of the reference (4 x u64 little-endian Montgomery limbs,

@@ -19,6 +19,7 @@ EXPORTS = [
     "jjs_verify_batch", "jjs_status_bitmap_device", "jjs_verify_batch_double", "jjs_verify_batch_vargen", "jjs_verify_batch_aggregate",
     "jjs_verify_mixed",
     "jjs_keyset_create", "jjs_keyset_destroy", "jjs_verify_keyed", "jjs_verify_keyed_device", "jjs_keyset_table_check",
+    "jjs_keyset_create_limited", "jjs_keyset_info",
     "jjs_init_limited", "jjs_memory_info",
     "jjs_verify_all", "jjs_verify_all_device", "jjs_verify_all_mixed", "jjs_verify_all_mixed_device",
     "jjs_verify_grouped", "jjs_verify_grouped_device",
@@ -116,6 +117,10 @@ def lib():
     L.jjs_verify_keyed_device.restype = C.c_int
     L.jjs_keyset_table_check.argtypes = [vp, C.c_int, vp, sz, vp]
     L.jjs_keyset_table_check.restype = C.c_int
+    L.jjs_keyset_create_limited.argtypes = [vp, C.c_int, vp, sz, sz, vp, C.POINTER(C.c_int)]
+    L.jjs_keyset_create_limited.restype = C.c_int
+    L.jjs_keyset_info.argtypes = [vp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_uint64)]
+    L.jjs_keyset_info.restype = C.c_int
     L.jjs_verify_all.argtypes = [vp, C.c_int, vp, vp, vp, sz, vp, C.POINTER(C.c_int)]
     L.jjs_verify_all.restype = C.c_int
     L.jjs_verify_all_device.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, sz, vp, vp, vp]

@@ -18,11 +18,13 @@ class JjsError(RuntimeError):
 
 
 class KeySet:
-    """A key set registered with BatchVerifier.keyset_create: its handle in the context, kind (SINGLE or DOUBLE), number of keys
-    and per-key status (0 valid, 2 InvalidPoint, 3 BytesError)."""
+    """A key set registered with BatchVerifier.keyset_create: its handle in the context, kind (SINGLE or DOUBLE), number of keys,
+    per-key status (0 valid, 2 InvalidPoint, 3 BytesError), and what jjs_keyset_info reports: the key-window width of its tables
+    (8..4, 0 for decoded points only) and the bytes it holds on each device."""
 
-    def __init__(self, handle, kind, n_keys, key_status):
+    def __init__(self, handle, kind, n_keys, key_status, key_window_bits=None, bytes_per_device=None):
         self.handle, self.kind, self.n_keys, self.key_status = handle, kind, n_keys, key_status
+        self.key_window_bits, self.bytes_per_device = key_window_bits, bytes_per_device
 
 
 def _u8(a, width, name):
@@ -344,15 +346,23 @@ class BatchVerifier:
                                                           d_status, d_c, d_agg, stream), "jjs_verify_aggregate_device")
 
     # ---- registered key sets ---------------------------------------------------------------------
-    def keyset_create(self, kind, pks):
-        """Register keys of kind SINGLE (pks: n x 32 bytes) or DOUBLE (n x 64) on every device (jjs_keyset_create)."""
+    def keyset_create(self, kind, pks, memory_limit=None):
+        """Register keys of kind SINGLE (pks: n x 32 bytes) or DOUBLE (n x 64) on every device: 8-bit key tables
+        (jjs_keyset_create), or with memory_limit the widest tables, else the decoded points only, that fit in that many bytes
+        per device (jjs_keyset_create_limited)."""
         if kind not in (SINGLE, DOUBLE):
             raise ValueError("key sets hold SINGLE or DOUBLE keys")
         pk = _u8(pks, PK_SIZE[kind], "pks")
         status = np.empty(pk.shape[0], dtype=np.uint8)
         handle = C.c_int(-1)
-        self._check(self._lib.jjs_keyset_create(self._ctx, kind, pk.ctypes.data, pk.shape[0], status.ctypes.data, C.byref(handle)), "jjs_keyset_create")
-        return KeySet(handle.value, kind, pk.shape[0], status)
+        if memory_limit is None:
+            self._check(self._lib.jjs_keyset_create(self._ctx, kind, pk.ctypes.data, pk.shape[0], status.ctypes.data, C.byref(handle)), "jjs_keyset_create")
+        else:
+            self._check(self._lib.jjs_keyset_create_limited(self._ctx, kind, pk.ctypes.data, pk.shape[0], int(memory_limit), status.ctypes.data,
+                                                            C.byref(handle)), "jjs_keyset_create_limited")
+        bits, held = C.c_int(-1), C.c_uint64(0)
+        self._check(self._lib.jjs_keyset_info(self._ctx, handle.value, C.byref(bits), C.byref(held)), "jjs_keyset_info")
+        return KeySet(handle.value, kind, pk.shape[0], status, bits.value, held.value)
 
     def keyset_destroy(self, ks):
         self._check(self._lib.jjs_keyset_destroy(self._ctx, ks.handle), "jjs_keyset_destroy")

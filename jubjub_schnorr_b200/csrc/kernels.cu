@@ -604,7 +604,8 @@ __global__ void __launch_bounds__(BLOCK) k_fb_check(const niels* table, int whic
 // ---- registered key sets (keyset.cuh) --------------------------------------------------------------------------------
 // Key points are numbered key-major (point p = key * nk + s, the order of the tables); the decoded points are slot-major
 // (s * n_keys + key, as k_decode writes them).
-// Table pass 1: thread p computes the window bases of key point p, bases[w * npts + p].
+// Table pass 1: thread p computes the window bases of key point p, bases[w * npts + p].  KW: the key-window width (keyset.cuh).
+template <int KW>
 __global__ void __launch_bounds__(BLOCK) k_keyset_bases(int variant, const fq* keys_u, const fq* keys_v, const uint8_t* kflags, size_t n_keys,
                                                         ext* bases) {
     const int nk = keyed_points(variant);
@@ -613,31 +614,35 @@ __global__ void __launch_bounds__(BLOCK) k_keyset_bases(int variant, const fq* k
     const size_t k = (size_t)(p % nk) * n_keys + p / nk;
     fq u, v;
     keyed_table_base(u, v, keys_u[k], keys_v[k], kflags[k]);
-    keyed_window_bases(bases + p, npts, u, v);
+    keyed_window_bases<KW>(bases + p, npts, u, v);
 }
 // Table pass 2: one thread per batch of KEYED_BATCH entries of one window of one key point.
-constexpr int KEYED_GROUPS = KEYED_ENTRIES / KEYED_BATCH;
+JJS_HD constexpr int keyed_groups(int kw) { return keyed_entries(kw) / KEYED_BATCH; }
+template <int KW>
 __global__ void __launch_bounds__(BLOCK) k_keyset_combine(const ext* bases, size_t npts, niels* table) {
+    constexpr int WINDOWS = keyed_windows(KW), ENTRIES = keyed_entries(KW), GROUPS = keyed_groups(KW);
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= npts * KEYED_WINDOWS * KEYED_GROUPS) return;
-    const size_t p = t / (KEYED_WINDOWS * KEYED_GROUPS);
-    const int r = (int)(t % (KEYED_WINDOWS * KEYED_GROUPS)), w = r / KEYED_GROUPS, g = r % KEYED_GROUPS;
-    keyed_combine_entries(table + p * KEYED_POINT_ENTRIES + (size_t)w * KEYED_ENTRIES + (size_t)g * KEYED_BATCH, bases[(size_t)w * npts + p],
-                          g * KEYED_BATCH + 1);
+    if (t >= npts * WINDOWS * GROUPS) return;
+    const size_t p = t / (WINDOWS * GROUPS);
+    const int r = (int)(t % (WINDOWS * GROUPS)), w = r / GROUPS, g = r % GROUPS;
+    keyed_combine_entries<KW>(table + p * keyed_point_entries(KW) + (size_t)w * ENTRIES + (size_t)g * KEYED_BATCH, bases[(size_t)w * npts + p],
+                              g * KEYED_BATCH + 1);
 }
-// the definition, entry by entry (jjs_keyset_table_check): flat index p * KEYED_POINT_ENTRIES + w * KEYED_ENTRIES + j - 1
+// the definition, entry by entry (jjs_keyset_table_check): flat index p * keyed_point_entries(KW) + w * keyed_entries(KW) + j - 1
+template <int KW>
 __global__ void __launch_bounds__(BLOCK) k_keyset_check(int variant, const fq* keys_u, const fq* keys_v, const uint8_t* kflags, size_t n_keys,
                                                         const niels* table, const uint32_t* entries, size_t n, uint32_t* mismatches) {
+    constexpr int ENTRIES = keyed_entries(KW), POINT_ENTRIES = keyed_point_entries(KW);
     const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
     const int nk = keyed_points(variant);
-    const size_t idx = (size_t)entries[t] % ((size_t)nk * n_keys * KEYED_POINT_ENTRIES), p = idx / KEYED_POINT_ENTRIES;
-    const int e = (int)(idx % KEYED_POINT_ENTRIES);
+    const size_t idx = (size_t)entries[t] % ((size_t)nk * n_keys * POINT_ENTRIES), p = idx / POINT_ENTRIES;
+    const int e = (int)(idx % POINT_ENTRIES);
     const size_t k = (size_t)(p % nk) * n_keys + p / nk;
     fq u, v;
     keyed_table_base(u, v, keys_u[k], keys_v[k], kflags[k]);
     niels ref;
-    keyed_table_entry(ref, u, v, e / KEYED_ENTRIES, e % KEYED_ENTRIES + 1);
+    keyed_table_entry<KW>(ref, u, v, e / ENTRIES, e % ENTRIES + 1);
     const niels& g = table[idx];
     if (!(fq_eq(ref.ypx, g.ypx) && fq_eq(ref.ymx, g.ymx) && fq_eq(ref.t2d, g.t2d))) atomicAdd(mismatches, 1u);
 }
@@ -653,7 +658,7 @@ __global__ void __launch_bounds__(BLOCK) k_keyed_gather(int variant, const fq* k
 #ifndef JJS_EQK_MINBLOCKS
 #define JJS_EQK_MINBLOCKS 4
 #endif
-template <int W = FB_W>
+template <int W, int KW>
 __global__ void __launch_bounds__(BLOCK, JJS_EQK_MINBLOCKS) k_equation_keyed(int variant, const fq* pts_u, const fq* pts_v, uint8_t* pflags, size_t n,
                                                                              const uint32_t* list, const uint32_t* lcount, WireField usc,
                                                                              const uint32_t* cwords, uint8_t* eqflags, const niels* ktab,
@@ -667,8 +672,8 @@ __global__ void __launch_bounds__(BLOCK, JJS_EQK_MINBLOCKS) k_equation_keyed(int
     const uint32_t key = key_index[item];   // in range: items under an unknown index never reach the work list
     bool need_r_test = false;
     const bool ok = key < n_keys &&
-                    stage_equation_keyed<W>(variant, eq, pts_u, pts_v, pflags, n, item, eq == 1 ? T.fb_gn : T.fb_g,
-                                         ktab + ((size_t)key * neq + eq) * KEYED_POINT_ENTRIES, usc, cwords, &need_r_test);
+                    stage_equation_keyed<W, KW>(variant, eq, pts_u, pts_v, pflags, n, item, eq == 1 ? T.fb_gn : T.fb_g,
+                                                ktab + ((size_t)key * neq + eq) * keyed_point_entries(KW), usc, cwords, &need_r_test);
     if (need_r_test) {
         int pk_slot, r_slot, base_slot;
         equation_slots(variant, eq, pk_slot, r_slot, base_slot);
@@ -882,9 +887,10 @@ inline Region region_of(const DeviceState& d, size_t first_item, size_t cap, int
 inline Region region_whole(const DeviceState& d) { return region_of(d, 0, d.chunk_items, 0); }
 inline Region region_half(const DeviceState& d, size_t j) { return region_of(d, (j & 1) * d.sub_items, d.sub_items, (int)(j & 1)); }
 
-// A registered key set (jjs_keyset_create), copied to every device of the context: the decoded key points slot-major as k_decode
-// writes them (point s of key k at s * n_keys + k), their flags, and the window tables key-major (keyset.cuh; the table of point
-// s of key k starts at entry (k * nk + s) * KEYED_POINT_ENTRIES).
+// A registered key set (jjs_keyset_create / _limited), copied to every device of the context: the decoded key points slot-major
+// as k_decode writes them (point s of key k at s * n_keys + k), their flags, and the window tables of width key_bits key-major
+// (keyset.cuh; the table of point s of key k starts at entry (k * nk + s) * keyed_point_entries(key_bits)).  key_bits 0: no
+// tables, the points only; items then run the per-item equation of run_chunk.
 struct KeySetDev {
     fq *u = nullptr, *v = nullptr;
     uint8_t* flags = nullptr;
@@ -892,6 +898,7 @@ struct KeySetDev {
 };
 struct KeySet {
     int variant = VAR_SINGLE;
+    int key_bits = KEYED_W;
     size_t n_keys = 0;
     std::vector<KeySetDev> dev;
 };
@@ -1370,7 +1377,8 @@ int run_chunk_aggregate(jjs_ctx* ctx, DeviceState& d, const Region& R, const uin
 
 // The pipeline for one chunk of m <= R.cap items under a registered key set (device pointers, key_index: the chunk's first
 // index).  The key slots are gathered from the key set instead of decoded; only the signature points go through k_decode,
-// with their subgroup test deferred.  Hash, deferred tests and status are the kernels of run_chunk.
+// with their subgroup test deferred.  Hash, deferred tests and status are the kernels of run_chunk; so is the equation under a
+// points-only set, which has no tables.
 int run_chunk_keyed(jjs_ctx* ctx, DeviceState& d, const Region& R, const KeySet& ks, const KeySetDev& kd, const uint32_t* key_index, const uint8_t* sig,
                     const uint8_t* msg, size_t m, uint8_t* status, uint8_t* c_out, cudaStream_t stream) {
     const int variant = ks.variant, nk = keyed_points(variant);
@@ -1388,10 +1396,14 @@ int run_chunk_keyed(jjs_ctx* ctx, DeviceState& d, const Region& R, const KeySet&
     ctx->launches += 2;
     int rc = enqueue_challenges(ctx, d, R, variant, m, fmsg, fu, stream, true);
     if (rc) return rc;
+    if (ks.key_bits == 0) return finish_chunk(ctx, d, R, variant, m, fu, status, c_out, stream);   // points only
     StageTimer t3(ctx, d.device, 3, stream);
     JJS_CUDA(ctx, cudaMemsetAsync(R.rcount, 0, sizeof(uint32_t), stream));
-    (d.fb_w == FB_W_SMALL ? k_equation_keyed<FB_W_SMALL> : k_equation_keyed<>)<<<blocks_for(nk * m), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, R.eqlist, R.rcount + 2, fu, R.cwords, R.eqflags,
-                                                              kd.table, key_index, ks.n_keys, T, R.rlist, R.rcount);
+    const auto keq = with_key_width(ks.key_bits, [&](auto kw) {
+        return d.fb_w == FB_W_SMALL ? k_equation_keyed<FB_W_SMALL, kw.value> : k_equation_keyed<FB_W, kw.value>;
+    });
+    keq<<<blocks_for(nk * m), BLOCK, 0, stream>>>(variant, R.pts_u, R.pts_v, R.pflags, m, R.eqlist, R.rcount + 2, fu, R.cwords, R.eqflags, kd.table,
+                                                  key_index, ks.n_keys, T, R.rlist, R.rcount);
     t3.stop(stream);
     StageTimer t5(ctx, d.device, 5, stream);
     k_rtest<<<blocks_for(nk * m), BLOCK, 0, stream>>>(R.pts_u, R.pts_v, R.pflags, R.rlist, R.rcount);
@@ -2346,9 +2358,9 @@ int run_small(jjs_ctx* ctx, const char* what, size_t in_bytes, size_t out_bytes,
 }
 
 // ---- registered key sets ----------------------------------------------------------------------------------------
-// Device memory of a key set of npts key points: decoded points and flags, and the tables.
+// Device memory of a key set of npts key points: decoded points and flags, and the tables of width kw (none for kw = 0).
 inline size_t keyset_point_bytes(size_t npts) { return npts * (2 * sizeof(fq) + 1); }
-inline size_t keyset_table_bytes(size_t npts) { return sizeof(niels) * npts * KEYED_POINT_ENTRIES; }
+inline size_t keyset_table_bytes(size_t npts, int kw) { return kw ? sizeof(niels) * npts * keyed_point_entries(kw) : 0; }
 
 struct DeviceTemp {   // scratch of one key-set build, freed on every path out
     DeviceState& d;
@@ -2357,25 +2369,40 @@ struct DeviceTemp {   // scratch of one key-set build, freed on every path out
     ~DeviceTemp() { dev_free(d, p, bytes); }
 };
 
-// Key set `ks` on device d: copy the wire keys in, decode them with the subgroup test, build the tables (keyset.cuh).
-// key_status (optional) receives 0 / 2 / 3 per key.
+// Everything a key set of npts key points at width kw allocates on a device, in order: what it keeps (points, flags, tables),
+// then the build's scratch (the wire keys and, with tables, the window bases of every key point).
+int alloc_keyset(DevAlloc& A, KeySetDev& kd, size_t npts, int kw, uint8_t** wire, uint8_t** bases) {
+    int rc = A(&kd.u, sizeof(fq) * npts);
+    if (!rc) rc = A(&kd.v, sizeof(fq) * npts);
+    if (!rc) rc = A(&kd.flags, npts);
+    if (!rc && kw) rc = A(&kd.table, keyset_table_bytes(npts, kw));
+    if (!rc) rc = A(wire, 32 * npts);
+    if (!rc && kw) rc = A(bases, sizeof(ext) * npts * keyed_windows(kw));
+    return rc;
+}
+// The most a key set of npts key points at width kw holds on a device, while its tables are built: a dry run of alloc_keyset.
+size_t keyset_peak(size_t npts, int kw) {
+    DevAlloc A{nullptr, nullptr};
+    KeySetDev kd;
+    uint8_t *wire = nullptr, *bases = nullptr;
+    alloc_keyset(A, kd, npts, kw, &wire, &bases);
+    return A.total;
+}
+
+// Key set `ks` on device d: copy the wire keys in, decode them with the subgroup test, build the tables (keyset.cuh) unless the
+// set holds points only.  key_status (optional) receives 0 / 2 / 3 per key.
 int keyset_build(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, KeySetDev& kd, const uint8_t* pk, uint8_t* key_status) {
     JJS_CUDA(ctx, cudaSetDevice(d.device));
-    const int nk = keyed_points(ks.variant);
+    const int nk = keyed_points(ks.variant), kw = ks.key_bits;
     const size_t npts = (size_t)nk * ks.n_keys;
-    DeviceTemp wire{d, 32 * npts}, bases{d, sizeof(ext) * npts * KEYED_WINDOWS};
+    DeviceTemp wire{d, 32 * npts}, bases{d, kw ? sizeof(ext) * npts * keyed_windows(kw) : 0};
     // a limited context refuses a key set that would cross its limit before allocating any of it
-    const size_t need = keyset_point_bytes(npts) + keyset_table_bytes(npts) + wire.bytes + bases.bytes;
+    const size_t need = keyset_peak(npts, kw);
     if (d.limit && d.held + need > d.limit)
         return fail(ctx, JJS_ERR_NOMEM, "key set: %zu bytes on device %d would exceed the context's memory limit of %zu bytes (%zu held)", need, d.device,
                     d.limit, d.held);
     DevAlloc A = dev_alloc(ctx, d);
-    int rc = A(&kd.u, sizeof(fq) * npts);
-    if (!rc) rc = A(&kd.v, sizeof(fq) * npts);
-    if (!rc) rc = A(&kd.flags, npts);
-    if (!rc) rc = A(&kd.table, keyset_table_bytes(npts));
-    if (!rc) rc = A(&wire.p, wire.bytes);
-    if (!rc) rc = A(&bases.p, bases.bytes);
+    int rc = alloc_keyset(A, kd, npts, kw, &wire.p, &bases.p);
     if (rc) return rc;
     cudaStream_t st = d.stream;
     // undecodable keys leave their coordinates unwritten; zero them so that gathering them copies defined values
@@ -2388,9 +2415,16 @@ int keyset_build(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, KeySetDev& kd, 
     f.f[1] = nk == 2 ? WireField{w + 32, 64} : WireField{nullptr, 0};
     f.f[2] = f.f[3] = WireField{nullptr, 0};
     k_decode<<<blocks_for(npts), BLOCK, 0, st>>>(f, nk, 0, ks.n_keys, kd.u, kd.v, kd.flags, d.tables(), 3u);
-    k_keyset_bases<<<blocks_for(npts), BLOCK, 0, st>>>(ks.variant, kd.u, kd.v, kd.flags, ks.n_keys, reinterpret_cast<ext*>(bases.p));
-    k_keyset_combine<<<blocks_for(npts * KEYED_WINDOWS * KEYED_GROUPS), BLOCK, 0, st>>>(reinterpret_cast<const ext*>(bases.p), npts, kd.table);
-    ctx->launches += 3;
+    ctx->launches++;
+    if (kw) {
+        with_key_width(kw, [&](auto kwc) {
+            constexpr int KW = kwc.value;
+            k_keyset_bases<KW><<<blocks_for(npts), BLOCK, 0, st>>>(ks.variant, kd.u, kd.v, kd.flags, ks.n_keys, reinterpret_cast<ext*>(bases.p));
+            k_keyset_combine<KW><<<blocks_for(npts * keyed_windows(KW) * keyed_groups(KW)), BLOCK, 0, st>>>(reinterpret_cast<const ext*>(bases.p), npts,
+                                                                                                            kd.table);
+        });
+        ctx->launches += 2;
+    }
     JJS_CUDA(ctx, cudaGetLastError());
     std::vector<uint8_t> flags;
     if (key_status) {
@@ -2402,6 +2436,18 @@ int keyset_build(jjs_ctx* ctx, DeviceState& d, const KeySet& ks, KeySetDev& kd, 
     return JJS_SUCCESS;
 }
 
+// The layout of jjs_keyset_create_limited for npts key points per device: the widest key-window width KEYED_MAX_W ..
+// KEYED_MIN_W whose peak (keyset_peak) is at most `budget` and, on a limited context, at most what the limit leaves on every
+// device; else points only (0) if that fits; else -1.  One width serves the whole set on every device.
+int pick_key_bits(const jjs_ctx* ctx, size_t npts, size_t budget) {
+    size_t room = budget;
+    for (const DeviceState& d : ctx->dev)
+        if (d.limit) room = std::min(room, d.limit > d.held ? d.limit - d.held : size_t(0));
+    for (int kw = KEYED_MAX_W; kw >= KEYED_MIN_W; kw--)
+        if (keyset_peak(npts, kw) <= room) return kw;
+    return keyset_peak(npts, 0) <= room ? 0 : -1;
+}
+
 void keyset_free(jjs_ctx* ctx, KeySet* ks) {
     const size_t npts = (size_t)keyed_points(ks->variant) * ks->n_keys;
     for (size_t k = 0; k < ks->dev.size(); k++) {
@@ -2411,9 +2457,38 @@ void keyset_free(jjs_ctx* ctx, KeySet* ks) {
         cudaSetDevice(d.device);
         cudaDeviceSynchronize();   // work enqueued by the device entry point may still read the tables
         dev_free(d, kd.u, sizeof(fq) * npts); dev_free(d, kd.v, sizeof(fq) * npts); dev_free(d, kd.flags, npts);
-        dev_free(d, kd.table, keyset_table_bytes(npts));
+        dev_free(d, kd.table, keyset_table_bytes(npts, ks->key_bits));
     }
     delete ks;
+}
+
+// Register a key set of kind `kind` at key-window width key_bits (0: points only) on every device: jjs_keyset_create and
+// jjs_keyset_create_limited after their argument checks.
+int keyset_register(jjs_ctx* ctx, int kind, int key_bits, const uint8_t* pk, size_t n_keys, uint8_t* key_status_or_null, int* keyset_out) {
+    KeySet* ks = new (std::nothrow) KeySet();
+    if (!ks) return fail(ctx, JJS_ERR_NOMEM, "key set: out of host memory");
+    ks->variant = kind;
+    ks->key_bits = key_bits;
+    ks->n_keys = n_keys;
+    ks->dev.resize(ctx->dev.size());
+    for (size_t k = 0; k < ctx->dev.size(); k++) {
+        int rc = keyset_build(ctx, ctx->dev[k], *ks, ks->dev[k], pk, k == 0 ? key_status_or_null : nullptr);
+        if (rc) {
+            keyset_free(ctx, ks);
+            return rc;
+        }
+    }
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    ctx->keysets.push_back(ks);
+    *keyset_out = (int)(ctx->keysets.size() - 1);
+    return JJS_SUCCESS;
+}
+// the arguments both create calls refuse
+int keyset_check_args(jjs_ctx* ctx, int kind, const uint8_t* pk, size_t n_keys, int* keyset_out) {
+    if (kind != JJS_KIND_SINGLE && kind != JJS_KIND_DOUBLE) return fail(ctx, JJS_ERR_ARGUMENT, "key sets hold single or double keys (kind %d)", kind);
+    if (n_keys == 0 || n_keys > 0xffffffffu) return fail(ctx, JJS_ERR_ARGUMENT, "n_keys must be in [1, 2^32)");
+    if (!pk || !keyset_out) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
+    return JJS_SUCCESS;
 }
 
 // The weights' seed: the caller's 32 bytes, or 32 fresh bytes from the operating system
@@ -2740,24 +2815,31 @@ JJS_API int jjs_profile_collect(jjs_ctx* ctx, double* stage_ms, uint64_t* stage_
 }
 JJS_API int jjs_keyset_create(jjs_ctx* ctx, int kind, const uint8_t* pk, size_t n_keys, uint8_t* key_status_or_null, int* keyset_out) {
     JJS_ENTER(ctx);
-    if (kind != JJS_KIND_SINGLE && kind != JJS_KIND_DOUBLE) return fail(ctx, JJS_ERR_ARGUMENT, "key sets hold single or double keys (kind %d)", kind);
-    if (n_keys == 0 || n_keys > 0xffffffffu) return fail(ctx, JJS_ERR_ARGUMENT, "n_keys must be in [1, 2^32)");
-    if (!pk || !keyset_out) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
-    KeySet* ks = new (std::nothrow) KeySet();
-    if (!ks) return fail(ctx, JJS_ERR_NOMEM, "key set: out of host memory");
-    ks->variant = kind;
-    ks->n_keys = n_keys;
-    ks->dev.resize(ctx->dev.size());
-    for (size_t k = 0; k < ctx->dev.size(); k++) {
-        int rc = keyset_build(ctx, ctx->dev[k], *ks, ks->dev[k], pk, k == 0 ? key_status_or_null : nullptr);
-        if (rc) {
-            keyset_free(ctx, ks);
-            return rc;
-        }
-    }
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    ctx->keysets.push_back(ks);
-    *keyset_out = (int)(ctx->keysets.size() - 1);
+    int rc = keyset_check_args(ctx, kind, pk, n_keys, keyset_out);
+    return rc ? rc : keyset_register(ctx, kind, KEYED_W, pk, n_keys, key_status_or_null, keyset_out);
+}
+JJS_API int jjs_keyset_create_limited(jjs_ctx* ctx, int kind, const uint8_t* pk, size_t n_keys, size_t bytes_per_device, uint8_t* key_status_or_null,
+                                      int* keyset_out) {
+    JJS_ENTER(ctx);
+    int rc = keyset_check_args(ctx, kind, pk, n_keys, keyset_out);
+    if (rc) return rc;
+    if (bytes_per_device == 0) return fail(ctx, JJS_ERR_ARGUMENT, "bytes_per_device must be positive");
+    const size_t npts = (size_t)keyed_points(kind) * n_keys;
+    const int key_bits = pick_key_bits(ctx, npts, bytes_per_device);
+    if (key_bits < 0)
+        return fail(ctx, JJS_ERR_NOMEM, "key set: even its decoded points (the smallest layout) need %zu bytes per device while they are built, beyond the "
+                    "budget of %zu bytes or what the context's memory limit leaves", keyset_peak(npts, 0), bytes_per_device);
+    return keyset_register(ctx, kind, key_bits, pk, n_keys, key_status_or_null, keyset_out);
+}
+JJS_API int jjs_keyset_info(const jjs_ctx* ctx, int keyset, int* key_window_bits, uint64_t* bytes_per_device) {
+    if (!ctx) return JJS_ERR_ARGUMENT;
+    if (!ctx->ready || ctx->dev.empty()) return JJS_ERR_CUDA;
+    jjs_ctx* c = const_cast<jjs_ctx*>(ctx);   // the handle table's lock and the error message
+    const KeySet* ks = keyset_lookup(c, keyset);
+    if (!ks) return fail(c, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
+    const size_t npts = (size_t)keyed_points(ks->variant) * ks->n_keys;
+    if (key_window_bits) *key_window_bits = ks->key_bits;
+    if (bytes_per_device) *bytes_per_device = keyset_point_bytes(npts) + keyset_table_bytes(npts, ks->key_bits);
     return JJS_SUCCESS;
 }
 JJS_API int jjs_keyset_destroy(jjs_ctx* ctx, int keyset) {
@@ -2792,6 +2874,7 @@ JJS_API int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* ent
     JJS_ENTER(ctx);
     const KeySet* ks = keyset_lookup(ctx, keyset);
     if (!ks) return fail(ctx, JJS_ERR_ARGUMENT, "unknown key set %d", keyset);
+    if (ks->key_bits == 0) return fail(ctx, JJS_ERR_ARGUMENT, "key set %d holds points only: no table", keyset);
     if (!mismatches) return fail(ctx, JJS_ERR_ARGUMENT, "null buffer");
     *mismatches = 0;
     if (n == 0) return JJS_SUCCESS;
@@ -2802,8 +2885,10 @@ JJS_API int jjs_keyset_table_check(jjs_ctx* ctx, int keyset, const uint32_t* ent
     uint32_t count = 0;
     int rc = run_small(ctx, "key-set table check", 4 * n, 4, srcs, bytes, 1, &count, [&](DeviceState& d, uint8_t* in, uint8_t* o) {
         cudaMemsetAsync(o, 0, 4, d.stream);
-        k_keyset_check<<<blocks_for(n), BLOCK, 0, d.stream>>>(ks->variant, kd.u, kd.v, kd.flags, ks->n_keys, kd.table, reinterpret_cast<const uint32_t*>(in),
-                                                             n, reinterpret_cast<uint32_t*>(o));
+        with_key_width(ks->key_bits, [&](auto kw) {
+            k_keyset_check<kw.value><<<blocks_for(n), BLOCK, 0, d.stream>>>(ks->variant, kd.u, kd.v, kd.flags, ks->n_keys, kd.table,
+                                                                          reinterpret_cast<const uint32_t*>(in), n, reinterpret_cast<uint32_t*>(o));
+        });
         ctx->launches++;
     });
     *mismatches = count;

@@ -95,6 +95,10 @@ extern "C" {
                                    d_msg32: *const u8, n: usize, d_status: *mut u8, d_c32_or_null: *mut u8,
                                    cuda_stream: *mut c_void) -> c_int;
     pub fn jjs_keyset_table_check(ctx: *mut jjs_ctx, keyset: c_int, entries: *const u32, n: usize, mismatches: *mut u32) -> c_int;
+    // key sets within a byte budget per device: the widest key-window width 8..4 that fits, else the decoded points only
+    pub fn jjs_keyset_create_limited(ctx: *mut jjs_ctx, kind: c_int, pk: *const u8, n_keys: usize, bytes_per_device: usize,
+                                     key_status_or_null: *mut u8, keyset_out: *mut c_int) -> c_int;
+    pub fn jjs_keyset_info(ctx: *const jjs_ctx, keyset: c_int, key_window_bits: *mut c_int, bytes_per_device: *mut u64) -> c_int;
     // NEW all-or-nothing verification of single / double items by one random linear combination (DESIGN.md section 12)
     pub fn jjs_verify_all(ctx: *mut jjs_ctx, kind: c_int, pk: *const u8, sig: *const u8, msg32: *const u8, n: usize,
                           seed32_or_null: *const u8, all_valid: *mut c_int) -> c_int;
